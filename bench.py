@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark: batched visibility sweep on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c2|c2s|c4]
+                    [--workload c2|c2s|c4] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (computeVisibility) over one batch of
 synthetic (map, source) pairs:
@@ -34,6 +34,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "Gcells/s visibility sweep (1000² grid, batched sources)"
+DUMP_BYTES = 60 * 10**6  # --dump-outputs budget: a full batch is 16 GB
 
 
 # ----------------------------------------------------------------------------
@@ -237,6 +238,20 @@ def ncu_traffic(workload_name, pairs):
         if d and j.get("kernel_source_hash") == kernel_source_hash():
             return d["dram_bytes_per_pair"] * pairs
     return None
+
+
+def dump_outputs(path, out_t):
+    """--dump-outputs: the fields of a fixed sample of the batch's pairs (PCG64 seed 0, as many as
+    DUMP_BYTES holds, in pair order) as DIR/visibility.npy [pairs, ny, nx], in the stored dtype, and
+    their indices in the batch as DIR/visibility_pairs.npy (float64), so that two builds can be
+    compared output for output."""
+    import torch
+    n = out_t.shape[0]
+    k = max(1, min(n, DUMP_BYTES // (out_t[0].numel() * out_t.element_size())))
+    idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "visibility.npy"), out_t[torch.from_numpy(idx).to(out_t.device)].cpu().numpy())
+    np.save(os.path.join(path, "visibility_pairs.npy"), idx.astype(np.float64))
 
 
 def bench_config(workload_name, desc, nx, ny, n, store, world):
@@ -689,7 +704,14 @@ def main():
     ap.add_argument("--no-penumbra", action="store_true")
     ap.add_argument("--no-giant", action="store_true")
     ap.add_argument("--no-legs", action="store_true", help="skip the C1 / C3 / ray-casting legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the fields of the last timed step to DIR/visibility.npy "
+                         "and their pair indices to DIR/visibility_pairs.npy (rank 0's batch only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -750,6 +772,8 @@ def main():
     with torch.cuda.stream(stream):
         for _ in range(args.warmup):
             step()
+        if args.dump_outputs:
+            out_t.fill_(float("nan"))  # what is dumped must come from the timed steps
     barrier()
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -766,6 +790,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.launches - launches0
     ctx.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_t)
     total_ms = evs[0].elapsed_time(evs[-1])
     step_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     if world > 1:
