@@ -168,6 +168,40 @@ vhp_status vhp_visibility_batch_runs(vhp_context *ctx, const uint8_t *occ, int n
 vhp_status vhp_runs_to_bits(const uint16_t *row_count, const uint64_t *pair_ptr, const uint16_t *trans,
                             int64_t npairs, int nx, int ny, uint32_t *out_bits);
 
+/* Merged visibility of SETS of light sources: ngroups groups, group g = sources
+ * [group_ptr[g], group_ptr[g+1]) of src_xy (group_ptr[0] = 0, non-decreasing), all on map
+ * group_map[g] (NULL -> map 0).  For every cell, over the group's sources k = 0, 1, ... (index
+ * WITHIN the group; duplicates count as separate entries):
+ *   vmax[g][y][x]   max_k of the field vhp_visibility_batch returns for source k (dtype; VHP_F32 =
+ *                   the fp64 maximum rounded once)          -- visibility_global_ after those sweeps
+ *   first[g][y][x]  smallest k whose sweep writes the cell with fp64 value >= threshold,
+ *                   VHP_NO_PARENT if none                   -- cameFrom_ after those sweeps
+ *   count[g][y][x]  number of k whose sweep writes the cell with fp64 value >= threshold
+ * "writes": every cell except source k's never-written border (column 0 unless sx == 0, row 0
+ * unless sy == 0).  Any output pointer may be NULL; at least one must be given.  The call writes
+ * every cell of the outputs it is given (empty groups: 0 / VHP_NO_PARENT / 0).
+ * Instead of K full fields per group, the sweeps fold straight into the group's outputs with
+ * atomics where the batched tile kernel runs and threshold > 0 (a dark cell costs no store); any
+ * other case (threshold <= 0, a few sweeps of a large map, the naive kernel) sweeps chunks of fields
+ * and folds them, with the same result.  Errors (VHP_ERR_INVALID_ARG): a source outside the grid,
+ * group_map out of range, group_ptr not starting at 0, decreasing, or a group of 2^31 sources or
+ * more, a NaN threshold, no output.  In the _dev form nsrc = group_ptr[ngroups] sizes the launch;
+ * a bad source or group layout is reported like an out-of-grid source of vhp_visibility_batch_dev
+ * (by the next synchronising call). */
+typedef struct vhp_merge_out {
+  void *vmax;
+  int32_t *first;
+  uint32_t *count;
+} vhp_merge_out;
+vhp_status vhp_visibility_merge_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                      const int32_t *src_xy, const int64_t *group_ptr,
+                                      const int32_t *group_map, int64_t ngroups, double threshold,
+                                      vhp_dtype dtype, const vhp_merge_out *out);
+vhp_status vhp_visibility_merge_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                          int ny, const int32_t *d_src_xy, const int64_t *d_group_ptr,
+                                          const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
+                                          double threshold, vhp_dtype dtype, const vhp_merge_out *d_out);
+
 /* ---- opt-in variants of the sweep (SURVEY 8f): the paper's MATLAB algorithm and the reference's
  * early-terminating queue variant.  Same layouts as vhp_visibility_batch.
  *   VHP_VARIANT_MATLAB  getAccessibilityMap.m (MATLAB_code/visibility/getAccessibilityMap.m:1-118):

@@ -42,6 +42,11 @@ class PlannerOut(C.Structure):
                 ("came", C.c_void_p), ("vis", C.c_void_p)]
 
 
+class MergeOut(C.Structure):
+    """struct vhp_merge_out: vmax (dtype), first (int32), count (uint32), each [group][ny][nx] or NULL."""
+    _fields_ = [("vmax", C.c_void_p), ("first", C.c_void_p), ("count", C.c_void_p)]
+
+
 class SweepVariant(C.Structure):
     """struct vhp_sweep_variant: model 1 = getAccessibilityMap.m (alpha, fac, light_strength),
     model 2 = computeVisibilityUsingQueue as an order-free rule (cutoff)."""
@@ -106,6 +111,10 @@ def load_library(build_if_missing: bool = True):
     lib.vhp_visibility_batch_runs.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_double, vp, vp, vp, i64,
                                               C.POINTER(i64)]
     lib.vhp_runs_to_bits.argtypes = [vp, vp, vp, i64, i32, i32, vp]
+    lib.vhp_visibility_merge_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, C.c_double, i32,
+                                               C.POINTER(MergeOut)]
+    lib.vhp_visibility_merge_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_double, i32,
+                                                   C.POINTER(MergeOut)]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
     for name in ("vhp_packed_pairs", "vhp_packed_bytes", "vhp_packed_pair_bytes"):
         getattr(lib, name).argtypes = [vp]
@@ -354,6 +363,42 @@ class Context:
             self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(),
             None if src_map_t is None else src_map_t.data_ptr(), src_xy_t.shape[0], float(threshold),
             out_bits_t.data_ptr()))
+
+    def visibility_merge_batch(self, occ, src_xy, group_ptr, threshold, group_map=None, dtype=F64,
+                               outputs=("vmax", "first", "count")):
+        """Merged visibility of groups of sources (vhp_visibility_merge_batch): group g = sources
+        src_xy[group_ptr[g]:group_ptr[g + 1]] on map group_map[g].  Returns a dict of the requested
+        outputs, (ngroups, ny, nx) each: vmax (max of the fields, dtype), first (int32, index within
+        the group of the first source whose sweep writes the cell with a value >= threshold, NO_PARENT
+        if none) and count (uint32, how many do)."""
+        occ = _occ_u8(occ)
+        nmaps, ny, nx = occ.shape
+        xy = np.ascontiguousarray(src_xy, dtype=np.int32).reshape(-1, 2)
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        ng = gp.shape[0] - 1
+        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
+        kinds = dict(vmax=np.float32 if dtype == F32 else np.float64, first=np.int32, count=np.uint32)
+        if set(outputs) - set(kinds):
+            raise ValueError(f"outputs are among {tuple(kinds)}")
+        r = {k: np.empty((max(ng, 0), ny, nx), kinds[k]) for k in outputs}
+        mo = MergeOut(*[_np_ptr(r.get(k)) for k in ("vmax", "first", "count")])
+        self._check(self.lib.vhp_visibility_merge_batch(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp),
+                                                        _np_ptr(gm), ng, float(threshold), dtype, C.byref(mo)))
+        return r
+
+    def visibility_merge_batch_dev(self, occ_t, src_xy_t, group_ptr_t, threshold, vmax_t=None, first_t=None,
+                                   count_t=None, group_map_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), src_xy_t int32 (nsrc, 2),
+        group_ptr_t int64 (ngroups + 1), outputs (ngroups, ny, nx): vmax_t float32/64, first_t int32,
+        count_t int32 (read as uint32); any may be None."""
+        nmaps, ny, nx = occ_t.shape
+        ng = group_ptr_t.shape[0] - 1
+        dtype = F32 if (vmax_t is not None and vmax_t.element_size() == 4) else F64
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        mo = MergeOut(ptr(vmax_t), ptr(first_t), ptr(count_t))
+        self._check(self.lib.vhp_visibility_merge_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), group_ptr_t.data_ptr(),
+            ptr(group_map_t), ng, src_xy_t.shape[0], float(threshold), dtype, C.byref(mo)))
 
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):

@@ -150,6 +150,8 @@ vhp_status check_device_error(vhp_context *ctx) {
   VHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   if (flag) {
     VHP_CUDA(ctx, cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
+    if (flag & 4)
+      return fail(ctx, VHP_ERR_INVALID_ARG, "inconsistent source groups (group_ptr / group_map)");
     return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
   }
   return VHP_OK;
@@ -688,12 +690,17 @@ int64_t bin_chunk_pairs(size_t cells, int64_t n) {
 // Batches the one-CTA tile kernel takes are swept straight into bits (kFmtBits: the field itself is
 // never stored); a non-positive threshold, a few pairs of a large map (grid mode) and the naive
 // kernel go through the fp64 field in ctx->b_bin (at most bin_chunk_pairs pairs).
-bool sweeps_into_bits(const vhp_context *ctx, int nx, int ny, int64_t np, double thr) {
+// Does a batch of np pairs run on the one-CTA tile kernel (not the naive kernel, not grid mode; see run_dev)?
+bool one_cta_tile_route(const vhp_context *ctx, int nx, int ny, int64_t np) {
   const size_t cells = (size_t)nx * ny;
-  return ctx->sweep_impl == 0 && ctx->bin_direct && thr > 0.0 && vhp_sweep_tile_supported(nx, ny) &&
+  return ctx->sweep_impl == 0 && vhp_sweep_tile_supported(nx, ny) &&
          !(ctx->grid_sweep == 2 && vhp_sweep_grid_supported(nx, ny)) &&
          !(ctx->grid_sweep == 1 && vhp_sweep_grid_supported(nx, ny) &&
            np <= std::min<int64_t>(16, (int64_t)(cells / 250000)));
+}
+
+bool sweeps_into_bits(const vhp_context *ctx, int nx, int ny, int64_t np, double thr) {
+  return ctx->bin_direct && thr > 0.0 && one_cta_tile_route(ctx, nx, ny, np);
 }
 
 vhp_status sweep_to_bits(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -888,6 +895,153 @@ vhp_status run_runs_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx
   ctx->tile_src = nullptr;
   ctx->last_result_bytes = ctx->last_d2h_bytes;
   if (result != VHP_OK) return result;
+  return check_device_error(ctx);
+}
+
+// ---- merged visibility of groups of sources (vhp_visibility_merge_batch) ----------------------------
+// The outputs are filled on the stream, the per-pair table (group, index in the group, map) is built from the CSR
+// layout, then either the sweeps fold straight into the outputs (kFmtMerge*: the one-CTA tile kernel takes the
+// batch and thr > 0, so cells of value 0 never need a visit) or chunks of pairs are swept into the fp64 field in
+// ctx->b_bin by any route of run_dev (grid mode, naive kernel, thr <= 0) and merge_fold_kernel folds them.
+vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
+                            const void *group_ptr, int64_t ngroups, int64_t nsrc, double thr, int dtype,
+                            const vhp_merge_out *out) {
+  if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
+  if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
+  if (nmaps < 1 || nx < 1 || ny < 1 || ngroups < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
+  if (ngroups > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: more than 2^31 - 1 groups");
+  if ((int64_t)nx * ny > (int64_t)1 << 30 || nx > 16384 || ny > 16384)
+    return fail(ctx, VHP_ERR_UNSUPPORTED, "grid larger than 16384 x 16384 is not supported");
+  if (dtype != VHP_F32 && dtype != VHP_F64) return fail(ctx, VHP_ERR_INVALID_ARG, "bad dtype");
+  if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: threshold is NaN");
+  if (!out->vmax && !out->first && !out->count)
+    return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: no output requested");
+  return VHP_OK;
+}
+
+VhpMergeDev merge_dev_of(const vhp_merge_out &o, vhp_dtype dtype) {
+  VhpMergeDev m;
+  m.vmax = o.vmax;
+  m.f32 = dtype == VHP_F32;
+  m.first = o.first;
+  m.count = o.count;
+  return m;
+}
+
+vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                         const int64_t *d_gptr, const int32_t *d_gmap, int64_t ngroups, int64_t nsrc, double thr,
+                         VhpMergeDev m) {
+  const size_t cells = (size_t)nx * ny;
+  VHP_CUDA(ctx, vhp_launch_merge_fill(m, (size_t)ngroups * cells, ctx->stream));
+  if (ngroups == 0 && nsrc == 0) return VHP_OK;
+  vhp_status st = ensure(ctx, ctx->b_merge, 12 * (size_t)std::max<int64_t>(nsrc, 1));
+  if (st != VHP_OK) return st;
+  int32_t *pg = (int32_t *)ctx->b_merge.p, *pk = pg + nsrc, *pm = pk + nsrc;
+  VHP_CUDA(ctx, vhp_launch_merge_table(d_gptr, d_gmap, ngroups, nsrc, nmaps, pg, pk, pm, ctx->d_err, ctx->sm_count,
+                                       ctx->stream, &ctx->launches));
+  if (nsrc == 0) return VHP_OK;
+  m.pair_group = pg;
+  m.pair_k = pk;
+  m.pair_map = pm;
+  if (thr > 0.0 && one_cta_tile_route(ctx, nx, ny, nsrc)) {
+    if ((st = ensure_rcp2(ctx, std::max(nx, ny) + 64)) != VHP_OK) return st;
+    if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
+    VHP_CUDA(ctx, vhp_launch_sweep_merge(ctx->tile, nx, ny, d_xy, m, nsrc, thr, ctx->rcp2_table, ctx->d_err,
+                                         ctx->stream, &ctx->launches));
+    return VHP_OK;
+  }
+  const int64_t chunk = bin_chunk_pairs(cells, nsrc);
+  if ((st = ensure(ctx, ctx->b_bin, (size_t)chunk * cells * 8)) != VHP_OK) return st;
+  for (int64_t p0 = 0; p0 < nsrc; p0 += chunk) {
+    const int64_t np = std::min(chunk, nsrc - p0);
+    if ((st = run_dev(ctx, Op::Sweep, d_occ, nmaps, nx, ny, d_xy + 2 * p0, pm + p0, np, VHP_F64, ctx->b_bin.p)) !=
+        VHP_OK)
+      return st;
+    VHP_CUDA(ctx, vhp_launch_merge_fold((const double *)ctx->b_bin.p, p0, np, nx, ny, d_xy, thr, m, ctx->sm_count,
+                                        ctx->stream, &ctx->launches));
+  }
+  return VHP_OK;
+}
+
+// host buffers: validate, upload maps and sources once, then runs of whole groups whose outputs fit 1 GB of device
+// memory (at least one group), each copied back with plain cudaMemcpyAsync (the merged result is already K times
+// smaller than the fields it folds)
+vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
+                          const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
+                          const vhp_merge_out *out) {
+  const char *what = "vhp_visibility_merge_batch";
+  if (ctx && gptr && ngroups >= 0) {
+    if (gptr[0] != 0) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(what) + ": group_ptr[0] must be 0");
+    for (int64_t g = 0; g < ngroups; ++g) {
+      if (gptr[g + 1] < gptr[g])
+        return fail(ctx, VHP_ERR_INVALID_ARG, std::string(what) + ": group_ptr decreases at group " + std::to_string(g));
+      if (gptr[g + 1] - gptr[g] >= ((int64_t)1 << 31))
+        return fail(ctx, VHP_ERR_INVALID_ARG,
+                    std::string(what) + ": group " + std::to_string(g) + " has 2^31 or more sources");
+    }
+  }
+  const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
+  vhp_status st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out);
+  if (st != VHP_OK) return st;
+  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, what)) != VHP_OK) return st;
+  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, what)) != VHP_OK) return st;
+  ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
+  ctx->last_transport_packed = 0;
+  if (ngroups == 0) return VHP_OK;
+  VHP_ON_DEVICE(ctx);
+  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8, occ_bytes = (size_t)nmaps * cells;
+  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
+  if ((st = ensure(ctx, ctx->b_src, 8 * (size_t)std::max<int64_t>(nsrc, 1))) != VHP_OK) return st;
+  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  if (nsrc > 0)
+    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, xy, (size_t)nsrc * 8, cudaMemcpyHostToDevice, ctx->stream));
+  ctx->planes_sticky = false;
+  ctx->tile_src = nullptr;
+  if (ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
+    if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
+    ctx->planes_sticky = true;
+  }
+  const size_t bv = out->vmax ? esz : 0, bf = out->first ? 4 : 0, bc = out->count ? 4 : 0;
+  const int64_t gchunk = std::min<int64_t>(ngroups, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / (cells * (bv + bf + bc)))));
+  vhp_status result = ensure(ctx, ctx->b_out[0], (size_t)gchunk * cells * (bv + bf + bc));
+  if (result == VHP_OK) result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gchunk + 1));
+  if (result == VHP_OK && gmap) result = ensure(ctx, ctx->b_map, 4 * (size_t)gchunk);
+  std::vector<int64_t> h_ptr((size_t)gchunk + 1);
+  const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
+  for (int64_t g0 = 0; g0 < ngroups && result == VHP_OK; g0 += gchunk) {
+    const int64_t gc = std::min(gchunk, ngroups - g0), a = gptr[g0];
+    for (int64_t i = 0; i <= gc; ++i) h_ptr[(size_t)i] = gptr[g0 + i] - a;
+    char *base = (char *)ctx->b_out[0].p;
+    VhpMergeDev m;
+    m.f32 = dtype == VHP_F32;
+    m.vmax = out->vmax ? base : nullptr;
+    m.first = out->first ? (int32_t *)(base + (size_t)gc * cells * bv) : nullptr;
+    m.count = out->count ? (uint32_t *)(base + (size_t)gc * cells * (bv + bf)) : nullptr;
+    cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
+                                    ctx->stream);
+    if (e == cudaSuccess && gmap)
+      e = cudaMemcpyAsync(ctx->b_map.p, gmap + g0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: upload of the group layout"); break; }
+    result = run_merge_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a,
+                           (const int64_t *)ctx->b_misc.p, gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc,
+                           gptr[g0 + gc] - a, thr, m);
+    if (result != VHP_OK) break;
+    const size_t n = (size_t)gc * cells, off = (size_t)g0 * cells;
+    if (out->vmax) e = cudaMemcpyAsync((char *)out->vmax + off * esz, m.vmax, n * esz, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->first)
+      e = cudaMemcpyAsync(out->first + off, m.first, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->count)
+      e = cudaMemcpyAsync(out->count + off, m.count, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: copy of the group outputs"); break; }
+    ctx->last_d2h_bytes += (int64_t)(n * (bv + bf + bc));
+  }
+  cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
+  ctx->planes_sticky = false;
+  ctx->tile_src = nullptr;
+  ctx->last_result_bytes = ctx->last_d2h_bytes;
+  if (result != VHP_OK) return result;
+  if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
   return check_device_error(ctx);
 }
 
@@ -1144,7 +1298,8 @@ void vhp_context_destroy(vhp_context *ctx) {
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
   if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
   VhpDevBuf *bufs[] = {&ctx->b_occ, &ctx->b_src, &ctx->b_map, &ctx->b_out[0], &ctx->b_out[1],
-                       &ctx->b_scratch, &ctx->b_planner, &ctx->b_misc, &ctx->b_grid, &ctx->b_bin};
+                       &ctx->b_scratch, &ctx->b_planner, &ctx->b_misc, &ctx->b_grid, &ctx->b_bin,
+                       &ctx->b_merge};
   for (VhpDevBuf *b : bufs)
     if (b->p) cudaFree(b->p);
   delete ctx->expand_pool;
@@ -1413,6 +1568,24 @@ vhp_status vhp_visibility_batch_bin_dev(vhp_context *ctx, const uint8_t *d_occ, 
   if (st != VHP_OK) return st;
   VHP_ON_DEVICE(ctx);
   return run_bin_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_src_map, npairs, threshold, d_out_bits);
+}
+
+vhp_status vhp_visibility_merge_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                      const int32_t *src_xy, const int64_t *group_ptr, const int32_t *group_map,
+                                      int64_t ngroups, double threshold, vhp_dtype dtype, const vhp_merge_out *out) {
+  return run_merge_host(ctx, occ, nmaps, nx, ny, src_xy, group_ptr, group_map, ngroups, threshold, dtype, out);
+}
+
+vhp_status vhp_visibility_merge_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                          const int32_t *d_src_xy, const int64_t *d_group_ptr,
+                                          const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
+                                          double threshold, vhp_dtype dtype, const vhp_merge_out *d_out) {
+  vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
+                                   d_out);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
+                       merge_dev_of(*d_out, dtype));
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

@@ -1,0 +1,142 @@
+// kernels_merge.cu -- merged visibility of groups of light sources (vhp_visibility_merge_batch): the per-pair
+// table of the CSR group layout, the output fill and the fold of fp64 fields into the group outputs.
+//
+// The fold is the route every size and threshold can take (the sweeps themselves run through run_dev: tile
+// kernel, grid mode or the naive kernel, into a chunk buffer); the direct route (kFmtMerge* of the tile kernel,
+// thr > 0) folds inside the sweep.  Both compute, per cell of group g over its sources k = 0, 1, ...:
+//   vmax  = max_k v_k                          (fp32: the fp64 maximum rounded once)
+//   first = min { k : k writes the cell, v_k >= thr }, -1 if none
+//   count = #{ k : k writes the cell, v_k >= thr }
+// where source (sx, sy) writes every cell but column 0 (unless sx == 0) and row 0 (unless sy == 0).
+#include <algorithm>
+#include <cstdint>
+
+#include "vhp_internal.h"
+
+namespace {
+
+constexpr int kErrGroups = 4; // d_err bit: inconsistent group layout / group map
+
+// Thread t < nsrc: pair t -> (group, index in group, map) by a binary search of group_ptr; thread t <= ngroups:
+// group_ptr[0] == 0, non-decreasing, groups below 2^31 sources, group_ptr[ngroups] == nsrc.
+__global__ void merge_table_kernel(const int64_t *__restrict__ gptr, const int32_t *__restrict__ gmap,
+                                   int64_t ngroups, int64_t nsrc, int nmaps, int32_t *__restrict__ pg,
+                                   int32_t *__restrict__ pk, int32_t *__restrict__ pmap, int *err) {
+  const int64_t n = nsrc > ngroups + 1 ? nsrc : ngroups + 1;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
+    if (t <= ngroups) {
+      const int64_t a = __ldg(gptr + t);
+      bool ok = t == 0 ? a == 0 : true;
+      if (t < ngroups) {
+        const int64_t b = __ldg(gptr + t + 1);
+        ok = ok && b >= a && b - a < ((int64_t)1 << 31);
+      } else {
+        ok = ok && a == nsrc;
+      }
+      if (!ok) atomicOr(err, kErrGroups);
+    }
+    if (t < nsrc) {
+      int64_t lo = 0, hi = ngroups; // largest g < ngroups with gptr[g] <= t
+      while (hi - lo > 1) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(gptr + mid) <= t) lo = mid;
+        else hi = mid;
+      }
+      int32_t g = -1, k = 0, m = 0;
+      if (ngroups > 0) {
+        const int64_t a = __ldg(gptr + lo), b = __ldg(gptr + lo + 1);
+        const int32_t mm = gmap ? __ldg(gmap + lo) : 0;
+        if (a <= t && t < b && mm >= 0 && mm < nmaps) {
+          g = (int32_t)lo;
+          k = (int32_t)(t - a);
+          m = mm;
+        }
+      }
+      if (g < 0) atomicOr(err, kErrGroups);
+      pg[t] = g;
+      pk[t] = k;
+      pmap[t] = m;
+    }
+  }
+}
+
+// One thread per cell of every group that has pairs in [p0, p0 + np): the thread of the group's first pair in
+// the chunk folds that group's pairs in order (no atomics; groups that span chunks continue where the last
+// chunk left them).
+template <bool F32>
+__global__ void merge_fold_kernel(const double *__restrict__ field, int64_t p0, int64_t np, int nx, size_t cells,
+                                  const int32_t *__restrict__ xy, double thr, VhpMergeDev m) {
+  const size_t total = (size_t)np * cells;
+  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total;
+       idx += (size_t)gridDim.x * blockDim.x) {
+    const int64_t j = (int64_t)(idx / cells);
+    const size_t c = idx - (size_t)j * cells;
+    const int64_t p = p0 + j;
+    const int32_t g = __ldg(m.pair_group + p);
+    if (g < 0 || (j > 0 && __ldg(m.pair_group + p - 1) == g)) continue;
+    const int x = (int)(c % nx), y = (int)(c / nx);
+    const size_t o = (size_t)g * cells + c;
+    double vm = 0.0;
+    float vf = 0.0f;
+    if (m.vmax) {
+      if (F32) vf = reinterpret_cast<const float *>(m.vmax)[o];
+      else vm = reinterpret_cast<const double *>(m.vmax)[o];
+    }
+    int32_t f = m.first ? m.first[o] : -1;
+    uint32_t cnt = m.count ? m.count[o] : 0u;
+    for (int64_t q = p; q < p0 + np && __ldg(m.pair_group + q) == g; ++q) {
+      const double v = __ldg(field + (size_t)(q - p0) * cells + c);
+      const int sx = __ldg(xy + 2 * q), sy = __ldg(xy + 2 * q + 1);
+      if (F32) vf = fmaxf(vf, __double2float_rn(v));
+      else vm = fmax(vm, v);
+      const bool writes = !((x == 0 && sx != 0) || (y == 0 && sy != 0));
+      if (writes && v >= thr) {
+        if (f < 0) f = __ldg(m.pair_k + q);
+        ++cnt;
+      }
+    }
+    if (m.vmax) {
+      if (F32) reinterpret_cast<float *>(m.vmax)[o] = vf;
+      else reinterpret_cast<double *>(m.vmax)[o] = vm;
+    }
+    if (m.first) m.first[o] = f;
+    if (m.count) m.count[o] = cnt;
+  }
+}
+
+unsigned grid_for(size_t n, int bs, int sm_count) {
+  return (unsigned)std::max<size_t>(1, std::min<size_t>((n + bs - 1) / bs, (size_t)sm_count * 32));
+}
+
+} // namespace
+
+cudaError_t vhp_launch_merge_table(const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t ngroups,
+                                   int64_t nsrc, int nmaps, int32_t *d_pair_group, int32_t *d_pair_k,
+                                   int32_t *d_pair_map, int *d_err, int sm_count, cudaStream_t st,
+                                   int64_t *launches) {
+  const int bs = 256;
+  merge_table_kernel<<<grid_for((size_t)std::max(nsrc, ngroups + 1), bs, sm_count), bs, 0, st>>>(
+      d_group_ptr, d_group_map, ngroups, nsrc, nmaps, d_pair_group, d_pair_k, d_pair_map, d_err);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t vhp_launch_merge_fill(const VhpMergeDev &m, size_t cells_total, cudaStream_t st) {
+  cudaError_t e = cudaSuccess;
+  if (m.vmax) e = cudaMemsetAsync(m.vmax, 0, cells_total * (m.f32 ? 4 : 8), st);
+  if (e == cudaSuccess && m.first) e = cudaMemsetAsync(m.first, 0xff, cells_total * 4, st); // VHP_NO_PARENT
+  if (e == cudaSuccess && m.count) e = cudaMemsetAsync(m.count, 0, cells_total * 4, st);
+  return e;
+}
+
+cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np, int nx, int ny,
+                                  const int32_t *d_src_xy, double thr, const VhpMergeDev &m, int sm_count,
+                                  cudaStream_t st, int64_t *launches) {
+  const size_t cells = (size_t)nx * ny;
+  const int bs = 256;
+  const unsigned grid = grid_for((size_t)np * cells, bs, sm_count);
+  if (m.f32) merge_fold_kernel<true><<<grid, bs, 0, st>>>(d_field, p0, np, nx, cells, d_src_xy, thr, m);
+  else merge_fold_kernel<false><<<grid, bs, 0, st>>>(d_field, p0, np, nx, cells, d_src_xy, thr, m);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}

@@ -42,6 +42,13 @@ sweep_tile_kernel(const TileArgs p) {
     return;
   }
   const int map = p.src_map ? __ldg(p.src_map + pair) : 0;
+  if constexpr (FMT == kFmtMerge64 || FMT == kFmtMerge32) { // fold into the outputs of the pair's group
+    const int g = __ldg(p.m_pg + pair);
+    if (g < 0) return; // a pair of an inconsistent group layout (the table kernel reported it)
+    if (threadIdx.x == 0) *reinterpret_cast<int2 *>(smem_raw + kMergeHdr) = make_int2(g, __ldg(p.m_pk + pair));
+    tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, reinterpret_cast<OutT *>(p.out), smem_raw);
+    return;
+  }
   // bit output: rows of (nx + 31) / 32 words
   const size_t per_pair = FMT == kFmtBits ? (size_t)((p.nx + 31) >> 5) * p.ny : (size_t)p.nx * p.ny;
   OutT *out = reinterpret_cast<OutT *>(p.out) + (size_t)pair * per_pair;
@@ -233,7 +240,50 @@ cudaError_t launch_tile_fmt(const TileArgs &p, int64_t npairs, cudaStream_t st) 
   }
 }
 
+// merged output (kFmtMerge*): fp64 staging whatever the dtype of vmax, the warp counts of the bit output
+template <int FMT>
+cudaError_t launch_tile_merge(const TileArgs &p, int64_t npairs, cudaStream_t st) {
+  switch (tile_warps_for(p.nx, p.ny, npairs)) {
+    case 1: return launch_tile_nw<double, 1, VHP_NW1_MINB, FMT>(p, npairs, st);
+    case 2: case 4: case 6: return launch_tile_nw<double, 4, VHP_NW4_MINB, FMT>(p, npairs, st);
+    default: return launch_tile_nw<double, 8, VHP_NW8_MINB, FMT>(p, npairs, st);
+  }
+}
+
 } // namespace
+
+cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
+                                   const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,
+                                   int *d_err, cudaStream_t st, int64_t *launches) {
+  if (!(thr > 0.0)) return cudaErrorInvalidValue; // cells of value 0 are never visited
+  TileArgs p;
+  p.pl = pl;
+  p.nx = nx;
+  p.ny = ny;
+  p.src_xy = d_src_xy;
+  p.src_map = m.pair_map;
+  p.out = const_cast<int32_t *>(m.pair_group); // a base for cell indices only
+  p.rtab = reinterpret_cast<const double2 *>(d_rcp2);
+  p.err = d_err;
+  p.vec = 0;
+  p.win_y0 = 0;
+  p.win_y1 = ny;
+  for (int q = 0; q < 4; ++q) p.halo[q] = nullptr;
+  p.g_edges = nullptr;
+  p.g_lm = p.g_prog = p.g_next_row = nullptr;
+  p.qmask = 0xF;
+  p.src_ctl = nullptr;
+  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
+  p.thr = thr;
+  p.m_vmax = m.vmax;
+  p.m_first = m.first;
+  p.m_count = m.count;
+  p.m_cells = (size_t)nx * ny;
+  p.m_pg = m.pair_group;
+  p.m_pk = m.pair_k;
+  if (launches) *launches += 1;
+  return m.f32 ? launch_tile_merge<kFmtMerge32>(p, npairs, st) : launch_tile_merge<kFmtMerge64>(p, npairs, st);
+}
 
 bool vhp_sweep_tile_supported(int nx, int ny) {
   return nx >= 1 && ny >= 1 && std::max(nx, ny) <= 16384 &&

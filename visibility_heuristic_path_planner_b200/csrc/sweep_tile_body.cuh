@@ -159,7 +159,13 @@ struct TileArgs {
   int *x_prog;
   int x_y0, x_y1;
   int remote_mask;
-  double thr; // kFmtBits: bit = (fp64 value >= thr), thr > 0
+  double thr; // kFmtBits: bit = (fp64 value >= thr), thr > 0; kFmtMerge*: the count / first threshold
+  // kFmtMerge*: the outputs of all groups ([group][ny][nx] each, any may be null) and the cells of one grid
+  void *m_vmax = nullptr;
+  int32_t *m_first = nullptr;
+  uint32_t *m_count = nullptr;
+  size_t m_cells = 0;
+  const int32_t *m_pg = nullptr, *m_pk = nullptr; // per pair: group (-1: skip the pair) and index within it
 };
 
 // how tile_sweep_cta is used
@@ -251,7 +257,47 @@ __device__ __forceinline__ void stg16_fill(double *q, double v) {
 // bit (x & 31) of word [y][x >> 5] = (fp64 value >= TileArgs::thr), rows of (nx + 31) / 32 words,
 // for thr > 0 and into a ZEROED buffer: cells below the threshold are not written at all, the
 // words around the source column (shared by the -x and +x quadrants) are or-ed in atomically.
-constexpr int kFmtValues = 0, kFmtBits = 2;
+// kFmtMerge64 / kFmtMerge32: the sweep is folded into the outputs of its GROUP of sources (vhp_visibility_merge_batch):
+// per cell with fp64 value v > 0, vmax = max(vmax, v) as an integer max on the bits (fp64, or fp32 of RN(v): non-negative
+// IEEE values order like their bit patterns and rounding is monotone), and where v >= thr (> 0), first = min(first, k)
+// and count += 1, k = the source's index within its group.  Cells of value 0 are not touched, which is why thr > 0.
+// Other CTAs sweep sources of the same group at the same time, so every write is a relaxed atomic (red), never a
+// plain store; count relies on the sweep storing each cell once (axis cells: the + quadrant only).  OutT is double
+// (the staging tiles hold the fp64 values); `out` is only a base for cell indices.
+constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4;
+constexpr int kMergeHdr = 224; // shared-memory header: {group, k} of the CTA's source (int2)
+
+__device__ __forceinline__ void red_max_u64(unsigned long long *a, unsigned long long v) {
+  asm volatile("red.relaxed.gpu.global.max.u64 [%0], %1;" :: "l"(a), "l"(v) : "memory");
+}
+__device__ __forceinline__ void red_max_u32(uint32_t *a, uint32_t v) {
+  asm volatile("red.relaxed.gpu.global.max.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
+}
+__device__ __forceinline__ void red_min_u32(uint32_t *a, uint32_t v) {
+  asm volatile("red.relaxed.gpu.global.min.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
+}
+__device__ __forceinline__ void red_add_u32(uint32_t *a, uint32_t v) {
+  asm volatile("red.relaxed.gpu.global.add.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
+}
+
+// fold value v of cell idx (y * nx + x) of this CTA's sweep into its group's outputs
+template <int FMT>
+__device__ __forceinline__ void merge_cell(const TileArgs &p, const ptrdiff_t idx, const double v) {
+  if (!(v > 0.0)) return;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int2 gk = *reinterpret_cast<const int2 *>(smem_raw + kMergeHdr);
+  const size_t o = (size_t)gk.x * p.m_cells + (size_t)idx;
+  if (p.m_vmax) {
+    if constexpr (FMT == kFmtMerge64)
+      red_max_u64(reinterpret_cast<unsigned long long *>(p.m_vmax) + o, (unsigned long long)__double_as_longlong(v));
+    else
+      red_max_u32(reinterpret_cast<uint32_t *>(p.m_vmax) + o, __float_as_uint(__double2float_rn(v)));
+  }
+  if (v >= p.thr) {
+    if (p.m_first) red_min_u32(reinterpret_cast<uint32_t *>(p.m_first) + o, (uint32_t)gk.y);
+    if (p.m_count) red_add_u32(p.m_count + o, 1u);
+  }
+}
 
 // staging tile: element (row r, column c) of a 32 x 32 tile (odd pitch: column-wise writes
 // and the row-wise read-out are both conflict-free)
@@ -416,7 +462,9 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   // before the global stores
   constexpr int kStepUnroll = NW == 1 ? VHP_STEP_UNROLL_1W : VHP_STEP_UNROLL;
   constexpr bool BITS = FMT == kFmtBits;
+  constexpr bool MERGE = FMT == kFmtMerge64 || FMT == kFmtMerge32;
   static_assert(!BITS || sizeof(OutT) == 4, "bit output: OutT is the 32-bit word");
+  static_assert(!MERGE || (sizeof(OutT) == 8 && !GE), "merge output: fp64 staging, one-CTA sweeps");
   auto publish = [&]() {
     if (GE) __threadfence(); // this lane's boundary-row stores, before lane 0 raises the flag
     __syncwarp();
@@ -512,6 +560,13 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
       if (!zero && cor >= p.thr) put_word(__ballot_sync(kAll, lane_st && colc), r0, rc);
       return;
     }
+    if constexpr (MERGE) { // the border row (if any) is 0: nothing to fold
+      if (!zero && cor > 0.0 && lane_st && colc) {
+        const ptrdiff_t i0c = ptr - out;
+        for (int r = r0; r <= rc; ++r) merge_cell<FMT>(p, i0c + r * rs, cor);
+      }
+      return;
+    }
     if (p.vec && nvx == 32 && (I > 0 || g.dirx > 0)) {
       // all 32 columns are stored and x0 is a multiple of 32: 128-bit stores
       constexpr int EPL = 16 / (int)sizeof(OutT), LPR = 32 / EPL; // elements per lane, lanes per row
@@ -604,6 +659,8 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
           if constexpr (BITS) {
             const uint32_t m = __ballot_sync(kAll, ge_thr(F));
             if (lane == s) wb = m;
+          } else if constexpr (MERGE) {
+            if (!decltype(masked)::value || (lane_st && s >= r0 && s <= rlast)) merge_cell<FMT>(p, q - out, F);
           } else if (!decltype(masked)::value || (lane_st && s >= r0 && s <= rlast)) {
             __stcs(q, to_out<OutT>(F));
           }
@@ -669,6 +726,11 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   __syncwarp();
   if constexpr (BITS) {
     put_word(wb & __ballot_sync(kAll, lane_st), r0, rlast);
+  } else if constexpr (MERGE) {
+    if (lane_st) {
+      const ptrdiff_t i0c = ptr - out;
+      for (int r = r0; r <= rlast; ++r) merge_cell<FMT>(p, i0c + r * rs, stage[stage_at(r, lane)]);
+    }
   } else if (lane_st) {
     OutT *q = ptr + r0 * rs;
 #pragma unroll kFillUnroll
@@ -698,7 +760,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
   TQuad *quads = reinterpret_cast<TQuad *>(smem_raw);
   // next tile row to hand out (NW > 1)
   int *next_row = GE ? p.g_next_row : reinterpret_cast<int *>(smem_raw + 240);
-  static_assert(4 * sizeof(TQuad) <= 240, "quadrant geometry overlaps the row counter");
+  static_assert(4 * sizeof(TQuad) <= kMergeHdr, "quadrant geometry overlaps the merge slot / row counter");
   uint32_t *bsum = reinterpret_cast<uint32_t *>(smem_raw + kTileHdr);
   const int nsum = tile_sum_words(nx) * ((ny + 31) >> 5);
   const int lmcap = tile_lm_cap(ny);
@@ -891,6 +953,21 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
           j = jn;
         }
       }
+    } else if constexpr (FMT == kFmtMerge64 || FMT == kFmtMerge32) {
+      // merge output: the lit spans of the value loop below, folded cell by cell (value 1.0); the never-written
+      // cells of those rows (x == 0 left of the source, row 0 below it) hold 0 and are left alone
+      static_assert(!GE, "merge output is a one-CTA sweep");
+      for (int y = ylo + warp; y <= yhi; y += NW) {
+        const bool upper = y >= sy;
+        if (!upper && y == 0) continue;
+        const int j = upper ? y - sy : sy - y;
+        const int nR = upper ? lit_run(0, j) : lit_run(3, j);
+        const int nL = upper ? lit_run(1, j) : lit_run(2, j);
+        if (nR == 0 && nL <= 1) continue;
+        const int xl = nL > 1 ? max(sx - (nL - 1), 1) : sx; // first lit column
+        const int xr = nR > 0 ? sx + nR - 1 : sx - 1;       // last lit column
+        for (int x = xl + lane; x <= xr; x += 32) merge_cell<FMT>(p, (ptrdiff_t)y * nx + x, 1.0);
+      }
     } else
     for (int y = max(ylo, p.win_y0) + wfirst; y <= min(yhi, p.win_y1 - 1); y += wstride) {
       const bool upper = y >= sy;
@@ -962,7 +1039,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
             const int rlast = min(min((J ? kTile : g.a) - 1, g.Ey - j0row), g.jw1 - j0row);
             const int ie = min(g.Ex, tile_start(g.a, Istop) - 1); // last local column of the run
             const int xa = g.dirx > 0 ? sx + i0 : sx - ie, xb = g.dirx > 0 ? sx + ie : sx - i0;
-            if constexpr (!BITS)
+            if constexpr (FMT == kFmtValues)
               fill_block<OutT>(out, nx, sy + g.diry * (j0row + r0), g.diry, rlast - r0 + 1, xa, xb,
                                to_out<OutT>(0.0), lane, p.vec != 0);
             if (Istop >= g.TX) return;

@@ -103,10 +103,11 @@ struct vhp_context {
   int sm_count = 0;
   int64_t launches = 0;
   std::string last_error;
-  // device-side error word (bit 0: a source / start / end outside the grid)
+  // device-side error word (bit 0: a source / start / end outside the grid, bit 2: inconsistent source groups)
   int *d_err = nullptr;
   // workspace buffers (grown on demand, reused across calls)
   VhpDevBuf b_occ, b_src, b_map, b_out[2], b_scratch, b_planner, b_misc, b_grid, b_bin;
+  VhpDevBuf b_merge; // vhp_visibility_merge_batch: per-pair table; host call: group layout too
   cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
   // 1/k table {rh, rl} of the tile kernel (double-double reciprocal), device resident
   double *rcp2_table = nullptr;
@@ -195,6 +196,33 @@ cudaError_t vhp_launch_sweep_tile(const VhpTilePlanes &pl, int nx, int ny, const
                                   int64_t *launches, const double *thr = nullptr, bool bits = false);
 // thr != null, bits: d_out = uint32 words, bit (x & 31) of word [pair][y][x >> 5] = (fp64 value >= thr);
 // needs thr > 0 (zeroes d_out, then writes only the cells at or above the threshold).
+
+// Merged visibility of groups of sources (vhp_visibility_merge_batch): the group outputs ([group][ny][nx], any may be
+// null; vmax fp32 when f32) and the per-pair table merge_table_kernel builds from the CSR group layout.
+struct VhpMergeDev {
+  void *vmax = nullptr;
+  int f32 = 0;
+  int32_t *first = nullptr;
+  uint32_t *count = nullptr;
+  const int32_t *pair_group = nullptr; // group of the pair, -1: the layout is inconsistent there (skip it)
+  const int32_t *pair_k = nullptr;     // index of the pair within its group
+  const int32_t *pair_map = nullptr;   // map of the pair (its group's)
+};
+// the sweeps fold straight into the group outputs (kFmtMerge*, one CTA per pair); needs thr > 0 and zero-filled
+// vmax / count, -1-filled first
+cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
+                                   const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,
+                                   int *d_err, cudaStream_t st, int64_t *launches);
+// kernels_merge.cu: the per-pair table (validates the layout: bit 4 of d_err), the output fill, and the fold of
+// np fp64 fields of pairs [p0, p0 + np) (what the fallback sweeps into a chunk buffer) into the group outputs
+cudaError_t vhp_launch_merge_table(const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t ngroups,
+                                   int64_t nsrc, int nmaps, int32_t *d_pair_group, int32_t *d_pair_k,
+                                   int32_t *d_pair_map, int *d_err, int sm_count, cudaStream_t st,
+                                   int64_t *launches);
+cudaError_t vhp_launch_merge_fill(const VhpMergeDev &m, size_t cells_total, cudaStream_t st);
+cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np, int nx, int ny,
+                                  const int32_t *d_src_xy, double thr, const VhpMergeDev &m, int sm_count,
+                                  cudaStream_t st, int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
