@@ -202,6 +202,25 @@ vhp_status vhp_visibility_merge_batch_dev(vhp_context *ctx, const uint8_t *d_occ
                                           const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
                                           double threshold, vhp_dtype dtype, const vhp_merge_out *d_out);
 
+/* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
+ *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
+ *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])
+ * i.e. bit-identical to the crop of the full field (the sweep's dependencies point towards the source, so
+ * the window depends on nothing outside it), never-written border included.  dtype as vhp_visibility_batch
+ * (VHP_F32 = the fp64 value rounded once).  0 <= radius <= 16383.  Work and traffic per pair scale with the
+ * window, not with the map: the batched tile kernel sweeps only the window, with its per-pair state sized by
+ * the window, so range-limited batches on maps up to 16384 x 16384 run on it.  The naive kernel, grid mode 2
+ * and windows too large for one CTA sweep whole fields and crop them, with the same result.
+ * Errors (VHP_ERR_INVALID_ARG): a radius out of range, a null out, a source outside the grid, a map index out
+ * of range; the _dev form reports the last two like vhp_visibility_batch_dev (by the next synchronising
+ * call) and reuses the bit planes of vhp_prepare_maps_dev. */
+vhp_status vhp_visibility_window_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                       const int32_t *src_xy, const int32_t *src_map, int64_t npairs,
+                                       int32_t radius, vhp_dtype dtype, void *out);
+vhp_status vhp_visibility_window_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                           const int32_t *d_src_xy, const int32_t *d_src_map, int64_t npairs,
+                                           int32_t radius, vhp_dtype dtype, void *d_out);
+
 /* ---- opt-in variants of the sweep (SURVEY 8f): the paper's MATLAB algorithm and the reference's
  * early-terminating queue variant.  Same layouts as vhp_visibility_batch.
  *   VHP_VARIANT_MATLAB  getAccessibilityMap.m (MATLAB_code/visibility/getAccessibilityMap.m:1-118):

@@ -115,6 +115,8 @@ def load_library(build_if_missing: bool = True):
                                                C.POINTER(MergeOut)]
     lib.vhp_visibility_merge_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_double, i32,
                                                    C.POINTER(MergeOut)]
+    for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
+        getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
     for name in ("vhp_packed_pairs", "vhp_packed_bytes", "vhp_packed_pair_bytes"):
         getattr(lib, name).argtypes = [vp]
@@ -279,17 +281,19 @@ class Context:
         return bad.value
 
     # ---- host (numpy) entry points ------------------------------------------
-    def _batch_host(self, fn, occ, src_xy, src_map, dtype, out=None):
+    def _batch_host(self, fn, occ, src_xy, src_map, dtype, out=None, pair_shape=None):
+        """pair_shape: the result of one pair, (ny, nx) by default."""
         occ = _occ_u8(occ)
         nmaps, ny, nx = occ.shape
         xy = np.ascontiguousarray(src_xy, dtype=np.int32).reshape(-1, 2)
         n = xy.shape[0]
         mp = None if src_map is None else np.ascontiguousarray(src_map, dtype=np.int32)
         odt = np.float32 if dtype == F32 else np.float64
+        shape = (n,) + (tuple(pair_shape) if pair_shape is not None else (ny, nx))
         if out is None:
-            out = np.empty((n, ny, nx), dtype=odt)
-        elif out.dtype != odt or out.shape != (n, ny, nx) or not out.flags.c_contiguous:
-            raise ValueError("out must be a C-contiguous (npairs, ny, nx) array of the result dtype")
+            out = np.empty(shape, dtype=odt)
+        elif out.dtype != odt or out.shape != shape or not out.flags.c_contiguous:
+            raise ValueError(f"out must be a C-contiguous {shape} array of the result dtype")
         self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(mp), n,
                        dtype, _np_ptr(out)))
         return out
@@ -298,6 +302,16 @@ class Context:
         """computeVisibility for every (map, source) pair -> (npairs, ny, nx).  `out`: an
         array to fill instead of a new one (pinned host memory gets the fastest transport)."""
         return self._batch_host(self.lib.vhp_visibility_batch, occ, src_xy, src_map, dtype, out)
+
+    def visibility_window_batch(self, occ, src_xy, radius, src_map=None, dtype=F64, out=None):
+        """Range-limited visibility (vhp_visibility_window_batch) -> (npairs, 2R+1, 2R+1): the window of
+        visibility_batch's field centred on each source, 0 where it leaves the grid."""
+        r = int(radius)
+        w = 2 * r + 1 if r >= 0 else 1  # (a negative radius is rejected by the library)
+
+        def fn(h, occ_p, nmaps, nx, ny, xy_p, mp_p, n, dt, out_p):
+            return self.lib.vhp_visibility_window_batch(h, occ_p, nmaps, nx, ny, xy_p, mp_p, n, r, dt, out_p)
+        return self._batch_host(fn, occ, src_xy, src_map, dtype, out, pair_shape=(w, w))
 
     def visibility_batch_packed(self, occ, src_xy, src_map=None, dtype=F64, handle=None):
         """computeVisibility for every pair, kept as a lossless packed handle
@@ -449,6 +463,16 @@ class Context:
         self._check(self.lib.vhp_visibility_batch_dev(
             self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(),
             None if src_map_t is None else src_map_t.data_ptr(), src_xy_t.shape[0], dtype,
+            out_t.data_ptr()))
+
+    def visibility_window_batch_dev(self, occ_t, src_xy_t, radius, out_t, src_map_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), src_xy_t int32 (n, 2),
+        out_t float32/64 (n, 2R+1, 2R+1), contiguous."""
+        nmaps, ny, nx = occ_t.shape
+        dtype = F32 if out_t.element_size() == 4 else F64
+        self._check(self.lib.vhp_visibility_window_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(),
+            None if src_map_t is None else src_map_t.data_ptr(), src_xy_t.shape[0], int(radius), dtype,
             out_t.data_ptr()))
 
     def raycast_batch_dev(self, occ_t, src_xy_t, out_t, src_map_t=None):

@@ -162,7 +162,7 @@ int grid_sweep_ctas(const vhp_context *ctx, int rows) {
   return std::max(2, std::min(2 * ctx->sm_count, (4 * (rows / 32 + 2) + 7) / 8));
 }
 
-enum class Op { Sweep, Raycast };
+enum class Op { Sweep, Raycast, Window };
 
 vhp_status run_dev(vhp_context *ctx, Op op, const uint8_t *d_occ, int nmaps, int nx, int ny,
                    const int32_t *d_xy, const int32_t *d_map, int64_t n, vhp_dtype dtype,
@@ -233,12 +233,64 @@ vhp_status run_dev(vhp_context *ctx, Op op, const uint8_t *d_occ, int nmaps, int
   return VHP_OK;
 }
 
+// pairs per chunk of fp64 fields (4 GB) where a route goes through whole fields (binary, merged and window outputs)
+int64_t bin_chunk_pairs(size_t cells, int64_t n) {
+  return std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(((size_t)4 << 30) / (cells * 8))));
+}
+
+// ---- range-limited windows (vhp_visibility_window_batch) ----------------------------------------
+// Direct: the one-CTA tile kernel sweeps only each pair's window (kFmtWindow).  Otherwise (the naive kernel, grid
+// mode forced, or a window whose state does not fit one CTA) chunks of full fields go through run_dev, which picks
+// grid mode or the naive kernel as for vhp_visibility_batch, and window_crop_kernel cuts the windows out.
+bool window_direct_route(const vhp_context *ctx, int nx, int ny, int radius) {
+  return ctx->sweep_impl == 0 && ctx->grid_sweep != 2 && vhp_sweep_window_supported(nx, ny, radius);
+}
+
+size_t window_pair_bytes(int radius, vhp_dtype dtype) {
+  const size_t w = 2 * (size_t)radius + 1;
+  return w * w * (dtype == VHP_F32 ? 4 : 8);
+}
+
+vhp_status run_window_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                          const int32_t *d_map, int64_t n, int radius, vhp_dtype dtype, void *d_out) {
+  if (n == 0) return VHP_OK;
+  vhp_status st;
+  if (window_direct_route(ctx, nx, ny, radius)) {
+    if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), radius + 1) + 64)) != VHP_OK) return st;
+    if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
+    VHP_CUDA(ctx, vhp_launch_sweep_window_batch(ctx->tile, nmaps, nx, ny, d_xy, d_map, n, radius, dtype, d_out,
+                                                ctx->rcp2_table, ctx->d_err, ctx->stream, &ctx->launches));
+    return VHP_OK;
+  }
+  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
+  const int64_t chunk = bin_chunk_pairs(cells, n);
+  if ((st = ensure(ctx, ctx->b_bin, (size_t)chunk * cells * esz)) != VHP_OK) return st;
+  if (d_map && (st = ensure(ctx, ctx->b_misc, 12 * (size_t)chunk)) != VHP_OK) return st;
+  for (int64_t p0 = 0; p0 < n; p0 += chunk) {
+    const int64_t np = std::min(chunk, n - p0);
+    const int32_t *xy = d_xy + 2 * p0, *mp = d_map ? d_map + p0 : nullptr;
+    if (mp) { // the full sweeps must not read beyond the maps
+      int32_t *sxy = (int32_t *)ctx->b_misc.p, *smp = sxy + 2 * chunk;
+      VHP_CUDA(ctx, vhp_launch_window_pairs(xy, mp, np, nmaps, sxy, smp, ctx->sm_count, ctx->stream, &ctx->launches));
+      xy = sxy;
+      mp = smp;
+    }
+    if ((st = run_dev(ctx, Op::Sweep, d_occ, nmaps, nx, ny, xy, mp, np, dtype, ctx->b_bin.p)) != VHP_OK) return st;
+    VHP_CUDA(ctx, vhp_launch_window_crop(ctx->b_bin.p, np, nx, ny, xy, radius, dtype,
+                                         (char *)d_out + (size_t)p0 * window_pair_bytes(radius, dtype),
+                                         ctx->sm_count, ctx->stream, &ctx->launches));
+  }
+  return VHP_OK;
+}
+
 // Plain transport of the host-buffer entry points: run in chunks of pairs from p_begin on and
 // overlap the D2H of chunk c with the kernel of chunk c+1 (two device buffers, copy stream).
+// Op::Window delivers the windows of `radius`, every other op whole fields.
 vhp_status run_host_plain(vhp_context *ctx, Op op, int nmaps, int nx, int ny, const int32_t *d_xy,
                           const int32_t *d_map, int64_t n, int64_t p_begin, vhp_dtype dtype,
-                          void *out) {
-  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
+                          void *out, int radius = 0) {
+  const size_t esz = dtype == VHP_F32 ? 4 : 8;
+  const size_t cells = op == Op::Window ? window_pair_bytes(radius, dtype) / esz : (size_t)nx * ny;
   vhp_status st;
   const size_t chunk_bytes_target = (size_t)1 << 30;
   int64_t chunk = std::max<int64_t>(1, (int64_t)(chunk_bytes_target / (cells * esz)));
@@ -262,8 +314,11 @@ vhp_status run_host_plain(vhp_context *ctx, Op op, int nmaps, int nx, int ny, co
       cudaError_t e = cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[b], 0);
       if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaStreamWaitEvent"); break; }
     }
-    result = run_dev(ctx, op, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
-                     d_map ? d_map + p0 : nullptr, np, dtype, ctx->b_out[b].p);
+    result = op == Op::Window
+                 ? run_window_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
+                                  d_map ? d_map + p0 : nullptr, np, radius, dtype, ctx->b_out[b].p)
+                 : run_dev(ctx, op, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
+                           d_map ? d_map + p0 : nullptr, np, dtype, ctx->b_out[b].p);
     if (result != VHP_OK) break;
     cudaError_t e = cudaEventRecord(ctx->ev_done[b], ctx->stream);
     if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_done[b], 0);
@@ -628,14 +683,15 @@ vhp_status run_host_to_packed(vhp_context *ctx, int nmaps, int nx, int ny, const
   return VHP_OK;
 }
 
-// host buffers: upload, run in chunks, deliver the results (packed or plain transport)
+// host buffers: upload, run in chunks, deliver the results (packed or plain transport; windows: plain)
 vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int nx, int ny,
                     const int32_t *xy, const int32_t *maps, int64_t n, vhp_dtype dtype,
-                    void *out) {
+                    void *out, int radius = 0) {
   vhp_status st = check_common(ctx, occ, nmaps, nx, ny, xy, n, dtype, out);
   if (st != VHP_OK) return st;
   st = check_points(ctx, xy, 2, maps, n, nmaps, nx, ny,
-                    op == Op::Sweep ? "vhp_visibility_batch" : "vhp_raycast_batch");
+                    op == Op::Sweep ? "vhp_visibility_batch"
+                                    : (op == Op::Window ? "vhp_visibility_window_batch" : "vhp_raycast_batch"));
   if (st != VHP_OK) return st;
   ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
   ctx->last_transport_packed = 0;
@@ -654,7 +710,7 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
                                   cudaMemcpyHostToDevice, ctx->stream));
   ctx->planes_sticky = false; // b_occ content changed
   ctx->tile_src = nullptr;
-  if (op == Op::Sweep && ctx->sweep_impl == 0 &&
+  if (op != Op::Raycast && ctx->sweep_impl == 0 &&
       (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
     // pack once for all chunks
     if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK)
@@ -663,16 +719,17 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
   }
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
   const int32_t *d_map = maps ? (const int32_t *)ctx->b_map.p : nullptr;
-  const size_t out_bytes = (size_t)n * cells * esz;
+  const size_t out_bytes = (size_t)n * (op == Op::Window ? window_pair_bytes(radius, dtype) : cells * esz);
   ctx->last_result_bytes = (int64_t)out_bytes;
   int64_t p_begin = 0;
   vhp_status result = VHP_OK;
   // small results are not worth the thread pool's wake-up
-  if (ctx->result_transport == 2 || (ctx->result_transport == 1 && out_bytes >= ((size_t)64 << 20))) {
+  if (op != Op::Window &&
+      (ctx->result_transport == 2 || (ctx->result_transport == 1 && out_bytes >= ((size_t)64 << 20)))) {
     result = run_host_packed(ctx, op, nmaps, nx, ny, d_xy, d_map, n, dtype, out, &p_begin);
   }
   if (result == VHP_OK && p_begin < n)
-    result = run_host_plain(ctx, op, nmaps, nx, ny, d_xy, d_map, n, p_begin, dtype, out);
+    result = run_host_plain(ctx, op, nmaps, nx, ny, d_xy, d_map, n, p_begin, dtype, out, radius);
   ctx->planes_sticky = false;
   ctx->tile_src = nullptr;
   if (result != VHP_OK) return result;
@@ -682,9 +739,6 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
 // ---- thresholded binary visibility ------------------------------------------------------------
 // Chunks of pairs: fp64 sweep into a device buffer, threshold_bits_kernel, and for host callers
 // the D2H of chunk c (copy stream, two bit buffers) under the sweeps of chunk c + 1.
-int64_t bin_chunk_pairs(size_t cells, int64_t n) {
-  return std::min<int64_t>(n, std::max<int64_t>(1, (int64_t)(((size_t)4 << 30) / (cells * 8))));
-}
 
 // Thresholded visibility of np pairs as bits (and, d_row_cnt != null, transition columns per row).
 // Batches the one-CTA tile kernel takes are swept straight into bits (kFmtBits: the field itself is
@@ -1366,6 +1420,25 @@ vhp_status vhp_visibility_batch(vhp_context *ctx, const uint8_t *occ, int nmaps,
                                 const int32_t *src_xy, const int32_t *src_map, int64_t npairs,
                                 vhp_dtype dtype, void *out) {
   return run_host(ctx, Op::Sweep, occ, nmaps, nx, ny, src_xy, src_map, npairs, dtype, out);
+}
+
+vhp_status vhp_visibility_window_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                       const int32_t *src_xy, const int32_t *src_map, int64_t npairs,
+                                       int32_t radius, vhp_dtype dtype, void *out) {
+  if (ctx && (radius < 0 || radius > 16383))
+    return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_window_batch: radius outside [0, 16383]");
+  return run_host(ctx, Op::Window, occ, nmaps, nx, ny, src_xy, src_map, npairs, dtype, out, radius);
+}
+
+vhp_status vhp_visibility_window_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                           const int32_t *d_src_xy, const int32_t *d_src_map, int64_t npairs,
+                                           int32_t radius, vhp_dtype dtype, void *d_out) {
+  vhp_status st = check_common(ctx, d_occ, nmaps, nx, ny, d_src_xy, npairs, dtype, d_out);
+  if (st != VHP_OK) return st;
+  if (radius < 0 || radius > 16383)
+    return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_window_batch_dev: radius outside [0, 16383]");
+  VHP_ON_DEVICE(ctx);
+  return run_window_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_src_map, npairs, radius, dtype, d_out);
 }
 
 vhp_status vhp_visibility_batch_packed(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,

@@ -49,6 +49,17 @@ sweep_tile_kernel(const TileArgs p) {
     tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, reinterpret_cast<OutT *>(p.out), smem_raw);
     return;
   }
+  if constexpr (FMT == kFmtWindow) { // the pair's window, addressed by absolute grid coordinates
+    if ((unsigned)map >= (unsigned)p.w_nmaps) {
+      if (threadIdx.x == 0) atomicOr(p.err, 1);
+      return;
+    }
+    const int W = 2 * p.w_r + 1;
+    OutT *out = reinterpret_cast<OutT *>(p.out) + (size_t)pair * W * W -
+                ((ptrdiff_t)(sy - p.w_r) * W + (sx - p.w_r));
+    tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, out, smem_raw);
+    return;
+  }
   // bit output: rows of (nx + 31) / 32 words
   const size_t per_pair = FMT == kFmtBits ? (size_t)((p.nx + 31) >> 5) * p.ny : (size_t)p.nx * p.ny;
   OutT *out = reinterpret_cast<OutT *>(p.out) + (size_t)pair * per_pair;
@@ -194,7 +205,8 @@ __global__ void ratio2_selftest_kernel(const double2 *__restrict__ tab, int kmax
 
 template <typename OutT, int NW, int MINB, int FMT = kFmtValues>
 cudaError_t launch_tile_nw(const TileArgs &p, int64_t npairs, cudaStream_t st) {
-  const size_t smem = tile_smem_bytes<OutT>(p.nx, p.ny, NW);
+  const size_t smem = FMT == kFmtWindow ? tile_smem_bytes_win<OutT>(p.nx, p.ny, p.w_r, NW)
+                                        : tile_smem_bytes<OutT>(p.nx, p.ny, NW);
   auto kern = sweep_tile_kernel<OutT, NW, MINB, FMT>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
@@ -250,7 +262,107 @@ cudaError_t launch_tile_merge(const TileArgs &p, int64_t npairs, cudaStream_t st
   }
 }
 
+// windows (kFmtWindow): the warp count of a map of the window's size.  8-warp CTAs are bound for 2 per SM (at 3 the
+// window code spills): they run windows wider than 512, whose shared memory admits about 2 anyway, or small batches.
+template <typename OutT>
+cudaError_t launch_tile_win(const TileArgs &p, int64_t npairs, cudaStream_t st) {
+  switch (tile_warps_for(win_side(p.nx, p.w_r), win_side(p.ny, p.w_r), npairs)) {
+    case 1: return launch_tile_nw<OutT, 1, VHP_NW1_MINB, kFmtWindow>(p, npairs, st);
+    case 2: case 4: case 6: return launch_tile_nw<OutT, 4, VHP_NW4_MINB, kFmtWindow>(p, npairs, st);
+    default: return launch_tile_nw<OutT, 8, 2, kFmtWindow>(p, npairs, st);
+  }
+}
+
+// fallback of the windows: window of pair p cut out of its full field, 0 outside the grid
+template <typename T>
+__global__ void window_crop_kernel(const T *__restrict__ field, int64_t np, int nx, int ny,
+                                   const int32_t *__restrict__ src_xy, int R, T *__restrict__ out) {
+  const int W = 2 * R + 1;
+  const size_t total = (size_t)np * W * W;
+  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total;
+       idx += (size_t)gridDim.x * blockDim.x) {
+    const size_t pair = idx / ((size_t)W * W);
+    const int rem = (int)(idx - pair * W * W), v = rem / W, u = rem - v * W;
+    const int x = __ldg(src_xy + 2 * pair) - R + u, y = __ldg(src_xy + 2 * pair + 1) - R + v;
+    out[idx] = ((unsigned)x < (unsigned)nx && (unsigned)y < (unsigned)ny)
+                   ? field[(pair * ny + y) * nx + x] : T(0);
+  }
+}
+
+// copy of the pairs with a map index out of range turned into a source outside the grid (which every sweep
+// route reports), so that the fallback never reads beyond the maps
+__global__ void window_pairs_kernel(const int32_t *__restrict__ src_xy, const int32_t *__restrict__ src_map,
+                                    int64_t np, int nmaps, int32_t *__restrict__ xy_out,
+                                    int32_t *__restrict__ map_out) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < np; i += (int64_t)gridDim.x * blockDim.x) {
+    const int m = src_map[i];
+    const bool ok = (unsigned)m < (unsigned)nmaps;
+    xy_out[2 * i] = ok ? src_xy[2 * i] : -1;
+    xy_out[2 * i + 1] = ok ? src_xy[2 * i + 1] : -1;
+    map_out[i] = ok ? m : 0;
+  }
+}
+
 } // namespace
+
+bool vhp_sweep_window_supported(int nx, int ny, int radius) {
+  return nx >= 1 && ny >= 1 && std::max(nx, ny) <= 16384 && radius >= 0 &&
+         tile_smem_bytes_win<double>(nx, ny, radius) <= 227u * 1024u;
+}
+
+cudaError_t vhp_launch_sweep_window_batch(const VhpTilePlanes &pl, int nmaps, int nx, int ny,
+                                          const int32_t *d_src_xy, const int32_t *d_src_map, int64_t npairs,
+                                          int radius, vhp_dtype dtype, void *d_out, const double *d_rcp2,
+                                          int *d_err, cudaStream_t st, int64_t *launches) {
+  TileArgs p;
+  p.pl = pl;
+  p.nx = nx;
+  p.ny = ny;
+  p.src_xy = d_src_xy;
+  p.src_map = d_src_map;
+  p.out = d_out;
+  p.rtab = reinterpret_cast<const double2 *>(d_rcp2);
+  p.err = d_err;
+  p.vec = 0; // window rows are not 16-byte aligned
+  p.win_y0 = 0;
+  p.win_y1 = ny;
+  for (int q = 0; q < 4; ++q) p.halo[q] = nullptr;
+  p.g_edges = nullptr;
+  p.g_lm = p.g_prog = p.g_next_row = nullptr;
+  p.qmask = 0xF;
+  p.src_ctl = nullptr;
+  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
+  p.thr = 0.0;
+  p.w_r = radius;
+  p.w_sw = win_sum_words(nx, radius);
+  p.w_nmaps = nmaps;
+  if (launches) *launches += 1;
+  return dtype == VHP_F32 ? launch_tile_win<float>(p, npairs, st) : launch_tile_win<double>(p, npairs, st);
+}
+
+cudaError_t vhp_launch_window_crop(const void *d_fields, int64_t np, int nx, int ny, const int32_t *d_src_xy,
+                                   int radius, vhp_dtype dtype, void *d_out, int sm_count, cudaStream_t st,
+                                   int64_t *launches) {
+  const size_t W = 2 * (size_t)radius + 1, total = (size_t)np * W * W;
+  const unsigned grid = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)sm_count * 16);
+  if (dtype == VHP_F32)
+    window_crop_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float *>(d_fields), np, nx, ny, d_src_xy,
+                                                    radius, static_cast<float *>(d_out));
+  else
+    window_crop_kernel<double><<<grid, 256, 0, st>>>(static_cast<const double *>(d_fields), np, nx, ny, d_src_xy,
+                                                     radius, static_cast<double *>(d_out));
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t vhp_launch_window_pairs(const int32_t *d_src_xy, const int32_t *d_src_map, int64_t np, int nmaps,
+                                    int32_t *d_xy_out, int32_t *d_map_out, int sm_count, cudaStream_t st,
+                                    int64_t *launches) {
+  const unsigned grid = (unsigned)std::min<int64_t>((np + 255) / 256, (int64_t)sm_count * 4);
+  window_pairs_kernel<<<grid, 256, 0, st>>>(d_src_xy, d_src_map, np, nmaps, d_xy_out, d_map_out);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
 
 cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
                                    const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,

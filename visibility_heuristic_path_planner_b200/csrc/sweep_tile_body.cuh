@@ -166,6 +166,9 @@ struct TileArgs {
   uint32_t *m_count = nullptr;
   size_t m_cells = 0;
   const int32_t *m_pg = nullptr, *m_pk = nullptr; // per pair: group (-1: skip the pair) and index within it
+  // kFmtWindow: radius R (windows of (2R+1)^2 per pair), block-summary words per window row (win_sum_words)
+  // and the number of maps (a pair on another map is reported like a source outside the grid)
+  int w_r = 0, w_sw = 0, w_nmaps = 0;
 };
 
 // how tile_sweep_cta is used
@@ -245,6 +248,30 @@ __host__ __device__ inline size_t tile_smem_bytes(int nx, int ny, int nwarps = k
          (size_t)nwarps * (kTile * kStagePitch * sizeof(OutT) + kWarpScratch * sizeof(double));
 }
 
+// Range-limited sweeps (kFmtWindow): every dependency of a cell points towards the source, so the
+// (2R+1)^2 window around it is swept on its own, in the map's absolute geometry (tile break points,
+// bit planes, summary, never-written border), and the per-CTA state is sized by the window.
+__host__ __device__ inline int win_side(int n, int R) { return n < 2 * R + 1 ? n : 2 * R + 1; }
+// block-summary words per block row and block rows a window can touch
+__host__ __device__ inline int win_sum_words(int nx, int R) {
+  const int nbx = (nx + 31) >> 5, span = (2 * R + 31) / 32 + 1;
+  const int b = nbx < span ? nbx : span, w = (b + 30) / 32 + 1;
+  return tile_sum_words(nx) < w ? tile_sum_words(nx) : w;
+}
+__host__ __device__ inline int win_sum_rows(int ny, int R) {
+  const int nby = (ny + 31) >> 5, span = (2 * R + 31) / 32 + 1;
+  return nby < span ? nby : span;
+}
+__host__ __device__ inline int win_sum_bytes(int nx, int ny, int R) {
+  return (4 * win_sum_words(nx, R) * win_sum_rows(ny, R) + 15) & ~15;
+}
+template <typename OutT>
+__host__ __device__ inline size_t tile_smem_bytes_win(int nx, int ny, int R, int nwarps = kTileWarps) {
+  return kTileHdr + win_sum_bytes(nx, ny, R) + 32 * (size_t)tile_lm_cap(win_side(ny, R)) +
+         sizeof(double) * (size_t)tile_edge_doubles(win_side(nx, R), nwarps) +
+         (size_t)nwarps * (kTile * kStagePitch * sizeof(OutT) + kWarpScratch * sizeof(double));
+}
+
 // 16-byte streaming store of one value replicated
 __device__ __forceinline__ void stg16_fill(float *q, float v) {
   __stcs(reinterpret_cast<float4 *>(q), make_float4(v, v, v, v));
@@ -264,7 +291,10 @@ __device__ __forceinline__ void stg16_fill(double *q, double v) {
 // Other CTAs sweep sources of the same group at the same time, so every write is a relaxed atomic (red), never a
 // plain store; count relies on the sweep storing each cell once (axis cells: the + quadrant only).  OutT is double
 // (the staging tiles hold the fp64 values); `out` is only a base for cell indices.
-constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4;
+// kFmtWindow: the field like kFmtValues, but only the (2R+1)^2 window around the source (TileArgs::w_r): each
+// quadrant's extents are clipped to R, `out` is shifted so that cell (x, y) sits at out[y * (2R+1) + x], stores
+// are scalar (window rows are not 16-byte aligned), and the window cells outside the grid are stored as 0.
+constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4, kFmtWindow = 5;
 constexpr int kMergeHdr = 224; // shared-memory header: {group, k} of the CTA's source (int2)
 
 __device__ __forceinline__ void red_max_u64(unsigned long long *a, unsigned long long v) {
@@ -308,14 +338,27 @@ __device__ __forceinline__ int tile_start(const int a, const int T) {
   return T ? a + kTile * (T - 1) : 0;
 }
 
+// Last local column / row to compute: the extent without the never-written border (x == 0 in the
+// -x quadrants, y == 0 in the -y quadrants).  A window (WIN) whose clipped extent stops short of the
+// grid's edge has no border cell.
+template <bool WIN = false>
+__device__ __forceinline__ int ext_cx(const TQuad &g, const int sx) {
+  return g.Ex - (g.dirx < 0 && (!WIN || g.Ex == sx));
+}
+template <bool WIN = false>
+__device__ __forceinline__ int ext_cy(const TQuad &g, const int sy) {
+  return g.Ey - (g.diry < 0 && (!WIN || g.Ey == sy));
+}
+
 // Does the block summary prove every cell tile (I, J) has to compute is free?  (A tile
 // with nothing to compute -- only border cells -- counts as free.)
+template <bool WIN = false>
 __device__ __forceinline__ bool tile_sum_free(const TQuad &g, const uint32_t *bsum, const int nbw,
                                               const int sx, const int sy, const int I,
                                               const int J) {
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
-  const int nvx = min(I ? kTile : g.a, g.Ex - (g.dirx < 0) - i0 + 1);
-  const int nvy = min(J ? kTile : g.a, g.Ey - (g.diry < 0) - j0 + 1);
+  const int nvx = min(I ? kTile : g.a, ext_cx<WIN>(g, sx) - i0 + 1);
+  const int nvy = min(J ? kTile : g.a, ext_cy<WIN>(g, sy) - j0 + 1);
   if (nvx <= 0 || nvy <= 0) return true;
   const int xa = sx + g.dirx * i0, xb = sx + g.dirx * (i0 + nvx - 1);
   const int ya = sy + g.diry * j0, yb = sy + g.diry * (j0 + nvy - 1);
@@ -344,6 +387,18 @@ __device__ __forceinline__ void fill_span(OutT *__restrict__ row, const int xa, 
   } else {
     for (int x = xa + lane; x <= xb; x += 32) __stcs(row + x, v);
   }
+}
+
+// q[0 .. n) = v by one warp, for any element-aligned q: scalar stores up to the first 16-byte boundary and
+// after the last one, 128-bit stores in between (window rows, kFmtWindow, start anywhere)
+template <typename OutT>
+__device__ __forceinline__ void fill_run(OutT *__restrict__ q, const int n, const OutT v, const int lane) {
+  constexpr int EPL = 16 / (int)sizeof(OutT);
+  const int head = min(n, (int)((16 - ((uintptr_t)q & 15)) & 15) / (int)sizeof(OutT));
+  if (lane < head) __stcs(q + lane, v);
+  const int nv = (n - head) / EPL, t0 = head + nv * EPL;
+  for (int k = lane; k < nv; k += 32) stg16_fill(q + head + k * EPL, v);
+  if (t0 + lane < n) __stcs(q + t0 + lane, v);
 }
 
 // rows y0, y0 + dy, ... (nrows of them), columns [xa, xb] = v by one warp.  Short spans (a dark run
@@ -400,6 +455,7 @@ struct TilePre {
   int sumfree;
 };
 
+template <bool WIN = false>
 __device__ __forceinline__ TilePre tile_prefetch(const TileArgs &p, const TQuad &g,
                                                  const uint32_t *__restrict__ rowpl,
                                                  const uint32_t *__restrict__ colpl,
@@ -411,9 +467,9 @@ __device__ __forceinline__ TilePre tile_prefetch(const TileArgs &p, const TQuad 
   t.sumfree = 0;
   const int wi = I ? kTile : g.a, wj = J ? kTile : g.a;
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
-  const int nvx = min(wi, g.Ex - (g.dirx < 0) - i0 + 1), nvy = min(wj, g.Ey - (g.diry < 0) - j0 + 1);
+  const int nvx = min(wi, ext_cx<WIN>(g, sx) - i0 + 1), nvy = min(wj, ext_cy<WIN>(g, sy) - j0 + 1);
   if (nvx > 0 && nvy > 0) {
-    t.sumfree = tile_sum_free(g, bsum, tile_sum_words(p.nx), sx, sy, I, J);
+    t.sumfree = tile_sum_free<WIN>(g, bsum, WIN ? p.w_sw : tile_sum_words(p.nx), sx, sy, I, J);
     if (!t.sumfree) {
       if (lane < nvy) { // row j0 + lane, bit b <-> local column i0 + b
         const uint32_t *rp =
@@ -484,12 +540,13 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
       if (lane == 0) atomicMax_system(xflag, I + 1);
     }
   };
-  const int nx = p.nx;
+  constexpr bool WIN = FMT == kFmtWindow;
+  const int nx = WIN ? 2 * p.w_r + 1 : p.nx; // row pitch of `out`
   const int wi = I ? kTile : g.a, wj = J ? kTile : g.a;          // tile extent
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
   const int il = i0 + lane, jr = j0 + lane;
   // the never-written border column / row is "occupied": exclude it from the compute extent
-  const int ExC = g.Ex - (g.dirx < 0), EyC = g.Ey - (g.diry < 0);
+  const int ExC = ext_cx<WIN>(g, sx), EyC = ext_cy<WIN>(g, sy);
   const int nvx = min(wi, ExC - i0 + 1), nvy = min(wj, EyC - j0 + 1); // columns / rows to compute
   const uint32_t cmask = nvx >= 32 ? ~0u : (nvx <= 0 ? 0u : (1u << nvx) - 1u);
   const uint32_t rmask = nvy >= 32 ? ~0u : (nvy <= 0 ? 0u : (1u << nvy) - 1u);
@@ -742,6 +799,9 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
 // written border get 0).  smem_raw: tile_smem_bytes<OutT>(nx, ny, NW) bytes, 16-aligned.
 // Ends with a block barrier.
 //
+// kFmtWindow: every cell of the (2R+1)^2 window exactly once instead (out: see kFmtWindow),
+// smem_raw: tile_smem_bytes_win<OutT>(nx, ny, R, NW) bytes.
+//
 // Grid mode (MODE != kSweepCta; one sweep of a giant map by many CTAs): kSweepGridInit, run by
 // one CTA, computes the staircase and writes it with the boundary rows, the progress flags and
 // the row counter to global memory; kSweepGridWork, launched after it with any number of
@@ -754,21 +814,25 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
                                                unsigned char *smem_raw) {
   constexpr bool GE = MODE != kSweepCta;
   constexpr bool BITS = FMT == kFmtBits;
+  constexpr bool WIN = FMT == kFmtWindow;
   static_assert(!GE || NW > 1, "grid mode uses the multi-warp boundary layout");
+  static_assert(!GE || !WIN, "window output is a one-CTA sweep");
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nx = p.nx, ny = p.ny;
+  const int opitch = WIN ? 2 * p.w_r + 1 : nx; // row pitch of `out`
   TQuad *quads = reinterpret_cast<TQuad *>(smem_raw);
   // next tile row to hand out (NW > 1)
   int *next_row = GE ? p.g_next_row : reinterpret_cast<int *>(smem_raw + 240);
   static_assert(4 * sizeof(TQuad) <= kMergeHdr, "quadrant geometry overlaps the merge slot / row counter");
   uint32_t *bsum = reinterpret_cast<uint32_t *>(smem_raw + kTileHdr);
   const int nsum = tile_sum_words(nx) * ((ny + 31) >> 5);
-  const int lmcap = tile_lm_cap(ny);
-  int *Lm = reinterpret_cast<int *>(smem_raw + kTileHdr + tile_sum_bytes(nx, ny));
+  const int sum_bytes = WIN ? win_sum_bytes(nx, ny, p.w_r) : tile_sum_bytes(nx, ny);
+  const int lmcap = tile_lm_cap(WIN ? win_side(ny, p.w_r) : ny);
+  int *Lm = reinterpret_cast<int *>(smem_raw + kTileHdr + sum_bytes);
   int *prog = GE ? p.g_prog : Lm + 4 * lmcap; // tiles finished (or lit) at the head of tile row (q, J)
-  double *const edges_s = reinterpret_cast<double *>(smem_raw + kTileHdr + tile_sum_bytes(nx, ny) + 32 * lmcap);
+  double *const edges_s = reinterpret_cast<double *>(smem_raw + kTileHdr + sum_bytes + 32 * lmcap);
   double *edges = GE ? p.g_edges : edges_s;
-  const int nedge = tile_edge_doubles(nx, NW);
+  const int nedge = tile_edge_doubles(WIN ? win_side(nx, p.w_r) : nx, NW);
   unsigned char *wbase = reinterpret_cast<unsigned char *>(GE ? edges_s : edges_s + nedge);
   double *wscr = reinterpret_cast<double *>(wbase) + warp * kWarpScratch;
   OutT *stage = reinterpret_cast<OutT *>(wbase + NW * kWarpScratch * sizeof(double)) +
@@ -784,6 +848,10 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       g.diry = (q < 2) ? 1 : -1;
       g.Ex = g.dirx > 0 ? nx - 1 - sx : sx;
       g.Ey = g.diry > 0 ? ny - 1 - sy : sy;
+      if (WIN) {
+        g.Ex = min(g.Ex, p.w_r);
+        g.Ey = min(g.Ey, p.w_r);
+      }
       // first tile width: the next tile column starts (+x) / ends (-x) on a multiple of 32
       g.a = g.dirx > 0 ? 32 - (sx & 31) : ((sx + 1) & 31);
       if (g.a == 0) g.a = 32;
@@ -812,7 +880,37 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       }
     }
   }
-  for (int i = tid; i < nsum; i += blockDim.x) bsum[i] = __ldg(p.pl.bsum + (size_t)map * nsum + i);
+  // bsq: the summary addressed by absolute block row and word (a window copies only the words it touches,
+  // rows of p.w_sw words)
+  const uint32_t *bsq = bsum;
+  if constexpr (WIN) {
+    const int R = p.w_r, nbw = tile_sum_words(nx), sw = p.w_sw;
+    const int wlo = (max(sx - R, 0) >> 5) >> 5, whi = (min(sx + R, nx - 1) >> 5) >> 5;
+    const int blo = max(sy - R, 0) >> 5, bhi = min(sy + R, ny - 1) >> 5;
+    const int nw = whi - wlo + 1, nwin = nw * (bhi - blo + 1);
+    const uint32_t *src = p.pl.bsum + (size_t)map * nsum + (size_t)blo * nbw + wlo;
+    for (int i = tid; i < nwin; i += blockDim.x) {
+      const int r = i / nw, c = i - r * nw;
+      bsum[r * sw + c] = __ldg(src + (size_t)r * nbw + c);
+    }
+    bsq = bsum - (blo * sw + wlo);
+    // window cells outside the grid are 0: the rows above / below it, then the columns left / right of it
+    const int W = 2 * R + 1, x0 = sx - R, y0 = sy - R;
+    const int ul = max(0, -x0), uh = min(W - 1, nx - 1 - x0), vl = max(0, -y0), vh = min(W - 1, ny - 1 - y0);
+    OutT *const wout = out + (ptrdiff_t)y0 * W + x0;
+    const OutT z = to_out<OutT>(0.0);
+    for (int v = warp; v < W; v += NW) {
+      OutT *const row = wout + (ptrdiff_t)v * W;
+      if (v < vl || v > vh) {
+        fill_run<OutT>(row, W, z, lane);
+      } else {
+        if (ul > 0) fill_run<OutT>(row, ul, z, lane);
+        if (uh < W - 1) fill_run<OutT>(row + uh + 1, W - 1 - uh, z, lane);
+      }
+    }
+  } else {
+    for (int i = tid; i < nsum; i += blockDim.x) bsum[i] = __ldg(p.pl.bsum + (size_t)map * nsum + i);
+  }
   if (MODE == kSweepCta)
     for (int i = tid; i < nedge; i += blockDim.x) edges[i] = 1.0; // virtual boundary
   __syncthreads();
@@ -822,14 +920,14 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
   }
 
   // ---- lit staircase: leading free tiles per tile row, then the running minimum ---------
-  const int nbw = tile_sum_words(nx);
+  const int nbw = WIN ? p.w_sw : tile_sum_words(nx);
   if (MODE != kSweepGridWork) {
   for (int q = 0; q < 4; ++q) {
     const TQuad &g = quads[q];
     for (int J = warp; J < g.TY; J += NW) {
       int L = 0;
       for (int Ib = 0; Ib < g.TX; Ib += 32) {
-        const bool fr = Ib + lane < g.TX && tile_sum_free(g, bsum, nbw, sx, sy, Ib + lane, J);
+        const bool fr = Ib + lane < g.TX && tile_sum_free<WIN>(g, bsq, nbw, sx, sy, Ib + lane, J);
         const unsigned m = __ballot_sync(kAll, fr);
         const int run = __ffs(~m) - 1; // leading ones (-1: all 32)
         L += run < 0 ? 32 : run;
@@ -975,14 +1073,21 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       const int nR = upper ? lit_run(0, j) : lit_run(3, j);
       const int nL = upper ? lit_run(1, j) : lit_run(2, j);
       if (nR == 0 && nL <= 1) continue;
-      OutT *row = out + (size_t)y * nx;
+      OutT *row = out + (size_t)y * opitch;
       const OutT v = to_out<OutT>((!upper && y == 0) ? 0.0 : 1.0); // y == 0 below the source: never written
       int xa = sx - (nL - 1), xb = sx + nR - 1;
       if (nL > 0 && xa == 0) { // x == 0 left of the source: never written
         if (lane == 0) __stcs(row, to_out<OutT>(0.0));
         xa = 1;
       }
-      if (nR > 0 && nL > 1) {
+      if (WIN) { // one run (the axis cell between the two quadrants' spans is lit whenever both are)
+        if (nR > 0 && nL > 1) {
+          fill_run<OutT>(row + xa, xb - xa + 1, v, lane);
+        } else {
+          if (nL > 1) fill_run<OutT>(row + xa, sx - xa, v, lane);
+          if (nR > 0) fill_run<OutT>(row + sx, xb - sx + 1, v, lane);
+        }
+      } else if (nR > 0 && nL > 1) {
         fill_span<OutT>(row, xa, xb, v, lane, p.vec);
       } else {
         if (nL > 1) fill_span<OutT>(row, xa, sx - 1, v, lane, p.vec);
@@ -999,11 +1104,11 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
     double Lv = 1.0, cor = 1.0; // left of the first tile: lit tiles or the virtual boundary
     int *xflag = nullptr; // grid mode across GPUs: the neighbour's flag of this row, if it is the exported one
     if (GE && reinterpret_cast<const short *>(smem_raw + 244)[q] == J) xflag = p.x_prog + q * lmcap + J;
-    TilePre pre = tile_prefetch(p, g, rowpl, colpl, bsum, sx, sy, I0, J, lane);
+    TilePre pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, I0, J, lane);
 #if VHP_DARK_TAIL
     // rows of this tile row that hold cells to compute (lane <-> row j0 + lane), as in process_tile
     const int j0row = tile_start(g.a, J);
-    const int nvyrow = min(J ? kTile : g.a, g.Ey - (g.diry < 0) - j0row + 1);
+    const int nvyrow = min(J ? kTile : g.a, ext_cy<WIN>(g, sy) - j0row + 1);
     const bool rowc_row = lane < nvyrow;
     int dark_seen = -1; // a boundary column >= the tile start known to be non-zero (finished row below)
 #endif
@@ -1020,7 +1125,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
         const int Iend = min(ld_acquire_shared(prog + q * lmcap + J - 1), g.TX); // finished below
         if (Iend > I) {
           const int i0 = tile_start(g.a, I);
-          const int ilim = min(g.Ex - (g.dirx < 0), tile_start(g.a, Iend) - 1);
+          const int ilim = min(ext_cx<WIN>(g, sx), tile_start(g.a, Iend) - 1);
           const double *rowB = edges + g.rowOff;
           int bad = -1;
           for (int ib = i0; ib <= ilim && bad < 0; ib += 32) {
@@ -1042,8 +1147,12 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
             if constexpr (FMT == kFmtValues)
               fill_block<OutT>(out, nx, sy + g.diry * (j0row + r0), g.diry, rlast - r0 + 1, xa, xb,
                                to_out<OutT>(0.0), lane, p.vec != 0);
+            if constexpr (WIN)
+              for (int r = r0; r <= rlast; ++r)
+                fill_run<OutT>(out + (ptrdiff_t)(sy + g.diry * (j0row + r)) * opitch + xa, xb - xa + 1,
+                               to_out<OutT>(0.0), lane);
             if (Istop >= g.TX) return;
-            pre = tile_prefetch(p, g, rowpl, colpl, bsum, sx, sy, Istop, J, lane);
+            pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, Istop, J, lane);
             I = Istop - 1;
             continue;
           }
@@ -1051,7 +1160,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       }
 #endif
       const TilePre cur = pre;
-      if (I + 1 < g.TX) pre = tile_prefetch(p, g, rowpl, colpl, bsum, sx, sy, I + 1, J, lane);
+      if (I + 1 < g.TX) pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, I + 1, J, lane);
       if (GE && J > 0 && ((p.remote_mask >> q) & 1) && J == g.Jlo) {
         // the row below lives on the neighbouring GPU: its flag arrives over NVLink.  A watchdog
         // (a few seconds) turns a lost neighbour into an error instead of a hung GPU.

@@ -197,6 +197,23 @@ cudaError_t vhp_launch_sweep_tile(const VhpTilePlanes &pl, int nx, int ny, const
 // thr != null, bits: d_out = uint32 words, bit (x & 31) of word [pair][y][x >> 5] = (fp64 value >= thr);
 // needs thr > 0 (zeroes d_out, then writes only the cells at or above the threshold).
 
+// Range-limited windows (vhp_visibility_window_batch): the one-CTA tile kernel sweeps only the (2R+1)^2 window
+// of each pair (kFmtWindow, shared memory sized by the window; supported: it fits one CTA), into d_out
+// [pair][2R+1][2R+1]; a map index out of range raises bit 0 of d_err like a source outside the grid.
+bool vhp_sweep_window_supported(int nx, int ny, int radius);
+cudaError_t vhp_launch_sweep_window_batch(const VhpTilePlanes &pl, int nmaps, int nx, int ny,
+                                          const int32_t *d_src_xy, const int32_t *d_src_map, int64_t npairs,
+                                          int radius, vhp_dtype dtype, void *d_out, const double *d_rcp2,
+                                          int *d_err, cudaStream_t st, int64_t *launches);
+// fallback: the windows of np pairs cut out of their full fields d_fields[np][ny][nx] (0 outside the grid), and the
+// copy of a batch's pairs whose out-of-range map indices become sources outside the grid
+cudaError_t vhp_launch_window_crop(const void *d_fields, int64_t np, int nx, int ny, const int32_t *d_src_xy,
+                                   int radius, vhp_dtype dtype, void *d_out, int sm_count, cudaStream_t st,
+                                   int64_t *launches);
+cudaError_t vhp_launch_window_pairs(const int32_t *d_src_xy, const int32_t *d_src_map, int64_t np, int nmaps,
+                                    int32_t *d_xy_out, int32_t *d_map_out, int sm_count, cudaStream_t st,
+                                    int64_t *launches);
+
 // Merged visibility of groups of sources (vhp_visibility_merge_batch): the group outputs ([group][ny][nx], any may be
 // null; vmax fp32 when f32) and the per-pair table merge_table_kernel builds from the CSR group layout.
 struct VhpMergeDev {
