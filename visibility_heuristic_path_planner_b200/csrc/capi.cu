@@ -115,16 +115,20 @@ vhp_status pack_tile(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, 
   return VHP_OK;
 }
 
+vhp_status check_grid_dtype(vhp_context *ctx, int nx, int ny, int dtype) {
+  if ((int64_t)nx * ny > (int64_t)1 << 30 || nx > 16384 || ny > 16384)
+    return fail(ctx, VHP_ERR_UNSUPPORTED, "grid larger than 16384 x 16384 is not supported");
+  if (dtype != VHP_F32 && dtype != VHP_F64) return fail(ctx, VHP_ERR_INVALID_ARG, "bad dtype");
+  return VHP_OK;
+}
+
 vhp_status check_common(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny,
                         const void *xy, int64_t n, int dtype, const void *out) {
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !xy || !out) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || n < 0)
     return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
-  if ((int64_t)nx * ny > (int64_t)1 << 30 || nx > 16384 || ny > 16384)
-    return fail(ctx, VHP_ERR_UNSUPPORTED, "grid larger than 16384 x 16384 is not supported");
-  if (dtype != VHP_F32 && dtype != VHP_F64) return fail(ctx, VHP_ERR_INVALID_ARG, "bad dtype");
-  return VHP_OK;
+  return check_grid_dtype(ctx, nx, ny, dtype);
 }
 
 // host-side validation of (x, y[, map]) items
@@ -162,6 +166,48 @@ int grid_sweep_ctas(const vhp_context *ctx, int rows) {
   return std::max(2, std::min(2 * ctx->sm_count, (4 * (rows / 32 + 2) + 7) / 8));
 }
 
+// May a single sweep of this map be spread over many CTAs?  (Maps too wide for the one-CTA kernel need it.)
+bool grid_mode_available(const vhp_context *ctx, int nx, int ny) {
+  return ctx->grid_sweep != 0 && vhp_sweep_grid_supported(nx, ny);
+}
+
+// Do the batched sweeps of this map read the bit planes (the tile kernel or grid mode, not the naive kernel)?
+bool sweeps_use_planes(const vhp_context *ctx, int nx, int ny) {
+  return ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny));
+}
+
+// Kernel of a batch of n whole-field sweeps.  A few sweeps of a large map run one at a time on the whole
+// GPU (grid mode, see vhp_strip_sweep_dev) instead of one CTA per pair.  (1000^2: up to 4 pairs, 2048^2
+// and up: 16; maps too wide for the one-CTA kernel's shared memory: up to 16 pairs whatever the size.)
+// Every route that claims to equal run_dev's fields (bits, merged outputs) asks this function.
+enum class SweepRoute { Tile, Grid, Naive };
+
+SweepRoute sweep_route(const vhp_context *ctx, int nx, int ny, int64_t n) {
+  if (ctx->sweep_impl != 0) return SweepRoute::Naive;
+  const bool tile_ok = vhp_sweep_tile_supported(nx, ny);
+  const int64_t grid_max = tile_ok ? std::min<int64_t>(16, (int64_t)((size_t)nx * ny / 250000)) : 16;
+  if (vhp_sweep_grid_supported(nx, ny) && (ctx->grid_sweep == 2 || (ctx->grid_sweep == 1 && n <= grid_max)))
+    return SweepRoute::Grid;
+  return tile_ok ? SweepRoute::Tile : SweepRoute::Naive;
+}
+
+// Range-limited windows sweep only the window on one CTA whatever the batch size, so only a forced grid
+// mode turns them away (their fallback goes through run_dev and sweep_route).
+bool window_direct_route(const vhp_context *ctx, int nx, int ny, int radius) {
+  return ctx->sweep_impl == 0 && ctx->grid_sweep != 2 && vhp_sweep_window_supported(nx, ny, radius);
+}
+
+// bit planes of map m of the packed batch (the grid kernels sweep "map 0")
+VhpTilePlanes planes_of_map(const vhp_context *ctx, size_t m, int nx, int ny) {
+  int wx, wy, nsum;
+  vhp_tile_plane_geometry(nx, ny, &wx, &wy, &nsum);
+  VhpTilePlanes pl = ctx->tile;
+  pl.rowF += m * pl.row_plane; pl.rowR += m * pl.row_plane;
+  pl.colF += m * pl.col_plane; pl.colR += m * pl.col_plane;
+  pl.bsum += m * (size_t)nsum;
+  return pl;
+}
+
 enum class Op { Sweep, Raycast, Window };
 
 vhp_status run_dev(vhp_context *ctx, Op op, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -175,60 +221,46 @@ vhp_status run_dev(vhp_context *ctx, Op op, const uint8_t *d_occ, int nmaps, int
   }
   const size_t esz = dtype == VHP_F32 ? 4 : 8;
   const size_t cells = (size_t)nx * ny;
-  // A few sweeps of a large map: one sweep at a time on the whole GPU (grid mode, see
-  // vhp_strip_sweep_dev) instead of one CTA per pair.  (1000^2: up to 4 pairs, 2048^2 and up: 16;
-  // maps too wide for the one-CTA kernel's shared memory: up to 16 pairs whatever the size.)
-  const bool tile_ok = vhp_sweep_tile_supported(nx, ny);
-  const bool use_grid =
-      ctx->sweep_impl == 0 && vhp_sweep_grid_supported(nx, ny) &&
-      (ctx->grid_sweep == 2 ||
-       (ctx->grid_sweep == 1 && n <= (tile_ok ? std::min<int64_t>(16, (int64_t)(cells / 250000)) : 16)));
-  if (ctx->sweep_impl == 0 && (tile_ok || use_grid)) {
-    vhp_status st = ensure_rcp2(ctx, std::max(nx, ny) + 64);
-    if (st != VHP_OK) return st;
-    if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
-    if (use_grid) {
-      std::vector<int32_t> h_xy(2 * (size_t)n), h_map;
-      VHP_CUDA(ctx, cudaMemcpyAsync(h_xy.data(), d_xy, h_xy.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-      if (d_map) {
-        h_map.resize((size_t)n);
-        VHP_CUDA(ctx, cudaMemcpyAsync(h_map.data(), d_map, h_map.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-      }
-      VHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-      if ((st = ensure(ctx, ctx->b_grid, vhp_sweep_grid_ws_bytes(nx, ny))) != VHP_OK) return st;
-      int wx, wy, nsum;
-      vhp_tile_plane_geometry(nx, ny, &wx, &wy, &nsum);
-      const int ctas = grid_sweep_ctas(ctx, ny);
-      for (int64_t k = 0; k < n; ++k) {
-        const int sx = h_xy[2 * k], sy = h_xy[2 * k + 1];
-        const int64_t m = d_map ? h_map[k] : 0;
-        if (sx < 0 || sx >= nx || sy < 0 || sy >= ny || m < 0 || m >= nmaps)
-          return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
-        VhpTilePlanes pl = ctx->tile; // planes of map m (the grid kernels sweep "map 0")
-        pl.rowF += m * pl.row_plane; pl.rowR += m * pl.row_plane;
-        pl.colF += m * pl.col_plane; pl.colR += m * pl.col_plane;
-        pl.bsum += m * (size_t)nsum;
-        VHP_CUDA(ctx, vhp_launch_sweep_window(pl, nx, ny, sx, sy, 0, ny, nullptr, dtype,
-                                              (char *)d_out + (size_t)k * cells * esz,
-                                              ctx->rcp2_table, ctx->d_err, ctx->b_grid.p, ctas,
-                                              ctx->stream, &ctx->launches));
-      }
-      return VHP_OK;
+  const SweepRoute route = sweep_route(ctx, nx, ny, n);
+  vhp_status st;
+  if (route == SweepRoute::Naive) {
+    // chunk so that the scratch fronts stay small
+    const int64_t chunk = 4096;
+    if ((st = ensure(ctx, ctx->b_scratch, vhp_sweep_naive_scratch_bytes(nx, ny, std::min(n, chunk)))) != VHP_OK)
+      return st;
+    for (int64_t p0 = 0; p0 < n; p0 += chunk) {
+      const int64_t np = std::min(chunk, n - p0);
+      VHP_CUDA(ctx, vhp_launch_sweep_naive(d_occ, nx, ny, d_xy + 2 * p0, d_map ? d_map + p0 : nullptr,
+                                           np, dtype, (char *)d_out + (size_t)p0 * nx * ny * esz,
+                                           (double *)ctx->b_scratch.p, ctx->d_err, ctx->stream,
+                                           &ctx->launches));
     }
+    return VHP_OK;
+  }
+  if ((st = ensure_rcp2(ctx, std::max(nx, ny) + 64)) != VHP_OK) return st;
+  if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
+  if (route == SweepRoute::Tile) {
     VHP_CUDA(ctx, vhp_launch_sweep_tile(ctx->tile, nx, ny, d_xy, d_map, n, dtype, d_out,
                                         ctx->rcp2_table, ctx->d_err, ctx->stream, &ctx->launches));
     return VHP_OK;
   }
-  // naive kernel: chunk so that the scratch fronts stay small
-  const int64_t chunk = 4096;
-  vhp_status st = ensure(ctx, ctx->b_scratch, vhp_sweep_naive_scratch_bytes(nx, ny, std::min(n, chunk)));
-  if (st != VHP_OK) return st;
-  for (int64_t p0 = 0; p0 < n; p0 += chunk) {
-    const int64_t np = std::min(chunk, n - p0);
-    VHP_CUDA(ctx, vhp_launch_sweep_naive(d_occ, nx, ny, d_xy + 2 * p0, d_map ? d_map + p0 : nullptr,
-                                         np, dtype, (char *)d_out + (size_t)p0 * nx * ny * esz,
-                                         (double *)ctx->b_scratch.p, ctx->d_err, ctx->stream,
-                                         &ctx->launches));
+  std::vector<int32_t> h_xy(2 * (size_t)n), h_map;
+  VHP_CUDA(ctx, cudaMemcpyAsync(h_xy.data(), d_xy, h_xy.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (d_map) {
+    h_map.resize((size_t)n);
+    VHP_CUDA(ctx, cudaMemcpyAsync(h_map.data(), d_map, h_map.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  VHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if ((st = ensure(ctx, ctx->b_grid, vhp_sweep_grid_ws_bytes(nx, ny))) != VHP_OK) return st;
+  const int ctas = grid_sweep_ctas(ctx, ny);
+  for (int64_t k = 0; k < n; ++k) {
+    const int sx = h_xy[2 * k], sy = h_xy[2 * k + 1];
+    const int64_t m = d_map ? h_map[k] : 0;
+    if (sx < 0 || sx >= nx || sy < 0 || sy >= ny || m < 0 || m >= nmaps)
+      return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
+    VHP_CUDA(ctx, vhp_launch_sweep_window(planes_of_map(ctx, (size_t)m, nx, ny), nx, ny, sx, sy, 0, ny, nullptr,
+                                          dtype, (char *)d_out + (size_t)k * cells * esz, ctx->rcp2_table,
+                                          ctx->d_err, ctx->b_grid.p, ctas, ctx->stream, &ctx->launches));
   }
   return VHP_OK;
 }
@@ -242,10 +274,6 @@ int64_t bin_chunk_pairs(size_t cells, int64_t n) {
 // Direct: the one-CTA tile kernel sweeps only each pair's window (kFmtWindow).  Otherwise (the naive kernel, grid
 // mode forced, or a window whose state does not fit one CTA) chunks of full fields go through run_dev, which picks
 // grid mode or the naive kernel as for vhp_visibility_batch, and window_crop_kernel cuts the windows out.
-bool window_direct_route(const vhp_context *ctx, int nx, int ny, int radius) {
-  return ctx->sweep_impl == 0 && ctx->grid_sweep != 2 && vhp_sweep_window_supported(nx, ny, radius);
-}
-
 size_t window_pair_bytes(int radius, vhp_dtype dtype) {
   const size_t w = 2 * (size_t)radius + 1;
   return w * w * (dtype == VHP_F32 ? 4 : 8);
@@ -283,61 +311,97 @@ vhp_status run_window_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int
   return VHP_OK;
 }
 
-// Plain transport of the host-buffer entry points: run in chunks of pairs from p_begin on and
-// overlap the D2H of chunk c with the kernel of chunk c+1 (two device buffers, copy stream).
-// Op::Window delivers the windows of `radius`, every other op whole fields.
-vhp_status run_host_plain(vhp_context *ctx, Op op, int nmaps, int nx, int ny, const int32_t *d_xy,
-                          const int32_t *d_map, int64_t n, int64_t p_begin, vhp_dtype dtype,
-                          void *out, int radius = 0) {
-  const size_t esz = dtype == VHP_F32 ? 4 : 8;
-  const size_t cells = op == Op::Window ? window_pair_bytes(radius, dtype) / esz : (size_t)nx * ny;
+// Upload of a host batch into b_occ / b_src / b_map: the maps, n items of item_bytes each and, when
+// maps is not null, n map indices.  Bit planes of an older content of b_occ (sticky ones of
+// vhp_prepare_maps_dev too) are dropped; pack: build them now, once for every chunk of the call.
+// The caller holds a PlanesGuard, which drops them again when the call returns.
+vhp_status stage_host_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const void *items,
+                            size_t item_bytes, int64_t n, const int32_t *maps, bool pack) {
+  const size_t occ_bytes = (size_t)nmaps * nx * ny;
   vhp_status st;
-  const size_t chunk_bytes_target = (size_t)1 << 30;
-  int64_t chunk = std::max<int64_t>(1, (int64_t)(chunk_bytes_target / (cells * esz)));
-  chunk = std::min(chunk, n - p_begin);
-  const size_t buf_bytes = (size_t)chunk * cells * esz;
-  if ((st = ensure(ctx, ctx->b_out[0], buf_bytes)) != VHP_OK) return st;
-  if (n - p_begin > chunk && (st = ensure(ctx, ctx->b_out[1], buf_bytes)) != VHP_OK) return st;
-  // pin the caller's buffer for full-rate async copies (ignore "already pinned").  Page-locking
-  // costs milliseconds: small results (a single 101 x 101 sweep is 80 KB) are copied as they are.
-  const size_t out_bytes = (size_t)(n - p_begin) * cells * esz;
-  char *const out_first = (char *)out + (size_t)p_begin * cells * esz;
-  const bool registered = out_bytes >= ((size_t)32 << 20) &&
-                          cudaHostRegister(out_first, out_bytes, cudaHostRegisterDefault) == cudaSuccess;
-  (void)cudaGetLastError();
-  vhp_status result = VHP_OK;
+  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
+  if ((st = ensure(ctx, ctx->b_src, item_bytes * (size_t)std::max<int64_t>(n, 1))) != VHP_OK) return st;
+  if (maps && (st = ensure(ctx, ctx->b_map, (size_t)n * 4)) != VHP_OK) return st;
+  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  if (n > 0)
+    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, items, (size_t)n * item_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  if (maps) VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, maps, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+  ctx->planes_sticky = false;
+  ctx->tile_src = nullptr;
+  if (!pack) return VHP_OK;
+  if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
+  ctx->planes_sticky = true;
+  return VHP_OK;
+}
+
+// The planes a host call packed point into b_occ, which the next call overwrites: drop them on every exit.
+struct PlanesGuard {
+  vhp_context *ctx;
+  explicit PlanesGuard(vhp_context *c) : ctx(c) {}
+  ~PlanesGuard() {
+    ctx->planes_sticky = false;
+    ctx->tile_src = nullptr;
+  }
+};
+
+// Delivery of pairs [p_begin, n) to the host buffer `out` in chunks of `chunk` pairs of pair_bytes each:
+// produce(p0, np, d_buf) computes a chunk into one of two device buffers on the stream, and the copy
+// stream takes it to `out` under the work of the next chunk.  Both streams are synchronised on every exit.
+template <class F>
+vhp_status pipelined_d2h(vhp_context *ctx, int64_t p_begin, int64_t n, int64_t chunk, size_t pair_bytes, void *out,
+                         F produce) {
+  vhp_status result = ensure(ctx, ctx->b_out[0], (size_t)chunk * pair_bytes);
+  if (result == VHP_OK && n - p_begin > chunk) result = ensure(ctx, ctx->b_out[1], (size_t)chunk * pair_bytes);
   int it = 0;
   for (int64_t p0 = p_begin; p0 < n && result == VHP_OK; p0 += chunk, ++it) {
     const int b = it & 1;
     const int64_t np = std::min(chunk, n - p0);
-    if (it >= 2) { // the copy that last read this buffer must be done
-      cudaError_t e = cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[b], 0);
-      if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaStreamWaitEvent"); break; }
-    }
-    result = op == Op::Window
-                 ? run_window_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
-                                  d_map ? d_map + p0 : nullptr, np, radius, dtype, ctx->b_out[b].p)
-                 : run_dev(ctx, op, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
-                           d_map ? d_map + p0 : nullptr, np, dtype, ctx->b_out[b].p);
-    if (result != VHP_OK) break;
-    cudaError_t e = cudaEventRecord(ctx->ev_done[b], ctx->stream);
+    cudaError_t e = cudaSuccess;
+    if (it >= 2) e = cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[b], 0); // the copy that last read buffer b is done
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaStreamWaitEvent"); break; }
+    if ((result = produce(p0, np, ctx->b_out[b].p)) != VHP_OK) break;
+    e = cudaEventRecord(ctx->ev_done[b], ctx->stream);
     if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_done[b], 0);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "event hand-over to the copy stream"); break; }
-    e = cudaMemcpyAsync((char *)out + (size_t)p0 * cells * esz, ctx->b_out[b].p,
-                                    (size_t)np * cells * esz, cudaMemcpyDeviceToHost,
-                                    ctx->copy_stream);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaMemcpyAsync D2H"); break; }
-    e = cudaEventRecord(ctx->ev_copied[b], ctx->copy_stream);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaEventRecord"); break; }
-    ctx->last_d2h_bytes += (int64_t)((size_t)np * cells * esz);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync((char *)out + (size_t)p0 * pair_bytes, ctx->b_out[b].p, (size_t)np * pair_bytes,
+                          cudaMemcpyDeviceToHost, ctx->copy_stream);
+    if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_copied[b], ctx->copy_stream);
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "D2H of a chunk: enqueue"); break; }
+    ctx->last_d2h_bytes += (int64_t)((size_t)np * pair_bytes);
   }
   cudaError_t e1 = cudaStreamSynchronize(ctx->copy_stream);
   cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-  if (registered) cudaHostUnregister(out_first);
   if (result != VHP_OK) return result;
   if (e1 != cudaSuccess) return cuda_fail(ctx, e1, "sync copy stream");
   if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
   return VHP_OK;
+}
+
+// Plain transport of the host-buffer entry points: run in chunks of pairs from p_begin on and
+// overlap the D2H of chunk c with the kernel of chunk c+1 (pipelined_d2h).
+// Op::Window delivers the windows of `radius`, every other op whole fields.
+vhp_status run_host_plain(vhp_context *ctx, Op op, int nmaps, int nx, int ny, const int32_t *d_xy,
+                          const int32_t *d_map, int64_t n, int64_t p_begin, vhp_dtype dtype,
+                          void *out, int radius = 0) {
+  const size_t pair_bytes =
+      op == Op::Window ? window_pair_bytes(radius, dtype) : (size_t)nx * ny * (dtype == VHP_F32 ? 4 : 8);
+  const int64_t chunk = std::min(std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / pair_bytes)), n - p_begin);
+  // pin the caller's buffer for full-rate async copies (ignore "already pinned").  Page-locking
+  // costs milliseconds: small results (a single 101 x 101 sweep is 80 KB) are copied as they are.
+  const size_t out_bytes = (size_t)(n - p_begin) * pair_bytes;
+  char *const out_first = (char *)out + (size_t)p_begin * pair_bytes;
+  const bool registered = out_bytes >= ((size_t)32 << 20) &&
+                          cudaHostRegister(out_first, out_bytes, cudaHostRegisterDefault) == cudaSuccess;
+  (void)cudaGetLastError();
+  const uint8_t *d_occ = (const uint8_t *)ctx->b_occ.p;
+  auto produce = [&](int64_t p0, int64_t np, void *buf) {
+    const int32_t *xy = d_xy + 2 * p0, *mp = d_map ? d_map + p0 : nullptr;
+    return op == Op::Window ? run_window_dev(ctx, d_occ, nmaps, nx, ny, xy, mp, np, radius, dtype, buf)
+                            : run_dev(ctx, op, d_occ, nmaps, nx, ny, xy, mp, np, dtype, buf);
+  };
+  const vhp_status result = pipelined_d2h(ctx, p_begin, n, chunk, pair_bytes, out, produce);
+  if (registered) cudaHostUnregister(out_first);
+  return result;
 }
 
 // Packed transport (result_transport.cu, host_expand.cpp): every chunk of results is packed on
@@ -697,26 +761,10 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
   ctx->last_transport_packed = 0;
   if (n == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
+  PlanesGuard planes_guard(ctx);
+  st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, n, maps, op != Op::Raycast && sweeps_use_planes(ctx, nx, ny));
+  if (st != VHP_OK) return st;
   const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
-  const size_t occ_bytes = (size_t)nmaps * cells;
-  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, (size_t)n * 2 * sizeof(int32_t))) != VHP_OK) return st;
-  if (maps && (st = ensure(ctx, ctx->b_map, (size_t)n * sizeof(int32_t))) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, xy, (size_t)n * 2 * sizeof(int32_t),
-                                cudaMemcpyHostToDevice, ctx->stream));
-  if (maps)
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, maps, (size_t)n * sizeof(int32_t),
-                                  cudaMemcpyHostToDevice, ctx->stream));
-  ctx->planes_sticky = false; // b_occ content changed
-  ctx->tile_src = nullptr;
-  if (op != Op::Raycast && ctx->sweep_impl == 0 &&
-      (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
-    // pack once for all chunks
-    if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK)
-      return st;
-    ctx->planes_sticky = true;
-  }
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
   const int32_t *d_map = maps ? (const int32_t *)ctx->b_map.p : nullptr;
   const size_t out_bytes = (size_t)n * (op == Op::Window ? window_pair_bytes(radius, dtype) : cells * esz);
@@ -730,8 +778,6 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
   }
   if (result == VHP_OK && p_begin < n)
     result = run_host_plain(ctx, op, nmaps, nx, ny, d_xy, d_map, n, p_begin, dtype, out, radius);
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
   if (result != VHP_OK) return result;
   return check_device_error(ctx);
 }
@@ -744,17 +790,8 @@ vhp_status run_host(vhp_context *ctx, Op op, const uint8_t *occ, int nmaps, int 
 // Batches the one-CTA tile kernel takes are swept straight into bits (kFmtBits: the field itself is
 // never stored); a non-positive threshold, a few pairs of a large map (grid mode) and the naive
 // kernel go through the fp64 field in ctx->b_bin (at most bin_chunk_pairs pairs).
-// Does a batch of np pairs run on the one-CTA tile kernel (not the naive kernel, not grid mode; see run_dev)?
-bool one_cta_tile_route(const vhp_context *ctx, int nx, int ny, int64_t np) {
-  const size_t cells = (size_t)nx * ny;
-  return ctx->sweep_impl == 0 && vhp_sweep_tile_supported(nx, ny) &&
-         !(ctx->grid_sweep == 2 && vhp_sweep_grid_supported(nx, ny)) &&
-         !(ctx->grid_sweep == 1 && vhp_sweep_grid_supported(nx, ny) &&
-           np <= std::min<int64_t>(16, (int64_t)(cells / 250000)));
-}
-
 bool sweeps_into_bits(const vhp_context *ctx, int nx, int ny, int64_t np, double thr) {
-  return ctx->bin_direct && thr > 0.0 && one_cta_tile_route(ctx, nx, ny, np);
+  return ctx->bin_direct && thr > 0.0 && sweep_route(ctx, nx, ny, np) == SweepRoute::Tile;
 }
 
 vhp_status sweep_to_bits(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -806,19 +843,11 @@ vhp_status run_bin_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx,
   ctx->last_transport_packed = 0;
   if (n == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
-  const size_t cells = (size_t)nx * ny, wpr = (size_t)(nx + 31) / 32, occ_bytes = (size_t)nmaps * cells;
-  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, (size_t)n * 8)) != VHP_OK) return st;
-  if (maps && (st = ensure(ctx, ctx->b_map, (size_t)n * 4)) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, xy, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  if (maps) VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, maps, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
-  if (ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
-    if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
-    ctx->planes_sticky = true;
-  }
+  PlanesGuard planes_guard(ctx);
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, n, maps, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
+    return st;
+  const size_t cells = (size_t)nx * ny, pair_bytes = (size_t)ny * ((nx + 31) / 32) * 4;
+  const uint8_t *d_occ = (const uint8_t *)ctx->b_occ.p;
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
   const int32_t *d_map = maps ? (const int32_t *)ctx->b_map.p : nullptr;
   // the sweep writes bits itself: four chunks (the D2H of one under the sweeps of the next), each
@@ -826,37 +855,13 @@ vhp_status run_bin_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx,
   const int64_t chunk = sweeps_into_bits(ctx, nx, ny, n, thr)
                             ? std::min<int64_t>(n, std::max<int64_t>((int64_t)ctx->sm_count * 6, (n + 3) / 4))
                             : bin_chunk_pairs(cells, n);
-  const size_t pair_words = (size_t)ny * wpr, chunk_bytes = (size_t)chunk * pair_words * 4;
-  vhp_status result = VHP_OK;
-  for (int b = 0; b < 2 && result == VHP_OK; ++b)
-    if (b == 0 || n > chunk) result = ensure(ctx, ctx->b_out[b], chunk_bytes);
-  int it = 0;
-  for (int64_t p0 = 0; p0 < n && result == VHP_OK; p0 += chunk, ++it) {
-    const int b = it & 1;
-    const int64_t np = std::min(chunk, n - p0);
-    cudaError_t e = cudaSuccess;
-    if (it >= 2) e = cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[b], 0); // bit buffer b is free again
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cudaStreamWaitEvent"); break; }
-    result = sweep_to_bits(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * p0,
-                           d_map ? d_map + p0 : nullptr, np, thr, (uint32_t *)ctx->b_out[b].p);
-    if (result != VHP_OK) break;
-    e = cudaEventRecord(ctx->ev_done[b], ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_done[b], 0);
-    if (e == cudaSuccess)
-      e = cudaMemcpyAsync(out_bits + (size_t)p0 * pair_words, ctx->b_out[b].p, (size_t)np * pair_words * 4,
-                          cudaMemcpyDeviceToHost, ctx->copy_stream);
-    if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_copied[b], ctx->copy_stream);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "binary visibility: enqueue"); break; }
-    ctx->last_d2h_bytes += (int64_t)((size_t)np * pair_words * 4);
-  }
-  cudaError_t e1 = cudaStreamSynchronize(ctx->copy_stream);
-  cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
-  ctx->last_result_bytes = (int64_t)((size_t)n * pair_words * 4);
+  auto produce = [&](int64_t p0, int64_t np, void *buf) {
+    return sweep_to_bits(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * p0, d_map ? d_map + p0 : nullptr, np, thr,
+                         (uint32_t *)buf);
+  };
+  const vhp_status result = pipelined_d2h(ctx, 0, n, chunk, pair_bytes, out_bits, produce);
+  ctx->last_result_bytes = (int64_t)((size_t)n * pair_bytes);
   if (result != VHP_OK) return result;
-  if (e1 != cudaSuccess) return cuda_fail(ctx, e1, "sync copy stream");
-  if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
   return check_device_error(ctx);
 }
 
@@ -878,19 +883,10 @@ vhp_status run_runs_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx
   pair_ptr[0] = 0;
   if (n == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
-  const size_t cells = (size_t)nx * ny, wpr = (size_t)(nx + 31) / 32, occ_bytes = (size_t)nmaps * cells;
-  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, (size_t)n * 8)) != VHP_OK) return st;
-  if (maps && (st = ensure(ctx, ctx->b_map, (size_t)n * 4)) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, xy, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  if (maps) VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, maps, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
-  if (ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
-    if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
-    ctx->planes_sticky = true;
-  }
+  PlanesGuard planes_guard(ctx);
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, n, maps, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
+    return st;
+  const size_t cells = (size_t)nx * ny, wpr = (size_t)(nx + 31) / 32;
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
   const int32_t *d_map = maps ? (const int32_t *)ctx->b_map.p : nullptr;
   // the sweep writes bits itself: a chunk is bounded by its bits (1 GB), not by an fp64 field
@@ -945,8 +941,6 @@ vhp_status run_runs_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx
     total = new_total;
   }
   (void)cudaStreamSynchronize(ctx->copy_stream); // (a failed chunk may have left its copies in flight)
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
   ctx->last_result_bytes = ctx->last_d2h_bytes;
   if (result != VHP_OK) return result;
   return check_device_error(ctx);
@@ -964,9 +958,8 @@ vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || ngroups < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
   if (ngroups > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: more than 2^31 - 1 groups");
-  if ((int64_t)nx * ny > (int64_t)1 << 30 || nx > 16384 || ny > 16384)
-    return fail(ctx, VHP_ERR_UNSUPPORTED, "grid larger than 16384 x 16384 is not supported");
-  if (dtype != VHP_F32 && dtype != VHP_F64) return fail(ctx, VHP_ERR_INVALID_ARG, "bad dtype");
+  const vhp_status st = check_grid_dtype(ctx, nx, ny, dtype);
+  if (st != VHP_OK) return st;
   if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: threshold is NaN");
   if (!out->vmax && !out->first && !out->count)
     return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: no output requested");
@@ -997,7 +990,7 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
   m.pair_group = pg;
   m.pair_k = pk;
   m.pair_map = pm;
-  if (thr > 0.0 && one_cta_tile_route(ctx, nx, ny, nsrc)) {
+  if (thr > 0.0 && sweep_route(ctx, nx, ny, nsrc) == SweepRoute::Tile) {
     if ((st = ensure_rcp2(ctx, std::max(nx, ny) + 64)) != VHP_OK) return st;
     if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
     VHP_CUDA(ctx, vhp_launch_sweep_merge(ctx->tile, nx, ny, d_xy, m, nsrc, thr, ctx->rcp2_table, ctx->d_err,
@@ -1043,18 +1036,11 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   ctx->last_transport_packed = 0;
   if (ngroups == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
-  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8, occ_bytes = (size_t)nmaps * cells;
-  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, 8 * (size_t)std::max<int64_t>(nsrc, 1))) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  if (nsrc > 0)
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, xy, (size_t)nsrc * 8, cudaMemcpyHostToDevice, ctx->stream));
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
-  if (ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
-    if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
-    ctx->planes_sticky = true;
-  }
+  PlanesGuard planes_guard(ctx);
+  // (the group maps are uploaded per run of groups below)
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
+    return st;
+  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
   const size_t bv = out->vmax ? esz : 0, bf = out->first ? 4 : 0, bc = out->count ? 4 : 0;
   const int64_t gchunk = std::min<int64_t>(ngroups, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / (cells * (bv + bf + bc)))));
   vhp_status result = ensure(ctx, ctx->b_out[0], (size_t)gchunk * cells * (bv + bf + bc));
@@ -1091,8 +1077,6 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     ctx->last_d2h_bytes += (int64_t)(n * (bv + bf + bc));
   }
   cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
   ctx->last_result_bytes = ctx->last_d2h_bytes;
   if (result != VHP_OK) return result;
   if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
@@ -1156,7 +1140,7 @@ vhp_status planner_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx
   if (nprob == 0) return VHP_OK;
   // maps too wide for the persistent single-CTA kernel still run on the grid route
   const bool cta_ok = vhp_planner_supported(nx, ny);
-  if (!cta_ok && !(ctx->grid_sweep != 0 && vhp_sweep_grid_supported(nx, ny)))
+  if (!cta_ok && !grid_mode_available(ctx, nx, ny))
     return fail(ctx, VHP_ERR_UNSUPPORTED, "planner: grid too large for the single-CTA kernel");
   if (ls_cap < max_iter + 2 || max_iter < 0)
     return fail(ctx, VHP_ERR_INVALID_ARG, "planner: ls_cap must be >= max_iter + 2");
@@ -1215,15 +1199,9 @@ vhp_status planner_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx
     float *vg32 = (dtype == VHP_F32 && o.vg) ? (float *)o.vg + q0 * cells : nullptr;
     float *vis32 = (dtype == VHP_F32 && o.vis) ? (float *)o.vis + q0 * cells : nullptr;
     if (grid_route) {
-      int wx, wy, nsum;
-      vhp_tile_plane_geometry(nx, ny, &wx, &wy, &nsum);
       for (int64_t k = 0; k < n; ++k) {
         const int64_t q = q0 + k;
-        const size_t m = d_pmap ? (size_t)h_pmap[q] : 0;
-        VhpTilePlanes pl = ctx->tile; // planes of map m (the grid kernels sweep "map 0")
-        pl.rowF += m * pl.row_plane; pl.rowR += m * pl.row_plane;
-        pl.colF += m * pl.col_plane; pl.colR += m * pl.col_plane;
-        pl.bsum += m * (size_t)nsum;
+        const VhpTilePlanes pl = planes_of_map(ctx, d_pmap ? (size_t)h_pmap[q] : 0, nx, ny);
         st = planner_grid_one(ctx, pl, nx, ny, &h_se[4 * q], thr, max_iter, ls_cap, vis + k * cells,
                               vg + k * cells, ws_hc + k * cells, came + k * cells, status + q, nb + q,
                               ls + 2 * (size_t)ls_cap * q, plen + q, pn + q,
@@ -1252,10 +1230,8 @@ vhp_status planner_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx
 vhp_status vhp_i_fail(vhp_context *ctx, vhp_status st, const std::string &msg) { return fail(ctx, st, msg); }
 vhp_status vhp_i_ensure_rcp2(vhp_context *ctx, int len) { return ensure_rcp2(ctx, len); }
 int vhp_i_grid_ctas(const vhp_context *ctx, int nx, int ny, int rows) {
-  const bool cta_ok = vhp_sweep_tile_supported(nx, ny);
-  const int mode = ctx->grid_sweep;
-  if (!cta_ok || (mode && vhp_sweep_grid_supported(nx, ny) &&
-                  (int64_t)nx * rows >= (mode > 1 ? 0 : (1 << 20))))
+  if (!vhp_sweep_tile_supported(nx, ny) ||
+      (grid_mode_available(ctx, nx, ny) && (int64_t)nx * rows >= (ctx->grid_sweep > 1 ? 0 : (1 << 20))))
     return grid_sweep_ctas(ctx, rows);
   return 1;
 }
@@ -1465,25 +1441,11 @@ vhp_status vhp_visibility_batch_packed(vhp_context *ctx, const uint8_t *occ, int
   h->chunks.clear();
   auto run = [&]() -> vhp_status {
     if (npairs == 0) return VHP_OK;
-    const size_t cells = (size_t)nx * ny, occ_bytes = (size_t)nmaps * cells;
-    vhp_status r;
-    if ((r = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return r;
-    if ((r = ensure(ctx, ctx->b_src, (size_t)npairs * 8)) != VHP_OK) return r;
-    if (src_map && (r = ensure(ctx, ctx->b_map, (size_t)npairs * 4)) != VHP_OK) return r;
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, src_xy, (size_t)npairs * 8, cudaMemcpyHostToDevice, ctx->stream));
-    if (src_map)
-      VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, src_map, (size_t)npairs * 4, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->planes_sticky = false;
-    ctx->tile_src = nullptr;
-    if (ctx->sweep_impl == 0 && (vhp_sweep_tile_supported(nx, ny) || vhp_sweep_grid_supported(nx, ny))) {
-      if ((r = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return r;
-      ctx->planes_sticky = true;
-    }
+    PlanesGuard planes_guard(ctx);
+    vhp_status r = stage_host_batch(ctx, occ, nmaps, nx, ny, src_xy, 8, npairs, src_map, sweeps_use_planes(ctx, nx, ny));
+    if (r != VHP_OK) return r;
     r = run_host_to_packed(ctx, nmaps, nx, ny, (const int32_t *)ctx->b_src.p,
                            src_map ? (const int32_t *)ctx->b_map.p : nullptr, npairs, dtype, h);
-    ctx->planes_sticky = false;
-    ctx->tile_src = nullptr;
     if (r != VHP_OK) return r;
     return check_device_error(ctx);
   };
@@ -1575,16 +1537,9 @@ vhp_status vhp_visibility_variant_batch(vhp_context *ctx, const uint8_t *occ, in
     return st;
   if (npairs == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
-  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8, occ_bytes = (size_t)nmaps * cells;
-  if ((st = ensure(ctx, ctx->b_occ, occ_bytes)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, (size_t)npairs * 8)) != VHP_OK) return st;
-  if (src_map && (st = ensure(ctx, ctx->b_map, (size_t)npairs * 4)) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, occ_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, src_xy, (size_t)npairs * 8, cudaMemcpyHostToDevice, ctx->stream));
-  if (src_map)
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, src_map, (size_t)npairs * 4, cudaMemcpyHostToDevice, ctx->stream));
-  ctx->planes_sticky = false; // b_occ content changed
-  ctx->tile_src = nullptr;
+  PlanesGuard planes_guard(ctx);
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, src_xy, 8, npairs, src_map, false)) != VHP_OK) return st;
+  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
   // results leave in chunks of at most 1 GB through one device buffer
   const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(npairs, (int64_t)(((size_t)1 << 30) / (cells * esz))));
   if ((st = ensure(ctx, ctx->b_out[0], (size_t)chunk * cells * esz)) != VHP_OK) return st;
@@ -1817,8 +1772,7 @@ vhp_status vhp_strip_sweep_dev(vhp_context *ctx, const uint8_t *d_occ, int nx, i
   if (sx < 0 || sx >= nx || sy < 0 || sy >= ny)
     return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_strip_sweep_dev: source outside the grid");
   if (dtype != VHP_F32 && dtype != VHP_F64) return fail(ctx, VHP_ERR_INVALID_ARG, "bad dtype");
-  const bool cta_ok = vhp_sweep_tile_supported(nx, ny);
-  if (!cta_ok && !(ctx->grid_sweep != 0 && vhp_sweep_grid_supported(nx, ny)))
+  if (!vhp_sweep_tile_supported(nx, ny) && !grid_mode_available(ctx, nx, ny))
     return fail(ctx, VHP_ERR_UNSUPPORTED, "vhp_strip_sweep_dev: grid too wide for the tile kernel");
   int32_t rows[4];
   vhp_window_halo_rows(nx, ny, sx, sy, y0, y1, rows);
@@ -1831,13 +1785,8 @@ vhp_status vhp_strip_sweep_dev(vhp_context *ctx, const uint8_t *d_occ, int nx, i
   if ((st = pack_tile(ctx, d_occ, 1, nx, ny, false)) != VHP_OK) return st;
   // Large windows are swept by many CTAs at once (grid mode): enough 8-warp CTAs for the tile
   // rows of the window, at most two per SM.
-  const int grid_mode = ctx->grid_sweep;
-  int grid_ctas = 1;
-  if (!cta_ok || (grid_mode && vhp_sweep_grid_supported(nx, ny) &&
-                  (int64_t)nx * (y1 - y0) >= (grid_mode > 1 ? 0 : (1 << 20)))) {
-    grid_ctas = grid_sweep_ctas(ctx, y1 - y0);
-    if ((st = ensure(ctx, ctx->b_grid, vhp_sweep_grid_ws_bytes(nx, ny))) != VHP_OK) return st;
-  }
+  const int grid_ctas = vhp_i_grid_ctas(ctx, nx, ny, y1 - y0);
+  if (grid_ctas > 1 && (st = ensure(ctx, ctx->b_grid, vhp_sweep_grid_ws_bytes(nx, ny))) != VHP_OK) return st;
   VHP_CUDA(ctx, vhp_launch_sweep_window(ctx->tile, nx, ny, sx, sy, y0, y1, d_halo, dtype,
                                         d_vis_strip, ctx->rcp2_table, ctx->d_err,
                                         grid_ctas > 1 ? ctx->b_grid.p : nullptr, grid_ctas,
@@ -1890,18 +1839,10 @@ vhp_status vhp_planner_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, in
       return st;
   if (nprob == 0) return VHP_OK;
   VHP_ON_DEVICE(ctx);
+  PlanesGuard planes_guard(ctx);
+  // (the planner kernels always read the bit planes, whatever VHP_SWEEP_IMPL says)
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, se_xy, 16, nprob, prob_map, true)) != VHP_OK) return st;
   const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
-  if ((st = ensure(ctx, ctx->b_occ, (size_t)nmaps * cells)) != VHP_OK) return st;
-  if ((st = ensure(ctx, ctx->b_src, (size_t)nprob * 16)) != VHP_OK) return st;
-  if (prob_map && (st = ensure(ctx, ctx->b_map, (size_t)nprob * 4)) != VHP_OK) return st;
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_occ.p, occ, (size_t)nmaps * cells, cudaMemcpyHostToDevice, ctx->stream));
-  VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_src.p, se_xy, (size_t)nprob * 16, cudaMemcpyHostToDevice, ctx->stream));
-  if (prob_map)
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_map.p, prob_map, (size_t)nprob * 4, cudaMemcpyHostToDevice, ctx->stream));
-  ctx->tile_src = nullptr;
-  ctx->planes_sticky = false;
-  if ((st = pack_tile(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, true)) != VHP_OK) return st;
-  ctx->planes_sticky = true;
   // device staging for the requested outputs, a chunk of problems at a time
   const size_t per_prob = (h.vis ? esz * cells : 0) + (h.vg ? esz * cells : 0) + (h.came ? 4 * cells : 0) +
                           4 + 4 + 8 + 4 + 2 * (size_t)ls_cap * 8 + 64;
@@ -1945,8 +1886,6 @@ vhp_status vhp_planner_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, in
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess && result == VHP_OK) result = cuda_fail(ctx, e, "planner sync");
   }
-  ctx->planes_sticky = false;
-  ctx->tile_src = nullptr;
   if (result != VHP_OK) return result;
   return check_device_error(ctx);
 }

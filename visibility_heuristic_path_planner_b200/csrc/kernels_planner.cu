@@ -527,13 +527,6 @@ cudaError_t vhp_launch_planner(const VhpTilePlanes &pl, int nx, int ny, const in
   p.fp.vec = ((uintptr_t)d_vis % 16 == 0 && nx % 2 == 0) ? 1 : 0;
   p.fp.win_y0 = 0;
   p.fp.win_y1 = ny;
-  for (int q = 0; q < 4; ++q) p.fp.halo[q] = nullptr;
-  p.fp.g_edges = nullptr;
-  p.fp.g_lm = p.fp.g_prog = p.fp.g_next_row = nullptr;
-  p.fp.qmask = 0xF;
-  p.fp.x_edges = nullptr; p.fp.x_prog = nullptr; p.fp.x_y0 = p.fp.x_y1 = 0; p.fp.remote_mask = 0;
-  p.fp.thr = 0.0;
-  p.fp.src_ctl = nullptr;
   p.se_xy = d_se_xy; p.prob_map = d_prob_map;
   p.thr = threshold; p.max_iter = max_iter; p.ls_cap = ls_cap;
   p.vis = d_vis; p.vg = d_vg; p.hc = d_hc; p.came = d_came;

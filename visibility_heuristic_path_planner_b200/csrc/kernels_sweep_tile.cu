@@ -326,13 +326,6 @@ cudaError_t vhp_launch_sweep_window_batch(const VhpTilePlanes &pl, int nmaps, in
   p.vec = 0; // window rows are not 16-byte aligned
   p.win_y0 = 0;
   p.win_y1 = ny;
-  for (int q = 0; q < 4; ++q) p.halo[q] = nullptr;
-  p.g_edges = nullptr;
-  p.g_lm = p.g_prog = p.g_next_row = nullptr;
-  p.qmask = 0xF;
-  p.src_ctl = nullptr;
-  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
-  p.thr = 0.0;
   p.w_r = radius;
   p.w_sw = win_sum_words(nx, radius);
   p.w_nmaps = nmaps;
@@ -380,12 +373,6 @@ cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, cons
   p.vec = 0;
   p.win_y0 = 0;
   p.win_y1 = ny;
-  for (int q = 0; q < 4; ++q) p.halo[q] = nullptr;
-  p.g_edges = nullptr;
-  p.g_lm = p.g_prog = p.g_next_row = nullptr;
-  p.qmask = 0xF;
-  p.src_ctl = nullptr;
-  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
   p.thr = thr;
   p.m_vmax = m.vmax;
   p.m_first = m.first;
@@ -466,13 +453,6 @@ cudaError_t vhp_launch_sweep_tile(const VhpTilePlanes &pl, int nx, int ny, const
   p.vec = ((uintptr_t)d_out % 16 == 0 && ((size_t)nx * esz) % 16 == 0) ? 1 : 0;
   p.win_y0 = 0;
   p.win_y1 = ny;
-  for (int q = 0; q < 4; ++q) p.halo[q] = nullptr;
-  p.g_edges = nullptr;
-  p.g_lm = p.g_prog = p.g_next_row = nullptr;
-  p.qmask = 0xF;
-  p.src_ctl = nullptr;
-  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
-  p.thr = 0.0;
   cudaError_t e;
   if (thr && bits) { // one bit per cell, (fp64 value >= thr), into a zeroed buffer
     if (!(*thr > 0.0)) return cudaErrorInvalidValue; // cells below the threshold are never written
@@ -531,8 +511,6 @@ cudaError_t launch_window(TileArgs &p, int sx, int sy, void *d_grid_ws, int grid
     if (launches) *launches += 2;
     return cudaGetLastError();
   }
-  p.g_edges = nullptr;
-  p.g_lm = p.g_prog = p.g_next_row = nullptr;
   const size_t smem = tile_smem_bytes<OutT>(p.nx, p.ny);
   cudaError_t e = cudaFuncSetAttribute(sweep_window_kernel<OutT>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -568,8 +546,6 @@ cudaError_t vhp_launch_sweep_window(const VhpTilePlanes &pl, int nx, int ny, int
   for (int q = 0; q < 4; ++q) p.halo[q] = d_halo ? d_halo[q] : nullptr;
   p.qmask = qmask;
   p.src_ctl = d_src_ctl;
-  p.x_edges = nullptr; p.x_prog = nullptr; p.x_y0 = p.x_y1 = 0; p.remote_mask = 0;
-  p.thr = 0.0;
   if (peer && d_grid_ws && grid_ctas > 1) { // peer hand-over exists in grid mode only
     const int lmcap = tile_lm_cap(ny);
     if (peer->x_ws) {

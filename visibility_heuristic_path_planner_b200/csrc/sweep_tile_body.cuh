@@ -130,19 +130,19 @@ struct TileArgs {
   // window mode: rows [win_y0, win_y1) only (whole grid: 0, ny); halo[q] = the fp64
   // visibility row (indexed by x) just below the first tile row of quadrant q, or null
   int win_y0, win_y1;
-  const double *halo[4];
+  const double *halo[4] = {nullptr, nullptr, nullptr, nullptr};
   // grid mode (one sweep spread over many CTAs): boundary rows, staircase, row progress and
   // the row counter live in global memory (null otherwise)
-  double *g_edges;
-  int *g_lm, *g_prog, *g_next_row;
+  double *g_edges = nullptr;
+  int *g_lm = nullptr, *g_prog = nullptr, *g_next_row = nullptr;
   // quadrants to run, bit q = Q(q+1) (0xF: all).  The strip-partitioned planner sweeps the +y
   // quadrants (Q1, Q2) and the -y quadrants (Q3, Q4) of a strip as two launches: the two
   // directions travel along the strips independently of each other.
-  int qmask;
+  int qmask = 0xF;
   // window / grid kernels only: {done, sx, sy, ...} in device memory.  Non-null: the source comes
   // from there and the launch is a no-op once `done` is set, so a planner iteration can be
   // enqueued (or captured in a CUDA graph) before the host knows the next source.
-  const int *src_ctl;
+  const int *src_ctl = nullptr;
   // grid mode across GPUs (strip-partitioned planner, one strip per rank): the boundary between
   // two strips is handed over tile by tile through peer memory instead of as a finished row.
   //   exporter: x_edges / x_prog = the boundary rows and progress flags of the NEIGHBOUR's
@@ -155,11 +155,11 @@ struct TileArgs {
   //   consumer: bit q of remote_mask = the boundary below quadrant q's first tile row arrives
   //     this way (its flag is raised with atomicMax by both sides, its boundary row is
   //     initialised only over the lit tiles, which nobody sends).
-  double *x_edges;
-  int *x_prog;
-  int x_y0, x_y1;
-  int remote_mask;
-  double thr; // kFmtBits: bit = (fp64 value >= thr), thr > 0; kFmtMerge*: the count / first threshold
+  double *x_edges = nullptr;
+  int *x_prog = nullptr;
+  int x_y0 = 0, x_y1 = 0;
+  int remote_mask = 0;
+  double thr = 0.0; // kFmtBits: bit = (fp64 value >= thr), thr > 0; kFmtMerge*: the count / first threshold
   // kFmtMerge*: the outputs of all groups ([group][ny][nx] each, any may be null) and the cells of one grid
   void *m_vmax = nullptr;
   int32_t *m_first = nullptr;
