@@ -202,6 +202,32 @@ vhp_status vhp_visibility_merge_batch_dev(vhp_context *ctx, const uint8_t *d_occ
                                           const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
                                           double threshold, vhp_dtype dtype, const vhp_merge_out *d_out);
 
+/* Range-limited merged visibility: what a set of sensors with sensing radius R covers together.  Inputs, group
+ * layout, outputs, dtype rules and errors are those of vhp_visibility_merge_batch, except that source k only
+ * contributes to the cells (x, y) in its range, dx = x - sx, dy = y - sy:
+ *   VHP_RANGE_BOX   |dx| <= R and |dy| <= R        (the cells of its vhp_visibility_window_batch window)
+ *   VHP_RANGE_DISK  dx*dx + dy*dy <= R*R           (integer arithmetic)
+ *   vmax[g][y][x]   max_k of (source k's field where the cell is in k's range, else 0)
+ *   first / count   the merge's "writes" rule narrowed to the range: the cell is in k's range, not on k's
+ *                   never-written border, and has fp64 value >= threshold
+ * Every in-range value equals the full field's (the box is closed under "upstream", the disk lies inside it), so
+ * VHP_RANGE_BOX with R >= max(nx, ny) - 1 is bit-identical to vhp_visibility_merge_batch, and R = 0 covers the
+ * source cells only.  Where threshold > 0 and the box fits one CTA of the batched tile kernel (maps up to
+ * 16384 x 16384 with small R), the sweeps of the boxes fold straight into the group outputs and dark cells cost
+ * nothing; otherwise chunks of fp64 windows (vhp_visibility_window_batch's routes) are folded, with the same
+ * result.  Additional errors (VHP_ERR_INVALID_ARG): radius outside [0, 16383], a shape other than the two. */
+typedef enum vhp_range_shape { VHP_RANGE_BOX = 0, VHP_RANGE_DISK = 1 } vhp_range_shape;
+vhp_status vhp_visibility_merge_range_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                            const int32_t *src_xy, const int64_t *group_ptr,
+                                            const int32_t *group_map, int64_t ngroups, int32_t radius,
+                                            int32_t shape, double threshold, vhp_dtype dtype,
+                                            const vhp_merge_out *out);
+vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                int ny, const int32_t *d_src_xy, const int64_t *d_group_ptr,
+                                                const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
+                                                int32_t radius, int32_t shape, double threshold,
+                                                vhp_dtype dtype, const vhp_merge_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

@@ -23,6 +23,7 @@ if os.environ.get("VHP_LIB_VARIANT"):
     LIB_PATH = os.path.join(PKG, "lib_" + os.environ["VHP_LIB_VARIANT"], "libvhp_b200.so")
 
 F32, F64 = 0, 1
+RANGE_BOX, RANGE_DISK = 0, 1
 NO_PARENT = -1
 STATUS_NAMES = {0: "OK", 1: "START_OOB", 2: "END_OOB", 3: "START_OCCUPIED",
                 4: "END_OCCUPIED", 5: "MAX_ITER", -1: "ERR_INVALID_ARG",
@@ -115,6 +116,10 @@ def load_library(build_if_missing: bool = True):
                                                C.POINTER(MergeOut)]
     lib.vhp_visibility_merge_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_double, i32,
                                                    C.POINTER(MergeOut)]
+    lib.vhp_visibility_merge_range_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, C.c_int32, C.c_int32,
+                                                     C.c_double, i32, C.POINTER(MergeOut)]
+    lib.vhp_visibility_merge_range_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_int32,
+                                                         C.c_int32, C.c_double, i32, C.POINTER(MergeOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -385,6 +390,18 @@ class Context:
         outputs, (ngroups, ny, nx) each: vmax (max of the fields, dtype), first (int32, index within
         the group of the first source whose sweep writes the cell with a value >= threshold, NO_PARENT
         if none) and count (uint32, how many do)."""
+        return self._merge_host(self.lib.vhp_visibility_merge_batch, (), occ, src_xy, group_ptr, threshold, group_map,
+                                dtype, outputs)
+
+    def visibility_merge_range_batch(self, occ, src_xy, group_ptr, threshold, radius, shape, group_map=None,
+                                     dtype=F64, outputs=("vmax", "first", "count")):
+        """Range-limited merged visibility (vhp_visibility_merge_range_batch): visibility_merge_batch where each
+        source only covers the cells in its range, |dx|, |dy| <= radius (shape RANGE_BOX) or
+        dx^2 + dy^2 <= radius^2 (RANGE_DISK)."""
+        return self._merge_host(self.lib.vhp_visibility_merge_range_batch, (int(radius), int(shape)), occ, src_xy,
+                                group_ptr, threshold, group_map, dtype, outputs)
+
+    def _merge_host(self, fn, extra, occ, src_xy, group_ptr, threshold, group_map, dtype, outputs):
         occ = _occ_u8(occ)
         nmaps, ny, nx = occ.shape
         xy = np.ascontiguousarray(src_xy, dtype=np.int32).reshape(-1, 2)
@@ -396,8 +413,8 @@ class Context:
             raise ValueError(f"outputs are among {tuple(kinds)}")
         r = {k: np.empty((max(ng, 0), ny, nx), kinds[k]) for k in outputs}
         mo = MergeOut(*[_np_ptr(r.get(k)) for k in ("vmax", "first", "count")])
-        self._check(self.lib.vhp_visibility_merge_batch(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp),
-                                                        _np_ptr(gm), ng, float(threshold), dtype, C.byref(mo)))
+        self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp), _np_ptr(gm), ng, *extra,
+                       float(threshold), dtype, C.byref(mo)))
         return r
 
     def visibility_merge_batch_dev(self, occ_t, src_xy_t, group_ptr_t, threshold, vmax_t=None, first_t=None,
@@ -405,14 +422,23 @@ class Context:
         """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), src_xy_t int32 (nsrc, 2),
         group_ptr_t int64 (ngroups + 1), outputs (ngroups, ny, nx): vmax_t float32/64, first_t int32,
         count_t int32 (read as uint32); any may be None."""
+        self._merge_dev(self.lib.vhp_visibility_merge_batch_dev, (), occ_t, src_xy_t, group_ptr_t, threshold, vmax_t,
+                        first_t, count_t, group_map_t)
+
+    def visibility_merge_range_batch_dev(self, occ_t, src_xy_t, group_ptr_t, threshold, radius, shape, vmax_t=None,
+                                         first_t=None, count_t=None, group_map_t=None):
+        """visibility_merge_range_batch on CUDA tensors (asynchronous), arguments as visibility_merge_batch_dev."""
+        self._merge_dev(self.lib.vhp_visibility_merge_range_batch_dev, (int(radius), int(shape)), occ_t, src_xy_t,
+                        group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t)
+
+    def _merge_dev(self, fn, extra, occ_t, src_xy_t, group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t):
         nmaps, ny, nx = occ_t.shape
         ng = group_ptr_t.shape[0] - 1
         dtype = F32 if (vmax_t is not None and vmax_t.element_size() == 4) else F64
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         mo = MergeOut(ptr(vmax_t), ptr(first_t), ptr(count_t))
-        self._check(self.lib.vhp_visibility_merge_batch_dev(
-            self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), group_ptr_t.data_ptr(),
-            ptr(group_map_t), ng, src_xy_t.shape[0], float(threshold), dtype, C.byref(mo)))
+        self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), group_ptr_t.data_ptr(),
+                       ptr(group_map_t), ng, src_xy_t.shape[0], *extra, float(threshold), dtype, C.byref(mo)))
 
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):

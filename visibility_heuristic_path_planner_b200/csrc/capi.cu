@@ -951,18 +951,30 @@ vhp_status run_runs_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx
 // layout, then either the sweeps fold straight into the outputs (kFmtMerge*: the one-CTA tile kernel takes the
 // batch and thr > 0, so cells of value 0 never need a visit) or chunks of pairs are swept into the fp64 field in
 // ctx->b_bin by any route of run_dev (grid mode, naive kernel, thr <= 0) and merge_fold_kernel folds them.
+// With a range (vhp_visibility_merge_range_batch) the direct route sweeps only each source's box
+// (kFmtMergeRange*, window_direct_route) and the fallback folds chunks of fp64 windows (run_window_dev, any of its
+// routes) with merge_window_fold_kernel.
+const char *merge_name(const VhpMergeRange *range) {
+  return range ? "vhp_visibility_merge_range_batch" : "vhp_visibility_merge_batch";
+}
+
 vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t ngroups, int64_t nsrc, double thr, int dtype,
-                            const vhp_merge_out *out) {
+                            const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
+  const std::string what = merge_name(range);
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || ngroups < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
-  if (ngroups > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: more than 2^31 - 1 groups");
+  if (ngroups > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": more than 2^31 - 1 groups");
   const vhp_status st = check_grid_dtype(ctx, nx, ny, dtype);
   if (st != VHP_OK) return st;
-  if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: threshold is NaN");
+  if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
   if (!out->vmax && !out->first && !out->count)
-    return fail(ctx, VHP_ERR_INVALID_ARG, "vhp_visibility_merge_batch: no output requested");
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
+  if (range && (range->radius < 0 || range->radius > 16383))
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": radius outside [0, 16383]");
+  if (range && range->shape != VHP_RANGE_BOX && range->shape != VHP_RANGE_DISK)
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": shape is neither VHP_RANGE_BOX nor VHP_RANGE_DISK");
   return VHP_OK;
 }
 
@@ -977,7 +989,7 @@ VhpMergeDev merge_dev_of(const vhp_merge_out &o, vhp_dtype dtype) {
 
 vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
                          const int64_t *d_gptr, const int32_t *d_gmap, int64_t ngroups, int64_t nsrc, double thr,
-                         VhpMergeDev m) {
+                         VhpMergeDev m, const VhpMergeRange *range = nullptr) {
   const size_t cells = (size_t)nx * ny;
   VHP_CUDA(ctx, vhp_launch_merge_fill(m, (size_t)ngroups * cells, ctx->stream));
   if (ngroups == 0 && nsrc == 0) return VHP_OK;
@@ -990,6 +1002,29 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
   m.pair_group = pg;
   m.pair_k = pk;
   m.pair_map = pm;
+  if (range) {
+    const int R = range->radius;
+    if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
+      if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), R + 1) + 64)) != VHP_OK) return st;
+      if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
+      VHP_CUDA(ctx, vhp_launch_sweep_merge(ctx->tile, nx, ny, d_xy, m, nsrc, thr, ctx->rcp2_table, ctx->d_err,
+                                           ctx->stream, &ctx->launches, range));
+      return VHP_OK;
+    }
+    // fp64 windows of up to 1 GB of pairs at a time
+    const size_t wbytes = window_pair_bytes(R, VHP_F64);
+    const int64_t chunk = std::min<int64_t>(nsrc, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / wbytes)));
+    if ((st = ensure(ctx, ctx->b_mwin, (size_t)chunk * wbytes)) != VHP_OK) return st;
+    for (int64_t p0 = 0; p0 < nsrc; p0 += chunk) {
+      const int64_t np = std::min(chunk, nsrc - p0);
+      if ((st = run_window_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * p0, pm + p0, np, R, VHP_F64, ctx->b_mwin.p)) !=
+          VHP_OK)
+        return st;
+      VHP_CUDA(ctx, vhp_launch_merge_window_fold((const double *)ctx->b_mwin.p, p0, np, nx, ny, d_xy, thr, *range, m,
+                                                 ctx->sm_count, ctx->stream, &ctx->launches));
+    }
+    return VHP_OK;
+  }
   if (thr > 0.0 && sweep_route(ctx, nx, ny, nsrc) == SweepRoute::Tile) {
     if ((st = ensure_rcp2(ctx, std::max(nx, ny) + 64)) != VHP_OK) return st;
     if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
@@ -1015,8 +1050,8 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
 // smaller than the fields it folds)
 vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
                           const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
-                          const vhp_merge_out *out) {
-  const char *what = "vhp_visibility_merge_batch";
+                          const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
+  const char *what = merge_name(range);
   if (ctx && gptr && ngroups >= 0) {
     if (gptr[0] != 0) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(what) + ": group_ptr[0] must be 0");
     for (int64_t g = 0; g < ngroups; ++g) {
@@ -1028,7 +1063,7 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     }
   }
   const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
-  vhp_status st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out);
+  vhp_status st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range);
   if (st != VHP_OK) return st;
   if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, what)) != VHP_OK) return st;
   if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, what)) != VHP_OK) return st;
@@ -1064,7 +1099,7 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: upload of the group layout"); break; }
     result = run_merge_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a,
                            (const int64_t *)ctx->b_misc.p, gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc,
-                           gptr[g0 + gc] - a, thr, m);
+                           gptr[g0 + gc] - a, thr, m, range);
     if (result != VHP_OK) break;
     const size_t n = (size_t)gc * cells, off = (size_t)g0 * cells;
     if (out->vmax) e = cudaMemcpyAsync((char *)out->vmax + off * esz, m.vmax, n * esz, cudaMemcpyDeviceToHost, ctx->stream);
@@ -1329,7 +1364,7 @@ void vhp_context_destroy(vhp_context *ctx) {
   if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
   VhpDevBuf *bufs[] = {&ctx->b_occ, &ctx->b_src, &ctx->b_map, &ctx->b_out[0], &ctx->b_out[1],
                        &ctx->b_scratch, &ctx->b_planner, &ctx->b_misc, &ctx->b_grid, &ctx->b_bin,
-                       &ctx->b_merge};
+                       &ctx->b_merge, &ctx->b_mwin};
   for (VhpDevBuf *b : bufs)
     if (b->p) cudaFree(b->p);
   delete ctx->expand_pool;
@@ -1614,6 +1649,34 @@ vhp_status vhp_visibility_merge_batch_dev(vhp_context *ctx, const uint8_t *d_occ
   VHP_ON_DEVICE(ctx);
   return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
                        merge_dev_of(*d_out, dtype));
+}
+
+vhp_status vhp_visibility_merge_range_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                            const int32_t *src_xy, const int64_t *group_ptr,
+                                            const int32_t *group_map, int64_t ngroups, int32_t radius,
+                                            int32_t shape, double threshold, vhp_dtype dtype,
+                                            const vhp_merge_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_merge_host(ctx, occ, nmaps, nx, ny, src_xy, group_ptr, group_map, ngroups, threshold, dtype, out,
+                        &range);
+}
+
+vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                int ny, const int32_t *d_src_xy, const int64_t *d_group_ptr,
+                                                const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
+                                                int32_t radius, int32_t shape, double threshold,
+                                                vhp_dtype dtype, const vhp_merge_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
+                                   d_out, &range);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
+                       merge_dev_of(*d_out, dtype), &range);
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

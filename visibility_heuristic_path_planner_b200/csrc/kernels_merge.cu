@@ -8,10 +8,13 @@
 //   first = min { k : k writes the cell, v_k >= thr }, -1 if none
 //   count = #{ k : k writes the cell, v_k >= thr }
 // where source (sx, sy) writes every cell but column 0 (unless sx == 0) and row 0 (unless sy == 0).
+// The range-limited form (vhp_visibility_merge_range_batch) counts v_k only where the cell is in k's range; its
+// fallback folds fp64 windows (merge_window_fold_kernel) instead of whole fields.
 #include <algorithm>
 #include <cstdint>
 
 #include "vhp_internal.h"
+#include "sweep_common.cuh"
 
 namespace {
 
@@ -104,6 +107,36 @@ __global__ void merge_fold_kernel(const double *__restrict__ field, int64_t p0, 
   }
 }
 
+// One thread per window cell of pairs [p0, p0 + np): cells in the grid and in the pair's range fold into its
+// group's outputs with the relaxed reductions of the direct route (kFmtMergeRange*), so the order of the pairs
+// does not matter.  r2: a cell (dx, dy) of the window is in range iff dx^2 + dy^2 <= r2 (box: 2 R^2).
+template <bool F32>
+__global__ void merge_window_fold_kernel(const double *__restrict__ win, int64_t p0, int64_t np, int nx, int ny,
+                                         int R, int r2, const int32_t *__restrict__ xy, double thr, VhpMergeDev m) {
+  const int W = 2 * R + 1;
+  const size_t ww = (size_t)W * W, total = (size_t)np * ww, cells = (size_t)nx * ny;
+  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total;
+       idx += (size_t)gridDim.x * blockDim.x) {
+    const int64_t q = p0 + (int64_t)(idx / ww);
+    const int rem = (int)(idx % ww), dy = rem / W - R, dx = rem % W - R;
+    const int sx = __ldg(xy + 2 * q), sy = __ldg(xy + 2 * q + 1), x = sx + dx, y = sy + dy;
+    if ((unsigned)x >= (unsigned)nx || (unsigned)y >= (unsigned)ny || dx * dx + dy * dy > r2) continue;
+    const int32_t g = __ldg(m.pair_group + q);
+    if (g < 0) continue;
+    const double v = __ldg(win + idx);
+    const size_t o = (size_t)g * cells + (size_t)y * nx + x;
+    if (m.vmax && v > 0.0) {
+      if (F32) red_max_u32(reinterpret_cast<uint32_t *>(m.vmax) + o, __float_as_uint(__double2float_rn(v)));
+      else red_max_u64(reinterpret_cast<unsigned long long *>(m.vmax) + o, (unsigned long long)__double_as_longlong(v));
+    }
+    const bool writes = !((x == 0 && sx != 0) || (y == 0 && sy != 0));
+    if (writes && v >= thr) {
+      if (m.first) red_min_u32(reinterpret_cast<uint32_t *>(m.first) + o, (uint32_t)__ldg(m.pair_k + q));
+      if (m.count) red_add_u32(m.count + o, 1u);
+    }
+  }
+}
+
 unsigned grid_for(size_t n, int bs, int sm_count) {
   return (unsigned)std::max<size_t>(1, std::min<size_t>((n + bs - 1) / bs, (size_t)sm_count * 32));
 }
@@ -137,6 +170,19 @@ cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np,
   const unsigned grid = grid_for((size_t)np * cells, bs, sm_count);
   if (m.f32) merge_fold_kernel<true><<<grid, bs, 0, st>>>(d_field, p0, np, nx, cells, d_src_xy, thr, m);
   else merge_fold_kernel<false><<<grid, bs, 0, st>>>(d_field, p0, np, nx, cells, d_src_xy, thr, m);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t vhp_launch_merge_window_fold(const double *d_win, int64_t p0, int64_t np, int nx, int ny,
+                                         const int32_t *d_src_xy, double thr, const VhpMergeRange &range,
+                                         const VhpMergeDev &m, int sm_count, cudaStream_t st, int64_t *launches) {
+  const int R = range.radius, r2 = range.shape == VHP_RANGE_DISK ? R * R : 2 * R * R;
+  const size_t W = 2 * (size_t)R + 1;
+  const int bs = 256;
+  const unsigned grid = grid_for((size_t)np * W * W, bs, sm_count);
+  if (m.f32) merge_window_fold_kernel<true><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m);
+  else merge_window_fold_kernel<false><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

@@ -42,7 +42,7 @@ sweep_tile_kernel(const TileArgs p) {
     return;
   }
   const int map = p.src_map ? __ldg(p.src_map + pair) : 0;
-  if constexpr (FMT == kFmtMerge64 || FMT == kFmtMerge32) { // fold into the outputs of the pair's group
+  if constexpr (fmt_merge(FMT)) { // fold into the outputs of the pair's group
     const int g = __ldg(p.m_pg + pair);
     if (g < 0) return; // a pair of an inconsistent group layout (the table kernel reported it)
     if (threadIdx.x == 0) *reinterpret_cast<int2 *>(smem_raw + kMergeHdr) = make_int2(g, __ldg(p.m_pk + pair));
@@ -205,8 +205,8 @@ __global__ void ratio2_selftest_kernel(const double2 *__restrict__ tab, int kmax
 
 template <typename OutT, int NW, int MINB, int FMT = kFmtValues>
 cudaError_t launch_tile_nw(const TileArgs &p, int64_t npairs, cudaStream_t st) {
-  const size_t smem = FMT == kFmtWindow ? tile_smem_bytes_win<OutT>(p.nx, p.ny, p.w_r, NW)
-                                        : tile_smem_bytes<OutT>(p.nx, p.ny, NW);
+  const size_t smem = fmt_clip(FMT) ? tile_smem_bytes_win<OutT>(p.nx, p.ny, p.w_r, NW)
+                                    : tile_smem_bytes<OutT>(p.nx, p.ny, NW);
   auto kern = sweep_tile_kernel<OutT, NW, MINB, FMT>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
@@ -270,6 +270,16 @@ cudaError_t launch_tile_win(const TileArgs &p, int64_t npairs, cudaStream_t st) 
     case 1: return launch_tile_nw<OutT, 1, VHP_NW1_MINB, kFmtWindow>(p, npairs, st);
     case 2: case 4: case 6: return launch_tile_nw<OutT, 4, VHP_NW4_MINB, kFmtWindow>(p, npairs, st);
     default: return launch_tile_nw<OutT, 8, 2, kFmtWindow>(p, npairs, st);
+  }
+}
+
+// range-limited merged output (kFmtMergeRange*): fp64 staging, the warp counts and bounds of the windows
+template <int FMT>
+cudaError_t launch_tile_merge_range(const TileArgs &p, int64_t npairs, cudaStream_t st) {
+  switch (tile_warps_for(win_side(p.nx, p.w_r), win_side(p.ny, p.w_r), npairs)) {
+    case 1: return launch_tile_nw<double, 1, VHP_NW1_MINB, FMT>(p, npairs, st);
+    case 2: case 4: case 6: return launch_tile_nw<double, 4, VHP_NW4_MINB, FMT>(p, npairs, st);
+    default: return launch_tile_nw<double, 8, 2, FMT>(p, npairs, st);
   }
 }
 
@@ -359,7 +369,7 @@ cudaError_t vhp_launch_window_pairs(const int32_t *d_src_xy, const int32_t *d_sr
 
 cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
                                    const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,
-                                   int *d_err, cudaStream_t st, int64_t *launches) {
+                                   int *d_err, cudaStream_t st, int64_t *launches, const VhpMergeRange *range) {
   if (!(thr > 0.0)) return cudaErrorInvalidValue; // cells of value 0 are never visited
   TileArgs p;
   p.pl = pl;
@@ -381,6 +391,14 @@ cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, cons
   p.m_pg = m.pair_group;
   p.m_pk = m.pair_k;
   if (launches) *launches += 1;
+  if (range) {
+    const int R = range->radius;
+    p.w_r = R;
+    p.w_sw = win_sum_words(nx, R);
+    p.w_r2 = range->shape == VHP_RANGE_DISK ? R * R : 2 * R * R;
+    return m.f32 ? launch_tile_merge_range<kFmtMergeRange32>(p, npairs, st)
+                 : launch_tile_merge_range<kFmtMergeRange64>(p, npairs, st);
+  }
   return m.f32 ? launch_tile_merge<kFmtMerge32>(p, npairs, st) : launch_tile_merge<kFmtMerge64>(p, npairs, st);
 }
 

@@ -167,8 +167,11 @@ struct TileArgs {
   size_t m_cells = 0;
   const int32_t *m_pg = nullptr, *m_pk = nullptr; // per pair: group (-1: skip the pair) and index within it
   // kFmtWindow: radius R (windows of (2R+1)^2 per pair), block-summary words per window row (win_sum_words)
-  // and the number of maps (a pair on another map is reported like a source outside the grid)
+  // and the number of maps (a pair on another map is reported like a source outside the grid); kFmtMergeRange*:
+  // R and w_sw, the sweep clipped to the box |dx|, |dy| <= R
   int w_r = 0, w_sw = 0, w_nmaps = 0;
+  // kFmtMergeRange*: a cell of the box is in range iff dx^2 + dy^2 <= w_r2 (disk: R^2; box: 2 R^2, every cell)
+  int w_r2 = 0;
 };
 
 // how tile_sweep_cta is used
@@ -294,31 +297,33 @@ __device__ __forceinline__ void stg16_fill(double *q, double v) {
 // kFmtWindow: the field like kFmtValues, but only the (2R+1)^2 window around the source (TileArgs::w_r): each
 // quadrant's extents are clipped to R, `out` is shifted so that cell (x, y) sits at out[y * (2R+1) + x], stores
 // are scalar (window rows are not 16-byte aligned), and the window cells outside the grid are stored as 0.
-constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4, kFmtWindow = 5;
+// kFmtMergeRange64 / kFmtMergeRange32 (vhp_visibility_merge_range_batch): kFmtMerge* with the sweep clipped to the box
+// |dx|, |dy| <= R like kFmtWindow (the box is closed under "upstream": its values are the full field's), cell indices
+// in map pitch, and only the cells in range (TileArgs::w_r2) folded.
+constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4, kFmtWindow = 5, kFmtMergeRange64 = 6,
+              kFmtMergeRange32 = 7;
 constexpr int kMergeHdr = 224; // shared-memory header: {group, k} of the CTA's source (int2)
 
-__device__ __forceinline__ void red_max_u64(unsigned long long *a, unsigned long long v) {
-  asm volatile("red.relaxed.gpu.global.max.u64 [%0], %1;" :: "l"(a), "l"(v) : "memory");
-}
-__device__ __forceinline__ void red_max_u32(uint32_t *a, uint32_t v) {
-  asm volatile("red.relaxed.gpu.global.max.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
-}
-__device__ __forceinline__ void red_min_u32(uint32_t *a, uint32_t v) {
-  asm volatile("red.relaxed.gpu.global.min.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
-}
-__device__ __forceinline__ void red_add_u32(uint32_t *a, uint32_t v) {
-  asm volatile("red.relaxed.gpu.global.add.u32 [%0], %1;" :: "l"(a), "r"(v) : "memory");
-}
+// the sweep folds into group outputs (merge_cell), and it does so only within a range
+__host__ __device__ constexpr bool fmt_range(int f) { return f == kFmtMergeRange64 || f == kFmtMergeRange32; }
+__host__ __device__ constexpr bool fmt_merge(int f) { return f == kFmtMerge64 || f == kFmtMerge32 || fmt_range(f); }
+// clipped geometry: each quadrant's extents are clipped to R and the per-CTA state is sized by the box
+// (tile_smem_bytes_win); the window output layout (pitch 2R+1, off-grid zeros) is kFmtWindow's alone
+__host__ __device__ constexpr bool fmt_clip(int f) { return f == kFmtWindow || fmt_range(f); }
 
-// fold value v of cell idx (y * nx + x) of this CTA's sweep into its group's outputs
+// fold value v of cell idx (y * nx + x) of this CTA's sweep into its group's outputs; (di, dj) = (|dx|, |dy|) of
+// the cell from the source, for the range test of kFmtMergeRange*
 template <int FMT>
-__device__ __forceinline__ void merge_cell(const TileArgs &p, const ptrdiff_t idx, const double v) {
+__device__ __forceinline__ void merge_cell(const TileArgs &p, const ptrdiff_t idx, const int di, const int dj,
+                                           const double v) {
   if (!(v > 0.0)) return;
+  if constexpr (fmt_range(FMT))
+    if (di * di + dj * dj > p.w_r2) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int2 gk = *reinterpret_cast<const int2 *>(smem_raw + kMergeHdr);
   const size_t o = (size_t)gk.x * p.m_cells + (size_t)idx;
   if (p.m_vmax) {
-    if constexpr (FMT == kFmtMerge64)
+    if constexpr (FMT == kFmtMerge64 || FMT == kFmtMergeRange64)
       red_max_u64(reinterpret_cast<unsigned long long *>(p.m_vmax) + o, (unsigned long long)__double_as_longlong(v));
     else
       red_max_u32(reinterpret_cast<uint32_t *>(p.m_vmax) + o, __float_as_uint(__double2float_rn(v)));
@@ -339,26 +344,26 @@ __device__ __forceinline__ int tile_start(const int a, const int T) {
 }
 
 // Last local column / row to compute: the extent without the never-written border (x == 0 in the
-// -x quadrants, y == 0 in the -y quadrants).  A window (WIN) whose clipped extent stops short of the
+// -x quadrants, y == 0 in the -y quadrants).  A clipped sweep (CLIP) whose extent stops short of the
 // grid's edge has no border cell.
-template <bool WIN = false>
+template <bool CLIP = false>
 __device__ __forceinline__ int ext_cx(const TQuad &g, const int sx) {
-  return g.Ex - (g.dirx < 0 && (!WIN || g.Ex == sx));
+  return g.Ex - (g.dirx < 0 && (!CLIP || g.Ex == sx));
 }
-template <bool WIN = false>
+template <bool CLIP = false>
 __device__ __forceinline__ int ext_cy(const TQuad &g, const int sy) {
-  return g.Ey - (g.diry < 0 && (!WIN || g.Ey == sy));
+  return g.Ey - (g.diry < 0 && (!CLIP || g.Ey == sy));
 }
 
 // Does the block summary prove every cell tile (I, J) has to compute is free?  (A tile
 // with nothing to compute -- only border cells -- counts as free.)
-template <bool WIN = false>
+template <bool CLIP = false>
 __device__ __forceinline__ bool tile_sum_free(const TQuad &g, const uint32_t *bsum, const int nbw,
                                               const int sx, const int sy, const int I,
                                               const int J) {
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
-  const int nvx = min(I ? kTile : g.a, ext_cx<WIN>(g, sx) - i0 + 1);
-  const int nvy = min(J ? kTile : g.a, ext_cy<WIN>(g, sy) - j0 + 1);
+  const int nvx = min(I ? kTile : g.a, ext_cx<CLIP>(g, sx) - i0 + 1);
+  const int nvy = min(J ? kTile : g.a, ext_cy<CLIP>(g, sy) - j0 + 1);
   if (nvx <= 0 || nvy <= 0) return true;
   const int xa = sx + g.dirx * i0, xb = sx + g.dirx * (i0 + nvx - 1);
   const int ya = sy + g.diry * j0, yb = sy + g.diry * (j0 + nvy - 1);
@@ -455,7 +460,7 @@ struct TilePre {
   int sumfree;
 };
 
-template <bool WIN = false>
+template <bool CLIP = false>
 __device__ __forceinline__ TilePre tile_prefetch(const TileArgs &p, const TQuad &g,
                                                  const uint32_t *__restrict__ rowpl,
                                                  const uint32_t *__restrict__ colpl,
@@ -467,9 +472,9 @@ __device__ __forceinline__ TilePre tile_prefetch(const TileArgs &p, const TQuad 
   t.sumfree = 0;
   const int wi = I ? kTile : g.a, wj = J ? kTile : g.a;
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
-  const int nvx = min(wi, ext_cx<WIN>(g, sx) - i0 + 1), nvy = min(wj, ext_cy<WIN>(g, sy) - j0 + 1);
+  const int nvx = min(wi, ext_cx<CLIP>(g, sx) - i0 + 1), nvy = min(wj, ext_cy<CLIP>(g, sy) - j0 + 1);
   if (nvx > 0 && nvy > 0) {
-    t.sumfree = tile_sum_free<WIN>(g, bsum, WIN ? p.w_sw : tile_sum_words(p.nx), sx, sy, I, J);
+    t.sumfree = tile_sum_free<CLIP>(g, bsum, CLIP ? p.w_sw : tile_sum_words(p.nx), sx, sy, I, J);
     if (!t.sumfree) {
       if (lane < nvy) { // row j0 + lane, bit b <-> local column i0 + b
         const uint32_t *rp =
@@ -518,7 +523,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   // before the global stores
   constexpr int kStepUnroll = NW == 1 ? VHP_STEP_UNROLL_1W : VHP_STEP_UNROLL;
   constexpr bool BITS = FMT == kFmtBits;
-  constexpr bool MERGE = FMT == kFmtMerge64 || FMT == kFmtMerge32;
+  constexpr bool MERGE = fmt_merge(FMT);
   static_assert(!BITS || sizeof(OutT) == 4, "bit output: OutT is the 32-bit word");
   static_assert(!MERGE || (sizeof(OutT) == 8 && !GE), "merge output: fp64 staging, one-CTA sweeps");
   auto publish = [&]() {
@@ -540,13 +545,13 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
       if (lane == 0) atomicMax_system(xflag, I + 1);
     }
   };
-  constexpr bool WIN = FMT == kFmtWindow;
-  const int nx = WIN ? 2 * p.w_r + 1 : p.nx; // row pitch of `out`
+  constexpr bool WIN = FMT == kFmtWindow, CLIP = fmt_clip(FMT);
+  const int nx = WIN ? 2 * p.w_r + 1 : p.nx; // row pitch of `out` (kFmtMergeRange*: the map's)
   const int wi = I ? kTile : g.a, wj = J ? kTile : g.a;          // tile extent
   const int i0 = tile_start(g.a, I), j0 = tile_start(g.a, J);
   const int il = i0 + lane, jr = j0 + lane;
   // the never-written border column / row is "occupied": exclude it from the compute extent
-  const int ExC = ext_cx<WIN>(g, sx), EyC = ext_cy<WIN>(g, sy);
+  const int ExC = ext_cx<CLIP>(g, sx), EyC = ext_cy<CLIP>(g, sy);
   const int nvx = min(wi, ExC - i0 + 1), nvy = min(wj, EyC - j0 + 1); // columns / rows to compute
   const uint32_t cmask = nvx >= 32 ? ~0u : (nvx <= 0 ? 0u : (1u << nvx) - 1u);
   const uint32_t rmask = nvy >= 32 ? ~0u : (nvy <= 0 ? 0u : (1u << nvy) - 1u);
@@ -620,7 +625,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
     if constexpr (MERGE) { // the border row (if any) is 0: nothing to fold
       if (!zero && cor > 0.0 && lane_st && colc) {
         const ptrdiff_t i0c = ptr - out;
-        for (int r = r0; r <= rc; ++r) merge_cell<FMT>(p, i0c + r * rs, cor);
+        for (int r = r0; r <= rc; ++r) merge_cell<FMT>(p, i0c + r * rs, il, j0 + r, cor);
       }
       return;
     }
@@ -717,7 +722,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
             const uint32_t m = __ballot_sync(kAll, ge_thr(F));
             if (lane == s) wb = m;
           } else if constexpr (MERGE) {
-            if (!decltype(masked)::value || (lane_st && s >= r0 && s <= rlast)) merge_cell<FMT>(p, q - out, F);
+            if (!decltype(masked)::value || (lane_st && s >= r0 && s <= rlast)) merge_cell<FMT>(p, q - out, il, j0 + s, F);
           } else if (!decltype(masked)::value || (lane_st && s >= r0 && s <= rlast)) {
             __stcs(q, to_out<OutT>(F));
           }
@@ -786,7 +791,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   } else if constexpr (MERGE) {
     if (lane_st) {
       const ptrdiff_t i0c = ptr - out;
-      for (int r = r0; r <= rlast; ++r) merge_cell<FMT>(p, i0c + r * rs, stage[stage_at(r, lane)]);
+      for (int r = r0; r <= rlast; ++r) merge_cell<FMT>(p, i0c + r * rs, il, j0 + r, stage[stage_at(r, lane)]);
     }
   } else if (lane_st) {
     OutT *q = ptr + r0 * rs;
@@ -800,7 +805,8 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
 // Ends with a block barrier.
 //
 // kFmtWindow: every cell of the (2R+1)^2 window exactly once instead (out: see kFmtWindow),
-// smem_raw: tile_smem_bytes_win<OutT>(nx, ny, R, NW) bytes.
+// smem_raw: tile_smem_bytes_win<OutT>(nx, ny, R, NW) bytes.  kFmtMergeRange*: the cells of the box |dx|, |dy| <= R
+// once each, in map pitch, smem_raw sized like kFmtWindow.
 //
 // Grid mode (MODE != kSweepCta; one sweep of a giant map by many CTAs): kSweepGridInit, run by
 // one CTA, computes the staircase and writes it with the boundary rows, the progress flags and
@@ -814,9 +820,9 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
                                                unsigned char *smem_raw) {
   constexpr bool GE = MODE != kSweepCta;
   constexpr bool BITS = FMT == kFmtBits;
-  constexpr bool WIN = FMT == kFmtWindow;
+  constexpr bool WIN = FMT == kFmtWindow, CLIP = fmt_clip(FMT);
   static_assert(!GE || NW > 1, "grid mode uses the multi-warp boundary layout");
-  static_assert(!GE || !WIN, "window output is a one-CTA sweep");
+  static_assert(!GE || !CLIP, "clipped sweeps are one-CTA sweeps");
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nx = p.nx, ny = p.ny;
   const int opitch = WIN ? 2 * p.w_r + 1 : nx; // row pitch of `out`
@@ -826,13 +832,13 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
   static_assert(4 * sizeof(TQuad) <= kMergeHdr, "quadrant geometry overlaps the merge slot / row counter");
   uint32_t *bsum = reinterpret_cast<uint32_t *>(smem_raw + kTileHdr);
   const int nsum = tile_sum_words(nx) * ((ny + 31) >> 5);
-  const int sum_bytes = WIN ? win_sum_bytes(nx, ny, p.w_r) : tile_sum_bytes(nx, ny);
-  const int lmcap = tile_lm_cap(WIN ? win_side(ny, p.w_r) : ny);
+  const int sum_bytes = CLIP ? win_sum_bytes(nx, ny, p.w_r) : tile_sum_bytes(nx, ny);
+  const int lmcap = tile_lm_cap(CLIP ? win_side(ny, p.w_r) : ny);
   int *Lm = reinterpret_cast<int *>(smem_raw + kTileHdr + sum_bytes);
   int *prog = GE ? p.g_prog : Lm + 4 * lmcap; // tiles finished (or lit) at the head of tile row (q, J)
   double *const edges_s = reinterpret_cast<double *>(smem_raw + kTileHdr + sum_bytes + 32 * lmcap);
   double *edges = GE ? p.g_edges : edges_s;
-  const int nedge = tile_edge_doubles(WIN ? win_side(nx, p.w_r) : nx, NW);
+  const int nedge = tile_edge_doubles(CLIP ? win_side(nx, p.w_r) : nx, NW);
   unsigned char *wbase = reinterpret_cast<unsigned char *>(GE ? edges_s : edges_s + nedge);
   double *wscr = reinterpret_cast<double *>(wbase) + warp * kWarpScratch;
   OutT *stage = reinterpret_cast<OutT *>(wbase + NW * kWarpScratch * sizeof(double)) +
@@ -848,7 +854,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       g.diry = (q < 2) ? 1 : -1;
       g.Ex = g.dirx > 0 ? nx - 1 - sx : sx;
       g.Ey = g.diry > 0 ? ny - 1 - sy : sy;
-      if (WIN) {
+      if (CLIP) {
         g.Ex = min(g.Ex, p.w_r);
         g.Ey = min(g.Ey, p.w_r);
       }
@@ -880,10 +886,10 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       }
     }
   }
-  // bsq: the summary addressed by absolute block row and word (a window copies only the words it touches,
-  // rows of p.w_sw words)
+  // bsq: the summary addressed by absolute block row and word (a clipped sweep copies only the words its box
+  // touches, rows of p.w_sw words)
   const uint32_t *bsq = bsum;
-  if constexpr (WIN) {
+  if constexpr (CLIP) {
     const int R = p.w_r, nbw = tile_sum_words(nx), sw = p.w_sw;
     const int wlo = (max(sx - R, 0) >> 5) >> 5, whi = (min(sx + R, nx - 1) >> 5) >> 5;
     const int blo = max(sy - R, 0) >> 5, bhi = min(sy + R, ny - 1) >> 5;
@@ -894,18 +900,20 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       bsum[r * sw + c] = __ldg(src + (size_t)r * nbw + c);
     }
     bsq = bsum - (blo * sw + wlo);
-    // window cells outside the grid are 0: the rows above / below it, then the columns left / right of it
-    const int W = 2 * R + 1, x0 = sx - R, y0 = sy - R;
-    const int ul = max(0, -x0), uh = min(W - 1, nx - 1 - x0), vl = max(0, -y0), vh = min(W - 1, ny - 1 - y0);
-    OutT *const wout = out + (ptrdiff_t)y0 * W + x0;
-    const OutT z = to_out<OutT>(0.0);
-    for (int v = warp; v < W; v += NW) {
-      OutT *const row = wout + (ptrdiff_t)v * W;
-      if (v < vl || v > vh) {
-        fill_run<OutT>(row, W, z, lane);
-      } else {
-        if (ul > 0) fill_run<OutT>(row, ul, z, lane);
-        if (uh < W - 1) fill_run<OutT>(row + uh + 1, W - 1 - uh, z, lane);
+    if constexpr (WIN) {
+      // window cells outside the grid are 0: the rows above / below it, then the columns left / right of it
+      const int W = 2 * R + 1, x0 = sx - R, y0 = sy - R;
+      const int ul = max(0, -x0), uh = min(W - 1, nx - 1 - x0), vl = max(0, -y0), vh = min(W - 1, ny - 1 - y0);
+      OutT *const wout = out + (ptrdiff_t)y0 * W + x0;
+      const OutT z = to_out<OutT>(0.0);
+      for (int v = warp; v < W; v += NW) {
+        OutT *const row = wout + (ptrdiff_t)v * W;
+        if (v < vl || v > vh) {
+          fill_run<OutT>(row, W, z, lane);
+        } else {
+          if (ul > 0) fill_run<OutT>(row, ul, z, lane);
+          if (uh < W - 1) fill_run<OutT>(row + uh + 1, W - 1 - uh, z, lane);
+        }
       }
     }
   } else {
@@ -920,14 +928,14 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
   }
 
   // ---- lit staircase: leading free tiles per tile row, then the running minimum ---------
-  const int nbw = WIN ? p.w_sw : tile_sum_words(nx);
+  const int nbw = CLIP ? p.w_sw : tile_sum_words(nx);
   if (MODE != kSweepGridWork) {
   for (int q = 0; q < 4; ++q) {
     const TQuad &g = quads[q];
     for (int J = warp; J < g.TY; J += NW) {
       int L = 0;
       for (int Ib = 0; Ib < g.TX; Ib += 32) {
-        const bool fr = Ib + lane < g.TX && tile_sum_free<WIN>(g, bsq, nbw, sx, sy, Ib + lane, J);
+        const bool fr = Ib + lane < g.TX && tile_sum_free<CLIP>(g, bsq, nbw, sx, sy, Ib + lane, J);
         const unsigned m = __ballot_sync(kAll, fr);
         const int run = __ffs(~m) - 1; // leading ones (-1: all 32)
         L += run < 0 ? 32 : run;
@@ -1051,7 +1059,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
           j = jn;
         }
       }
-    } else if constexpr (FMT == kFmtMerge64 || FMT == kFmtMerge32) {
+    } else if constexpr (fmt_merge(FMT)) {
       // merge output: the lit spans of the value loop below, folded cell by cell (value 1.0); the never-written
       // cells of those rows (x == 0 left of the source, row 0 below it) hold 0 and are left alone
       static_assert(!GE, "merge output is a one-CTA sweep");
@@ -1064,7 +1072,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
         if (nR == 0 && nL <= 1) continue;
         const int xl = nL > 1 ? max(sx - (nL - 1), 1) : sx; // first lit column
         const int xr = nR > 0 ? sx + nR - 1 : sx - 1;       // last lit column
-        for (int x = xl + lane; x <= xr; x += 32) merge_cell<FMT>(p, (ptrdiff_t)y * nx + x, 1.0);
+        for (int x = xl + lane; x <= xr; x += 32) merge_cell<FMT>(p, (ptrdiff_t)y * nx + x, abs(x - sx), j, 1.0);
       }
     } else
     for (int y = max(ylo, p.win_y0) + wfirst; y <= min(yhi, p.win_y1 - 1); y += wstride) {
@@ -1104,11 +1112,11 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
     double Lv = 1.0, cor = 1.0; // left of the first tile: lit tiles or the virtual boundary
     int *xflag = nullptr; // grid mode across GPUs: the neighbour's flag of this row, if it is the exported one
     if (GE && reinterpret_cast<const short *>(smem_raw + 244)[q] == J) xflag = p.x_prog + q * lmcap + J;
-    TilePre pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, I0, J, lane);
+    TilePre pre = tile_prefetch<CLIP>(p, g, rowpl, colpl, bsq, sx, sy, I0, J, lane);
 #if VHP_DARK_TAIL
     // rows of this tile row that hold cells to compute (lane <-> row j0 + lane), as in process_tile
     const int j0row = tile_start(g.a, J);
-    const int nvyrow = min(J ? kTile : g.a, ext_cy<WIN>(g, sy) - j0row + 1);
+    const int nvyrow = min(J ? kTile : g.a, ext_cy<CLIP>(g, sy) - j0row + 1);
     const bool rowc_row = lane < nvyrow;
     int dark_seen = -1; // a boundary column >= the tile start known to be non-zero (finished row below)
 #endif
@@ -1125,7 +1133,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
         const int Iend = min(ld_acquire_shared(prog + q * lmcap + J - 1), g.TX); // finished below
         if (Iend > I) {
           const int i0 = tile_start(g.a, I);
-          const int ilim = min(ext_cx<WIN>(g, sx), tile_start(g.a, Iend) - 1);
+          const int ilim = min(ext_cx<CLIP>(g, sx), tile_start(g.a, Iend) - 1);
           const double *rowB = edges + g.rowOff;
           int bad = -1;
           for (int ib = i0; ib <= ilim && bad < 0; ib += 32) {
@@ -1152,7 +1160,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
                 fill_run<OutT>(out + (ptrdiff_t)(sy + g.diry * (j0row + r)) * opitch + xa, xb - xa + 1,
                                to_out<OutT>(0.0), lane);
             if (Istop >= g.TX) return;
-            pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, Istop, J, lane);
+            pre = tile_prefetch<CLIP>(p, g, rowpl, colpl, bsq, sx, sy, Istop, J, lane);
             I = Istop - 1;
             continue;
           }
@@ -1160,7 +1168,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       }
 #endif
       const TilePre cur = pre;
-      if (I + 1 < g.TX) pre = tile_prefetch<WIN>(p, g, rowpl, colpl, bsq, sx, sy, I + 1, J, lane);
+      if (I + 1 < g.TX) pre = tile_prefetch<CLIP>(p, g, rowpl, colpl, bsq, sx, sy, I + 1, J, lane);
       if (GE && J > 0 && ((p.remote_mask >> q) & 1) && J == g.Jlo) {
         // the row below lives on the neighbouring GPU: its flag arrives over NVLink.  A watchdog
         // (a few seconds) turns a lost neighbour into an error instead of a hung GPU.

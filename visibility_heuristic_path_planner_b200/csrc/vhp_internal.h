@@ -108,6 +108,9 @@ struct vhp_context {
   // workspace buffers (grown on demand, reused across calls)
   VhpDevBuf b_occ, b_src, b_map, b_out[2], b_scratch, b_planner, b_misc, b_grid, b_bin;
   VhpDevBuf b_merge; // vhp_visibility_merge_batch: per-pair table; host call: group layout too
+  // vhp_visibility_merge_range_batch, fallback: the fp64 windows of a chunk of pairs (apart from b_bin and b_misc,
+  // which the window routes use themselves)
+  VhpDevBuf b_mwin;
   cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
   // 1/k table {rh, rl} of the tile kernel (double-double reciprocal), device resident
   double *rcp2_table = nullptr;
@@ -225,11 +228,18 @@ struct VhpMergeDev {
   const int32_t *pair_k = nullptr;     // index of the pair within its group
   const int32_t *pair_map = nullptr;   // map of the pair (its group's)
 };
+// range of vhp_visibility_merge_range_batch: 0 <= radius <= 16383, shape VHP_RANGE_BOX / VHP_RANGE_DISK
+struct VhpMergeRange {
+  int radius = 0;
+  int shape = VHP_RANGE_BOX;
+};
 // the sweeps fold straight into the group outputs (kFmtMerge*, one CTA per pair); needs thr > 0 and zero-filled
-// vmax / count, -1-filled first
+// vmax / count, -1-filled first.  range: sweep only each pair's box and fold only its cells in range
+// (kFmtMergeRange*; supported where vhp_sweep_window_supported holds)
 cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
                                    const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,
-                                   int *d_err, cudaStream_t st, int64_t *launches);
+                                   int *d_err, cudaStream_t st, int64_t *launches,
+                                   const VhpMergeRange *range = nullptr);
 // kernels_merge.cu: the per-pair table (validates the layout: bit 4 of d_err), the output fill, and the fold of
 // np fp64 fields of pairs [p0, p0 + np) (what the fallback sweeps into a chunk buffer) into the group outputs
 cudaError_t vhp_launch_merge_table(const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t ngroups,
@@ -240,6 +250,11 @@ cudaError_t vhp_launch_merge_fill(const VhpMergeDev &m, size_t cells_total, cuda
 cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np, int nx, int ny,
                                   const int32_t *d_src_xy, double thr, const VhpMergeDev &m, int sm_count,
                                   cudaStream_t st, int64_t *launches);
+// the fold of np fp64 windows d_win[np][2R+1][2R+1] of pairs [p0, p0 + np) (vhp_visibility_window_batch's layout)
+// into the group outputs, cells in range only (relaxed red atomics: any order gives the same result)
+cudaError_t vhp_launch_merge_window_fold(const double *d_win, int64_t p0, int64_t np, int nx, int ny,
+                                         const int32_t *d_src_xy, double thr, const VhpMergeRange &range,
+                                         const VhpMergeDev &m, int sm_count, cudaStream_t st, int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
