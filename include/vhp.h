@@ -228,6 +228,55 @@ vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t 
                                                 int32_t radius, int32_t shape, double threshold,
                                                 vhp_dtype dtype, const vhp_merge_out *d_out);
 
+/* Greedy sensor placement: which k of a set of candidate positions cover the most cells together.  nprob
+ * independent problems in the CSR layout of vhp_visibility_merge_batch: problem q has the candidates
+ * [group_ptr[q], group_ptr[q+1]) of cand_xy on map group_map[q] (NULL -> map 0); radius R, shape and threshold as in
+ * vhp_visibility_merge_range_batch.
+ *   S(c)  the cells where candidate c would add 1 to vhp_visibility_merge_range_batch's count: in range, not on c's
+ *         never-written border, fp64 value of vhp_visibility_batch's field >= threshold
+ *   T_q   the cells whose bit is set in target ([prob][ny][ceil(nx/32)] uint32, the layout of
+ *         vhp_visibility_batch_bin; bits beyond nx are ignored); NULL: every cell.  "Add k sensors to those already
+ *         placed" is the complement of their coverage as the target.
+ * Greedy, U = {} and for r = 0 .. k-1: gain(c) = |S(c) & T_q \ U| for every candidate of the problem; p = argmax,
+ * ties to the smallest index within the group; if gain(p) == 0 stop (npicked = r), else U |= S(p).  Duplicates are
+ * separate entries.  Every decision is an integer comparison, so the result is exact.  Outputs (any may be NULL, at
+ * least one must be given):
+ *   pick[q][r]     index within the group of the r-th pick, -1 from npicked on            (int32 [prob][k])
+ *   gain[q][r]     cells the r-th pick newly covers, 0 from npicked on; non-increasing    (uint32 [prob][k])
+ *   npicked[q]                                                                            (int32 [prob])
+ *   covered[q]     U after the last pick, every cell of the union (in the target or not), bits beyond nx 0
+ *                  ([prob][ny][ceil(nx/32)] uint32) = count > 0 of vhp_visibility_merge_range_batch on the picks
+ * so sum of gain = |U & T|.  Within (1 - 1/e) of the best k-subset.
+ * Routes.  Phase 1 stores each candidate's S(c) as bits over its box clipped to the grid: min(2R+1, ny) rows and
+ * min(ceil(nx/32), (2R+31)/32 + 1) words aligned to the map's 32-column words.  Where threshold > 0 and the box fits one
+ * CTA of the batched tile kernel, the sweep of each box writes those bits itself; otherwise (threshold <= 0, the naive
+ * kernel, grid mode 2, boxes too large) chunks of fp64 windows, or whole fields where a window would be larger than the
+ * map, are thresholded into them.  Phase 2 runs min(k, nsrc) rounds of two kernels each on the device with no host
+ * synchronisation: one takes every problem's pick, one updates exactly the gains of the candidates whose box meets it.
+ * Workspace (device, grown on demand and kept by the context): 4 * nsrc * rows * words bytes of candidate bits, plus
+ * 4 * ny * ceil(nx/32) + 4 * rows * words bytes per problem; the host form runs problems in batches that fit 4 GB
+ * (at least one problem).  A failed allocation returns VHP_ERR_CUDA and names the bytes.
+ * Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_merge_range_batch (radius outside [0, 16383], an unknown
+ * shape, a NaN threshold, a candidate outside the grid, a bad group layout, group_map out of range), k < 0, no
+ * output.  k == 0 is valid (npicked 0, covered all zero).  The _dev form takes nsrc = group_ptr[nprob] and reports a
+ * bad candidate or group layout like vhp_visibility_merge_batch_dev, by the next synchronising call. */
+typedef struct vhp_cover_out {
+  int32_t *pick;
+  uint32_t *gain;
+  int32_t *npicked;
+  uint32_t *covered;
+} vhp_cover_out;
+vhp_status vhp_visibility_cover_greedy_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                             const int32_t *cand_xy, const int64_t *group_ptr,
+                                             const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
+                                             int32_t shape, double threshold, const uint32_t *target,
+                                             const vhp_cover_out *out);
+vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                 const int32_t *d_cand_xy, const int64_t *d_group_ptr,
+                                                 const int32_t *d_group_map, int64_t nprob, int64_t nsrc, int32_t k,
+                                                 int32_t radius, int32_t shape, double threshold,
+                                                 const uint32_t *d_target, const vhp_cover_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

@@ -48,6 +48,12 @@ class MergeOut(C.Structure):
     _fields_ = [("vmax", C.c_void_p), ("first", C.c_void_p), ("count", C.c_void_p)]
 
 
+class CoverOut(C.Structure):
+    """struct vhp_cover_out: pick (int32 [prob][k]), gain (uint32 [prob][k]), npicked (int32 [prob]), covered
+    (uint32 [prob][ny][ceil(nx/32)]), each may be NULL."""
+    _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("covered", C.c_void_p)]
+
+
 class SweepVariant(C.Structure):
     """struct vhp_sweep_variant: model 1 = getAccessibilityMap.m (alpha, fac, light_strength),
     model 2 = computeVisibilityUsingQueue as an order-free rule (cutoff)."""
@@ -120,6 +126,10 @@ def load_library(build_if_missing: bool = True):
                                                      C.c_double, i32, C.POINTER(MergeOut)]
     lib.vhp_visibility_merge_range_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_int32,
                                                          C.c_int32, C.c_double, i32, C.POINTER(MergeOut)]
+    lib.vhp_visibility_cover_greedy_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, C.c_int32, C.c_int32,
+                                                      C.c_int32, C.c_double, vp, C.POINTER(CoverOut)]
+    lib.vhp_visibility_cover_greedy_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_int32,
+                                                          C.c_int32, C.c_int32, C.c_double, vp, C.POINTER(CoverOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -440,6 +450,47 @@ class Context:
         self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), group_ptr_t.data_ptr(),
                        ptr(group_map_t), ng, src_xy_t.shape[0], *extra, float(threshold), dtype, C.byref(mo)))
 
+    def visibility_cover_greedy_batch(self, occ, cand_xy, group_ptr, k, threshold, radius, shape, group_map=None,
+                                      target=None):
+        """Greedy sensor placement (vhp_visibility_cover_greedy_batch): per problem q (candidates
+        cand_xy[group_ptr[q]:group_ptr[q + 1]] on map group_map[q]) the k candidates, picked one by one, that each add
+        the most cells to what the earlier picks cover, within the candidate's range (radius, shape as
+        visibility_merge_range_batch) at fp64 value >= threshold.  target: bool (nprob, ny, nx), the cells that count
+        (None: all).  Returns pick (int32 (nprob, k), index within the group, -1 after the last pick), gain (uint32
+        (nprob, k), cells newly covered), npicked (int32 (nprob,)) and covered (uint32 (nprob, ny, ceil(nx/32)), the
+        bits of the union, see unpack_bits)."""
+        occ = _occ_u8(occ)
+        nmaps, ny, nx = occ.shape
+        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        npb = gp.shape[0] - 1
+        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
+        tb = None if target is None else pack_bits(np.asarray(target, bool).reshape(max(npb, 0), ny, nx))
+        k = int(k)
+        n = max(npb, 0)
+        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint32),
+                 npicked=np.empty(n, np.int32), covered=np.empty((n, ny, (nx + 31) // 32), np.uint32))
+        co = CoverOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "covered")])
+        self._check(self.lib.vhp_visibility_cover_greedy_batch(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy),
+                                                                _np_ptr(gp), _np_ptr(gm), npb, k, int(radius),
+                                                                int(shape), float(threshold), _np_ptr(tb),
+                                                                C.byref(co)))
+        return r
+
+    def visibility_cover_greedy_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape,
+                                          pick_t=None, gain_t=None, npicked_t=None, covered_t=None, group_map_t=None,
+                                          target_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2),
+        group_ptr_t int64 (nprob + 1), target_t int32 (nprob, ny, ceil(nx/32)) packed bits or None; outputs pick_t,
+        gain_t int32 (nprob, k), npicked_t int32 (nprob,), covered_t int32 (nprob, ny, ceil(nx/32)); any may be None."""
+        nmaps, ny, nx = occ_t.shape
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        co = CoverOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(covered_t))
+        self._check(self.lib.vhp_visibility_cover_greedy_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
+            group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
+            ptr(target_t), C.byref(co)))
+
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):
         """Opt-in sweep variants (vhp_visibility_variant_batch): VARIANT_MATLAB =
@@ -545,6 +596,16 @@ def unpack_bits(bits, nx):
     """uint32 (..., ceil(nx/32)) bit-packed rows -> bool (..., nx)."""
     b = np.ascontiguousarray(bits).view(np.uint8)
     return np.unpackbits(b, axis=-1, bitorder="little")[..., :nx].astype(bool)
+
+
+def pack_bits(cells):
+    """bool (..., nx) -> uint32 (..., ceil(nx/32)) bit-packed rows (bit x & 31 of word x >> 5), the inverse of
+    unpack_bits."""
+    cells = np.asarray(cells, bool)
+    nx = cells.shape[-1]
+    pad = np.zeros(cells.shape[:-1] + (32 * ((nx + 31) // 32),), bool)
+    pad[..., :nx] = cells
+    return np.ascontiguousarray(np.packbits(pad, axis=-1, bitorder="little")).view("<u4")
 
 
 def torch_context(device: int, stream) -> Context:

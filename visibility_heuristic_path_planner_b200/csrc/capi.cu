@@ -958,6 +958,14 @@ const char *merge_name(const VhpMergeRange *range) {
   return range ? "vhp_visibility_merge_range_batch" : "vhp_visibility_merge_batch";
 }
 
+vhp_status check_range(vhp_context *ctx, const std::string &what, const VhpMergeRange &range) {
+  if (range.radius < 0 || range.radius > 16383)
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": radius outside [0, 16383]");
+  if (range.shape != VHP_RANGE_BOX && range.shape != VHP_RANGE_DISK)
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": shape is neither VHP_RANGE_BOX nor VHP_RANGE_DISK");
+  return VHP_OK;
+}
+
 vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t ngroups, int64_t nsrc, double thr, int dtype,
                             const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
@@ -971,11 +979,7 @@ vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx
   if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
   if (!out->vmax && !out->first && !out->count)
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
-  if (range && (range->radius < 0 || range->radius > 16383))
-    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": radius outside [0, 16383]");
-  if (range && range->shape != VHP_RANGE_BOX && range->shape != VHP_RANGE_DISK)
-    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": shape is neither VHP_RANGE_BOX nor VHP_RANGE_DISK");
-  return VHP_OK;
+  return range ? check_range(ctx, what, *range) : VHP_OK;
 }
 
 VhpMergeDev merge_dev_of(const vhp_merge_out &o, vhp_dtype dtype) {
@@ -1045,6 +1049,19 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
   return VHP_OK;
 }
 
+// host-side validation of a CSR group layout
+vhp_status check_groups_host(vhp_context *ctx, const std::string &what, const int64_t *gptr, int64_t ngroups) {
+  if (!ctx || !gptr || ngroups < 0) return VHP_OK; // (the argument checks report these)
+  if (gptr[0] != 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": group_ptr[0] must be 0");
+  for (int64_t g = 0; g < ngroups; ++g) {
+    if (gptr[g + 1] < gptr[g])
+      return fail(ctx, VHP_ERR_INVALID_ARG, what + ": group_ptr decreases at group " + std::to_string(g));
+    if (gptr[g + 1] - gptr[g] >= ((int64_t)1 << 31))
+      return fail(ctx, VHP_ERR_INVALID_ARG, what + ": group " + std::to_string(g) + " has 2^31 or more sources");
+  }
+  return VHP_OK;
+}
+
 // host buffers: validate, upload maps and sources once, then runs of whole groups whose outputs fit 1 GB of device
 // memory (at least one group), each copied back with plain cudaMemcpyAsync (the merged result is already K times
 // smaller than the fields it folds)
@@ -1052,18 +1069,10 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
                           const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
                           const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
   const char *what = merge_name(range);
-  if (ctx && gptr && ngroups >= 0) {
-    if (gptr[0] != 0) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(what) + ": group_ptr[0] must be 0");
-    for (int64_t g = 0; g < ngroups; ++g) {
-      if (gptr[g + 1] < gptr[g])
-        return fail(ctx, VHP_ERR_INVALID_ARG, std::string(what) + ": group_ptr decreases at group " + std::to_string(g));
-      if (gptr[g + 1] - gptr[g] >= ((int64_t)1 << 31))
-        return fail(ctx, VHP_ERR_INVALID_ARG,
-                    std::string(what) + ": group " + std::to_string(g) + " has 2^31 or more sources");
-    }
-  }
+  vhp_status st = check_groups_host(ctx, what, gptr, ngroups);
+  if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
-  vhp_status st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range);
+  st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range);
   if (st != VHP_OK) return st;
   if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, what)) != VHP_OK) return st;
   if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, what)) != VHP_OK) return st;
@@ -1110,6 +1119,176 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
     if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: copy of the group outputs"); break; }
     ctx->last_d2h_bytes += (int64_t)(n * (bv + bf + bc));
+  }
+  cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
+  ctx->last_result_bytes = ctx->last_d2h_bytes;
+  if (result != VHP_OK) return result;
+  if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
+  return check_device_error(ctx);
+}
+
+// ---- greedy coverage placement (vhp_visibility_cover_greedy_batch) --------------------------------------
+// Phase 1 stores every candidate's coverage bits over its box (VhpCoverBox): the direct route sweeps the boxes
+// straight into bits (kFmtCoverBits: threshold > 0 and window_direct_route), the fallback folds chunks of fp64
+// windows (run_window_dev, any of its routes) or, where a window would be larger than the map, of whole fields
+// (run_dev) with cover_fold_kernel.  Phase 2 (kernels_cover.cu) runs min(k, nsrc) greedy rounds on the device.
+const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
+
+vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
+                            const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k, const VhpMergeRange &range,
+                            double thr, const vhp_cover_out *out) {
+  const std::string what = kCoverName;
+  if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
+  if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
+  if (nmaps < 1 || nx < 1 || ny < 1 || nprob < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
+  if (nprob > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": more than 2^31 - 1 problems");
+  const vhp_status st = check_grid_dtype(ctx, nx, ny, VHP_F64);
+  if (st != VHP_OK) return st;
+  if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
+  if (k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": k < 0");
+  if (!out->pick && !out->gain && !out->npicked && !out->covered)
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
+  return check_range(ctx, what, range);
+}
+
+VhpCoverDev cover_dev_of(const vhp_cover_out &o) {
+  VhpCoverDev c;
+  c.pick = o.pick;
+  c.gain = o.gain;
+  c.npicked = o.npicked;
+  c.covered = o.covered;
+  return c;
+}
+
+// a workspace buffer of the rounds; a failed allocation names its size
+vhp_status ensure_cover(vhp_context *ctx, VhpDevBuf &b, size_t bytes, const char *what) {
+  if (ensure(ctx, b, bytes) == VHP_OK) return VHP_OK;
+  (void)cudaGetLastError();
+  return fail(ctx, VHP_ERR_CUDA, std::string(kCoverName) + ": " + what + " of " + std::to_string(bytes) +
+                                     " bytes: " + ctx->last_error);
+}
+
+vhp_status run_cover_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                         const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
+                         const VhpMergeRange &range, double thr, const uint32_t *d_target, const VhpCoverDev &out) {
+  const int R = std::min(range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
+  const bool disk = range.shape == VHP_RANGE_DISK;
+  const int r2 = range.radius * range.radius;
+  const int64_t rounds = std::min<int64_t>(k, nsrc);
+  uint32_t *bits = nullptr;
+  int32_t *pg = nullptr, *pk = nullptr;
+  int disk_r2 = -1; // the direct route stores the whole box: the rounds apply the disk
+  vhp_status st;
+  if (nprob > 0 || nsrc > 0) {
+    if ((st = ensure(ctx, ctx->b_merge, 12 * (size_t)std::max<int64_t>(nsrc, 1))) != VHP_OK) return st;
+    pg = (int32_t *)ctx->b_merge.p;
+    pk = pg + nsrc;
+    int32_t *pm = pk + nsrc;
+    VHP_CUDA(ctx, vhp_launch_merge_table(d_gptr, d_gmap, nprob, nsrc, nmaps, pg, pk, pm, ctx->d_err, ctx->sm_count,
+                                         ctx->stream, &ctx->launches));
+    if (rounds > 0 && nprob > 0) {
+      const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
+      if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits")) != VHP_OK)
+        return st;
+      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R), "workspace")) != VHP_OK)
+        return st;
+      bits = (uint32_t *)ctx->b_cover.p;
+      if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
+        if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), R + 1) + 64)) != VHP_OK) return st;
+        if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
+        VHP_CUDA(ctx, vhp_launch_sweep_cover(ctx->tile, nx, ny, d_xy, pm, nsrc, R, thr, bits, ctx->rcp2_table,
+                                             ctx->d_err, ctx->stream, &ctx->launches));
+        if (disk) disk_r2 = r2;
+      } else {
+        // fp64 windows, or whole fields where a window would be larger than the map, up to 1 GB at a time
+        const bool win = (2 * (size_t)R + 1) * (2 * (size_t)R + 1) <= (size_t)nx * ny;
+        const size_t vbytes = win ? window_pair_bytes(R, VHP_F64) : (size_t)nx * ny * 8;
+        const int64_t chunk = std::min<int64_t>(nsrc, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / vbytes)));
+        if ((st = ensure(ctx, ctx->b_mwin, (size_t)chunk * vbytes)) != VHP_OK) return st;
+        for (int64_t p0 = 0; p0 < nsrc; p0 += chunk) {
+          const int64_t np = std::min(chunk, nsrc - p0);
+          st = win ? run_window_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * p0, pm + p0, np, R, VHP_F64, ctx->b_mwin.p)
+                   : run_dev(ctx, Op::Sweep, d_occ, nmaps, nx, ny, d_xy + 2 * p0, pm + p0, np, VHP_F64, ctx->b_mwin.p);
+          if (st != VHP_OK) return st;
+          VHP_CUDA(ctx, vhp_launch_cover_fold((const double *)ctx->b_mwin.p, win ? R : -1, p0, np, nx, ny, R, disk, r2,
+                                              d_xy, thr, bits, ctx->sm_count, ctx->stream, &ctx->launches));
+        }
+      }
+    }
+  }
+  VHP_CUDA(ctx, vhp_launch_cover_greedy(bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, pg, pk, d_target, k,
+                                        ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream, &ctx->launches));
+  return VHP_OK;
+}
+
+// host buffers: validate, upload maps and candidates once, then runs of whole problems whose device memory (candidate
+// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync
+vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
+                          const int64_t *gptr, const int32_t *gmap, int64_t nprob, int32_t k,
+                          const VhpMergeRange &range, double thr, const uint32_t *target, const vhp_cover_out *out) {
+  vhp_status st = check_groups_host(ctx, kCoverName, gptr, nprob);
+  if (st != VHP_OK) return st;
+  const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
+  if ((st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out)) != VHP_OK) return st;
+  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, kCoverName)) != VHP_OK) return st;
+  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, nprob, nmaps, nx, ny, kCoverName)) != VHP_OK) return st;
+  ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
+  ctx->last_transport_packed = 0;
+  if (nprob == 0) return VHP_OK;
+  VHP_ON_DEVICE(ctx);
+  PlanesGuard planes_guard(ctx);
+  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
+    return st;
+  const size_t plane = (size_t)ny * ((nx + 31) / 32);
+  const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(range.radius, std::max(nx, ny) - 1), 0, 0);
+  const size_t box = (size_t)b.H * b.W * 4, budget = (size_t)4 << 30;
+  const size_t bp = out->pick ? 4 * (size_t)k : 0, bg = out->gain ? 4 * (size_t)k : 0, bn = out->npicked ? 4 : 0;
+  const size_t bc = out->covered ? plane * 4 : 0, bt = target ? plane * 4 : 0;
+  // device bytes of problem q: its candidates' bits, state, new, outputs, target
+  auto prob_bytes = [&](int64_t q) {
+    return (size_t)(gptr[q + 1] - gptr[q]) * (box + 16) + plane * 4 + box + bp + bg + bn + bc + bt + 64;
+  };
+  std::vector<int64_t> h_ptr;
+  const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
+  vhp_status result = VHP_OK;
+  for (int64_t q0 = 0, gc = 0; q0 < nprob && result == VHP_OK; q0 += gc) {
+    size_t bytes = prob_bytes(q0);
+    for (gc = 1; q0 + gc < nprob && bytes + prob_bytes(q0 + gc) <= budget; ++gc) bytes += prob_bytes(q0 + gc);
+    const int64_t a = gptr[q0];
+    h_ptr.resize((size_t)gc + 1);
+    for (int64_t i = 0; i <= gc; ++i) h_ptr[(size_t)i] = gptr[q0 + i] - a;
+    if ((result = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + bn + bc) + 256)) != VHP_OK) break;
+    if ((result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gc + 1))) != VHP_OK) break;
+    if (gmap && (result = ensure(ctx, ctx->b_map, 4 * (size_t)gc)) != VHP_OK) break;
+    if (target && (result = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) break;
+    char *base = (char *)ctx->b_out[0].p;
+    VhpCoverDev o;
+    o.pick = out->pick ? (int32_t *)base : nullptr;
+    o.gain = out->gain ? (uint32_t *)(base + gc * bp) : nullptr;
+    o.npicked = out->npicked ? (int32_t *)(base + gc * (bp + bg)) : nullptr;
+    o.covered = out->covered ? (uint32_t *)(base + gc * (bp + bg + bn)) : nullptr;
+    cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
+                                    ctx->stream);
+    if (e == cudaSuccess && gmap)
+      e = cudaMemcpyAsync(ctx->b_map.p, gmap + q0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && target)
+      e = cudaMemcpyAsync(ctx->b_out[1].p, target + (size_t)q0 * plane, (size_t)gc * bt, cudaMemcpyHostToDevice,
+                          ctx->stream);
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: upload of the problems"); break; }
+    result = run_cover_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a, (const int64_t *)ctx->b_misc.p,
+                           gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc, gptr[q0 + gc] - a, k, range, thr,
+                           target ? (const uint32_t *)ctx->b_out[1].p : nullptr, o);
+    if (result != VHP_OK) break;
+    if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->gain)
+      e = cudaMemcpyAsync(out->gain + q0 * k, o.gain, gc * bg, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->npicked)
+      e = cudaMemcpyAsync(out->npicked + q0, o.npicked, gc * bn, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->covered)
+      e = cudaMemcpyAsync(out->covered + q0 * plane, o.covered, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: copy of the outputs"); break; }
+    ctx->last_d2h_bytes += (int64_t)(gc * (bp + bg + bn + bc));
   }
   cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
   ctx->last_result_bytes = ctx->last_d2h_bytes;
@@ -1364,7 +1543,7 @@ void vhp_context_destroy(vhp_context *ctx) {
   if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
   VhpDevBuf *bufs[] = {&ctx->b_occ, &ctx->b_src, &ctx->b_map, &ctx->b_out[0], &ctx->b_out[1],
                        &ctx->b_scratch, &ctx->b_planner, &ctx->b_misc, &ctx->b_grid, &ctx->b_bin,
-                       &ctx->b_merge, &ctx->b_mwin};
+                       &ctx->b_merge, &ctx->b_mwin, &ctx->b_cover, &ctx->b_cover_ws};
   for (VhpDevBuf *b : bufs)
     if (b->p) cudaFree(b->p);
   delete ctx->expand_pool;
@@ -1677,6 +1856,34 @@ vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t 
   VHP_ON_DEVICE(ctx);
   return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
                        merge_dev_of(*d_out, dtype), &range);
+}
+
+vhp_status vhp_visibility_cover_greedy_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                             const int32_t *cand_xy, const int64_t *group_ptr,
+                                             const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
+                                             int32_t shape, double threshold, const uint32_t *target,
+                                             const vhp_cover_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, target,
+                        out);
+}
+
+vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                 const int32_t *d_cand_xy, const int64_t *d_group_ptr,
+                                                 const int32_t *d_group_map, int64_t nprob, int64_t nsrc, int32_t k,
+                                                 int32_t radius, int32_t shape, double threshold,
+                                                 const uint32_t *d_target, const vhp_cover_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  vhp_status st = check_cover_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
+                                   threshold, d_out);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  return run_cover_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
+                       threshold, d_target, cover_dev_of(*d_out));
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

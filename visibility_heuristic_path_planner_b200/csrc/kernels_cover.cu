@@ -1,0 +1,381 @@
+// kernels_cover.cu -- greedy coverage placement (vhp_visibility_cover_greedy_batch): the fallback that turns fp64
+// values into candidate coverage bits, and the greedy rounds over those bits.
+//
+// A candidate's coverage set S(c) is stored as bits over its box (VhpCoverBox, vhp_internal.h).  Per problem q the
+// rounds keep state_q = ~target_q | U (the cells that no longer count) and, per candidate, gain(c) = |S(c) \ state|.
+// A round is two launches and no host synchronisation:
+//   apply  (one CTA per problem): take the argmax of the problem's key slot, record the pick, write
+//          new = S(p) \ state into a per-problem scratch over p's box, OR S(p) into state (and `covered`);
+//   update (32 candidates per CTA): a candidate whose box meets the pick's takes gain -= |S(c) & new| over the
+//          intersection (a warp per such candidate, lanes over rows), then every candidate puts its key into the slot.
+// The key (gain << 32) | ~index makes atomicMax pick the largest gain and, among equal gains, the smallest index
+// within the group.  Every quantity is an integer, so the result does not depend on the order of the atomics.
+#include <algorithm>
+#include <cstdint>
+
+#include "vhp_internal.h"
+
+namespace {
+
+constexpr unsigned kAll = 0xffffffffu;
+constexpr int kCand = 32;  // candidates per CTA of the init / update kernels (lane l of warp 0 <-> candidate l)
+constexpr int kWarps = 8;  // warps per CTA of those kernels
+constexpr int kApplyThreads = 512;
+
+struct CoverGeo {
+  int nx, ny, R, nw; // R: the radius clamped for the geometry; nw = ceil(nx / 32)
+};
+
+// bits lo .. hi of a word (any lo, hi; empty if lo > hi after clamping to [0, 31])
+__device__ __forceinline__ uint32_t span_mask(int lo, int hi) {
+  lo = max(lo, 0);
+  hi = min(hi, 31);
+  return lo > hi ? 0u : ((~0u >> (31 - hi)) & (~0u << lo));
+}
+
+__device__ __forceinline__ int isqrt_floor(int v) {
+  int h = (int)sqrt((double)v);
+  while (h * h > v) --h;
+  while ((h + 1) * (h + 1) <= v) ++h;
+  return h;
+}
+
+__device__ __forceinline__ uint32_t warp_sum(uint32_t v) {
+#pragma unroll
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(kAll, v, o);
+  return v;
+}
+
+// slot[g] = max(slot[g], key) for the valid lanes of a warp: one atomic when they share a problem
+__device__ __forceinline__ void put_keys(const bool valid, const int32_t g, const unsigned long long key,
+                                         unsigned long long *slot) {
+  const unsigned vm = __ballot_sync(kAll, valid);
+  if (!vm) return;
+  const int lead = __ffs(vm) - 1, lane = threadIdx.x & 31;
+  const int32_t g0 = __shfl_sync(kAll, g, lead);
+  if (__all_sync(kAll, !valid || g == g0)) {
+    unsigned long long m = valid ? key : 0ull;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const unsigned long long t = __shfl_xor_sync(kAll, m, o);
+      m = t > m ? t : m;
+    }
+    if (lane == lead) atomicMax(slot + g0, m);
+  } else if (valid) {
+    atomicMax(slot + g, key);
+  }
+}
+
+__device__ __forceinline__ unsigned long long key_of(uint32_t gain, int32_t k) {
+  return ((unsigned long long)gain << 32) | (uint32_t)~k;
+}
+
+// Fallback of phase 1: one thread per box word of pairs [p0, p0 + np).
+__global__ void cover_fold_kernel(const double *__restrict__ val, int win_r, int64_t p0, int64_t np, CoverGeo G,
+                                  bool disk, int r2, const int32_t *__restrict__ xy, double thr,
+                                  uint32_t *__restrict__ bits) {
+  const VhpCoverBox b0 = vhp_cover_box(G.nx, G.ny, G.R, 0, 0);
+  const size_t hw = (size_t)b0.H * b0.W, total = (size_t)np * hw;
+  const int P = 2 * win_r + 1;
+  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total;
+       idx += (size_t)gridDim.x * blockDim.x) {
+    const int64_t j = (int64_t)(idx / hw), q = p0 + j;
+    const int i = (int)(idx - (size_t)j * hw), rr = i / b0.W, w = i - rr * b0.W;
+    const int sx = __ldg(xy + 2 * q), sy = __ldg(xy + 2 * q + 1);
+    uint32_t m = 0;
+    if ((unsigned)sx < (unsigned)G.nx && (unsigned)sy < (unsigned)G.ny) {
+      const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, sx, sy);
+      const int y = b.y0 + rr, dy = y - sy;
+      if (abs(dy) <= G.R) {
+        // row y of the value source: a window centred on the candidate, or the whole field
+        const double *row = win_r >= 0 ? val + (size_t)j * P * P + (ptrdiff_t)(dy + win_r) * P - (sx - win_r)
+                                       : val + (size_t)j * G.nx * G.ny + (size_t)y * G.nx;
+        const bool row_writes = !(y == 0 && sy != 0);
+        for (int bit = 0; bit < 32; ++bit) {
+          const int x = 32 * (b.w0 + w) + bit, dx = x - sx;
+          if (x >= G.nx || abs(dx) > G.R || (disk && dx * dx + dy * dy > r2)) continue;
+          if (row_writes && !(x == 0 && sx != 0) && __ldg(row + x) >= thr) m |= 1u << bit;
+        }
+      }
+    }
+    bits[(size_t)q * hw + i] = m;
+  }
+}
+
+__global__ void cover_state_kernel(const uint32_t *__restrict__ target, size_t n, uint32_t *__restrict__ state) {
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    state[i] = ~__ldg(target + i);
+}
+
+// gain(c) = |S(c) \ state| of 32 candidates per CTA (a warp per candidate, lanes over rows); disk_r2 >= 0: the disk
+// mask dx^2 + dy^2 <= disk_r2 is applied to the bits in place first.  Then the keys of round 0, and first[q] = the
+// problem's candidate of index 0 (the rounds read no group_ptr: the host form's copy of it may be gone by then).
+__global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__restrict__ bits, int64_t nsrc, CoverGeo G,
+                                                                 int disk_r2, const int32_t *__restrict__ xy,
+                                                                 const int32_t *__restrict__ pg,
+                                                                 const int32_t *__restrict__ pk,
+                                                                 const uint32_t *__restrict__ state,
+                                                                 uint32_t *__restrict__ gain,
+                                                                 unsigned long long *slot, int64_t *first) {
+  __shared__ uint32_t sg[kCand];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t base = blockIdx.x * (int64_t)kCand;
+  const VhpCoverBox b0 = vhp_cover_box(G.nx, G.ny, G.R, 0, 0);
+  const size_t hw = (size_t)b0.H * b0.W;
+  for (int j = warp; j < kCand; j += kWarps) {
+    const int64_t c = base + j;
+    uint32_t acc = 0;
+    const int32_t g = c < nsrc ? __ldg(pg + c) : -1;
+    if (g >= 0) {
+      const int sx = __ldg(xy + 2 * c), sy = __ldg(xy + 2 * c + 1);
+      const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, sx, sy);
+      uint32_t *bc = bits + (size_t)c * hw;
+      const uint32_t *sq = state + (size_t)g * G.ny * G.nw;
+      for (int r = lane; r < b.H; r += 32) {
+        const int y = b.y0 + r;
+        int xa = 0, xb = -1; // the disk's columns on row y
+        if (disk_r2 >= 0) {
+          const int v = disk_r2 - (y - sy) * (y - sy);
+          if (v >= 0) {
+            const int h = isqrt_floor(v);
+            xa = sx - h;
+            xb = sx + h;
+          }
+        }
+        uint32_t *row = bc + (size_t)r * b.W;
+        const uint32_t *srow = sq + (size_t)y * G.nw + b.w0;
+        for (int w = 0; w < b.W; ++w) {
+          uint32_t m = row[w];
+          if (disk_r2 >= 0 && m) {
+            const int x0 = 32 * (b.w0 + w);
+            const uint32_t mm = m & span_mask(xa - x0, xb - x0);
+            if (mm != m) row[w] = mm;
+            m = mm;
+          }
+          if (m) acc += __popc(m & ~__ldg(srow + w));
+        }
+      }
+      acc = warp_sum(acc);
+    }
+    if (lane == 0) sg[j] = acc;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    const int64_t c = base + lane;
+    const int32_t g = c < nsrc ? __ldg(pg + c) : -1;
+    const uint32_t gn = sg[lane];
+    const int32_t kc = g >= 0 ? __ldg(pk + c) : -1;
+    if (c < nsrc) gain[c] = gn;
+    if (kc == 0) first[g] = c;
+    put_keys(g >= 0, g, key_of(gn, kc), slot);
+  }
+}
+
+// Round r, one CTA per problem: take the slot's pick (gain 0 or a finished problem: done), record it, and update the
+// problem's state over the pick's box.
+__global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32_t *__restrict__ bits,
+                                                                    const int64_t *__restrict__ first, int64_t nsrc,
+                                                                    CoverGeo G,
+                                                                    const int32_t *__restrict__ xy, int32_t r,
+                                                                    int32_t k, unsigned long long *slot, int64_t *cur,
+                                                                    int *done, uint32_t *__restrict__ state,
+                                                                    uint32_t *__restrict__ newb, VhpCoverDev out) {
+  const int64_t q = blockIdx.x;
+  if (done[q]) return;
+  const unsigned long long key = slot[q];
+  __syncthreads(); // every thread has read the slot before thread 0 resets it
+  const uint32_t gn = (uint32_t)(key >> 32), idx = ~(uint32_t)key;
+  const int64_t c = first[q] + idx;
+  if (gn == 0 || first[q] < 0 || c >= nsrc) { // (the last two: an inconsistent group layout, reported by the table)
+    if (threadIdx.x == 0) done[q] = 1;
+    return;
+  }
+  if (threadIdx.x == 0) {
+    if (out.pick) out.pick[q * k + r] = (int32_t)idx;
+    if (out.gain) out.gain[q * k + r] = gn;
+    if (out.npicked) out.npicked[q] = r + 1;
+    cur[q] = c;
+    slot[q] = 0;
+  }
+  const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, __ldg(xy + 2 * c), __ldg(xy + 2 * c + 1));
+  const int hw = b.H * b.W;
+  const uint32_t *bc = bits + (size_t)c * hw;
+  const size_t plane = (size_t)G.ny * G.nw;
+  uint32_t *sq = state + (size_t)q * plane, *nq = newb + (size_t)q * hw;
+  uint32_t *cov = out.covered ? out.covered + (size_t)q * plane : nullptr;
+  for (int i = threadIdx.x; i < hw; i += blockDim.x) {
+    const int rr = i / b.W, w = i - rr * b.W;
+    const size_t o = (size_t)(b.y0 + rr) * G.nw + b.w0 + w;
+    const uint32_t m = __ldg(bc + i), s = sq[o];
+    nq[i] = m & ~s;
+    if (m) {
+      sq[o] = s | m;
+      if (cov) cov[o] |= m;
+    }
+  }
+}
+
+// After round r's apply: exact gain update of the candidates whose box meets their problem's pick, then the keys of
+// round r + 1.  Candidates of finished problems do nothing; a candidate of gain 0 keeps it.
+__global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_t *__restrict__ bits, int64_t nsrc,
+                                                                   CoverGeo G, const int32_t *__restrict__ xy,
+                                                                   const int32_t *__restrict__ pg,
+                                                                   const int32_t *__restrict__ pk,
+                                                                   const int64_t *__restrict__ cur,
+                                                                   const int *__restrict__ done,
+                                                                   const uint32_t *__restrict__ newb,
+                                                                   uint32_t *__restrict__ gain,
+                                                                   unsigned long long *slot) {
+  __shared__ uint32_t sdec[kCand];
+  __shared__ unsigned sov;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t base = blockIdx.x * (int64_t)kCand;
+  const VhpCoverBox b0 = vhp_cover_box(G.nx, G.ny, G.R, 0, 0);
+  const size_t hw = (size_t)b0.H * b0.W;
+  bool valid = false;
+  int32_t g = -1;
+  uint32_t gn = 0;
+  if (warp == 0) {
+    const int64_t c = base + lane;
+    g = c < nsrc ? pg[c] : -1;
+    valid = g >= 0 && !done[g];
+    bool ov = false;
+    if (valid) {
+      gn = gain[c];
+      const int64_t p = cur[g];
+      if (gn > 0) {
+        const VhpCoverBox cb = vhp_cover_box(G.nx, G.ny, G.R, xy[2 * c], xy[2 * c + 1]);
+        const VhpCoverBox pb = vhp_cover_box(G.nx, G.ny, G.R, xy[2 * p], xy[2 * p + 1]);
+        ov = abs(cb.y0 - pb.y0) < b0.H && abs(cb.w0 - pb.w0) < b0.W;
+      }
+    }
+    sdec[lane] = 0;
+    const unsigned m = __ballot_sync(kAll, ov);
+    if (lane == 0) sov = m;
+  }
+  __syncthreads();
+  const unsigned ovm = sov;
+  int rank = 0;
+  for (unsigned m = ovm; m; m &= m - 1, ++rank) {
+    if (rank % kWarps != warp) continue;
+    const int j = __ffs(m) - 1;
+    const int64_t c = base + j;
+    const int32_t q = pg[c];
+    const int64_t p = cur[q];
+    const VhpCoverBox cb = vhp_cover_box(G.nx, G.ny, G.R, xy[2 * c], xy[2 * c + 1]);
+    const VhpCoverBox pb = vhp_cover_box(G.nx, G.ny, G.R, xy[2 * p], xy[2 * p + 1]);
+    const int ra = max(cb.y0, pb.y0), rb = min(cb.y0, pb.y0) + b0.H;
+    const int wa = max(cb.w0, pb.w0), wb = min(cb.w0, pb.w0) + b0.W;
+    uint32_t acc = 0;
+    for (int y = ra + lane; y < rb; y += 32) {
+      const uint32_t *nr = newb + (size_t)q * hw + (size_t)(y - pb.y0) * b0.W - pb.w0;
+      const uint32_t *br = bits + (size_t)c * hw + (size_t)(y - cb.y0) * b0.W - cb.w0;
+      for (int w = wa; w < wb; ++w) {
+        const uint32_t n = nr[w];
+        if (n) acc += __popc(__ldg(br + w) & n);
+      }
+    }
+    acc = warp_sum(acc);
+    if (lane == 0) sdec[j] = acc;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    const int64_t c = base + lane;
+    if (valid && sdec[lane]) {
+      gn -= sdec[lane];
+      gain[c] = gn;
+    }
+    put_keys(valid, g, key_of(gn, valid ? pk[c] : 0), slot);
+  }
+}
+
+unsigned grid_for(size_t n, int bs, int sm_count) {
+  return (unsigned)std::max<size_t>(1, std::min<size_t>((n + bs - 1) / bs, (size_t)sm_count * 32));
+}
+
+size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src], slot [prob], cur [prob], first [prob],
+// done [prob]
+struct CoverWs {
+  uint32_t *state, *newb, *gain;
+  unsigned long long *slot;
+  int64_t *cur, *first;
+  int *done;
+  size_t bytes;
+};
+CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R) {
+  const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
+  const size_t np = (size_t)nprob, plane = (size_t)ny * ((nx + 31) / 32);
+  const size_t o_new = align256(np * plane * 4), o_gain = o_new + align256(np * b.H * b.W * 4);
+  const size_t o_slot = o_gain + align256((size_t)nsrc * 4), o_cur = o_slot + align256(np * 8);
+  const size_t o_first = o_cur + align256(np * 8), o_done = o_first + align256(np * 8);
+  char *p = static_cast<char *>(base);
+  CoverWs w{};
+  w.bytes = o_done + align256(np * 4);
+  if (!p) return w;
+  w.state = (uint32_t *)p;
+  w.newb = (uint32_t *)(p + o_new);
+  w.gain = (uint32_t *)(p + o_gain);
+  w.slot = (unsigned long long *)(p + o_slot);
+  w.cur = (int64_t *)(p + o_cur);
+  w.first = (int64_t *)(p + o_first);
+  w.done = (int *)(p + o_done);
+  return w;
+}
+
+} // namespace
+
+cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, int64_t np, int nx, int ny, int R,
+                                  bool disk, int r2, const int32_t *d_xy, double thr, uint32_t *d_bits, int sm_count,
+                                  cudaStream_t st, int64_t *launches) {
+  const CoverGeo G{nx, ny, R, (nx + 31) / 32};
+  const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
+  const int bs = 256;
+  cover_fold_kernel<<<grid_for((size_t)np * b.H * b.W, bs, sm_count), bs, 0, st>>>(d_val, win_r, p0, np, G, disk, r2,
+                                                                                   d_xy, thr, d_bits);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R) {
+  return cover_ws(nullptr, nprob, nsrc, nx, ny, R).bytes;
+}
+
+cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
+                                    int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                    const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
+                                    const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches) {
+  const CoverGeo G{nx, ny, R, (nx + 31) / 32};
+  const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
+  cudaError_t e = cudaSuccess;
+  if (out.pick) e = cudaMemsetAsync(out.pick, 0xff, np * k * 4, st); // -1 from npicked on
+  if (e == cudaSuccess && out.gain) e = cudaMemsetAsync(out.gain, 0, np * k * 4, st);
+  if (e == cudaSuccess && out.npicked) e = cudaMemsetAsync(out.npicked, 0, np * 4, st);
+  if (e == cudaSuccess && out.covered) e = cudaMemsetAsync(out.covered, 0, np * plane * 4, st);
+  const int64_t rounds = std::min<int64_t>(k, nsrc);
+  if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
+  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R);
+  if (d_target) {
+    cover_state_kernel<<<grid_for(np * plane, 256, sm_count), 256, 0, st>>>(d_target, np * plane, ws.state);
+    if (launches) *launches += 1;
+  } else {
+    e = cudaMemsetAsync(ws.state, 0, np * plane * 4, st);
+  }
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.slot, 0, np * 8, st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.done, 0, np * 4, st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0xff, np * 8, st);
+  if (e != cudaSuccess) return e;
+  const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
+  cover_init_kernel<<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
+                                                  ws.gain, ws.slot, ws.first);
+  for (int32_t r = 0; r < rounds; ++r) {
+    cover_apply_kernel<<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k, ws.slot, ws.cur,
+                                                                  ws.done, ws.state, ws.newb, out);
+    if (r + 1 < rounds)
+      cover_update_kernel<<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
+                                                        ws.done, ws.newb, ws.gain, ws.slot);
+  }
+  if (launches) *launches += 2 * rounds;
+  return cudaGetLastError();
+}

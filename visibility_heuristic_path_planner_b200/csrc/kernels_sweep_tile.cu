@@ -60,6 +60,12 @@ sweep_tile_kernel(const TileArgs p) {
     tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, out, smem_raw);
     return;
   }
+  if constexpr (FMT == kFmtCoverBits) { // the candidate's box bits (VhpCoverBox), addressed by absolute grid coordinates
+    const VhpCoverBox b = vhp_cover_box(p.nx, p.ny, p.w_r, sx, sy);
+    uint32_t *out = reinterpret_cast<uint32_t *>(p.out) + (size_t)pair * b.H * b.W - ((ptrdiff_t)b.y0 * b.W + b.w0);
+    tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, reinterpret_cast<OutT *>(out), smem_raw);
+    return;
+  }
   // bit output: rows of (nx + 31) / 32 words
   const size_t per_pair = FMT == kFmtBits ? (size_t)((p.nx + 31) >> 5) * p.ny : (size_t)p.nx * p.ny;
   OutT *out = reinterpret_cast<OutT *>(p.out) + (size_t)pair * per_pair;
@@ -283,6 +289,15 @@ cudaError_t launch_tile_merge_range(const TileArgs &p, int64_t npairs, cudaStrea
   }
 }
 
+// candidate coverage bits (kFmtCoverBits): the warp counts and bounds of the windows
+cudaError_t launch_tile_cover(const TileArgs &p, int64_t npairs, cudaStream_t st) {
+  switch (tile_warps_for(win_side(p.nx, p.w_r), win_side(p.ny, p.w_r), npairs)) {
+    case 1: return launch_tile_nw<float, 1, VHP_NW1_MINB, kFmtCoverBits>(p, npairs, st);
+    case 2: case 4: case 6: return launch_tile_nw<float, 4, VHP_NW4_MINB, kFmtCoverBits>(p, npairs, st);
+    default: return launch_tile_nw<float, 8, 2, kFmtCoverBits>(p, npairs, st);
+  }
+}
+
 // fallback of the windows: window of pair p cut out of its full field, 0 outside the grid
 template <typename T>
 __global__ void window_crop_kernel(const T *__restrict__ field, int64_t np, int nx, int ny,
@@ -400,6 +415,32 @@ cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, cons
                  : launch_tile_merge_range<kFmtMergeRange64>(p, npairs, st);
   }
   return m.f32 ? launch_tile_merge<kFmtMerge32>(p, npairs, st) : launch_tile_merge<kFmtMerge64>(p, npairs, st);
+}
+
+cudaError_t vhp_launch_sweep_cover(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
+                                   const int32_t *d_src_map, int64_t npairs, int radius, double thr, uint32_t *d_bits,
+                                   const double *d_rcp2, int *d_err, cudaStream_t st, int64_t *launches) {
+  if (!(thr > 0.0)) return cudaErrorInvalidValue; // cells below the threshold are never written
+  const VhpCoverBox b = vhp_cover_box(nx, ny, radius, 0, 0);
+  cudaError_t e = cudaMemsetAsync(d_bits, 0, (size_t)npairs * b.H * b.W * sizeof(uint32_t), st);
+  if (e != cudaSuccess) return e;
+  TileArgs p;
+  p.pl = pl;
+  p.nx = nx;
+  p.ny = ny;
+  p.src_xy = d_src_xy;
+  p.src_map = d_src_map;
+  p.out = d_bits;
+  p.rtab = reinterpret_cast<const double2 *>(d_rcp2);
+  p.err = d_err;
+  p.vec = 0;
+  p.win_y0 = 0;
+  p.win_y1 = ny;
+  p.thr = thr;
+  p.w_r = radius;
+  p.w_sw = win_sum_words(nx, radius);
+  if (launches) *launches += 1;
+  return launch_tile_cover(p, npairs, st);
 }
 
 bool vhp_sweep_tile_supported(int nx, int ny) {

@@ -300,8 +300,12 @@ __device__ __forceinline__ void stg16_fill(double *q, double v) {
 // kFmtMergeRange64 / kFmtMergeRange32 (vhp_visibility_merge_range_batch): kFmtMerge* with the sweep clipped to the box
 // |dx|, |dy| <= R like kFmtWindow (the box is closed under "upstream": its values are the full field's), cell indices
 // in map pitch, and only the cells in range (TileArgs::w_r2) folded.
+// kFmtCoverBits (vhp_visibility_cover_greedy_batch): kFmtBits's bit stores with kFmtMergeRange*'s clipped geometry, in
+// the candidate's box layout (VhpCoverBox: rows of vhp_cover_words(nx, R) words, `out` shifted by the box origin, so
+// the addressing is the whole-map bit layout's with another row pitch); only the box |dx|, |dy| <= R is stored, the
+// disk is applied afterwards.
 constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4, kFmtWindow = 5, kFmtMergeRange64 = 6,
-              kFmtMergeRange32 = 7;
+              kFmtMergeRange32 = 7, kFmtCoverBits = 8;
 constexpr int kMergeHdr = 224; // shared-memory header: {group, k} of the CTA's source (int2)
 
 // the sweep folds into group outputs (merge_cell), and it does so only within a range
@@ -309,7 +313,9 @@ __host__ __device__ constexpr bool fmt_range(int f) { return f == kFmtMergeRange
 __host__ __device__ constexpr bool fmt_merge(int f) { return f == kFmtMerge64 || f == kFmtMerge32 || fmt_range(f); }
 // clipped geometry: each quadrant's extents are clipped to R and the per-CTA state is sized by the box
 // (tile_smem_bytes_win); the window output layout (pitch 2R+1, off-grid zeros) is kFmtWindow's alone
-__host__ __device__ constexpr bool fmt_clip(int f) { return f == kFmtWindow || fmt_range(f); }
+__host__ __device__ constexpr bool fmt_clip(int f) { return f == kFmtWindow || fmt_range(f) || f == kFmtCoverBits; }
+// one bit per cell (v >= thr), into a zeroed buffer
+__host__ __device__ constexpr bool fmt_bits(int f) { return f == kFmtBits || f == kFmtCoverBits; }
 
 // fold value v of cell idx (y * nx + x) of this CTA's sweep into its group's outputs; (di, dj) = (|dx|, |dy|) of
 // the cell from the source, for the range test of kFmtMergeRange*
@@ -522,7 +528,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   // the row above may start its tile I as soon as rowE holds this tile's top row: publish
   // before the global stores
   constexpr int kStepUnroll = NW == 1 ? VHP_STEP_UNROLL_1W : VHP_STEP_UNROLL;
-  constexpr bool BITS = FMT == kFmtBits;
+  constexpr bool BITS = fmt_bits(FMT);
   constexpr bool MERGE = fmt_merge(FMT);
   static_assert(!BITS || sizeof(OutT) == 4, "bit output: OutT is the 32-bit word");
   static_assert(!MERGE || (sizeof(OutT) == 8 && !GE), "merge output: fp64 staging, one-CTA sweeps");
@@ -592,7 +598,7 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
   // bit output: the tile's columns of one row are (part of) ONE word, since tile columns start on
   // multiples of 32 except the first one of a quadrant, which ends on one
   const int xw = g.dirx > 0 ? sx + i0 : sx - i0; // column of lane 0
-  const int wpr = (nx + 31) >> 5;
+  const int wpr = FMT == kFmtCoverBits ? vhp_cover_words(p.nx, p.w_r) : (nx + 31) >> 5; // words per row of `out`
   auto put_word = [&](const uint32_t m, const int rfirst, const int rend) { // m: bit l <-> column il
     const uint32_t w = g.dirx > 0 ? m << (xw & 31) : __brev(m) >> (31 - (xw & 31));
     if (lane >= rfirst && lane <= rend && w) { // lane <-> row j0 + lane
@@ -806,7 +812,8 @@ __device__ __forceinline__ void process_tile(const TileArgs &p, const TQuad &g, 
 //
 // kFmtWindow: every cell of the (2R+1)^2 window exactly once instead (out: see kFmtWindow),
 // smem_raw: tile_smem_bytes_win<OutT>(nx, ny, R, NW) bytes.  kFmtMergeRange*: the cells of the box |dx|, |dy| <= R
-// once each, in map pitch, smem_raw sized like kFmtWindow.
+// once each, in map pitch, smem_raw sized like kFmtWindow.  kFmtCoverBits: the bits of that box, `out` as kFmtBits's
+// with the box's row pitch.
 //
 // Grid mode (MODE != kSweepCta; one sweep of a giant map by many CTAs): kSweepGridInit, run by
 // one CTA, computes the staircase and writes it with the boundary rows, the progress flags and
@@ -819,7 +826,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
                                                const int sy, OutT *__restrict__ out,
                                                unsigned char *smem_raw) {
   constexpr bool GE = MODE != kSweepCta;
-  constexpr bool BITS = FMT == kFmtBits;
+  constexpr bool BITS = fmt_bits(FMT);
   constexpr bool WIN = FMT == kFmtWindow, CLIP = fmt_clip(FMT);
   static_assert(!GE || NW > 1, "grid mode uses the multi-warp boundary layout");
   static_assert(!GE || !CLIP, "clipped sweeps are one-CTA sweeps");
@@ -1027,7 +1034,7 @@ __device__ __forceinline__ void tile_sweep_cta(const TileArgs &p, const int map,
       // word masks once and then stores them row after row.  (Row by row, with the staircase
       // looked up per row, the all-lit headline batch spent 135 instructions per row.)
       static_assert(!GE, "bit output is a one-CTA sweep");
-      const int wprl = (nx + 31) >> 5;
+      const int wprl = FMT == kFmtCoverBits ? vhp_cover_words(nx, p.w_r) : (nx + 31) >> 5;
       uint32_t *const wout = reinterpret_cast<uint32_t *>(out);
       int seg = 0;
       for (int half = 0; half < 2 && 1.0 >= p.thr; ++half) {

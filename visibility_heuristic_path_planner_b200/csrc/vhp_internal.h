@@ -111,6 +111,8 @@ struct vhp_context {
   // vhp_visibility_merge_range_batch, fallback: the fp64 windows of a chunk of pairs (apart from b_bin and b_misc,
   // which the window routes use themselves)
   VhpDevBuf b_mwin;
+  // vhp_visibility_cover_greedy_batch: the candidates' coverage bits, and the workspace of the greedy rounds
+  VhpDevBuf b_cover, b_cover_ws;
   cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
   // 1/k table {rh, rl} of the tile kernel (double-double reciprocal), device resident
   double *rcp2_table = nullptr;
@@ -255,6 +257,56 @@ cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np,
 cudaError_t vhp_launch_merge_window_fold(const double *d_win, int64_t p0, int64_t np, int nx, int ny,
                                          const int32_t *d_src_xy, double thr, const VhpMergeRange &range,
                                          const VhpMergeDev &m, int sm_count, cudaStream_t st, int64_t *launches);
+
+// Greedy coverage placement (vhp_visibility_cover_greedy_batch).  The coverage bits of a candidate at (sx, sy) are
+// stored over its box, clipped to the grid: H = min(2R+1, ny) rows from row y0 and W words (the span rule of
+// win_sum_words) from word w0 of the map's 32-column words, so cell (x, y) is bit x & 31 of word
+// (y - y0) * W + (x >> 5) - w0.  R is the radius clamped to max(nx, ny) - 1, which leaves the box unchanged.  Every
+// box has the same H x W words; a candidate outside the grid gets the box of the nearest cell.
+struct VhpCoverBox {
+  int y0, w0, H, W;
+};
+__host__ __device__ inline int vhp_cover_words(int nx, int R) {
+  const int nw = (nx + 31) >> 5, span = (2 * R + 31) / 32 + 1;
+  return nw < span ? nw : span;
+}
+__host__ __device__ inline VhpCoverBox vhp_cover_box(int nx, int ny, int R, int sx, int sy) {
+  sx = sx < 0 ? 0 : (sx >= nx ? nx - 1 : sx);
+  sy = sy < 0 ? 0 : (sy >= ny ? ny - 1 : sy);
+  VhpCoverBox b;
+  b.H = ny < 2 * R + 1 ? ny : 2 * R + 1;
+  b.W = vhp_cover_words(nx, R);
+  const int y0 = sy - R < 0 ? 0 : sy - R, w0 = (sx - R < 0 ? 0 : sx - R) >> 5, nw = (nx + 31) >> 5;
+  b.y0 = y0 < ny - b.H ? y0 : ny - b.H;
+  b.w0 = w0 < nw - b.W ? w0 : nw - b.W;
+  return b;
+}
+// Phase 1, direct route (thr > 0, vhp_sweep_window_supported): the one-CTA tile kernel sweeps each candidate's box
+// straight into its bits (kFmtCoverBits; zeroes d_bits first, the box only, no disk).  Pair p's map is d_src_map[p].
+cudaError_t vhp_launch_sweep_cover(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
+                                   const int32_t *d_src_map, int64_t npairs, int radius, double thr, uint32_t *d_bits,
+                                   const double *d_rcp2, int *d_err, cudaStream_t st, int64_t *launches);
+// kernels_cover.cu.  Fallback of phase 1: the bits of pairs [p0, p0 + np) from their fp64 values, win_r >= 0: windows
+// [np][2 win_r + 1]^2 centred on the candidate, win_r < 0: whole fields [np][ny][nx]; each bit is the cell's range
+// test (box of radius R, disk dx^2 + dy^2 <= r2 if disk), "writes" test and v >= thr.
+cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, int64_t np, int nx, int ny, int R,
+                                  bool disk, int r2, const int32_t *d_xy, double thr, uint32_t *d_bits, int sm_count,
+                                  cudaStream_t st, int64_t *launches);
+// Phase 2, the greedy rounds over the bits of nsrc candidates (table of vhp_launch_merge_table) of nprob problems.
+struct VhpCoverDev {
+  int32_t *pick = nullptr;   // [prob][k]
+  uint32_t *gain = nullptr;  // [prob][k]
+  int32_t *npicked = nullptr; // [prob]
+  uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
+};
+// workspace bytes of the rounds beyond the candidate bits
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R);
+// outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
+// route's sweep stores the whole box); d_target (may be null): [prob][ny][ceil(nx/32)] bits of the cells to cover
+cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
+                                    int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                    const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
+                                    const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
