@@ -329,7 +329,8 @@ def test_binary_thresholds_on_field_values(vhp, oracle, monkeypatch):
 def test_binary_direct_all_warp_counts(vhp, n):
     """The bit-writing sweep at the batch sizes that select the 4-warp and the 1-warp kernels, with
     sources on word boundaries, corners and edges: equal to the fp64 field of the same library
-    (itself bit-exact against the oracle at these batch sizes) compared with >= threshold."""
+    compared with >= threshold (the fields of those instances are checked against the oracle in
+    test_gpu_warps.py, at these and other batch sizes)."""
     rng = np.random.default_rng(n)
     c = vhp.Context(0)
     for nx, ny, nobs in ((101, 101, 10), (64, 50, 5), (97, 130, 0), (33, 32, 1), (160, 45, 12)):

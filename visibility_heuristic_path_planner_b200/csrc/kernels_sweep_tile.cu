@@ -237,7 +237,10 @@ int tile_warps_for(int nx, int ny, int64_t npairs) {
 
 template <typename OutT>
 cudaError_t launch_tile(const TileArgs &p, int64_t npairs, cudaStream_t st) {
-  switch (tile_warps_for(p.nx, p.ny, npairs)) {
+  int nw = tile_warps_for(p.nx, p.ny, npairs);
+  // a forced 10 or 16 whose CTA does not fit shared memory runs 8 warps (vhp_sweep_tile_supported checked those)
+  if (tile_smem_bytes<OutT>(p.nx, p.ny, nw) > 227u * 1024u) nw = 8;
+  switch (nw) {
     case 1: return launch_tile_nw<OutT, 1, VHP_NW1_MINB>(p, npairs, st);
     case 2: return launch_tile_nw<OutT, 2, 12>(p, npairs, st);
     case 4: return launch_tile_nw<OutT, 4, VHP_NW4_MINB>(p, npairs, st);
