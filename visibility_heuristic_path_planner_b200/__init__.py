@@ -506,20 +506,21 @@ class Context:
         return self._batch_host(self.lib.vhp_raycast_batch, occ, src_xy, src_map, dtype, out)
 
     def planner_batch(self, occ, start_end, prob_map=None, threshold=0.5, max_iter=100,
-                      dtype=F64, fields=True):
+                      dtype=F64, fields=True, ls_cap=None):
         """solve() + reconstructPath() for every problem.  Returns a dict of numpy
         arrays (status, nb_sources, light_sources, path_len, path_n, path[, vg,
-        came, vis])."""
+        came, vis]).  ls_cap: entries per problem of light_sources and path (default
+        max_iter + 2, the least the library accepts)."""
         occ = _occ_u8(occ)
         nmaps, ny, nx = occ.shape
         se = np.ascontiguousarray(start_end, dtype=np.int32).reshape(-1, 4)
         n = se.shape[0]
         mp = None if prob_map is None else np.ascontiguousarray(prob_map, dtype=np.int32)
-        cap = int(max_iter) + 2
+        cap = int(max_iter) + 2 if ls_cap is None else int(ls_cap)
         ft = np.float32 if dtype == F32 else np.float64
         r = dict(status=np.zeros(n, np.int32), nb_sources=np.zeros(n, np.int32),
-                 light_sources=np.zeros((n, cap, 2), np.int32), path_len=np.zeros(n),
-                 path_n=np.zeros(n, np.int32), path=np.zeros((n, cap, 2), np.int32))
+                 light_sources=np.zeros((n, max(cap, 0), 2), np.int32), path_len=np.zeros(n),
+                 path_n=np.zeros(n, np.int32), path=np.zeros((n, max(cap, 0), 2), np.int32))
         if fields:
             r.update(vg=np.zeros((n, ny, nx), ft), came=np.zeros((n, ny, nx), np.int32),
                      vis=np.zeros((n, ny, nx), ft))
@@ -530,6 +531,33 @@ class Context:
                                                _np_ptr(se), _np_ptr(mp), n, float(threshold),
                                                int(max_iter), cap, dtype, C.byref(po)))
         return r
+
+    PLANNER_OUTPUTS = ("status", "nb_sources", "light_sources", "path_len", "path_n", "path", "vg", "came", "vis")
+
+    def planner_batch_dev(self, occ_t, start_end_t, prob_map_t=None, threshold=0.5, max_iter=100, ls_cap=None,
+                          dtype=F64, **outputs):
+        """planner_batch on CUDA tensors (asynchronous, returns nothing): occ_t uint8 (nmaps, ny, nx),
+        start_end_t int32 (nprob, 4), prob_map_t int32 (nprob,) or None.  Outputs by keyword, each a
+        contiguous CUDA tensor or omitted: status, nb_sources, path_n int32 (nprob,), path_len float64
+        (nprob,), light_sources, path int32 (nprob, ls_cap, 2), came int32 (nprob, ny, nx), vg, vis (nprob,
+        ny, nx) of dtype.  With no output at all the library gets a NULL output struct."""
+        unknown = set(outputs) - set(self.PLANNER_OUTPUTS)
+        if unknown:
+            raise ValueError(f"unknown planner outputs {sorted(unknown)}; they are among {self.PLANNER_OUTPUTS}")
+        for k in ("vg", "vis"):
+            t = outputs.get(k)
+            if t is not None and t.element_size() != (4 if dtype == F32 else 8):
+                raise ValueError(f"{k} must be of the dtype of the call")
+        nmaps, ny, nx = occ_t.shape
+        cap = int(max_iter) + 2 if ls_cap is None else int(ls_cap)
+        po = None
+        if any(t is not None for t in outputs.values()):
+            po = C.byref(PlannerOut(*[None if outputs.get(k) is None else outputs[k].data_ptr()
+                                      for k in self.PLANNER_OUTPUTS]))
+        self._check(self.lib.vhp_planner_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, start_end_t.data_ptr(),
+            None if prob_map_t is None else prob_map_t.data_ptr(), start_end_t.shape[0], float(threshold),
+            int(max_iter), cap, dtype, po))
 
     # ---- device (torch) entry points ----------------------------------------
     def visibility_batch_dev(self, occ_t, src_xy_t, out_t, src_map_t=None):

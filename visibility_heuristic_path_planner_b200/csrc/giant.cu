@@ -90,6 +90,10 @@ struct vhp_giant {
   cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
   bool graph_failed = false;
+  // what the capture baked into the sweep nodes: the context's ratio table (ensure_rcp2 frees it
+  // when it grows) and its grid-sweep mode (vhp_i_grid_ctas fixes the CTA count)
+  const double *graph_rcp2 = nullptr;
+  int graph_grid_sweep = -1;
   // NCCL timing trace (env VHP_GIANT_TRACE or stats requested in mode 2)
   bool trace = false;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> trace_ev;
@@ -251,6 +255,8 @@ vhp_status enqueue_iteration(vhp_giant *g, unsigned long long cond, int use_cond
 // CUDA graph: one WHILE node whose body is one iteration; the step kernel sets the condition.
 vhp_status build_graph(vhp_giant *g) {
   cudaStream_t S = g->ctx->stream;
+  g->graph_rcp2 = g->ctx->rcp2_table;
+  g->graph_grid_sweep = g->ctx->grid_sweep;
   GCUDA(g, cudaGraphCreate(&g->graph, 0));
   cudaGraphConditionalHandle handle;
   GCUDA(g, cudaGraphConditionalHandleCreate(&handle, g->graph, 1, cudaGraphCondAssignDefault));
@@ -298,6 +304,11 @@ vhp_status run_loop(vhp_giant *g, int max_iter, int *iters_out) {
   int mode = g->loop_mode;
   if (mode == 0) mode = g->world > 1 ? 2 : 1;
   if (mode == 1 && g->world > 1) mode = 2; // NCCL calls are not captured
+  if ((g->exec || g->graph_failed) &&
+      (g->graph_rcp2 != g->ctx->rcp2_table || g->graph_grid_sweep != g->ctx->grid_sweep)) {
+    drop_graph(g); // its sweeps would read a freed table or run a stale CTA count: capture again
+    g->graph_failed = false;
+  }
   if (mode == 1 && !g->exec && !g->graph_failed) {
     const vhp_status st = build_graph(g);
     if (st != VHP_OK) { // e.g. a driver without conditional nodes: fall back to batches
