@@ -277,6 +277,49 @@ vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t
                                                  int32_t radius, int32_t shape, double threshold,
                                                  const uint32_t *d_target, const vhp_cover_out *d_out);
 
+/* Weighted greedy sensor placement: which k candidates cover the most summed importance together.  Problems,
+ * candidates, group_map, radius, shape, threshold and S(c) are exactly those of vhp_visibility_cover_greedy_batch.
+ *   W_q   weights ([prob][ny][nx] uint8, unpadded, no alignment needed): the importance W_q(x) in [0, 255] of cell x
+ *         to problem q; NULL: every cell weighs 1.
+ * Greedy, U = {} and for r = 0 .. k-1: gain(c) = sum of W_q(x) over x in S(c) \ U for every candidate of the problem;
+ * p = argmax, ties to the smallest index within the group; if gain(p) == 0 stop (npicked = r), else U |= S(p).
+ * Duplicates are separate entries.  Every gain is an exact integer sum and every decision an integer comparison, so
+ * the result does not depend on the order of atomics or blocks.  Outputs (any may be NULL, at least one must be given):
+ *   pick[q][r]     index within the group of the r-th pick, -1 from npicked on            (int32 [prob][k])
+ *   gain[q][r]     summed weight the r-th pick newly covers, 0 from npicked on            (uint64 [prob][k])
+ *   npicked[q]                                                                            (int32 [prob])
+ *   covered[q]     U after the last pick, every cell of the union whatever its weight, bits beyond nx 0
+ *                  ([prob][ny][ceil(nx/32)] uint32)
+ * so sum of gain = sum of W over U, gains are non-increasing, and the result is within (1 - 1/e) of the best k-subset
+ * (weighted coverage is monotone submodular).  There is no target: weights in {0, 1} are the target of
+ * vhp_visibility_cover_greedy_batch (and give its result), and "add k sensors to those already placed" is weights
+ * zeroed on their coverage.
+ * Gains fit 36 bits (at most 2^28 cells of weight 255), which leaves 28 bits of the 64-bit argmax key for the index:
+ * nsrc >= 2^28 is VHP_ERR_INVALID_ARG (the nsrc argument of the _dev form, group_ptr[nprob] of the host form),
+ * checked before any candidate is read.
+ * Routes and phase 1 are those of vhp_visibility_cover_greedy_batch; the rounds also read a copy of the weights in
+ * 32-byte rows per 32-column word.  Workspace: that of vhp_visibility_cover_greedy_batch, plus 4 * nsrc bytes (uint64
+ * gains) and 32 * ny * ceil(nx/32) bytes per problem; the host form's 4 GB batches also count each problem's ny * nx
+ * weight bytes.  Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_cover_greedy_batch, and the 2^28 limit.
+ * k == 0 is valid. */
+typedef struct vhp_cover_weighted_out {
+  int32_t *pick;
+  uint64_t *gain;
+  int32_t *npicked;
+  uint32_t *covered;
+} vhp_cover_weighted_out;
+vhp_status vhp_visibility_cover_greedy_weighted_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                      const int32_t *cand_xy, const int64_t *group_ptr,
+                                                      const int32_t *group_map, int64_t nprob, int32_t k,
+                                                      int32_t radius, int32_t shape, double threshold,
+                                                      const uint8_t *weights, const vhp_cover_weighted_out *out);
+vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                          int ny, const int32_t *d_cand_xy,
+                                                          const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                                          int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
+                                                          int32_t shape, double threshold, const uint8_t *d_weights,
+                                                          const vhp_cover_weighted_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

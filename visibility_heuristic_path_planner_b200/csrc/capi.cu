@@ -8,6 +8,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "vhp_internal.h"
@@ -1132,12 +1133,18 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
 // straight into bits (kFmtCoverBits: threshold > 0 and window_direct_route), the fallback folds chunks of fp64
 // windows (run_window_dev, any of its routes) or, where a window would be larger than the map, of whole fields
 // (run_dev) with cover_fold_kernel.  Phase 2 (kernels_cover.cu) runs min(k, nsrc) greedy rounds on the device.
+// The weighted call (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
+const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
+// the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
+constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
+// Out: vhp_cover_out or vhp_cover_weighted_out
+template <class Out>
 vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k, const VhpMergeRange &range,
-                            double thr, const vhp_cover_out *out) {
-  const std::string what = kCoverName;
+                            double thr, const Out *out, const char *name = kCoverName) {
+  const std::string what = name;
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || nprob < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
@@ -1151,8 +1158,22 @@ vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx
   return check_range(ctx, what, range);
 }
 
-VhpCoverDev cover_dev_of(const vhp_cover_out &o) {
-  VhpCoverDev c;
+// the cover call's checks, then the weighted key's limit on nsrc (before any candidate is read)
+vhp_status check_cover_weighted_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
+                                     const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
+                                     const VhpMergeRange &range, double thr, const vhp_cover_weighted_out *out) {
+  const vhp_status st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr, out,
+                                         kCoverWeightedName);
+  if (st != VHP_OK) return st;
+  if (nsrc >= kCoverWeightedMaxSrc)
+    return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverWeightedName) + ": 2^28 or more candidates");
+  return VHP_OK;
+}
+
+// Out: vhp_cover_out or vhp_cover_weighted_out, Dev: VhpCoverDev or VhpCoverWeightedDev
+template <class Dev, class Out>
+Dev cover_dev_of(const Out &o) {
+  Dev c;
   c.pick = o.pick;
   c.gain = o.gain;
   c.npicked = o.npicked;
@@ -1161,44 +1182,54 @@ VhpCoverDev cover_dev_of(const vhp_cover_out &o) {
 }
 
 // a workspace buffer of the rounds; a failed allocation names its size
-vhp_status ensure_cover(vhp_context *ctx, VhpDevBuf &b, size_t bytes, const char *what) {
+vhp_status ensure_cover(vhp_context *ctx, VhpDevBuf &b, size_t bytes, const char *what, const char *name) {
   if (ensure(ctx, b, bytes) == VHP_OK) return VHP_OK;
   (void)cudaGetLastError();
-  return fail(ctx, VHP_ERR_CUDA, std::string(kCoverName) + ": " + what + " of " + std::to_string(bytes) +
+  return fail(ctx, VHP_ERR_CUDA, std::string(name) + ": " + what + " of " + std::to_string(bytes) +
                                      " bytes: " + ctx->last_error);
 }
 
-vhp_status run_cover_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
-                         const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                         const VhpMergeRange &range, double thr, const uint32_t *d_target, const VhpCoverDev &out) {
+// what phase 1 leaves for the rounds
+struct CoverBits {
+  uint32_t *bits = nullptr;
+  int32_t *pg = nullptr, *pk = nullptr; // candidate -> problem, index within it (vhp_launch_merge_table)
+  int R = 0;                            // the geometry's radius
+  int disk_r2 = -1;                     // >= 0: the direct route stored the whole box, the rounds apply the disk
+};
+
+// Phase 1 of both cover calls: the table, the workspace of the rounds (ws_bytes) and every candidate's coverage bits
+vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                            const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
+                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb) {
+  const char *name = weighted ? kCoverWeightedName : kCoverName;
   const int R = std::min(range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
   const bool disk = range.shape == VHP_RANGE_DISK;
   const int r2 = range.radius * range.radius;
   const int64_t rounds = std::min<int64_t>(k, nsrc);
-  uint32_t *bits = nullptr;
-  int32_t *pg = nullptr, *pk = nullptr;
-  int disk_r2 = -1; // the direct route stores the whole box: the rounds apply the disk
+  cb.R = R;
   vhp_status st;
   if (nprob > 0 || nsrc > 0) {
     if ((st = ensure(ctx, ctx->b_merge, 12 * (size_t)std::max<int64_t>(nsrc, 1))) != VHP_OK) return st;
-    pg = (int32_t *)ctx->b_merge.p;
-    pk = pg + nsrc;
-    int32_t *pm = pk + nsrc;
-    VHP_CUDA(ctx, vhp_launch_merge_table(d_gptr, d_gmap, nprob, nsrc, nmaps, pg, pk, pm, ctx->d_err, ctx->sm_count,
-                                         ctx->stream, &ctx->launches));
+    cb.pg = (int32_t *)ctx->b_merge.p;
+    cb.pk = cb.pg + nsrc;
+    int32_t *pm = cb.pk + nsrc;
+    VHP_CUDA(ctx, vhp_launch_merge_table(d_gptr, d_gmap, nprob, nsrc, nmaps, cb.pg, cb.pk, pm, ctx->d_err,
+                                         ctx->sm_count, ctx->stream, &ctx->launches));
     if (rounds > 0 && nprob > 0) {
       const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
-      if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits")) != VHP_OK)
+      if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits", name)) !=
+          VHP_OK)
         return st;
-      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R), "workspace")) != VHP_OK)
+      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, weighted), "workspace",
+                             name)) != VHP_OK)
         return st;
-      bits = (uint32_t *)ctx->b_cover.p;
+      uint32_t *bits = cb.bits = (uint32_t *)ctx->b_cover.p;
       if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
         if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), R + 1) + 64)) != VHP_OK) return st;
         if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
         VHP_CUDA(ctx, vhp_launch_sweep_cover(ctx->tile, nx, ny, d_xy, pm, nsrc, R, thr, bits, ctx->rcp2_table,
                                              ctx->d_err, ctx->stream, &ctx->launches));
-        if (disk) disk_r2 = r2;
+        if (disk) cb.disk_r2 = r2;
       } else {
         // fp64 windows, or whole fields where a window would be larger than the map, up to 1 GB at a time
         const bool win = (2 * (size_t)R + 1) * (2 * (size_t)R + 1) <= (size_t)nx * ny;
@@ -1216,22 +1247,57 @@ vhp_status run_cover_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
       }
     }
   }
-  VHP_CUDA(ctx, vhp_launch_cover_greedy(bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, pg, pk, d_target, k,
-                                        ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream, &ctx->launches));
+  return VHP_OK;
+}
+
+vhp_status run_cover_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                         const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
+                         const VhpMergeRange &range, double thr, const uint32_t *d_target, const VhpCoverDev &out) {
+  CoverBits cb;
+  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
+                                         false, cb);
+  if (st != VHP_OK) return st;
+  VHP_CUDA(ctx, vhp_launch_cover_greedy(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk, d_target,
+                                        k, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream, &ctx->launches));
+  return VHP_OK;
+}
+
+vhp_status run_cover_weighted_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                  const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
+                                  int64_t nsrc, int32_t k, const VhpMergeRange &range, double thr,
+                                  const uint8_t *d_weights, const VhpCoverWeightedDev &out) {
+  CoverBits cb;
+  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
+                                         true, cb);
+  if (st != VHP_OK) return st;
+  VHP_CUDA(ctx, vhp_launch_cover_greedy_weighted(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk,
+                                                 d_weights, k, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
+                                                 &ctx->launches));
   return VHP_OK;
 }
 
 // host buffers: validate, upload maps and candidates once, then runs of whole problems whose device memory (candidate
-// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync
+// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync.  kW: the
+// weighted call, extra = weights ([prob][ny][nx] uint8), else extra = target ([prob][ny][ceil(nx/32)] uint32); either
+// may be null.
+template <bool kW>
 vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
                           const int64_t *gptr, const int32_t *gmap, int64_t nprob, int32_t k,
-                          const VhpMergeRange &range, double thr, const uint32_t *target, const vhp_cover_out *out) {
-  vhp_status st = check_groups_host(ctx, kCoverName, gptr, nprob);
+                          const VhpMergeRange &range, double thr, const void *extra,
+                          const typename std::conditional<kW, vhp_cover_weighted_out, vhp_cover_out>::type *out) {
+  using Dev = typename std::conditional<kW, VhpCoverWeightedDev, VhpCoverDev>::type;
+  using Gain = typename std::remove_pointer<decltype(Dev::gain)>::type;
+  const char *name = kW ? kCoverWeightedName : kCoverName;
+  vhp_status st = check_groups_host(ctx, name, gptr, nprob);
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
-  if ((st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out)) != VHP_OK) return st;
-  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, kCoverName)) != VHP_OK) return st;
-  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, nprob, nmaps, nx, ny, kCoverName)) != VHP_OK) return st;
+  if constexpr (kW)
+    st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
+  else
+    st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
+  if (st != VHP_OK) return st;
+  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, name)) != VHP_OK) return st;
+  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, nprob, nmaps, nx, ny, name)) != VHP_OK) return st;
   ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
   ctx->last_transport_packed = 0;
   if (nprob == 0) return VHP_OK;
@@ -1242,12 +1308,14 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   const size_t plane = (size_t)ny * ((nx + 31) / 32);
   const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(range.radius, std::max(nx, ny) - 1), 0, 0);
   const size_t box = (size_t)b.H * b.W * 4, budget = (size_t)4 << 30;
-  const size_t bp = out->pick ? 4 * (size_t)k : 0, bg = out->gain ? 4 * (size_t)k : 0, bn = out->npicked ? 4 : 0;
-  const size_t bc = out->covered ? plane * 4 : 0, bt = target ? plane * 4 : 0;
-  // device bytes of problem q: its candidates' bits, state, new, outputs, target
-  auto prob_bytes = [&](int64_t q) {
-    return (size_t)(gptr[q + 1] - gptr[q]) * (box + 16) + plane * 4 + box + bp + bg + bn + bc + bt + 64;
-  };
+  const size_t bp = out->pick ? 4 * (size_t)k : 0, bg = out->gain ? sizeof(Gain) * (size_t)k : 0;
+  const size_t bn = out->npicked ? 4 : 0, bc = out->covered ? plane * 4 : 0;
+  const size_t bt = extra ? (kW ? (size_t)ny * nx : plane * 4) : 0;
+  // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
+  // the weighted rounds' 32-byte rows of weights)
+  const size_t per_src = box + 12 + sizeof(Gain), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
+                                                             (kW ? plane * 32 : 0);
+  auto prob_bytes = [&](int64_t q) { return (size_t)(gptr[q + 1] - gptr[q]) * per_src + per_prob; };
   std::vector<int64_t> h_ptr;
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
   vhp_status result = VHP_OK;
@@ -1260,24 +1328,31 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     if ((result = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + bn + bc) + 256)) != VHP_OK) break;
     if ((result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gc + 1))) != VHP_OK) break;
     if (gmap && (result = ensure(ctx, ctx->b_map, 4 * (size_t)gc)) != VHP_OK) break;
-    if (target && (result = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) break;
+    if (extra && (result = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) break;
     char *base = (char *)ctx->b_out[0].p;
-    VhpCoverDev o;
+    const size_t o_gain = (gc * bp + sizeof(Gain) - 1) & ~(sizeof(Gain) - 1); // uint64 gains: 8-byte aligned
+    Dev o;
     o.pick = out->pick ? (int32_t *)base : nullptr;
-    o.gain = out->gain ? (uint32_t *)(base + gc * bp) : nullptr;
-    o.npicked = out->npicked ? (int32_t *)(base + gc * (bp + bg)) : nullptr;
-    o.covered = out->covered ? (uint32_t *)(base + gc * (bp + bg + bn)) : nullptr;
+    o.gain = out->gain ? (Gain *)(base + o_gain) : nullptr;
+    o.npicked = out->npicked ? (int32_t *)(base + o_gain + gc * bg) : nullptr;
+    o.covered = out->covered ? (uint32_t *)(base + o_gain + gc * (bg + bn)) : nullptr;
     cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
                                     ctx->stream);
     if (e == cudaSuccess && gmap)
       e = cudaMemcpyAsync(ctx->b_map.p, gmap + q0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess && target)
-      e = cudaMemcpyAsync(ctx->b_out[1].p, target + (size_t)q0 * plane, (size_t)gc * bt, cudaMemcpyHostToDevice,
-                          ctx->stream);
+    if (e == cudaSuccess && extra)
+      e = cudaMemcpyAsync(ctx->b_out[1].p, (const char *)extra + (size_t)q0 * bt, (size_t)gc * bt,
+                          cudaMemcpyHostToDevice, ctx->stream);
     if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: upload of the problems"); break; }
-    result = run_cover_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a, (const int64_t *)ctx->b_misc.p,
-                           gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc, gptr[q0 + gc] - a, k, range, thr,
-                           target ? (const uint32_t *)ctx->b_out[1].p : nullptr, o);
+    const uint8_t *d_occ = (const uint8_t *)ctx->b_occ.p;
+    const int64_t *d_gptr = (const int64_t *)ctx->b_misc.p;
+    const int32_t *d_gmap = gmap ? (const int32_t *)ctx->b_map.p : nullptr;
+    if constexpr (kW)
+      result = run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a,
+                                      k, range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, o);
+    else
+      result = run_cover_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k, range,
+                             thr, extra ? (const uint32_t *)ctx->b_out[1].p : nullptr, o);
     if (result != VHP_OK) break;
     if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && out->gain)
@@ -1866,8 +1941,8 @@ vhp_status vhp_visibility_cover_greedy_batch(vhp_context *ctx, const uint8_t *oc
   VhpMergeRange range;
   range.radius = radius;
   range.shape = shape;
-  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, target,
-                        out);
+  return run_cover_host<false>(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold,
+                               target, out);
 }
 
 vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -1883,7 +1958,36 @@ vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t
   if (st != VHP_OK) return st;
   VHP_ON_DEVICE(ctx);
   return run_cover_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
-                       threshold, d_target, cover_dev_of(*d_out));
+                       threshold, d_target, cover_dev_of<VhpCoverDev>(*d_out));
+}
+
+vhp_status vhp_visibility_cover_greedy_weighted_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                      const int32_t *cand_xy, const int64_t *group_ptr,
+                                                      const int32_t *group_map, int64_t nprob, int32_t k,
+                                                      int32_t radius, int32_t shape, double threshold,
+                                                      const uint8_t *weights, const vhp_cover_weighted_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_cover_host<true>(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold,
+                              weights, out);
+}
+
+vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                          int ny, const int32_t *d_cand_xy,
+                                                          const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                                          int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
+                                                          int32_t shape, double threshold, const uint8_t *d_weights,
+                                                          const vhp_cover_weighted_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  vhp_status st = check_cover_weighted_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
+                                            threshold, d_out);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  return run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
+                                threshold, d_weights, cover_dev_of<VhpCoverWeightedDev>(*d_out));
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

@@ -10,8 +10,13 @@
 //          intersection (a warp per such candidate, lanes over rows), then every candidate puts its key into the slot.
 // The key (gain << 32) | ~index makes atomicMax pick the largest gain and, among equal gains, the smallest index
 // within the group.  Every quantity is an integer, so the result does not depend on the order of the atomics.
+//
+// The weighted rounds (vhp_visibility_cover_greedy_weighted_batch) are the same kernels instantiated with kW = true:
+// state starts as {W == 0} (cover_weight_kernel, which also copies the weights into a plane of 32-byte rows per word),
+// gains are uint64 sums of the weights of the set bits (weight_sum), and the key is (gain << 28) | (2^28 - 1 - index).
 #include <algorithm>
 #include <cstdint>
+#include <type_traits>
 
 #include "vhp_internal.h"
 
@@ -21,6 +26,13 @@ constexpr unsigned kAll = 0xffffffffu;
 constexpr int kCand = 32;  // candidates per CTA of the init / update kernels (lane l of warp 0 <-> candidate l)
 constexpr int kWarps = 8;  // warps per CTA of those kernels
 constexpr int kApplyThreads = 512;
+
+constexpr int kIdxBits = 28; // index bits of the weighted key: gains fit the other 36 (2^28 cells of weight <= 255)
+constexpr unsigned long long kIdxMask = (1ull << kIdxBits) - 1;
+
+// gain of a candidate: a cell count, or a sum of uint8 weights
+template <bool kW>
+using GainT = typename std::conditional<kW, uint64_t, uint32_t>::type;
 
 struct CoverGeo {
   int nx, ny, R, nw; // R: the radius clamped for the geometry; nw = ceil(nx / 32)
@@ -46,6 +58,23 @@ __device__ __forceinline__ uint32_t warp_sum(uint32_t v) {
   return v;
 }
 
+__device__ __forceinline__ uint64_t warp_sum(uint64_t v) {
+#pragma unroll
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(kAll, v, o);
+  return v;
+}
+
+// sum of the weights of the set bits of m; w: the word's 32 weights (32-byte aligned), bit b <-> byte b.  Each nibble
+// of m becomes a {0, 1} byte selector for __dp4a.
+__device__ __forceinline__ uint32_t weight_sum(uint32_t m, const uint8_t *w) {
+  const uint4 a = __ldg(reinterpret_cast<const uint4 *>(w)), b = __ldg(reinterpret_cast<const uint4 *>(w) + 1);
+  const uint32_t v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  uint32_t s = 0;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) s = __dp4a(v[j], (((m >> (4 * j)) & 0xfu) * 0x00204081u) & 0x01010101u, s);
+  return s;
+}
+
 // slot[g] = max(slot[g], key) for the valid lanes of a warp: one atomic when they share a problem
 __device__ __forceinline__ void put_keys(const bool valid, const int32_t g, const unsigned long long key,
                                          unsigned long long *slot) {
@@ -68,6 +97,9 @@ __device__ __forceinline__ void put_keys(const bool valid, const int32_t g, cons
 
 __device__ __forceinline__ unsigned long long key_of(uint32_t gain, int32_t k) {
   return ((unsigned long long)gain << 32) | (uint32_t)~k;
+}
+__device__ __forceinline__ unsigned long long key_of(uint64_t gain, int32_t k) {
+  return ((unsigned long long)gain << kIdxBits) | (kIdxMask - (uint32_t)k);
 }
 
 // Fallback of phase 1: one thread per box word of pairs [p0, p0 + np).
@@ -107,24 +139,59 @@ __global__ void cover_state_kernel(const uint32_t *__restrict__ target, size_t n
     state[i] = ~__ldg(target + i);
 }
 
+// Weighted rounds, before init: wpad[q][y][w][0..31] = W_q of the word's 32 columns (0 beyond nx; weights null: 1) and
+// state = {W == 0}, bits beyond nx included.  A thread per 4 columns (8 lanes per word): 4-byte stores, and the word's
+// zero-weight bits gathered over its 8 lanes with shuffles.
+__global__ void cover_weight_kernel(const uint8_t *__restrict__ wts, int64_t nprob, CoverGeo G,
+                                    uint8_t *__restrict__ wpad, uint32_t *__restrict__ state) {
+  const int lane = threadIdx.x & 31;
+  const size_t n4 = (size_t)nprob * G.ny * G.nw * 8, step = (size_t)gridDim.x * blockDim.x;
+  // the loop is uniform over the warp (i0 is its first thread's index), so every lane takes part in the shuffles
+  for (size_t i0 = blockIdx.x * (size_t)blockDim.x + threadIdx.x - lane; i0 < n4; i0 += step) {
+    const size_t i = i0 + lane; // 4-column group i & 7 of word i >> 3
+    uint32_t z = 0;
+    if (i < n4) {
+      const size_t word = i >> 3, row = word / G.nw; // row = q * ny + y
+      const int x = 32 * (int)(word - row * G.nw) + 4 * (int)(i & 7);
+      uint32_t v = 0;
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        uint32_t c = 0;
+        if (x + b < G.nx) c = wts ? __ldg(wts + row * G.nx + x + b) : 1u;
+        v |= c << (8 * b);
+        z |= (uint32_t)(c == 0) << b;
+      }
+      reinterpret_cast<uint32_t *>(wpad)[i] = v;
+    }
+    uint32_t m = z << (4 * (lane & 7));
+    m |= __shfl_xor_sync(kAll, m, 1);
+    m |= __shfl_xor_sync(kAll, m, 2);
+    m |= __shfl_xor_sync(kAll, m, 4);
+    if ((lane & 7) == 0 && i < n4) state[i >> 3] = m;
+  }
+}
+
 // gain(c) = |S(c) \ state| of 32 candidates per CTA (a warp per candidate, lanes over rows); disk_r2 >= 0: the disk
 // mask dx^2 + dy^2 <= disk_r2 is applied to the bits in place first.  Then the keys of round 0, and first[q] = the
 // problem's candidate of index 0 (the rounds read no group_ptr: the host form's copy of it may be gone by then).
+// kW: the gain sums the weights of wpad (cover_weight_kernel's plane) instead of counting cells.
+template <bool kW>
 __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__restrict__ bits, int64_t nsrc, CoverGeo G,
                                                                  int disk_r2, const int32_t *__restrict__ xy,
                                                                  const int32_t *__restrict__ pg,
                                                                  const int32_t *__restrict__ pk,
                                                                  const uint32_t *__restrict__ state,
-                                                                 uint32_t *__restrict__ gain,
-                                                                 unsigned long long *slot, int64_t *first) {
-  __shared__ uint32_t sg[kCand];
+                                                                 GainT<kW> *__restrict__ gain,
+                                                                 unsigned long long *slot, int64_t *first,
+                                                                 const uint8_t *__restrict__ wpad) {
+  __shared__ GainT<kW> sg[kCand];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t base = blockIdx.x * (int64_t)kCand;
   const VhpCoverBox b0 = vhp_cover_box(G.nx, G.ny, G.R, 0, 0);
   const size_t hw = (size_t)b0.H * b0.W;
   for (int j = warp; j < kCand; j += kWarps) {
     const int64_t c = base + j;
-    uint32_t acc = 0;
+    GainT<kW> acc = 0;
     const int32_t g = c < nsrc ? __ldg(pg + c) : -1;
     if (g >= 0) {
       const int sx = __ldg(xy + 2 * c), sy = __ldg(xy + 2 * c + 1);
@@ -152,7 +219,12 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
             if (mm != m) row[w] = mm;
             m = mm;
           }
-          if (m) acc += __popc(m & ~__ldg(srow + w));
+          if constexpr (kW) {
+            const uint32_t v = m ? m & ~__ldg(srow + w) : 0u;
+            if (v) acc += weight_sum(v, wpad + (((size_t)g * G.ny + y) * G.nw + b.w0 + w) * 32);
+          } else {
+            if (m) acc += __popc(m & ~__ldg(srow + w));
+          }
         }
       }
       acc = warp_sum(acc);
@@ -163,7 +235,7 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
   if (warp == 0) {
     const int64_t c = base + lane;
     const int32_t g = c < nsrc ? __ldg(pg + c) : -1;
-    const uint32_t gn = sg[lane];
+    const GainT<kW> gn = sg[lane];
     const int32_t kc = g >= 0 ? __ldg(pk + c) : -1;
     if (c < nsrc) gain[c] = gn;
     if (kc == 0) first[g] = c;
@@ -173,18 +245,28 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
 
 // Round r, one CTA per problem: take the slot's pick (gain 0 or a finished problem: done), record it, and update the
 // problem's state over the pick's box.
+template <bool kW>
 __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32_t *__restrict__ bits,
                                                                     const int64_t *__restrict__ first, int64_t nsrc,
                                                                     CoverGeo G,
                                                                     const int32_t *__restrict__ xy, int32_t r,
                                                                     int32_t k, unsigned long long *slot, int64_t *cur,
                                                                     int *done, uint32_t *__restrict__ state,
-                                                                    uint32_t *__restrict__ newb, VhpCoverDev out) {
+                                                                    uint32_t *__restrict__ newb,
+                                                                    VhpCoverDevT<GainT<kW>> out) {
   const int64_t q = blockIdx.x;
   if (done[q]) return;
   const unsigned long long key = slot[q];
   __syncthreads(); // every thread has read the slot before thread 0 resets it
-  const uint32_t gn = (uint32_t)(key >> 32), idx = ~(uint32_t)key;
+  GainT<kW> gn;
+  uint32_t idx;
+  if constexpr (kW) {
+    gn = key >> kIdxBits;
+    idx = (uint32_t)(kIdxMask - (key & kIdxMask));
+  } else {
+    gn = (uint32_t)(key >> 32);
+    idx = ~(uint32_t)key;
+  }
   const int64_t c = first[q] + idx;
   if (gn == 0 || first[q] < 0 || c >= nsrc) { // (the last two: an inconsistent group layout, reported by the table)
     if (threadIdx.x == 0) done[q] = 1;
@@ -216,7 +298,9 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
 }
 
 // After round r's apply: exact gain update of the candidates whose box meets their problem's pick, then the keys of
-// round r + 1.  Candidates of finished problems do nothing; a candidate of gain 0 keeps it.
+// round r + 1.  Candidates of finished problems do nothing; a candidate of gain 0 keeps it.  kW: the weights of
+// wpad's words, loaded only for words where S(c) & new is not 0.
+template <bool kW>
 __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_t *__restrict__ bits, int64_t nsrc,
                                                                    CoverGeo G, const int32_t *__restrict__ xy,
                                                                    const int32_t *__restrict__ pg,
@@ -224,9 +308,10 @@ __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_
                                                                    const int64_t *__restrict__ cur,
                                                                    const int *__restrict__ done,
                                                                    const uint32_t *__restrict__ newb,
-                                                                   uint32_t *__restrict__ gain,
-                                                                   unsigned long long *slot) {
-  __shared__ uint32_t sdec[kCand];
+                                                                   GainT<kW> *__restrict__ gain,
+                                                                   unsigned long long *slot,
+                                                                   const uint8_t *__restrict__ wpad) {
+  __shared__ GainT<kW> sdec[kCand];
   __shared__ unsigned sov;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t base = blockIdx.x * (int64_t)kCand;
@@ -234,7 +319,7 @@ __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_
   const size_t hw = (size_t)b0.H * b0.W;
   bool valid = false;
   int32_t g = -1;
-  uint32_t gn = 0;
+  GainT<kW> gn = 0;
   if (warp == 0) {
     const int64_t c = base + lane;
     g = c < nsrc ? pg[c] : -1;
@@ -266,13 +351,18 @@ __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_
     const VhpCoverBox pb = vhp_cover_box(G.nx, G.ny, G.R, xy[2 * p], xy[2 * p + 1]);
     const int ra = max(cb.y0, pb.y0), rb = min(cb.y0, pb.y0) + b0.H;
     const int wa = max(cb.w0, pb.w0), wb = min(cb.w0, pb.w0) + b0.W;
-    uint32_t acc = 0;
+    GainT<kW> acc = 0;
     for (int y = ra + lane; y < rb; y += 32) {
       const uint32_t *nr = newb + (size_t)q * hw + (size_t)(y - pb.y0) * b0.W - pb.w0;
       const uint32_t *br = bits + (size_t)c * hw + (size_t)(y - cb.y0) * b0.W - cb.w0;
       for (int w = wa; w < wb; ++w) {
         const uint32_t n = nr[w];
-        if (n) acc += __popc(__ldg(br + w) & n);
+        if constexpr (kW) {
+          const uint32_t m = n ? __ldg(br + w) & n : 0u;
+          if (m) acc += weight_sum(m, wpad + (((size_t)q * G.ny + y) * G.nw + w) * 32);
+        } else {
+          if (n) acc += __popc(__ldg(br + w) & n);
+        }
       }
     }
     acc = warp_sum(acc);
@@ -295,33 +385,82 @@ unsigned grid_for(size_t n, int bs, int sm_count) {
 
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
-// workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src], slot [prob], cur [prob], first [prob],
-// done [prob]
+// workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src] (uint32, weighted uint64), slot [prob],
+// cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]
 struct CoverWs {
-  uint32_t *state, *newb, *gain;
+  uint32_t *state, *newb;
+  void *gain;
   unsigned long long *slot;
   int64_t *cur, *first;
   int *done;
+  uint8_t *wpad;
   size_t bytes;
 };
-CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R) {
+CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted) {
   const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
   const size_t np = (size_t)nprob, plane = (size_t)ny * ((nx + 31) / 32);
   const size_t o_new = align256(np * plane * 4), o_gain = o_new + align256(np * b.H * b.W * 4);
-  const size_t o_slot = o_gain + align256((size_t)nsrc * 4), o_cur = o_slot + align256(np * 8);
+  const size_t o_slot = o_gain + align256((size_t)nsrc * (weighted ? 8 : 4)), o_cur = o_slot + align256(np * 8);
   const size_t o_first = o_cur + align256(np * 8), o_done = o_first + align256(np * 8);
+  const size_t o_wpad = o_done + align256(np * 4);
   char *p = static_cast<char *>(base);
   CoverWs w{};
-  w.bytes = o_done + align256(np * 4);
+  w.bytes = o_wpad + (weighted ? align256(np * plane * 32) : 0);
   if (!p) return w;
   w.state = (uint32_t *)p;
   w.newb = (uint32_t *)(p + o_new);
-  w.gain = (uint32_t *)(p + o_gain);
+  w.gain = p + o_gain;
   w.slot = (unsigned long long *)(p + o_slot);
   w.cur = (int64_t *)(p + o_cur);
   w.first = (int64_t *)(p + o_first);
   w.done = (int *)(p + o_done);
+  w.wpad = weighted ? (uint8_t *)(p + o_wpad) : nullptr;
   return w;
+}
+
+// the rounds of both calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null: all 1)
+template <bool kW>
+cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
+                          const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
+                          const uint32_t *d_target, const uint8_t *d_weights, int32_t k, void *d_ws,
+                          const VhpCoverDevT<GainT<kW>> &out, int sm_count, cudaStream_t st, int64_t *launches) {
+  const CoverGeo G{nx, ny, R, (nx + 31) / 32};
+  const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
+  cudaError_t e = cudaSuccess;
+  if (out.pick) e = cudaMemsetAsync(out.pick, 0xff, np * k * 4, st); // -1 from npicked on
+  if (e == cudaSuccess && out.gain) e = cudaMemsetAsync(out.gain, 0, np * k * sizeof(GainT<kW>), st);
+  if (e == cudaSuccess && out.npicked) e = cudaMemsetAsync(out.npicked, 0, np * 4, st);
+  if (e == cudaSuccess && out.covered) e = cudaMemsetAsync(out.covered, 0, np * plane * 4, st);
+  const int64_t rounds = std::min<int64_t>(k, nsrc);
+  if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
+  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW);
+  GainT<kW> *gain = (GainT<kW> *)ws.gain;
+  if (kW) {
+    cover_weight_kernel<<<grid_for(np * plane * 8, 256, sm_count), 256, 0, st>>>(d_weights, nprob, G, ws.wpad,
+                                                                                 ws.state);
+    if (launches) *launches += 1;
+  } else if (d_target) {
+    cover_state_kernel<<<grid_for(np * plane, 256, sm_count), 256, 0, st>>>(d_target, np * plane, ws.state);
+    if (launches) *launches += 1;
+  } else {
+    e = cudaMemsetAsync(ws.state, 0, np * plane * 4, st);
+  }
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.slot, 0, np * 8, st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.done, 0, np * 4, st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0xff, np * 8, st);
+  if (e != cudaSuccess) return e;
+  const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
+  cover_init_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
+                                                      gain, ws.slot, ws.first, ws.wpad);
+  for (int32_t r = 0; r < rounds; ++r) {
+    cover_apply_kernel<kW><<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k, ws.slot,
+                                                                      ws.cur, ws.done, ws.state, ws.newb, out);
+    if (r + 1 < rounds)
+      cover_update_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
+                                                            ws.done, ws.newb, gain, ws.slot, ws.wpad);
+  }
+  if (launches) *launches += 2 * rounds;
+  return cudaGetLastError();
 }
 
 } // namespace
@@ -338,44 +477,23 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
   return cudaGetLastError();
 }
 
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R) {
-  return cover_ws(nullptr, nprob, nsrc, nx, ny, R).bytes;
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted) {
+  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted).bytes;
 }
 
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
                                     int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
                                     const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
                                     const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches) {
-  const CoverGeo G{nx, ny, R, (nx + 31) / 32};
-  const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
-  cudaError_t e = cudaSuccess;
-  if (out.pick) e = cudaMemsetAsync(out.pick, 0xff, np * k * 4, st); // -1 from npicked on
-  if (e == cudaSuccess && out.gain) e = cudaMemsetAsync(out.gain, 0, np * k * 4, st);
-  if (e == cudaSuccess && out.npicked) e = cudaMemsetAsync(out.npicked, 0, np * 4, st);
-  if (e == cudaSuccess && out.covered) e = cudaMemsetAsync(out.covered, 0, np * plane * 4, st);
-  const int64_t rounds = std::min<int64_t>(k, nsrc);
-  if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
-  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R);
-  if (d_target) {
-    cover_state_kernel<<<grid_for(np * plane, 256, sm_count), 256, 0, st>>>(d_target, np * plane, ws.state);
-    if (launches) *launches += 1;
-  } else {
-    e = cudaMemsetAsync(ws.state, 0, np * plane * 4, st);
-  }
-  if (e == cudaSuccess) e = cudaMemsetAsync(ws.slot, 0, np * 8, st);
-  if (e == cudaSuccess) e = cudaMemsetAsync(ws.done, 0, np * 4, st);
-  if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0xff, np * 8, st);
-  if (e != cudaSuccess) return e;
-  const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
-  cover_init_kernel<<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
-                                                  ws.gain, ws.slot, ws.first);
-  for (int32_t r = 0; r < rounds; ++r) {
-    cover_apply_kernel<<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k, ws.slot, ws.cur,
-                                                                  ws.done, ws.state, ws.newb, out);
-    if (r + 1 < rounds)
-      cover_update_kernel<<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
-                                                        ws.done, ws.newb, ws.gain, ws.slot);
-  }
-  if (launches) *launches += 2 * rounds;
-  return cudaGetLastError();
+  return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, d_target,
+                              nullptr, k, d_ws, out, sm_count, st, launches);
+}
+
+cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
+                                             int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                             const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, void *d_ws,
+                                             const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
+                                             int64_t *launches) {
+  return launch_rounds<true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
+                             d_weights, k, d_ws, out, sm_count, st, launches);
 }

@@ -293,20 +293,30 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
                                   bool disk, int r2, const int32_t *d_xy, double thr, uint32_t *d_bits, int sm_count,
                                   cudaStream_t st, int64_t *launches);
 // Phase 2, the greedy rounds over the bits of nsrc candidates (table of vhp_launch_merge_table) of nprob problems.
-struct VhpCoverDev {
+// Gain is uint32 (cells) for the cover call, uint64 (summed weights) for the weighted call.
+template <class Gain>
+struct VhpCoverDevT {
   int32_t *pick = nullptr;   // [prob][k]
-  uint32_t *gain = nullptr;  // [prob][k]
+  Gain *gain = nullptr;      // [prob][k]
   int32_t *npicked = nullptr; // [prob]
   uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
 };
-// workspace bytes of the rounds beyond the candidate bits
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R);
+using VhpCoverDev = VhpCoverDevT<uint32_t>;
+using VhpCoverWeightedDev = VhpCoverDevT<uint64_t>;
+// workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane)
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted);
 // outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
 // route's sweep stores the whole box); d_target (may be null): [prob][ny][ceil(nx/32)] bits of the cells to cover
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
                                     int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
                                     const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
                                     const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches);
+// the weighted rounds: d_weights (may be null: every cell weighs 1) [prob][ny][nx] uint8; nsrc < 2^28
+cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
+                                             int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                             const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, void *d_ws,
+                                             const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
+                                             int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
