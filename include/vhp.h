@@ -320,6 +320,49 @@ vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, cons
                                                           int32_t shape, double threshold, const uint8_t *d_weights,
                                                           const vhp_cover_weighted_out *d_out);
 
+/* Redundant (m-fold) greedy sensor placement: which k candidates see the most summed importance, where a cell counts
+ * until m of the picks cover it (coverage that survives a failed sensor, two or three views of a target, overlapping
+ * camera views).  Problems, candidates, group_map, radius, shape, threshold, S(c) and the weights W_q (NULL: every
+ * cell weighs 1) are exactly those of vhp_visibility_cover_greedy_weighted_batch.  m in [1, 255].
+ *   f(A) = sum over x of W_q(x) * min(cnt_A(x), m), cnt_A(x) = the number of picks in A whose S covers x
+ * Greedy, A = {} and every cnt 0, for r = 0 .. k-1: gain(c) = sum of W_q(x) over x in S(c) with cnt(x) < m for every
+ * candidate of the problem not yet picked; p = argmax, ties to the smallest index within the group; if gain(p) == 0
+ * stop (npicked = r), else cnt += 1 over S(p), saturating at m.  A candidate is picked at most once.  Duplicates are
+ * separate entries, so with m >= 2 two identical candidates can both be picked.  Every gain is an exact integer sum and
+ * every decision an integer comparison.  Outputs (any may be NULL, at least one must be given):
+ *   pick[q][r]     index within the group of the r-th pick, -1 from npicked on            (int32 [prob][k])
+ *   gain[q][r]     summed weight the r-th pick adds to f, 0 from npicked on               (uint64 [prob][k])
+ *   npicked[q]                                                                            (int32 [prob])
+ *   count[q]       min(m, number of picks whose S covers the cell), every cell whatever its weight
+ *                  ([prob][ny][nx] uint8) = min(m, count) of vhp_visibility_merge_range_batch on the picks
+ * so gains are non-increasing, sum of gain = sum over x of W_q(x) * count(x), and the result is within (1 - 1/e) of
+ * the best k-subset (f is monotone submodular).  m = 1 gives exactly the pick, gain and npicked of
+ * vhp_visibility_cover_greedy_weighted_batch, and count is its covered unpacked.  There is no target: weights in
+ * {0, 1} are the target.
+ * Routes, phase 1 and the 2^28 limit are those of vhp_visibility_cover_greedy_weighted_batch; the rounds also keep a
+ * uint8 counter per cell in 32-byte rows per 32-column word.  Workspace: that of
+ * vhp_visibility_cover_greedy_weighted_batch plus 32 * ny * ceil(nx/32) bytes per problem; the host form's 4 GB batches
+ * also count each problem's ny * nx count bytes.  Errors (VHP_ERR_INVALID_ARG): those of
+ * vhp_visibility_cover_greedy_weighted_batch (the 2^28 limit checked before any candidate is read), m outside
+ * [1, 255], no output.  k == 0 is valid (npicked 0, count all zero). */
+typedef struct vhp_cover_mfold_out {
+  int32_t *pick;
+  uint64_t *gain;
+  int32_t *npicked;
+  uint8_t *count;
+} vhp_cover_mfold_out;
+vhp_status vhp_visibility_cover_greedy_mfold_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                   const int32_t *cand_xy, const int64_t *group_ptr,
+                                                   const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
+                                                   int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                                   const vhp_cover_mfold_out *out);
+vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                       int ny, const int32_t *d_cand_xy, const int64_t *d_group_ptr,
+                                                       const int32_t *d_group_map, int64_t nprob, int64_t nsrc,
+                                                       int32_t k, int32_t radius, int32_t shape, double threshold,
+                                                       const uint8_t *d_weights, int32_t m,
+                                                       const vhp_cover_mfold_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

@@ -60,6 +60,12 @@ class CoverWeightedOut(C.Structure):
     _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("covered", C.c_void_p)]
 
 
+class CoverMfoldOut(C.Structure):
+    """struct vhp_cover_mfold_out: pick (int32 [prob][k]), gain (uint64 [prob][k]), npicked (int32 [prob]), count
+    (uint8 [prob][ny][nx]), each may be NULL."""
+    _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("count", C.c_void_p)]
+
+
 class SweepVariant(C.Structure):
     """struct vhp_sweep_variant: model 1 = getAccessibilityMap.m (alpha, fac, light_strength),
     model 2 = computeVisibilityUsingQueue as an order-free rule (cutoff)."""
@@ -142,6 +148,12 @@ def load_library(build_if_missing: bool = True):
     lib.vhp_visibility_cover_greedy_weighted_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64,
                                                                    C.c_int32, C.c_int32, C.c_int32, C.c_double, vp,
                                                                    C.POINTER(CoverWeightedOut)]
+    lib.vhp_visibility_cover_greedy_mfold_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, C.c_int32,
+                                                            C.c_int32, C.c_int32, C.c_double, vp, C.c_int32,
+                                                            C.POINTER(CoverMfoldOut)]
+    lib.vhp_visibility_cover_greedy_mfold_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64,
+                                                                C.c_int32, C.c_int32, C.c_int32, C.c_double, vp,
+                                                                C.c_int32, C.POINTER(CoverMfoldOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -545,6 +557,48 @@ class Context:
             self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
             group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
             ptr(weights_t), C.byref(co)))
+
+    def visibility_cover_greedy_mfold_batch(self, occ, cand_xy, group_ptr, k, m, threshold, radius, shape,
+                                            weights=None, group_map=None):
+        """Redundant (m-fold) greedy sensor placement (vhp_visibility_cover_greedy_mfold_batch): as
+        visibility_cover_greedy_weighted_batch, but a cell's weight counts until m (1..255) picks cover it, so each
+        round takes the candidate, not yet picked, whose cells covered fewer than m times weigh the most.  Returns pick
+        (int32 (nprob, k)), gain (uint64 (nprob, k), summed weight the pick adds), npicked (int32 (nprob,)) and count
+        (uint8 (nprob, ny, nx), min(m, number of picks covering the cell))."""
+        occ = _occ_u8(occ)
+        nmaps, ny, nx = occ.shape
+        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        npb = gp.shape[0] - 1
+        n = max(npb, 0)
+        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
+        if weights is not None:
+            w = np.asarray(weights)
+            if w.dtype != np.uint8 or w.shape != (n, ny, nx):
+                raise ValueError(f"weights must be uint8 of shape {(n, ny, nx)}, got {w.dtype} {w.shape}")
+            weights = np.ascontiguousarray(w)
+        k = int(k)
+        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint64),
+                 npicked=np.empty(n, np.int32), count=np.empty((n, ny, nx), np.uint8))
+        co = CoverMfoldOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "count")])
+        self._check(self.lib.vhp_visibility_cover_greedy_mfold_batch(
+            self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp), _np_ptr(gm), npb, k, int(radius),
+            int(shape), float(threshold), _np_ptr(weights), int(m), C.byref(co)))
+        return r
+
+    def visibility_cover_greedy_mfold_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, k, m, threshold, radius, shape,
+                                                pick_t=None, gain_t=None, npicked_t=None, count_t=None,
+                                                group_map_t=None, weights_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2),
+        group_ptr_t int64 (nprob + 1), weights_t uint8 (nprob, ny, nx) or None; outputs pick_t int32 (nprob, k),
+        gain_t int64 / uint64 (nprob, k), npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx); any may be None."""
+        nmaps, ny, nx = occ_t.shape
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        co = CoverMfoldOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(count_t))
+        self._check(self.lib.vhp_visibility_cover_greedy_mfold_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
+            group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
+            ptr(weights_t), int(m), C.byref(co)))
 
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):

@@ -1133,13 +1133,20 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
 // straight into bits (kFmtCoverBits: threshold > 0 and window_direct_route), the fallback folds chunks of fp64
 // windows (run_window_dev, any of its routes) or, where a window would be larger than the map, of whole fields
 // (run_dev) with cover_fold_kernel.  Phase 2 (kernels_cover.cu) runs min(k, nsrc) greedy rounds on the device.
-// The weighted call (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds.
+// The weighted call (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds, the
+// m-fold call (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
 const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
+const char *const kCoverMfoldName = "vhp_visibility_cover_greedy_mfold_batch";
 // the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
 constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
-// Out: vhp_cover_out or vhp_cover_weighted_out
+// the per-cell output of each cover call: the covered bits, or the m-fold call's counts
+void *cover_cells(const vhp_cover_out *o) { return o->covered; }
+void *cover_cells(const vhp_cover_weighted_out *o) { return o->covered; }
+void *cover_cells(const vhp_cover_mfold_out *o) { return o->count; }
+
+// Out: vhp_cover_out, vhp_cover_weighted_out or vhp_cover_mfold_out
 template <class Out>
 vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k, const VhpMergeRange &range,
@@ -1153,20 +1160,33 @@ vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx
   if (st != VHP_OK) return st;
   if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
   if (k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": k < 0");
-  if (!out->pick && !out->gain && !out->npicked && !out->covered)
+  if (!out->pick && !out->gain && !out->npicked && !cover_cells(out))
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
   return check_range(ctx, what, range);
 }
 
 // the cover call's checks, then the weighted key's limit on nsrc (before any candidate is read)
+template <class Out>
 vhp_status check_cover_weighted_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                                      const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
-                                     const VhpMergeRange &range, double thr, const vhp_cover_weighted_out *out) {
+                                     const VhpMergeRange &range, double thr, const Out *out,
+                                     const char *name = kCoverWeightedName) {
   const vhp_status st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr, out,
-                                         kCoverWeightedName);
+                                         name);
   if (st != VHP_OK) return st;
   if (nsrc >= kCoverWeightedMaxSrc)
-    return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverWeightedName) + ": 2^28 or more candidates");
+    return fail(ctx, VHP_ERR_INVALID_ARG, std::string(name) + ": 2^28 or more candidates");
+  return VHP_OK;
+}
+
+// the weighted call's checks, then m
+vhp_status check_cover_mfold_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
+                                  const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
+                                  const VhpMergeRange &range, double thr, int32_t m, const vhp_cover_mfold_out *out) {
+  const vhp_status st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr,
+                                                  out, kCoverMfoldName);
+  if (st != VHP_OK) return st;
+  if (m < 1 || m > 255) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverMfoldName) + ": m outside [1, 255]");
   return VHP_OK;
 }
 
@@ -1197,11 +1217,11 @@ struct CoverBits {
   int disk_r2 = -1;                     // >= 0: the direct route stored the whole box, the rounds apply the disk
 };
 
-// Phase 1 of both cover calls: the table, the workspace of the rounds (ws_bytes) and every candidate's coverage bits
+// Phase 1 of the cover calls: the table, the workspace of the rounds (ws_bytes) and every candidate's coverage bits
 vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
                             const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb) {
-  const char *name = weighted ? kCoverWeightedName : kCoverName;
+                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb, bool mfold = false) {
+  const char *name = mfold ? kCoverMfoldName : weighted ? kCoverWeightedName : kCoverName;
   const int R = std::min(range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
   const bool disk = range.shape == VHP_RANGE_DISK;
   const int r2 = range.radius * range.radius;
@@ -1220,8 +1240,8 @@ vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, i
       if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits", name)) !=
           VHP_OK)
         return st;
-      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, weighted), "workspace",
-                             name)) != VHP_OK)
+      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, weighted, mfold),
+                             "workspace", name)) != VHP_OK)
         return st;
       uint32_t *bits = cb.bits = (uint32_t *)ctx->b_cover.p;
       if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
@@ -1276,22 +1296,41 @@ vhp_status run_cover_weighted_dev(vhp_context *ctx, const uint8_t *d_occ, int nm
   return VHP_OK;
 }
 
+vhp_status run_cover_mfold_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                               const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
+                               const VhpMergeRange &range, double thr, const uint8_t *d_weights, int32_t m,
+                               const VhpCoverMfoldDev &out) {
+  CoverBits cb;
+  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
+                                         true, cb, true);
+  if (st != VHP_OK) return st;
+  VHP_CUDA(ctx, vhp_launch_cover_greedy_mfold(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk,
+                                              d_weights, k, m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
+                                              &ctx->launches));
+  return VHP_OK;
+}
+
 // host buffers: validate, upload maps and candidates once, then runs of whole problems whose device memory (candidate
-// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync.  kW: the
-// weighted call, extra = weights ([prob][ny][nx] uint8), else extra = target ([prob][ny][ceil(nx/32)] uint32); either
-// may be null.
-template <bool kW>
+// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync.  Out picks
+// the call: vhp_cover_out, extra = target ([prob][ny][ceil(nx/32)] uint32); vhp_cover_weighted_out, extra = weights
+// ([prob][ny][nx] uint8); vhp_cover_mfold_out, extra = weights and m, and count ([prob][ny][nx] uint8) instead of
+// covered.  extra may be null.
+template <class Out>
 vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
                           const int64_t *gptr, const int32_t *gmap, int64_t nprob, int32_t k,
-                          const VhpMergeRange &range, double thr, const void *extra,
-                          const typename std::conditional<kW, vhp_cover_weighted_out, vhp_cover_out>::type *out) {
-  using Dev = typename std::conditional<kW, VhpCoverWeightedDev, VhpCoverDev>::type;
+                          const VhpMergeRange &range, double thr, const void *extra, const Out *out, int32_t m = 1) {
+  constexpr bool kM = std::is_same<Out, vhp_cover_mfold_out>::value;
+  constexpr bool kW = kM || std::is_same<Out, vhp_cover_weighted_out>::value;
+  using Dev = typename std::conditional<
+      kM, VhpCoverMfoldDev, typename std::conditional<kW, VhpCoverWeightedDev, VhpCoverDev>::type>::type;
   using Gain = typename std::remove_pointer<decltype(Dev::gain)>::type;
-  const char *name = kW ? kCoverWeightedName : kCoverName;
+  const char *name = kM ? kCoverMfoldName : kW ? kCoverWeightedName : kCoverName;
   vhp_status st = check_groups_host(ctx, name, gptr, nprob);
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
-  if constexpr (kW)
+  if constexpr (kM)
+    st = check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, m, out);
+  else if constexpr (kW)
     st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
   else
     st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
@@ -1309,12 +1348,12 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(range.radius, std::max(nx, ny) - 1), 0, 0);
   const size_t box = (size_t)b.H * b.W * 4, budget = (size_t)4 << 30;
   const size_t bp = out->pick ? 4 * (size_t)k : 0, bg = out->gain ? sizeof(Gain) * (size_t)k : 0;
-  const size_t bn = out->npicked ? 4 : 0, bc = out->covered ? plane * 4 : 0;
+  const size_t bn = out->npicked ? 4 : 0, bc = cover_cells(out) ? (kM ? (size_t)ny * nx : plane * 4) : 0;
   const size_t bt = extra ? (kW ? (size_t)ny * nx : plane * 4) : 0;
   // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
-  // the weighted rounds' 32-byte rows of weights)
+  // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters)
   const size_t per_src = box + 12 + sizeof(Gain), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
-                                                             (kW ? plane * 32 : 0);
+                                                             (kW ? plane * 32 : 0) + (kM ? plane * 32 : 0);
   auto prob_bytes = [&](int64_t q) { return (size_t)(gptr[q + 1] - gptr[q]) * per_src + per_prob; };
   std::vector<int64_t> h_ptr;
   const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
@@ -1335,7 +1374,11 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     o.pick = out->pick ? (int32_t *)base : nullptr;
     o.gain = out->gain ? (Gain *)(base + o_gain) : nullptr;
     o.npicked = out->npicked ? (int32_t *)(base + o_gain + gc * bg) : nullptr;
-    o.covered = out->covered ? (uint32_t *)(base + o_gain + gc * (bg + bn)) : nullptr;
+    char *cells = cover_cells(out) ? base + o_gain + gc * (bg + bn) : nullptr;
+    if constexpr (kM)
+      o.count = (uint8_t *)cells;
+    else
+      o.covered = (uint32_t *)cells;
     cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
                                     ctx->stream);
     if (e == cudaSuccess && gmap)
@@ -1347,7 +1390,10 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     const uint8_t *d_occ = (const uint8_t *)ctx->b_occ.p;
     const int64_t *d_gptr = (const int64_t *)ctx->b_misc.p;
     const int32_t *d_gmap = gmap ? (const int32_t *)ctx->b_map.p : nullptr;
-    if constexpr (kW)
+    if constexpr (kM)
+      result = run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k,
+                                   range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o);
+    else if constexpr (kW)
       result = run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a,
                                       k, range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, o);
     else
@@ -1359,8 +1405,8 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
       e = cudaMemcpyAsync(out->gain + q0 * k, o.gain, gc * bg, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && out->npicked)
       e = cudaMemcpyAsync(out->npicked + q0, o.npicked, gc * bn, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && out->covered)
-      e = cudaMemcpyAsync(out->covered + q0 * plane, o.covered, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && cells)
+      e = cudaMemcpyAsync((char *)cover_cells(out) + q0 * bc, cells, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
     if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: copy of the outputs"); break; }
     ctx->last_d2h_bytes += (int64_t)(gc * (bp + bg + bn + bc));
@@ -1941,8 +1987,8 @@ vhp_status vhp_visibility_cover_greedy_batch(vhp_context *ctx, const uint8_t *oc
   VhpMergeRange range;
   range.radius = radius;
   range.shape = shape;
-  return run_cover_host<false>(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold,
-                               target, out);
+  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, target,
+                        out);
 }
 
 vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -1969,8 +2015,8 @@ vhp_status vhp_visibility_cover_greedy_weighted_batch(vhp_context *ctx, const ui
   VhpMergeRange range;
   range.radius = radius;
   range.shape = shape;
-  return run_cover_host<true>(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold,
-                              weights, out);
+  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
+                        out);
 }
 
 vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
@@ -1988,6 +2034,40 @@ vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, cons
   VHP_ON_DEVICE(ctx);
   return run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
                                 threshold, d_weights, cover_dev_of<VhpCoverWeightedDev>(*d_out));
+}
+
+vhp_status vhp_visibility_cover_greedy_mfold_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                   const int32_t *cand_xy, const int64_t *group_ptr,
+                                                   const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
+                                                   int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                                   const vhp_cover_mfold_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
+                        out, m);
+}
+
+vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                       int ny, const int32_t *d_cand_xy, const int64_t *d_group_ptr,
+                                                       const int32_t *d_group_map, int64_t nprob, int64_t nsrc,
+                                                       int32_t k, int32_t radius, int32_t shape, double threshold,
+                                                       const uint8_t *d_weights, int32_t m,
+                                                       const vhp_cover_mfold_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  vhp_status st = check_cover_mfold_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
+                                         threshold, m, d_out);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  VhpCoverMfoldDev o;
+  o.pick = d_out->pick;
+  o.gain = d_out->gain;
+  o.npicked = d_out->npicked;
+  o.count = d_out->count;
+  return run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
+                             threshold, d_weights, m, o);
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

@@ -14,6 +14,11 @@
 // The weighted rounds (vhp_visibility_cover_greedy_weighted_batch) are the same kernels instantiated with kW = true:
 // state starts as {W == 0} (cover_weight_kernel, which also copies the weights into a plane of 32-byte rows per word),
 // gains are uint64 sums of the weights of the set bits (weight_sum), and the key is (gain << 28) | (2^28 - 1 - index).
+//
+// The m-fold rounds (vhp_visibility_cover_greedy_mfold_batch) are the weighted rounds with the apply step instantiated
+// with kM = true: a per-problem plane of uint8 counters cnt(x) = min(m, picks whose S covers x) in wpad's layout, and
+// state |= new, new = the cells that reach m this round (so a cell's weight leaves the gains only then).  Init and
+// update are the weighted instances as they are: a gain is still sum W over S(c) \ state, and it changes only by new.
 #include <algorithm>
 #include <cstdint>
 #include <type_traits>
@@ -244,8 +249,10 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
 }
 
 // Round r, one CTA per problem: take the slot's pick (gain 0 or a finished problem: done), record it, and update the
-// problem's state over the pick's box.
-template <bool kW>
+// problem's state over the pick's box.  kM (m-fold, with kW): cnt += 1 over S(p) saturating at mfold (cnt: the
+// counter plane, wpad's layout), new = the cells that reach mfold now and are not in state, state |= new, and the
+// pick's gain is zeroed (with mfold >= 2 it keeps gain on its own cells).  gain, cnt and mfold are unused otherwise.
+template <bool kW, bool kM>
 __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32_t *__restrict__ bits,
                                                                     const int64_t *__restrict__ first, int64_t nsrc,
                                                                     CoverGeo G,
@@ -253,7 +260,8 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
                                                                     int32_t k, unsigned long long *slot, int64_t *cur,
                                                                     int *done, uint32_t *__restrict__ state,
                                                                     uint32_t *__restrict__ newb,
-                                                                    VhpCoverDevT<GainT<kW>> out) {
+                                                                    VhpCoverDevT<GainT<kW>> out, GainT<kW> *gain,
+                                                                    uint8_t *__restrict__ cnt, int mfold) {
   const int64_t q = blockIdx.x;
   if (done[q]) return;
   const unsigned long long key = slot[q];
@@ -278,6 +286,7 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
     if (out.npicked) out.npicked[q] = r + 1;
     cur[q] = c;
     slot[q] = 0;
+    if constexpr (kM) gain[c] = 0;
   }
   const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, __ldg(xy + 2 * c), __ldg(xy + 2 * c + 1));
   const int hw = b.H * b.W;
@@ -289,10 +298,63 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
     const int rr = i / b.W, w = i - rr * b.W;
     const size_t o = (size_t)(b.y0 + rr) * G.nw + b.w0 + w;
     const uint32_t m = __ldg(bc + i), s = sq[o];
-    nq[i] = m & ~s;
-    if (m) {
-      sq[o] = s | m;
-      if (cov) cov[o] |= m;
+    if constexpr (kM) {
+      uint32_t nw = 0;
+      if (m) {
+        // the word's 32 counters, byte b <-> bit b; each nibble of m becomes a {0, 1} byte selector (weight_sum)
+        uint4 *cw = reinterpret_cast<uint4 *>(cnt + ((size_t)q * plane + o) * 32);
+        uint4 a = cw[0], b2 = cw[1];
+        uint32_t v[8] = {a.x, a.y, a.z, a.w, b2.x, b2.y, b2.z, b2.w};
+        const uint32_t top = (uint32_t)(mfold - 1) * 0x01010101u, lim = top + 0x01010101u;
+        uint32_t eq = 0; // bits whose counter is mfold - 1 before this pick
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const uint32_t sel = (((m >> (4 * j)) & 0xfu) * 0x00204081u) & 0x01010101u;
+          eq |= ((((__vcmpeq4(v[j], top) & 0x01010101u) * 0x01020408u) >> 24) & 0xfu) << (4 * j);
+          v[j] += sel & __vcmpltu4(v[j], lim); // counters < mfold <= 255: no carry between bytes
+        }
+        cw[0] = make_uint4(v[0], v[1], v[2], v[3]);
+        cw[1] = make_uint4(v[4], v[5], v[6], v[7]);
+        nw = m & ~s & eq;
+        if (nw) sq[o] = s | nw;
+      }
+      nq[i] = nw;
+    } else {
+      nq[i] = m & ~s;
+      if (m) {
+        sq[o] = s | m;
+        if (cov) cov[o] |= m;
+      }
+    }
+  }
+}
+
+// m-fold output: count[row][x] = cnt[row][x] for rows (problem, y) of the padded counter plane (32 bytes per word).
+// A thread per 16 columns: one aligned 16-byte load, and stores as wide as the destination's alignment allows (the
+// caller's rows are nx bytes, so a row of count starts 16-byte aligned only where row * nx is a multiple of 16).
+__global__ void cover_count_kernel(const uint8_t *__restrict__ cnt, size_t nrows, int nx, int nw,
+                                   uint8_t *__restrict__ count) {
+  const int nch = (nx + 15) >> 4;
+  const size_t n = nrows * nch;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    const size_t row = i / nch;
+    const int x = 16 * (int)(i - row * nch);
+    const uint4 v = __ldg(reinterpret_cast<const uint4 *>(cnt + row * nw * 32 + x));
+    uint8_t *dst = count + row * nx + x;
+    const unsigned a = (unsigned)reinterpret_cast<uintptr_t>(dst) & 15u;
+    if (x + 16 <= nx && a == 0) {
+      *reinterpret_cast<uint4 *>(dst) = v;
+    } else if (x + 16 <= nx && (a & 3u) == 0) {
+      uint32_t *d = reinterpret_cast<uint32_t *>(dst);
+      d[0] = v.x;
+      d[1] = v.y;
+      d[2] = v.z;
+      d[3] = v.w;
+    } else {
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int b = 0; b < 16; ++b)
+        if (x + b < nx) dst[b] = (uint8_t)(w[b >> 2] >> (8 * (b & 3)));
     }
   }
 }
@@ -386,26 +448,26 @@ unsigned grid_for(size_t n, int bs, int sm_count) {
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 // workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src] (uint32, weighted uint64), slot [prob],
-// cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]
+// cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]; m-fold (weighted too): cnt, wpad's layout
 struct CoverWs {
   uint32_t *state, *newb;
   void *gain;
   unsigned long long *slot;
   int64_t *cur, *first;
   int *done;
-  uint8_t *wpad;
+  uint8_t *wpad, *cnt;
   size_t bytes;
 };
-CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted) {
+CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold) {
   const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
   const size_t np = (size_t)nprob, plane = (size_t)ny * ((nx + 31) / 32);
   const size_t o_new = align256(np * plane * 4), o_gain = o_new + align256(np * b.H * b.W * 4);
   const size_t o_slot = o_gain + align256((size_t)nsrc * (weighted ? 8 : 4)), o_cur = o_slot + align256(np * 8);
   const size_t o_first = o_cur + align256(np * 8), o_done = o_first + align256(np * 8);
-  const size_t o_wpad = o_done + align256(np * 4);
+  const size_t o_wpad = o_done + align256(np * 4), o_cnt = o_wpad + (weighted ? align256(np * plane * 32) : 0);
   char *p = static_cast<char *>(base);
   CoverWs w{};
-  w.bytes = o_wpad + (weighted ? align256(np * plane * 32) : 0);
+  w.bytes = o_cnt + (mfold ? align256(np * plane * 32) : 0);
   if (!p) return w;
   w.state = (uint32_t *)p;
   w.newb = (uint32_t *)(p + o_new);
@@ -415,15 +477,18 @@ CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R,
   w.first = (int64_t *)(p + o_first);
   w.done = (int *)(p + o_done);
   w.wpad = weighted ? (uint8_t *)(p + o_wpad) : nullptr;
+  w.cnt = mfold ? (uint8_t *)(p + o_cnt) : nullptr;
   return w;
 }
 
-// the rounds of both calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null: all 1)
-template <bool kW>
+// the rounds of the three calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null:
+// all 1), kM (with kW) counts each cell until mfold picks cover it and writes d_count (may be null) at the end
+template <bool kW, bool kM = false>
 cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                           const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
-                          const uint32_t *d_target, const uint8_t *d_weights, int32_t k, void *d_ws,
-                          const VhpCoverDevT<GainT<kW>> &out, int sm_count, cudaStream_t st, int64_t *launches) {
+                          const uint32_t *d_target, const uint8_t *d_weights, int32_t k, int mfold, void *d_ws,
+                          const VhpCoverDevT<GainT<kW>> &out, uint8_t *d_count, int sm_count, cudaStream_t st,
+                          int64_t *launches) {
   const CoverGeo G{nx, ny, R, (nx + 31) / 32};
   const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
   cudaError_t e = cudaSuccess;
@@ -432,8 +497,9 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   if (e == cudaSuccess && out.npicked) e = cudaMemsetAsync(out.npicked, 0, np * 4, st);
   if (e == cudaSuccess && out.covered) e = cudaMemsetAsync(out.covered, 0, np * plane * 4, st);
   const int64_t rounds = std::min<int64_t>(k, nsrc);
+  if (e == cudaSuccess && d_count && rounds <= 0) e = cudaMemsetAsync(d_count, 0, np * ny * nx, st); // no pick
   if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
-  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW);
+  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW, kM);
   GainT<kW> *gain = (GainT<kW> *)ws.gain;
   if (kW) {
     cover_weight_kernel<<<grid_for(np * plane * 8, 256, sm_count), 256, 0, st>>>(d_weights, nprob, G, ws.wpad,
@@ -448,18 +514,26 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   if (e == cudaSuccess) e = cudaMemsetAsync(ws.slot, 0, np * 8, st);
   if (e == cudaSuccess) e = cudaMemsetAsync(ws.done, 0, np * 4, st);
   if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0xff, np * 8, st);
+  if (e == cudaSuccess && kM) e = cudaMemsetAsync(ws.cnt, 0, np * plane * 32, st);
   if (e != cudaSuccess) return e;
   const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
   cover_init_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
                                                       gain, ws.slot, ws.first, ws.wpad);
   for (int32_t r = 0; r < rounds; ++r) {
-    cover_apply_kernel<kW><<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k, ws.slot,
-                                                                      ws.cur, ws.done, ws.state, ws.newb, out);
+    cover_apply_kernel<kW, kM><<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k,
+                                                                          ws.slot, ws.cur, ws.done, ws.state, ws.newb,
+                                                                          out, gain, ws.cnt, mfold);
     if (r + 1 < rounds)
       cover_update_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
                                                             ws.done, ws.newb, gain, ws.slot, ws.wpad);
   }
   if (launches) *launches += 2 * rounds;
+  if (kM && d_count) {
+    const size_t nrows = np * ny;
+    cover_count_kernel<<<grid_for(nrows * ((nx + 15) / 16), 256, sm_count), 256, 0, st>>>(ws.cnt, nrows, nx, G.nw,
+                                                                                          d_count);
+    if (launches) *launches += 1;
+  }
   return cudaGetLastError();
 }
 
@@ -477,8 +551,8 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
   return cudaGetLastError();
 }
 
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted) {
-  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted).bytes;
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold) {
+  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold, mfold).bytes;
 }
 
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
@@ -486,7 +560,7 @@ cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t npro
                                     const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
                                     const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches) {
   return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, d_target,
-                              nullptr, k, d_ws, out, sm_count, st, launches);
+                              nullptr, k, 1, d_ws, out, nullptr, sm_count, st, launches);
 }
 
 cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
@@ -495,5 +569,18 @@ cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int
                                              const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
                                              int64_t *launches) {
   return launch_rounds<true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
-                             d_weights, k, d_ws, out, sm_count, st, launches);
+                             d_weights, k, 1, d_ws, out, nullptr, sm_count, st, launches);
+}
+
+cudaError_t vhp_launch_cover_greedy_mfold(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
+                                          int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                          const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, int m,
+                                          void *d_ws, const VhpCoverMfoldDev &out, int sm_count, cudaStream_t st,
+                                          int64_t *launches) {
+  VhpCoverWeightedDev o;
+  o.pick = out.pick;
+  o.gain = out.gain;
+  o.npicked = out.npicked;
+  return launch_rounds<true, true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
+                                   d_weights, k, m, d_ws, o, out.count, sm_count, st, launches);
 }

@@ -303,8 +303,16 @@ struct VhpCoverDevT {
 };
 using VhpCoverDev = VhpCoverDevT<uint32_t>;
 using VhpCoverWeightedDev = VhpCoverDevT<uint64_t>;
-// workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane)
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted);
+// the m-fold call's outputs: gains as the weighted call's, count instead of covered
+struct VhpCoverMfoldDev {
+  int32_t *pick = nullptr;    // [prob][k]
+  uint64_t *gain = nullptr;   // [prob][k]
+  int32_t *npicked = nullptr; // [prob]
+  uint8_t *count = nullptr;   // [prob][ny][nx], min(m, picks whose S covers the cell)
+};
+// workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane; m-fold:
+// those of the weighted rounds and a counter plane of the padded plane's size)
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold = false);
 // outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
 // route's sweep stores the whole box); d_target (may be null): [prob][ny][ceil(nx/32)] bits of the cells to cover
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
@@ -317,6 +325,12 @@ cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int
                                              const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, void *d_ws,
                                              const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
                                              int64_t *launches);
+// the m-fold rounds: the weighted rounds, where a cell's weight counts until m in [1, 255] picks cover it
+cudaError_t vhp_launch_cover_greedy_mfold(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
+                                          int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
+                                          const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, int m,
+                                          void *d_ws, const VhpCoverMfoldDev &out, int sm_count, cudaStream_t st,
+                                          int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
