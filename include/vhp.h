@@ -363,6 +363,44 @@ vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const u
                                                        const uint8_t *d_weights, int32_t m,
                                                        const vhp_cover_mfold_out *d_out);
 
+/* Directional greedy sensor placement: cameras with a field of view, and fleets that mix sensing ranges.  Everything
+ * is vhp_visibility_cover_greedy_mfold_batch (problems, candidates, group_map, radius R, shape, threshold, weights,
+ * m, the greedy, ties, outputs, the 2^28 limit, k == 0), with each candidate's S(c) narrowed to its view:
+ *   S_view(c) = S(c) & view(c)
+ * views ([nsrc][5] int32) holds (r, ax, ay, bx, by) for each candidate.  Directions are in the grid's (x, y), x the
+ * column and y the row: a positive cross(a, b) turns from increasing column towards increasing row, which is clockwise
+ * on an image drawn with row 0 at the top.  With dx = x - sx, dy = y - sy, d = (dx, dy) and cross(u, v) = u.x * v.y - u.y * v.x (64-bit), view(c)
+ * is the cells with
+ *   range      the call's shape with radius r: |dx|, |dy| <= r (VHP_RANGE_BOX) or dx^2 + dy^2 <= r^2 (VHP_RANGE_DISK);
+ *              0 <= r <= R, the call's radius (R still sets the box of the candidate bits and the workspace)
+ *   direction  c1 = cross(a, d) and c2 = cross(d, b):
+ *              cross(a, b) > 0 (the sector from a towards b is under 180 degrees): c1 >= 0 and c2 >= 0;
+ *              cross(a, b) < 0, or cross(a, b) == 0 and dot(a, b) < 0 (180 degrees or more): c1 >= 0 or c2 >= 0;
+ *              cross(a, b) == 0 and dot(a, b) > 0 (a and b point the same way, a == b included): every direction;
+ *              d = (0, 0), the sensor's own cell, is always in it.
+ * The sectors are defined by integer vectors alone, so the result is exact and order-independent.  Every view
+ * omnidirectional (a == b) with r = R gives exactly vhp_visibility_cover_greedy_mfold_batch's pick, gain, npicked
+ * and count.
+ * Routes and phase 1 are those of vhp_visibility_cover_greedy_mfold_batch; one more kernel then masks each candidate's
+ * bits in place, once, before the rounds.  Workspace: that of vhp_visibility_cover_greedy_mfold_batch; the host form
+ * uploads the views with the candidates and its 4 GB batches also count each candidate's 20 view bytes.
+ * Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_cover_greedy_mfold_batch; views NULL with nsrc > 0; a view
+ * with r outside [0, R], a or b equal to (0, 0), or a component outside [-32767, 32767].  The host form checks the
+ * views before any candidate is read.  The _dev form reports a bad view like a bad candidate, by the next
+ * synchronising call with its own message, and that candidate covers nothing; with k == 0 or no problem the views
+ * are not read. */
+vhp_status vhp_visibility_cover_greedy_view_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                  const int32_t *cand_xy, const int32_t *views,
+                                                  const int64_t *group_ptr, const int32_t *group_map, int64_t nprob,
+                                                  int32_t k, int32_t radius, int32_t shape, double threshold,
+                                                  const uint8_t *weights, int32_t m, const vhp_cover_mfold_out *out);
+vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                      int ny, const int32_t *d_cand_xy, const int32_t *d_views,
+                                                      const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                                      int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
+                                                      int32_t shape, double threshold, const uint8_t *d_weights,
+                                                      int32_t m, const vhp_cover_mfold_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

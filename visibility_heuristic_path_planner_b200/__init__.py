@@ -154,6 +154,12 @@ def load_library(build_if_missing: bool = True):
     lib.vhp_visibility_cover_greedy_mfold_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64,
                                                                 C.c_int32, C.c_int32, C.c_int32, C.c_double, vp,
                                                                 C.c_int32, C.POINTER(CoverMfoldOut)]
+    lib.vhp_visibility_cover_greedy_view_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, C.c_int32,
+                                                           C.c_int32, C.c_int32, C.c_double, vp, C.c_int32,
+                                                           C.POINTER(CoverMfoldOut)]
+    lib.vhp_visibility_cover_greedy_view_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64,
+                                                               C.c_int32, C.c_int32, C.c_int32, C.c_double, vp,
+                                                               C.c_int32, C.POINTER(CoverMfoldOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -600,6 +606,52 @@ class Context:
             group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
             ptr(weights_t), int(m), C.byref(co)))
 
+    def visibility_cover_greedy_view_batch(self, occ, cand_xy, views, group_ptr, k, m, threshold, radius, shape,
+                                           weights=None, group_map=None):
+        """Directional greedy sensor placement (vhp_visibility_cover_greedy_view_batch): as
+        visibility_cover_greedy_mfold_batch, with each candidate's coverage narrowed to its view.  views: int32
+        (nsrc, 5), (r, ax, ay, bx, by) per candidate: range r (0 <= r <= radius) in the call's shape and the sector
+        from a = (ax, ay) to b = (bx, by), in the grid's (x, y) = (column, row); see sensor_views.  Returns pick, gain,
+        npicked and count as visibility_cover_greedy_mfold_batch."""
+        occ = _occ_u8(occ)
+        nmaps, ny, nx = occ.shape
+        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
+        vw = np.ascontiguousarray(views, dtype=np.int32).reshape(-1, 5)
+        if vw.shape[0] != xy.shape[0]:
+            raise ValueError(f"views must have one row per candidate ({xy.shape[0]}), got {vw.shape[0]}")
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        npb = gp.shape[0] - 1
+        n = max(npb, 0)
+        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
+        if weights is not None:
+            w = np.asarray(weights)
+            if w.dtype != np.uint8 or w.shape != (n, ny, nx):
+                raise ValueError(f"weights must be uint8 of shape {(n, ny, nx)}, got {w.dtype} {w.shape}")
+            weights = np.ascontiguousarray(w)
+        k = int(k)
+        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint64),
+                 npicked=np.empty(n, np.int32), count=np.empty((n, ny, nx), np.uint8))
+        co = CoverMfoldOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "count")])
+        self._check(self.lib.vhp_visibility_cover_greedy_view_batch(
+            self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(vw), _np_ptr(gp), _np_ptr(gm), npb, k,
+            int(radius), int(shape), float(threshold), _np_ptr(weights), int(m), C.byref(co)))
+        return r
+
+    def visibility_cover_greedy_view_batch_dev(self, occ_t, cand_xy_t, views_t, group_ptr_t, k, m, threshold, radius,
+                                               shape, pick_t=None, gain_t=None, npicked_t=None, count_t=None,
+                                               group_map_t=None, weights_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2), views_t
+        int32 (nsrc, 5), group_ptr_t int64 (nprob + 1), weights_t uint8 (nprob, ny, nx) or None; outputs pick_t int32
+        (nprob, k), gain_t int64 / uint64 (nprob, k), npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx); any may
+        be None.  A bad view is reported by the next synchronising call."""
+        nmaps, ny, nx = occ_t.shape
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        co = CoverMfoldOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(count_t))
+        self._check(self.lib.vhp_visibility_cover_greedy_view_batch_dev(
+            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), ptr(views_t), group_ptr_t.data_ptr(),
+            ptr(group_map_t), group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape),
+            float(threshold), ptr(weights_t), int(m), C.byref(co)))
+
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):
         """Opt-in sweep variants (vhp_visibility_variant_batch): VARIANT_MATLAB =
@@ -743,6 +795,36 @@ def pack_bits(cells):
     pad = np.zeros(cells.shape[:-1] + (32 * ((nx + 31) // 32),), bool)
     pad[..., :nx] = cells
     return np.ascontiguousarray(np.packbits(pad, axis=-1, bitorder="little")).view("<u4")
+
+
+def sensor_views(heading_deg, fov_deg, radius, scale=32767):
+    """Views for visibility_cover_greedy_view_batch: int32 (n, 5) rows (r, ax, ay, bx, by) from headings and fields of
+    view in degrees (scalars or arrays, broadcast together).  Angles are measured from +x (the column) towards +y (the
+    row).  a = round(scale * dir(heading - fov / 2)) and b = round(scale * dir(heading + fov / 2)); fov >= 360 gives
+    a == b = round(scale * dir(heading)), every direction.  The library sees only these integer vectors: they, not the
+    angles, define the view, so a sector edge is the rounded direction (at scale 32767 within about 2e-3 degrees).
+    Raises ValueError when fov <= 0, scale is outside [1, 32767], or fov < 360 but the rounded a and b point the same
+    way, which the library would read as every direction."""
+    h, f, r = np.broadcast_arrays(np.asarray(heading_deg, np.float64), np.asarray(fov_deg, np.float64),
+                                  np.asarray(radius, np.int64))
+    h, f, r = h.reshape(-1), f.reshape(-1), r.reshape(-1)
+    if not 1 <= int(scale) <= 32767:
+        raise ValueError(f"scale must be in [1, 32767], got {scale}")
+    if (f <= 0).any():
+        raise ValueError("fov must be positive")
+    full = f >= 360
+    half = np.where(full, 0.0, f / 2)
+    ta, tb = np.radians(h - half), np.radians(h + half)
+    a = np.rint(int(scale) * np.stack([np.cos(ta), np.sin(ta)], 1)).astype(np.int64)
+    b = np.rint(int(scale) * np.stack([np.cos(tb), np.sin(tb)], 1)).astype(np.int64)
+    cross = a[:, 0] * b[:, 1] - a[:, 1] * b[:, 0]
+    dot = a[:, 0] * b[:, 0] + a[:, 1] * b[:, 1]
+    same = (cross == 0) & (dot > 0) & ~full
+    if same.any():
+        i = int(np.flatnonzero(same)[0])
+        raise ValueError(f"fov {f[i]} at heading {h[i]}: the rounded sector edges point the same way "
+                         f"(a = {tuple(a[i])}, b = {tuple(b[i])}); use a larger fov or scale")
+    return np.ascontiguousarray(np.concatenate([r[:, None], a, b], 1).astype(np.int32))
 
 
 def torch_context(device: int, stream) -> Context:

@@ -157,6 +157,10 @@ vhp_status check_device_error(vhp_context *ctx) {
     VHP_CUDA(ctx, cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
     if (flag & 4)
       return fail(ctx, VHP_ERR_INVALID_ARG, "inconsistent source groups (group_ptr / group_map)");
+    if (flag & 8)
+      return fail(ctx, VHP_ERR_INVALID_ARG,
+                  "a candidate's view (r, ax, ay, bx, by) is invalid: r outside [0, radius], a or b (0, 0), or a "
+                  "component outside [-32767, 32767]");
     return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
   }
   return VHP_OK;
@@ -1134,10 +1138,13 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
 // windows (run_window_dev, any of its routes) or, where a window would be larger than the map, of whole fields
 // (run_dev) with cover_fold_kernel.  Phase 2 (kernels_cover.cu) runs min(k, nsrc) greedy rounds on the device.
 // The weighted call (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds, the
-// m-fold call (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters.
+// m-fold call (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters, and
+// the view call (vhp_visibility_cover_greedy_view_batch) the m-fold call with each candidate's bits masked by its view
+// in between.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
 const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
 const char *const kCoverMfoldName = "vhp_visibility_cover_greedy_mfold_batch";
+const char *const kCoverViewName = "vhp_visibility_cover_greedy_view_batch";
 // the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
 constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
@@ -1190,6 +1197,33 @@ vhp_status check_cover_mfold_args(vhp_context *ctx, const void *occ, int nmaps, 
   return VHP_OK;
 }
 
+// the m-fold call's checks, then the views' buffer (their values: check_views_host, or bit 3 of d_err on the device)
+vhp_status check_cover_view_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
+                                 const void *views, const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
+                                 const VhpMergeRange &range, double thr, int32_t m, const vhp_cover_mfold_out *out) {
+  const vhp_status st = check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr, m,
+                                               out);
+  if (st != VHP_OK) return st;
+  if (nsrc > 0 && !views) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverViewName) + ": views is NULL");
+  return VHP_OK;
+}
+
+// host-side validation of the views [n][5] = (r, ax, ay, bx, by), the rule of cover_view_kernel
+vhp_status check_views_host(vhp_context *ctx, const int32_t *views, int64_t n, int radius) {
+  for (int64_t i = 0; i < n; ++i) {
+    const int32_t *v = views + 5 * i;
+    const char *bad = nullptr;
+    if (v[0] < 0 || v[0] > radius) bad = "r outside [0, radius]";
+    for (int j = 1; j < 5 && !bad; ++j)
+      if (v[j] < -32767 || v[j] > 32767) bad = "a component outside [-32767, 32767]";
+    if (!bad && ((v[1] == 0 && v[2] == 0) || (v[3] == 0 && v[4] == 0))) bad = "a or b is (0, 0)";
+    if (bad)
+      return fail(ctx, VHP_ERR_INVALID_ARG,
+                  std::string(kCoverViewName) + ": view of candidate " + std::to_string(i) + ": " + bad);
+  }
+  return VHP_OK;
+}
+
 // Out: vhp_cover_out or vhp_cover_weighted_out, Dev: VhpCoverDev or VhpCoverWeightedDev
 template <class Dev, class Out>
 Dev cover_dev_of(const Out &o) {
@@ -1220,8 +1254,9 @@ struct CoverBits {
 // Phase 1 of the cover calls: the table, the workspace of the rounds (ws_bytes) and every candidate's coverage bits
 vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
                             const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb, bool mfold = false) {
-  const char *name = mfold ? kCoverMfoldName : weighted ? kCoverWeightedName : kCoverName;
+                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb, bool mfold = false,
+                            const char *call = nullptr) {
+  const char *name = call ? call : mfold ? kCoverMfoldName : weighted ? kCoverWeightedName : kCoverName;
   const int R = std::min(range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
   const bool disk = range.shape == VHP_RANGE_DISK;
   const int r2 = range.radius * range.radius;
@@ -1310,27 +1345,50 @@ vhp_status run_cover_mfold_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps
   return VHP_OK;
 }
 
+// the view call: phase 1, the bits masked by the views (range r_c in the call's shape, so the rounds apply no disk),
+// then the m-fold rounds
+vhp_status run_cover_view_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
+                              const int32_t *d_views, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
+                              int64_t nsrc, int32_t k, const VhpMergeRange &range, double thr,
+                              const uint8_t *d_weights, int32_t m, const VhpCoverMfoldDev &out) {
+  CoverBits cb;
+  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
+                                         true, cb, true, kCoverViewName);
+  if (st != VHP_OK) return st;
+  if (cb.bits)
+    VHP_CUDA(ctx, vhp_launch_cover_view(cb.bits, nsrc, nx, ny, cb.R, range.radius, range.shape == VHP_RANGE_DISK, d_xy,
+                                        d_views, ctx->d_err, ctx->sm_count, ctx->stream, &ctx->launches));
+  VHP_CUDA(ctx, vhp_launch_cover_greedy_mfold(cb.bits, nsrc, nprob, nx, ny, cb.R, -1, d_xy, cb.pg, cb.pk, d_weights,
+                                              k, m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
+                                              &ctx->launches));
+  return VHP_OK;
+}
+
 // host buffers: validate, upload maps and candidates once, then runs of whole problems whose device memory (candidate
 // bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync.  Out picks
 // the call: vhp_cover_out, extra = target ([prob][ny][ceil(nx/32)] uint32); vhp_cover_weighted_out, extra = weights
 // ([prob][ny][nx] uint8); vhp_cover_mfold_out, extra = weights and m, and count ([prob][ny][nx] uint8) instead of
-// covered.  extra may be null.
+// covered.  extra may be null.  view (with vhp_cover_mfold_out): the view call, views [nsrc][5] uploaded with the
+// candidates.
 template <class Out>
 vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
                           const int64_t *gptr, const int32_t *gmap, int64_t nprob, int32_t k,
-                          const VhpMergeRange &range, double thr, const void *extra, const Out *out, int32_t m = 1) {
+                          const VhpMergeRange &range, double thr, const void *extra, const Out *out, int32_t m = 1,
+                          bool view = false, const int32_t *views = nullptr) {
   constexpr bool kM = std::is_same<Out, vhp_cover_mfold_out>::value;
   constexpr bool kW = kM || std::is_same<Out, vhp_cover_weighted_out>::value;
   using Dev = typename std::conditional<
       kM, VhpCoverMfoldDev, typename std::conditional<kW, VhpCoverWeightedDev, VhpCoverDev>::type>::type;
   using Gain = typename std::remove_pointer<decltype(Dev::gain)>::type;
-  const char *name = kM ? kCoverMfoldName : kW ? kCoverWeightedName : kCoverName;
+  const char *name = view ? kCoverViewName : kM ? kCoverMfoldName : kW ? kCoverWeightedName : kCoverName;
   vhp_status st = check_groups_host(ctx, name, gptr, nprob);
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
-  if constexpr (kM)
-    st = check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, m, out);
-  else if constexpr (kW)
+  if constexpr (kM) {
+    st = view ? check_cover_view_args(ctx, occ, nmaps, nx, ny, xy, views, gptr, nprob, nsrc, k, range, thr, m, out)
+              : check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, m, out);
+    if (st == VHP_OK && view) st = check_views_host(ctx, views, nsrc, range.radius);
+  } else if constexpr (kW)
     st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
   else
     st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
@@ -1344,6 +1402,10 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   PlanesGuard planes_guard(ctx);
   if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
     return st;
+  if (view && nsrc > 0) {
+    if ((st = ensure(ctx, ctx->b_views, 20 * (size_t)nsrc)) != VHP_OK) return st;
+    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_views.p, views, 20 * (size_t)nsrc, cudaMemcpyHostToDevice, ctx->stream));
+  }
   const size_t plane = (size_t)ny * ((nx + 31) / 32);
   const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(range.radius, std::max(nx, ny) - 1), 0, 0);
   const size_t box = (size_t)b.H * b.W * 4, budget = (size_t)4 << 30;
@@ -1351,8 +1413,8 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   const size_t bn = out->npicked ? 4 : 0, bc = cover_cells(out) ? (kM ? (size_t)ny * nx : plane * 4) : 0;
   const size_t bt = extra ? (kW ? (size_t)ny * nx : plane * 4) : 0;
   // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
-  // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters)
-  const size_t per_src = box + 12 + sizeof(Gain), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
+  // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters; views: 20 bytes)
+  const size_t per_src = box + 12 + sizeof(Gain) + (view ? 20 : 0), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
                                                              (kW ? plane * 32 : 0) + (kM ? plane * 32 : 0);
   auto prob_bytes = [&](int64_t q) { return (size_t)(gptr[q + 1] - gptr[q]) * per_src + per_prob; };
   std::vector<int64_t> h_ptr;
@@ -1391,8 +1453,12 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     const int64_t *d_gptr = (const int64_t *)ctx->b_misc.p;
     const int32_t *d_gmap = gmap ? (const int32_t *)ctx->b_map.p : nullptr;
     if constexpr (kM)
-      result = run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k,
-                                   range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o);
+      result = view ? run_cover_view_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, (const int32_t *)ctx->b_views.p + 5 * a,
+                                         d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k, range, thr,
+                                         extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o)
+                    : run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc,
+                                          gptr[q0 + gc] - a, k, range, thr,
+                                          extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o);
     else if constexpr (kW)
       result = run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a,
                                       k, range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, o);
@@ -1664,7 +1730,7 @@ void vhp_context_destroy(vhp_context *ctx) {
   if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
   VhpDevBuf *bufs[] = {&ctx->b_occ, &ctx->b_src, &ctx->b_map, &ctx->b_out[0], &ctx->b_out[1],
                        &ctx->b_scratch, &ctx->b_planner, &ctx->b_misc, &ctx->b_grid, &ctx->b_bin,
-                       &ctx->b_merge, &ctx->b_mwin, &ctx->b_cover, &ctx->b_cover_ws};
+                       &ctx->b_merge, &ctx->b_mwin, &ctx->b_cover, &ctx->b_cover_ws, &ctx->b_views};
   for (VhpDevBuf *b : bufs)
     if (b->p) cudaFree(b->p);
   delete ctx->expand_pool;
@@ -2068,6 +2134,40 @@ vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const u
   o.count = d_out->count;
   return run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
                              threshold, d_weights, m, o);
+}
+
+vhp_status vhp_visibility_cover_greedy_view_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                                  const int32_t *cand_xy, const int32_t *views,
+                                                  const int64_t *group_ptr, const int32_t *group_map, int64_t nprob,
+                                                  int32_t k, int32_t radius, int32_t shape, double threshold,
+                                                  const uint8_t *weights, int32_t m, const vhp_cover_mfold_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
+                        out, m, true, views);
+}
+
+vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
+                                                      int ny, const int32_t *d_cand_xy, const int32_t *d_views,
+                                                      const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                                      int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
+                                                      int32_t shape, double threshold, const uint8_t *d_weights,
+                                                      int32_t m, const vhp_cover_mfold_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  vhp_status st = check_cover_view_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_views, d_group_ptr, nprob, nsrc, k,
+                                        range, threshold, m, d_out);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  VhpCoverMfoldDev o;
+  o.pick = d_out->pick;
+  o.gain = d_out->gain;
+  o.npicked = d_out->npicked;
+  o.count = d_out->count;
+  return run_cover_view_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_views, d_group_ptr, d_group_map, nprob, nsrc, k,
+                            range, threshold, d_weights, m, o);
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

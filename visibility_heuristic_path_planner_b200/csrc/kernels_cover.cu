@@ -19,6 +19,9 @@
 // with kM = true: a per-problem plane of uint8 counters cnt(x) = min(m, picks whose S covers x) in wpad's layout, and
 // state |= new, new = the cells that reach m this round (so a cell's weight leaves the gains only then).  Init and
 // update are the weighted instances as they are: a gain is still sum W over S(c) \ state, and it changes only by new.
+//
+// The view call (vhp_visibility_cover_greedy_view_batch) narrows every S(c) to its candidate's view once, in place,
+// with cover_view_kernel between phase 1 and the m-fold rounds; the rounds cannot tell masked bits from swept ones.
 #include <algorithm>
 #include <cstdint>
 #include <type_traits>
@@ -359,6 +362,91 @@ __global__ void cover_count_kernel(const uint8_t *__restrict__ cnt, size_t nrows
   }
 }
 
+// floor and ceiling of n / d, d != 0 (C division truncates toward zero)
+__device__ __forceinline__ long long floor_div(long long n, long long d) {
+  const long long q = n / d;
+  return (n % d != 0 && ((n < 0) != (d < 0))) ? q - 1 : q;
+}
+__device__ __forceinline__ long long ceil_div(long long n, long long d) {
+  const long long q = n / d;
+  return (n % d != 0 && ((n < 0) == (d < 0))) ? q + 1 : q;
+}
+
+constexpr int kViewInf = 1 << 20; // beyond any dx of a box (|dx| <= 16383 + 31)
+
+// the dx of a row with u * dx <= v, as [lo, hi] clamped to [-kViewInf, kViewInf] (empty: lo > hi)
+__device__ __forceinline__ void half_plane(long long u, long long v, int &lo, int &hi) {
+  lo = -kViewInf;
+  hi = kViewInf;
+  if (u > 0) {
+    hi = (int)max(min(floor_div(v, u), (long long)kViewInf), (long long)-kViewInf);
+  } else if (u < 0) {
+    lo = (int)max(min(ceil_div(v, u), (long long)kViewInf), (long long)-kViewInf);
+  } else if (v < 0) {
+    lo = 1;
+    hi = 0;
+  }
+}
+
+// The view call, after phase 1: S(c) &= view(c) in place, a warp per candidate, lanes over its box's rows.  view(c) =
+// range r (the call's shape) and the sector of a = (ax, ay), b = (bx, by): cross(a, d) >= 0 and cross(d, b) >= 0 under
+// 180 degrees (cross(a, b) > 0), either one from 180 degrees on (cross(a, b) < 0, or 0 with dot(a, b) < 0), every d
+// when a and b point the same way.  On a row each half-plane is one dx interval, so the row's view is at most two.  A
+// bad view (r outside [0, radius], a or b zero or a component outside [-32767, 32767]) raises bit 3 of err and clears
+// the candidate's bits.  Only words that change are stored.
+__global__ void __launch_bounds__(kWarps * 32) cover_view_kernel(uint32_t *__restrict__ bits, int64_t nsrc, CoverGeo G,
+                                                                 int radius, bool disk,
+                                                                 const int32_t *__restrict__ xy,
+                                                                 const int32_t *__restrict__ views, int *err) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const VhpCoverBox b0 = vhp_cover_box(G.nx, G.ny, G.R, 0, 0);
+  const size_t hw = (size_t)b0.H * b0.W;
+  for (int64_t c = blockIdx.x * (int64_t)kWarps + warp; c < nsrc; c += (int64_t)gridDim.x * kWarps) {
+    const int sx = __ldg(xy + 2 * c), sy = __ldg(xy + 2 * c + 1);
+    const int32_t *v = views + 5 * c;
+    const int r = __ldg(v), ax = __ldg(v + 1), ay = __ldg(v + 2), bx = __ldg(v + 3), by = __ldg(v + 4);
+    const auto comp_ok = [](int t) { return t >= -32767 && t <= 32767; };
+    const bool ok = r >= 0 && r <= radius && comp_ok(ax) && comp_ok(ay) && comp_ok(bx) && comp_ok(by) &&
+                    (ax | ay) != 0 && (bx | by) != 0;
+    if (!ok && lane == 0) atomicOr(err, 8);
+    const long long cab = (long long)ax * by - (long long)ay * bx, dab = (long long)ax * bx + (long long)ay * by;
+    const int mode = cab > 0 ? 0 : (cab < 0 || dab < 0) ? 1 : 2; // intersection, union, every direction
+    const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, sx, sy);
+    uint32_t *bc = bits + (size_t)c * hw;
+    for (int rr = lane; rr < b.H; rr += 32) {
+      const int dy = b.y0 + rr - sy;
+      int lo1 = 1, hi1 = 0, lo2 = 1, hi2 = 0; // the row's view: [lo1, hi1] | [lo2, hi2] in dx
+      if (ok && abs(dy) <= r) {
+        const int h = disk ? isqrt_floor(r * r - dy * dy) : r;
+        lo1 = -h;
+        hi1 = h;
+        if (mode != 2) {
+          int la, ha, lb, hb;
+          half_plane(ay, (long long)ax * dy, la, ha);   // cross(a, d) >= 0: ay * dx <= ax * dy
+          half_plane(-by, -(long long)bx * dy, lb, hb); // cross(d, b) >= 0: by * dx >= bx * dy
+          if (mode == 0) {
+            lo1 = max(lo1, max(la, lb));
+            hi1 = min(hi1, min(ha, hb));
+          } else {
+            lo2 = max(lo1, lb);
+            hi2 = min(hi1, hb);
+            lo1 = max(lo1, la);
+            hi1 = min(hi1, ha);
+          }
+        }
+      }
+      uint32_t *row = bc + (size_t)rr * b.W;
+      for (int w = 0; w < b.W; ++w) {
+        const uint32_t m = row[w];
+        if (!m) continue;
+        const int o = sx - 32 * (b.w0 + w); // bit of dx = 0
+        const uint32_t mm = m & (span_mask(o + lo1, o + hi1) | span_mask(o + lo2, o + hi2));
+        if (mm != m) row[w] = mm;
+      }
+    }
+  }
+}
+
 // After round r's apply: exact gain update of the candidates whose box meets their problem's pick, then the keys of
 // round r + 1.  Candidates of finished problems do nothing; a candidate of gain 0 keeps it.  kW: the weights of
 // wpad's words, loaded only for words where S(c) & new is not 0.
@@ -547,6 +635,18 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
   const int bs = 256;
   cover_fold_kernel<<<grid_for((size_t)np * b.H * b.W, bs, sm_count), bs, 0, st>>>(d_val, win_r, p0, np, G, disk, r2,
                                                                                    d_xy, thr, d_bits);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t vhp_launch_cover_view(uint32_t *d_bits, int64_t nsrc, int nx, int ny, int R, int radius, bool disk,
+                                  const int32_t *d_xy, const int32_t *d_views, int *d_err, int sm_count,
+                                  cudaStream_t st, int64_t *launches) {
+  if (nsrc <= 0) return cudaSuccess;
+  const CoverGeo G{nx, ny, R, (nx + 31) / 32};
+  cover_view_kernel<<<grid_for((size_t)nsrc * 32, kWarps * 32, sm_count), kWarps * 32, 0, st>>>(d_bits, nsrc, G, radius,
+                                                                                             disk, d_xy, d_views,
+                                                                                             d_err);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

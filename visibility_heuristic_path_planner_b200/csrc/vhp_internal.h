@@ -103,7 +103,8 @@ struct vhp_context {
   int sm_count = 0;
   int64_t launches = 0;
   std::string last_error;
-  // device-side error word (bit 0: a source / start / end outside the grid, bit 2: inconsistent source groups)
+  // device-side error word (bit 0: a source / start / end outside the grid, bit 2: inconsistent source groups,
+  // bit 3: a bad view of vhp_visibility_cover_greedy_view_batch_dev)
   int *d_err = nullptr;
   // workspace buffers (grown on demand, reused across calls)
   VhpDevBuf b_occ, b_src, b_map, b_out[2], b_scratch, b_planner, b_misc, b_grid, b_bin;
@@ -113,6 +114,8 @@ struct vhp_context {
   VhpDevBuf b_mwin;
   // vhp_visibility_cover_greedy_batch: the candidates' coverage bits, and the workspace of the greedy rounds
   VhpDevBuf b_cover, b_cover_ws;
+  // vhp_visibility_cover_greedy_view_batch: the candidates' views, uploaded with the candidates
+  VhpDevBuf b_views;
   cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
   // 1/k table {rh, rl} of the tile kernel (double-double reciprocal), device resident
   double *rcp2_table = nullptr;
@@ -331,6 +334,12 @@ cudaError_t vhp_launch_cover_greedy_mfold(uint32_t *d_bits, int64_t nsrc, int64_
                                           const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, int m,
                                           void *d_ws, const VhpCoverMfoldDev &out, int sm_count, cudaStream_t st,
                                           int64_t *launches);
+// the view call, between phase 1 and the m-fold rounds (which then run with disk_r2 = -1): every candidate's bits
+// &= its view, d_views [nsrc][5] = (r, ax, ay, bx, by): range r in [0, radius] in the call's shape (disk or box), and
+// the sector of a and b.  A bad view raises bit 3 of d_err and clears the candidate's bits.
+cudaError_t vhp_launch_cover_view(uint32_t *d_bits, int64_t nsrc, int nx, int ny, int R, int radius, bool disk,
+                                  const int32_t *d_xy, const int32_t *d_views, int *d_err, int sm_count,
+                                  cudaStream_t st, int64_t *launches);
 
 // opt-in sweep variants (kernels_sweep_variant.cu): model 1 getAccessibilityMap.m (alpha, fac),
 // model 2 computeVisibilityUsingQueue as an order-free rule (cutoff)
