@@ -401,6 +401,32 @@ vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const ui
                                                       int32_t shape, double threshold, const uint8_t *d_weights,
                                                       int32_t m, const vhp_cover_mfold_out *d_out);
 
+/* Directional merged visibility: what a set of cameras with headings and fields of view covers together, the
+ * evaluation counterpart of vhp_visibility_cover_greedy_view_batch.  Everything is vhp_visibility_merge_range_batch
+ * (inputs, groups, group_map, radius R, shape, threshold, dtype, the outputs and the "writes" rule), with source k's
+ * range narrowed to its view, views[k] = (r, ax, ay, bx, by) ([nsrc][5] int32), by exactly the rule of
+ * vhp_visibility_cover_greedy_view_batch (range r <= R in the call's shape, the sector of a and b by integer cross
+ * products, the sensor's own cell always in it):
+ *   vmax[g][y][x]   max_k of (source k's field where the cell is in view(k), else 0)
+ *   first / count   the range merge's rule further narrowed to view(k)
+ * Every view omnidirectional (a == b) with r = R gives exactly vhp_visibility_merge_range_batch's outputs.  For a
+ * singleton group {c}, count is 1 exactly on S_view(c) of the view cover call, and min(m, count) over its picks is
+ * that call's count.  Routes and launches are those of vhp_visibility_merge_range_batch; the host form uploads the
+ * views with the sources.
+ * Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_merge_range_batch; views NULL with nsrc > 0; a view with r
+ * outside [0, R], a or b equal to (0, 0), or a component outside [-32767, 32767].  The host form checks the views
+ * before any source is read.  The _dev form reports a bad view by the next synchronising call with its own message,
+ * and that source contributes nothing; with no groups the views are not read. */
+vhp_status vhp_visibility_merge_view_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                           const int32_t *src_xy, const int32_t *views, const int64_t *group_ptr,
+                                           const int32_t *group_map, int64_t ngroups, int32_t radius, int32_t shape,
+                                           double threshold, vhp_dtype dtype, const vhp_merge_out *out);
+vhp_status vhp_visibility_merge_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                               const int32_t *d_src_xy, const int32_t *d_views,
+                                               const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                               int64_t ngroups, int64_t nsrc, int32_t radius, int32_t shape,
+                                               double threshold, vhp_dtype dtype, const vhp_merge_out *d_out);
+
 /* Range-limited visibility: for every (map, source) pair the (2R+1) x (2R+1) window centred on the source,
  *   out[p][v][u] = visibility_(sx - R + u, sy - R + v) of vhp_visibility_batch for pair p where that cell lies
  *                  inside the grid, 0 where it does not                           (u, v in [0, 2R])

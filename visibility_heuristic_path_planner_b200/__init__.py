@@ -138,6 +138,10 @@ def load_library(build_if_missing: bool = True):
                                                      C.c_double, i32, C.POINTER(MergeOut)]
     lib.vhp_visibility_merge_range_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_int32,
                                                          C.c_int32, C.c_double, i32, C.POINTER(MergeOut)]
+    lib.vhp_visibility_merge_view_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, C.c_int32, C.c_int32,
+                                                    C.c_double, i32, C.POINTER(MergeOut)]
+    lib.vhp_visibility_merge_view_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64, C.c_int32,
+                                                        C.c_int32, C.c_double, i32, C.POINTER(MergeOut)]
     lib.vhp_visibility_cover_greedy_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, C.c_int32, C.c_int32,
                                                       C.c_int32, C.c_double, vp, C.POINTER(CoverOut)]
     lib.vhp_visibility_cover_greedy_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, i64, i64, C.c_int32,
@@ -441,10 +445,22 @@ class Context:
         return self._merge_host(self.lib.vhp_visibility_merge_range_batch, (int(radius), int(shape)), occ, src_xy,
                                 group_ptr, threshold, group_map, dtype, outputs)
 
-    def _merge_host(self, fn, extra, occ, src_xy, group_ptr, threshold, group_map, dtype, outputs):
+    def visibility_merge_view_batch(self, occ, src_xy, views, group_ptr, threshold, radius, shape, group_map=None,
+                                    dtype=F64, outputs=("vmax", "first", "count")):
+        """Directional merged visibility (vhp_visibility_merge_view_batch): visibility_merge_range_batch where each
+        source only covers the cells in its view.  views: int32 (nsrc, 5), (r, ax, ay, bx, by) per source, the rule of
+        visibility_cover_greedy_view_batch (see sensor_views)."""
+        vw = np.ascontiguousarray(views, dtype=np.int32).reshape(-1, 5)
+        return self._merge_host(self.lib.vhp_visibility_merge_view_batch, (int(radius), int(shape)), occ, src_xy,
+                                group_ptr, threshold, group_map, dtype, outputs, views=vw)
+
+    def _merge_host(self, fn, extra, occ, src_xy, group_ptr, threshold, group_map, dtype, outputs, views=None):
         occ = _occ_u8(occ)
         nmaps, ny, nx = occ.shape
         xy = np.ascontiguousarray(src_xy, dtype=np.int32).reshape(-1, 2)
+        if views is not None and views.shape[0] != xy.shape[0]:
+            raise ValueError(f"views must have one row per source ({xy.shape[0]}), got {views.shape[0]}")
+        lead = () if views is None else (_np_ptr(views),)
         gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
         ng = gp.shape[0] - 1
         gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
@@ -453,7 +469,7 @@ class Context:
             raise ValueError(f"outputs are among {tuple(kinds)}")
         r = {k: np.empty((max(ng, 0), ny, nx), kinds[k]) for k in outputs}
         mo = MergeOut(*[_np_ptr(r.get(k)) for k in ("vmax", "first", "count")])
-        self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp), _np_ptr(gm), ng, *extra,
+        self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), *lead, _np_ptr(gp), _np_ptr(gm), ng, *extra,
                        float(threshold), dtype, C.byref(mo)))
         return r
 
@@ -471,13 +487,22 @@ class Context:
         self._merge_dev(self.lib.vhp_visibility_merge_range_batch_dev, (int(radius), int(shape)), occ_t, src_xy_t,
                         group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t)
 
-    def _merge_dev(self, fn, extra, occ_t, src_xy_t, group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t):
+    def visibility_merge_view_batch_dev(self, occ_t, src_xy_t, views_t, group_ptr_t, threshold, radius, shape,
+                                        vmax_t=None, first_t=None, count_t=None, group_map_t=None):
+        """visibility_merge_view_batch on CUDA tensors (asynchronous), arguments as visibility_merge_batch_dev plus
+        views_t int32 (nsrc, 5).  A bad view is reported by the next synchronising call."""
+        self._merge_dev(self.lib.vhp_visibility_merge_view_batch_dev, (int(radius), int(shape)), occ_t, src_xy_t,
+                        group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t, views_t=views_t)
+
+    def _merge_dev(self, fn, extra, occ_t, src_xy_t, group_ptr_t, threshold, vmax_t, first_t, count_t, group_map_t,
+                   views_t=False):
         nmaps, ny, nx = occ_t.shape
         ng = group_ptr_t.shape[0] - 1
         dtype = F32 if (vmax_t is not None and vmax_t.element_size() == 4) else F64
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         mo = MergeOut(ptr(vmax_t), ptr(first_t), ptr(count_t))
-        self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), group_ptr_t.data_ptr(),
+        lead = () if views_t is False else (ptr(views_t),)
+        self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, src_xy_t.data_ptr(), *lead, group_ptr_t.data_ptr(),
                        ptr(group_map_t), ng, src_xy_t.shape[0], *extra, float(threshold), dtype, C.byref(mo)))
 
     def visibility_cover_greedy_batch(self, occ, cand_xy, group_ptr, k, threshold, radius, shape, group_map=None,
@@ -798,7 +823,7 @@ def pack_bits(cells):
 
 
 def sensor_views(heading_deg, fov_deg, radius, scale=32767):
-    """Views for visibility_cover_greedy_view_batch: int32 (n, 5) rows (r, ax, ay, bx, by) from headings and fields of
+    """Views for visibility_cover_greedy_view_batch and visibility_merge_view_batch: int32 (n, 5) rows (r, ax, ay, bx, by) from headings and fields of
     view in degrees (scalars or arrays, broadcast together).  Angles are measured from +x (the column) towards +y (the
     row).  a = round(scale * dir(heading - fov / 2)) and b = round(scale * dir(heading + fov / 2)); fov >= 360 gives
     a == b = round(scale * dir(heading)), every direction.  The library sees only these integer vectors: they, not the

@@ -161,6 +161,10 @@ vhp_status check_device_error(vhp_context *ctx) {
       return fail(ctx, VHP_ERR_INVALID_ARG,
                   "a candidate's view (r, ax, ay, bx, by) is invalid: r outside [0, radius], a or b (0, 0), or a "
                   "component outside [-32767, 32767]");
+    if (flag & 16)
+      return fail(ctx, VHP_ERR_INVALID_ARG,
+                  "a source's view (r, ax, ay, bx, by) is invalid: r outside [0, radius], a or b (0, 0), or a "
+                  "component outside [-32767, 32767]; that source contributed nothing");
     return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
   }
   return VHP_OK;
@@ -958,9 +962,11 @@ vhp_status run_runs_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx
 // ctx->b_bin by any route of run_dev (grid mode, naive kernel, thr <= 0) and merge_fold_kernel folds them.
 // With a range (vhp_visibility_merge_range_batch) the direct route sweeps only each source's box
 // (kFmtMergeRange*, window_direct_route) and the fallback folds chunks of fp64 windows (run_window_dev, any of its
-// routes) with merge_window_fold_kernel.
-const char *merge_name(const VhpMergeRange *range) {
-  return range ? "vhp_visibility_merge_range_batch" : "vhp_visibility_merge_batch";
+// routes) with merge_window_fold_kernel.  With views (vhp_visibility_merge_view_batch) both routes of the range form
+// fold only each source's cells in its view (kFmtMergeView*, merge_window_fold_kernel<F32, true>).
+const char *const kMergeViewName = "vhp_visibility_merge_view_batch";
+const char *merge_name(const VhpMergeRange *range, bool view = false) {
+  return view ? kMergeViewName : range ? "vhp_visibility_merge_range_batch" : "vhp_visibility_merge_batch";
 }
 
 vhp_status check_range(vhp_context *ctx, const std::string &what, const VhpMergeRange &range) {
@@ -973,8 +979,9 @@ vhp_status check_range(vhp_context *ctx, const std::string &what, const VhpMerge
 
 vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t ngroups, int64_t nsrc, double thr, int dtype,
-                            const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
-  const std::string what = merge_name(range);
+                            const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false,
+                            const void *views = nullptr) {
+  const std::string what = merge_name(range, view);
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || ngroups < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
@@ -984,7 +991,30 @@ vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx
   if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
   if (!out->vmax && !out->first && !out->count)
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
-  return range ? check_range(ctx, what, *range) : VHP_OK;
+  if (range) {
+    const vhp_status sr = check_range(ctx, what, *range);
+    if (sr != VHP_OK) return sr;
+  }
+  if (view && nsrc > 0 && !views) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": views is NULL");
+  return VHP_OK;
+}
+
+// host-side validation of the views [n][5] = (r, ax, ay, bx, by), the rule of cover_view_kernel and MergeView; name / item: the
+// call and what a view belongs to, for the message
+vhp_status check_views_host(vhp_context *ctx, const int32_t *views, int64_t n, int radius, const char *name,
+                            const char *item) {
+  for (int64_t i = 0; i < n; ++i) {
+    const int32_t *v = views + 5 * i;
+    const char *bad = nullptr;
+    if (v[0] < 0 || v[0] > radius) bad = "r outside [0, radius]";
+    for (int j = 1; j < 5 && !bad; ++j)
+      if (v[j] < -32767 || v[j] > 32767) bad = "a component outside [-32767, 32767]";
+    if (!bad && ((v[1] == 0 && v[2] == 0) || (v[3] == 0 && v[4] == 0))) bad = "a or b is (0, 0)";
+    if (bad)
+      return fail(ctx, VHP_ERR_INVALID_ARG,
+                  std::string(name) + ": view of " + item + " " + std::to_string(i) + ": " + bad);
+  }
+  return VHP_OK;
 }
 
 VhpMergeDev merge_dev_of(const vhp_merge_out &o, vhp_dtype dtype) {
@@ -1013,7 +1043,8 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
   m.pair_map = pm;
   if (range) {
     const int R = range->radius;
-    if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
+    if (thr > 0.0 && window_direct_route(ctx, nx, ny, R) &&
+        (!range->views || vhp_sweep_merge_view_supported(nx, ny, R))) {
       if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), R + 1) + 64)) != VHP_OK) return st;
       if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
       VHP_CUDA(ctx, vhp_launch_sweep_merge(ctx->tile, nx, ny, d_xy, m, nsrc, thr, ctx->rcp2_table, ctx->d_err,
@@ -1030,7 +1061,7 @@ vhp_status run_merge_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int 
           VHP_OK)
         return st;
       VHP_CUDA(ctx, vhp_launch_merge_window_fold((const double *)ctx->b_mwin.p, p0, np, nx, ny, d_xy, thr, *range, m,
-                                                 ctx->sm_count, ctx->stream, &ctx->launches));
+                                                 ctx->d_err, ctx->sm_count, ctx->stream, &ctx->launches));
     }
     return VHP_OK;
   }
@@ -1069,16 +1100,19 @@ vhp_status check_groups_host(vhp_context *ctx, const std::string &what, const in
 
 // host buffers: validate, upload maps and sources once, then runs of whole groups whose outputs fit 1 GB of device
 // memory (at least one group), each copied back with plain cudaMemcpyAsync (the merged result is already K times
-// smaller than the fields it folds)
+// smaller than the fields it folds).  view: vhp_visibility_merge_view_batch, views [nsrc][5] uploaded with the
+// sources.
 vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
                           const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
-                          const vhp_merge_out *out, const VhpMergeRange *range = nullptr) {
-  const char *what = merge_name(range);
+                          const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false,
+                          const int32_t *views = nullptr) {
+  const char *what = merge_name(range, view);
   vhp_status st = check_groups_host(ctx, what, gptr, ngroups);
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
-  st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range);
+  st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range, view, views);
   if (st != VHP_OK) return st;
+  if (view && (st = check_views_host(ctx, views, nsrc, range->radius, what, "source")) != VHP_OK) return st;
   if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, what)) != VHP_OK) return st;
   if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, what)) != VHP_OK) return st;
   ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
@@ -1089,6 +1123,10 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   // (the group maps are uploaded per run of groups below)
   if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
     return st;
+  if (view && nsrc > 0) {
+    if ((st = ensure(ctx, ctx->b_views, 20 * (size_t)nsrc)) != VHP_OK) return st;
+    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_views.p, views, 20 * (size_t)nsrc, cudaMemcpyHostToDevice, ctx->stream));
+  }
   const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
   const size_t bv = out->vmax ? esz : 0, bf = out->first ? 4 : 0, bc = out->count ? 4 : 0;
   const int64_t gchunk = std::min<int64_t>(ngroups, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / (cells * (bv + bf + bc)))));
@@ -1111,9 +1149,12 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
     if (e == cudaSuccess && gmap)
       e = cudaMemcpyAsync(ctx->b_map.p, gmap + g0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
     if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: upload of the group layout"); break; }
+    VhpMergeRange run_range;
+    if (range) run_range = *range;
+    if (view) run_range.views = (const int32_t *)ctx->b_views.p + 5 * a;
     result = run_merge_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a,
                            (const int64_t *)ctx->b_misc.p, gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc,
-                           gptr[g0 + gc] - a, thr, m, range);
+                           gptr[g0 + gc] - a, thr, m, range ? &run_range : nullptr);
     if (result != VHP_OK) break;
     const size_t n = (size_t)gc * cells, off = (size_t)g0 * cells;
     if (out->vmax) e = cudaMemcpyAsync((char *)out->vmax + off * esz, m.vmax, n * esz, cudaMemcpyDeviceToHost, ctx->stream);
@@ -1205,22 +1246,6 @@ vhp_status check_cover_view_args(vhp_context *ctx, const void *occ, int nmaps, i
                                                out);
   if (st != VHP_OK) return st;
   if (nsrc > 0 && !views) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverViewName) + ": views is NULL");
-  return VHP_OK;
-}
-
-// host-side validation of the views [n][5] = (r, ax, ay, bx, by), the rule of cover_view_kernel
-vhp_status check_views_host(vhp_context *ctx, const int32_t *views, int64_t n, int radius) {
-  for (int64_t i = 0; i < n; ++i) {
-    const int32_t *v = views + 5 * i;
-    const char *bad = nullptr;
-    if (v[0] < 0 || v[0] > radius) bad = "r outside [0, radius]";
-    for (int j = 1; j < 5 && !bad; ++j)
-      if (v[j] < -32767 || v[j] > 32767) bad = "a component outside [-32767, 32767]";
-    if (!bad && ((v[1] == 0 && v[2] == 0) || (v[3] == 0 && v[4] == 0))) bad = "a or b is (0, 0)";
-    if (bad)
-      return fail(ctx, VHP_ERR_INVALID_ARG,
-                  std::string(kCoverViewName) + ": view of candidate " + std::to_string(i) + ": " + bad);
-  }
   return VHP_OK;
 }
 
@@ -1387,7 +1412,7 @@ vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   if constexpr (kM) {
     st = view ? check_cover_view_args(ctx, occ, nmaps, nx, ny, xy, views, gptr, nprob, nsrc, k, range, thr, m, out)
               : check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, m, out);
-    if (st == VHP_OK && view) st = check_views_host(ctx, views, nsrc, range.radius);
+    if (st == VHP_OK && view) st = check_views_host(ctx, views, nsrc, range.radius, kCoverViewName, "candidate");
   } else if constexpr (kW)
     st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
   else
@@ -2039,6 +2064,34 @@ vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t 
   range.shape = shape;
   vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
                                    d_out, &range);
+  if (st != VHP_OK) return st;
+  VHP_ON_DEVICE(ctx);
+  return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
+                       merge_dev_of(*d_out, dtype), &range);
+}
+
+vhp_status vhp_visibility_merge_view_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                           const int32_t *src_xy, const int32_t *views, const int64_t *group_ptr,
+                                           const int32_t *group_map, int64_t ngroups, int32_t radius, int32_t shape,
+                                           double threshold, vhp_dtype dtype, const vhp_merge_out *out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  return run_merge_host(ctx, occ, nmaps, nx, ny, src_xy, group_ptr, group_map, ngroups, threshold, dtype, out,
+                        &range, true, views);
+}
+
+vhp_status vhp_visibility_merge_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                               const int32_t *d_src_xy, const int32_t *d_views,
+                                               const int64_t *d_group_ptr, const int32_t *d_group_map,
+                                               int64_t ngroups, int64_t nsrc, int32_t radius, int32_t shape,
+                                               double threshold, vhp_dtype dtype, const vhp_merge_out *d_out) {
+  VhpMergeRange range;
+  range.radius = radius;
+  range.shape = shape;
+  range.views = d_views;
+  vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
+                                   d_out, &range, true, d_views);
   if (st != VHP_OK) return st;
   VHP_ON_DEVICE(ctx);
   return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,

@@ -9,7 +9,8 @@
 //   count = #{ k : k writes the cell, v_k >= thr }
 // where source (sx, sy) writes every cell but column 0 (unless sx == 0) and row 0 (unless sy == 0).
 // The range-limited form (vhp_visibility_merge_range_batch) counts v_k only where the cell is in k's range; its
-// fallback folds fp64 windows (merge_window_fold_kernel) instead of whole fields.
+// fallback folds fp64 windows (merge_window_fold_kernel) instead of whole fields, and so does the fallback of the view
+// form (vhp_visibility_merge_view_batch), with only the cells in each source's view (MergeView).
 #include <algorithm>
 #include <cstdint>
 
@@ -19,6 +20,7 @@
 namespace {
 
 constexpr int kErrGroups = 4; // d_err bit: inconsistent group layout / group map
+constexpr int kErrView = 16;  // d_err bit: a bad view of vhp_visibility_merge_view_batch_dev
 
 // Thread t < nsrc: pair t -> (group, index in group, map) by a binary search of group_ptr; thread t <= ngroups:
 // group_ptr[0] == 0, non-decreasing, groups below 2^31 sources, group_ptr[ngroups] == nsrc.
@@ -109,10 +111,12 @@ __global__ void merge_fold_kernel(const double *__restrict__ field, int64_t p0, 
 
 // One thread per window cell of pairs [p0, p0 + np): cells in the grid and in the pair's range fold into its
 // group's outputs with the relaxed reductions of the direct route (kFmtMergeRange*), so the order of the pairs
-// does not matter.  r2: a cell (dx, dy) of the window is in range iff dx^2 + dy^2 <= r2 (box: 2 R^2).
-template <bool F32>
+// does not matter.  r2: a cell (dx, dy) of the window is in range iff dx^2 + dy^2 <= r2 (box: 2 R^2).  VIEW: only
+// the cells in the pair's view views[q] fold instead; a bad view folds nothing and raises error value 16.
+template <bool F32, bool VIEW>
 __global__ void merge_window_fold_kernel(const double *__restrict__ win, int64_t p0, int64_t np, int nx, int ny,
-                                         int R, int r2, const int32_t *__restrict__ xy, double thr, VhpMergeDev m) {
+                                         int R, int r2, const int32_t *__restrict__ xy, double thr, VhpMergeDev m,
+                                         const int32_t *__restrict__ views, bool disk, int *err) {
   const int W = 2 * R + 1;
   const size_t ww = (size_t)W * W, total = (size_t)np * ww, cells = (size_t)nx * ny;
   for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total;
@@ -120,7 +124,17 @@ __global__ void merge_window_fold_kernel(const double *__restrict__ win, int64_t
     const int64_t q = p0 + (int64_t)(idx / ww);
     const int rem = (int)(idx % ww), dy = rem / W - R, dx = rem % W - R;
     const int sx = __ldg(xy + 2 * q), sy = __ldg(xy + 2 * q + 1), x = sx + dx, y = sy + dy;
-    if ((unsigned)x >= (unsigned)nx || (unsigned)y >= (unsigned)ny || dx * dx + dy * dy > r2) continue;
+    if constexpr (VIEW) { // (a pair of an inconsistent group layout reads no view)
+      MergeView w;
+      if (__ldg(m.pair_group + q) < 0) continue;
+      if (!merge_view_decode(views + 5 * q, R, disk, w)) {
+        if (rem == 0) atomicOr(err, kErrView);
+        continue;
+      }
+      if ((unsigned)x >= (unsigned)nx || (unsigned)y >= (unsigned)ny || !merge_view_has(w, dx, dy)) continue;
+    } else {
+      if ((unsigned)x >= (unsigned)nx || (unsigned)y >= (unsigned)ny || dx * dx + dy * dy > r2) continue;
+    }
     const int32_t g = __ldg(m.pair_group + q);
     if (g < 0) continue;
     const double v = __ldg(win + idx);
@@ -176,13 +190,22 @@ cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np,
 
 cudaError_t vhp_launch_merge_window_fold(const double *d_win, int64_t p0, int64_t np, int nx, int ny,
                                          const int32_t *d_src_xy, double thr, const VhpMergeRange &range,
-                                         const VhpMergeDev &m, int sm_count, cudaStream_t st, int64_t *launches) {
+                                         const VhpMergeDev &m, int *d_err, int sm_count, cudaStream_t st,
+                                         int64_t *launches) {
   const int R = range.radius, r2 = range.shape == VHP_RANGE_DISK ? R * R : 2 * R * R;
   const size_t W = 2 * (size_t)R + 1;
   const int bs = 256;
   const unsigned grid = grid_for((size_t)np * W * W, bs, sm_count);
-  if (m.f32) merge_window_fold_kernel<true><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m);
-  else merge_window_fold_kernel<false><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m);
+  const int32_t *v = range.views;
+  const bool disk = range.shape == VHP_RANGE_DISK;
+  if (v && m.f32)
+    merge_window_fold_kernel<true, true><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m, v, disk, d_err);
+  else if (v)
+    merge_window_fold_kernel<false, true><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m, v, disk, d_err);
+  else if (m.f32)
+    merge_window_fold_kernel<true, false><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m, v, disk, d_err);
+  else
+    merge_window_fold_kernel<false, false><<<grid, bs, 0, st>>>(d_win, p0, np, nx, ny, R, r2, d_src_xy, thr, m, v, disk, d_err);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

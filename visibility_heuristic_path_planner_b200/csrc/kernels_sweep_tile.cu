@@ -45,6 +45,18 @@ sweep_tile_kernel(const TileArgs p) {
   if constexpr (fmt_merge(FMT)) { // fold into the outputs of the pair's group
     const int g = __ldg(p.m_pg + pair);
     if (g < 0) return; // a pair of an inconsistent group layout (the table kernel reported it)
+    if constexpr (fmt_view(FMT)) { // the source's view into the tail; a bad one (error value 16) folds nothing
+      MergeView w;
+      if (!merge_view_decode(p.m_views + 5 * pair, p.w_r, p.m_disk != 0, w)) {
+        if (threadIdx.x == 0) atomicOr(p.err, 16);
+        return;
+      }
+      if (threadIdx.x == 0) {
+        uint32_t dsmem;
+        asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dsmem));
+        *reinterpret_cast<int4 *>(smem_raw + dsmem - kViewTail) = make_int4(w.key | (sy * p.nx + sx), w.range, w.a, w.b);
+      }
+    }
     if (threadIdx.x == 0) *reinterpret_cast<int2 *>(smem_raw + kMergeHdr) = make_int2(g, __ldg(p.m_pk + pair));
     tile_sweep_cta<OutT, NW, kSweepCta, FMT>(p, map, sx, sy, reinterpret_cast<OutT *>(p.out), smem_raw);
     return;
@@ -211,7 +223,7 @@ __global__ void ratio2_selftest_kernel(const double2 *__restrict__ tab, int kmax
 
 template <typename OutT, int NW, int MINB, int FMT = kFmtValues>
 cudaError_t launch_tile_nw(const TileArgs &p, int64_t npairs, cudaStream_t st) {
-  const size_t smem = fmt_clip(FMT) ? tile_smem_bytes_win<OutT>(p.nx, p.ny, p.w_r, NW)
+  const size_t smem = fmt_clip(FMT) ? tile_smem_bytes_win<OutT>(p.nx, p.ny, p.w_r, NW) + (fmt_view(FMT) ? kViewTail : 0)
                                     : tile_smem_bytes<OutT>(p.nx, p.ny, NW);
   auto kern = sweep_tile_kernel<OutT, NW, MINB, FMT>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -282,7 +294,7 @@ cudaError_t launch_tile_win(const TileArgs &p, int64_t npairs, cudaStream_t st) 
   }
 }
 
-// range-limited merged output (kFmtMergeRange*): fp64 staging, the warp counts and bounds of the windows
+// range-limited merged output (kFmtMergeRange*, kFmtMergeView*): fp64 staging, the warp counts and bounds of the windows
 template <int FMT>
 cudaError_t launch_tile_merge_range(const TileArgs &p, int64_t npairs, cudaStream_t st) {
   switch (tile_warps_for(win_side(p.nx, p.w_r), win_side(p.ny, p.w_r), npairs)) {
@@ -336,6 +348,11 @@ __global__ void window_pairs_kernel(const int32_t *__restrict__ src_xy, const in
 bool vhp_sweep_window_supported(int nx, int ny, int radius) {
   return nx >= 1 && ny >= 1 && std::max(nx, ny) <= 16384 && radius >= 0 &&
          tile_smem_bytes_win<double>(nx, ny, radius) <= 227u * 1024u;
+}
+
+bool vhp_sweep_merge_view_supported(int nx, int ny, int radius) {
+  return vhp_sweep_window_supported(nx, ny, radius) &&
+         tile_smem_bytes_win<double>(nx, ny, radius) + kViewTail <= 227u * 1024u;
 }
 
 cudaError_t vhp_launch_sweep_window_batch(const VhpTilePlanes &pl, int nmaps, int nx, int ny,
@@ -414,6 +431,12 @@ cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, cons
     p.w_r = R;
     p.w_sw = win_sum_words(nx, R);
     p.w_r2 = range->shape == VHP_RANGE_DISK ? R * R : 2 * R * R;
+    if (range->views) {
+      p.m_views = range->views;
+      p.m_disk = range->shape == VHP_RANGE_DISK;
+      return m.f32 ? launch_tile_merge_range<kFmtMergeView32>(p, npairs, st)
+                   : launch_tile_merge_range<kFmtMergeView64>(p, npairs, st);
+    }
     return m.f32 ? launch_tile_merge_range<kFmtMergeRange32>(p, npairs, st)
                  : launch_tile_merge_range<kFmtMergeRange64>(p, npairs, st);
   }

@@ -139,10 +139,16 @@ struct TileArgs {
   // quadrants (Q1, Q2) and the -y quadrants (Q3, Q4) of a strip as two launches: the two
   // directions travel along the strips independently of each other.
   int qmask = 0xF;
+  // kFmtMergeView*: the call's shape is the disk (in the padding in front of src_ctl, so that no other member moves)
+  int m_disk = 0;
   // window / grid kernels only: {done, sx, sy, ...} in device memory.  Non-null: the source comes
   // from there and the launch is a no-op once `done` is set, so a planner iteration can be
   // enqueued (or captured in a CUDA graph) before the host knows the next source.
-  const int *src_ctl = nullptr;
+  // kFmtMergeView* (the batched tile kernel, which never reads src_ctl): the views [pair][5] = (r, ax, ay, bx, by).
+  union {
+    const int *src_ctl = nullptr;
+    const int32_t *m_views;
+  };
   // grid mode across GPUs (strip-partitioned planner, one strip per rank): the boundary between
   // two strips is handed over tile by tile through peer memory instead of as a finished row.
   //   exporter: x_edges / x_prog = the boundary rows and progress flags of the NEIGHBOUR's
@@ -304,12 +310,20 @@ __device__ __forceinline__ void stg16_fill(double *q, double v) {
 // the candidate's box layout (VhpCoverBox: rows of vhp_cover_words(nx, R) words, `out` shifted by the box origin, so
 // the addressing is the whole-map bit layout's with another row pitch); only the box |dx|, |dy| <= R is stored, the
 // disk is applied afterwards.
+// kFmtMergeView64 / kFmtMergeView32 (vhp_visibility_merge_view_batch): kFmtMergeRange*, with only the cells of the box in
+// the source's view (MergeView, TileArgs::m_views) folded.  The CTA's decoded view sits in kViewTail bytes after the
+// layout of kFmtMergeRange* (the end of the dynamic shared memory), its key holding the source's cell index.
 constexpr int kFmtValues = 0, kFmtBits = 2, kFmtMerge64 = 3, kFmtMerge32 = 4, kFmtWindow = 5, kFmtMergeRange64 = 6,
-              kFmtMergeRange32 = 7, kFmtCoverBits = 8;
+              kFmtMergeRange32 = 7, kFmtCoverBits = 8, kFmtMergeView64 = 9, kFmtMergeView32 = 10;
 constexpr int kMergeHdr = 224; // shared-memory header: {group, k} of the CTA's source (int2)
 
-// the sweep folds into group outputs (merge_cell), and it does so only within a range
-__host__ __device__ constexpr bool fmt_range(int f) { return f == kFmtMergeRange64 || f == kFmtMergeRange32; }
+constexpr int kViewTail = 16;  // kFmtMergeView*: shared-memory tail, the CTA's MergeView
+
+// the sweep folds into group outputs (merge_cell), and it does so only within a range (and a view)
+__host__ __device__ constexpr bool fmt_view(int f) { return f == kFmtMergeView64 || f == kFmtMergeView32; }
+__host__ __device__ constexpr bool fmt_range(int f) {
+  return f == kFmtMergeRange64 || f == kFmtMergeRange32 || fmt_view(f);
+}
 __host__ __device__ constexpr bool fmt_merge(int f) { return f == kFmtMerge64 || f == kFmtMerge32 || fmt_range(f); }
 // clipped geometry: each quadrant's extents are clipped to R and the per-CTA state is sized by the box
 // (tile_smem_bytes_win); the window output layout (pitch 2R+1, off-grid zeros) is kFmtWindow's alone
@@ -318,18 +332,26 @@ __host__ __device__ constexpr bool fmt_clip(int f) { return f == kFmtWindow || f
 __host__ __device__ constexpr bool fmt_bits(int f) { return f == kFmtBits || f == kFmtCoverBits; }
 
 // fold value v of cell idx (y * nx + x) of this CTA's sweep into its group's outputs; (di, dj) = (|dx|, |dy|) of
-// the cell from the source, for the range test of kFmtMergeRange*
+// the cell from the source, for the range test of kFmtMergeRange*.  kFmtMergeView* recovers the signs from idx and
+// the source's index s: with |dx| < nx, idx - s = dy * nx + dx is >= 0 exactly when dy >= 0 (dj > 0).
 template <int FMT>
 __device__ __forceinline__ void merge_cell(const TileArgs &p, const ptrdiff_t idx, const int di, const int dj,
                                            const double v) {
   if (!(v > 0.0)) return;
-  if constexpr (fmt_range(FMT))
-    if (di * di + dj * dj > p.w_r2) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
+  if constexpr (fmt_view(FMT)) {
+    uint32_t dsmem;
+    asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dsmem));
+    const int4 t = *reinterpret_cast<const int4 *>(smem_raw + dsmem - kViewTail);
+    const int delta = (int)idx - (t.x & 0x7fffffff), dy = delta >= 0 ? dj : -dj;
+    if (!merge_view_has(MergeView{t.x, t.y, t.z, t.w}, delta - dy * p.nx, dy)) return;
+  } else if constexpr (fmt_range(FMT)) {
+    if (di * di + dj * dj > p.w_r2) return;
+  }
   const int2 gk = *reinterpret_cast<const int2 *>(smem_raw + kMergeHdr);
   const size_t o = (size_t)gk.x * p.m_cells + (size_t)idx;
   if (p.m_vmax) {
-    if constexpr (FMT == kFmtMerge64 || FMT == kFmtMergeRange64)
+    if constexpr (FMT == kFmtMerge64 || FMT == kFmtMergeRange64 || FMT == kFmtMergeView64)
       red_max_u64(reinterpret_cast<unsigned long long *>(p.m_vmax) + o, (unsigned long long)__double_as_longlong(v));
     else
       red_max_u32(reinterpret_cast<uint32_t *>(p.m_vmax) + o, __float_as_uint(__double2float_rn(v)));

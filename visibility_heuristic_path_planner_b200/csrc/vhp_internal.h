@@ -104,7 +104,8 @@ struct vhp_context {
   int64_t launches = 0;
   std::string last_error;
   // device-side error word (bit 0: a source / start / end outside the grid, bit 2: inconsistent source groups,
-  // bit 3: a bad view of vhp_visibility_cover_greedy_view_batch_dev)
+  // bit 3: a bad view of vhp_visibility_cover_greedy_view_batch_dev, bit 4: a bad view of
+  // vhp_visibility_merge_view_batch_dev)
   int *d_err = nullptr;
   // workspace buffers (grown on demand, reused across calls)
   VhpDevBuf b_occ, b_src, b_map, b_out[2], b_scratch, b_planner, b_misc, b_grid, b_bin;
@@ -209,6 +210,9 @@ cudaError_t vhp_launch_sweep_tile(const VhpTilePlanes &pl, int nx, int ny, const
 // of each pair (kFmtWindow, shared memory sized by the window; supported: it fits one CTA), into d_out
 // [pair][2R+1][2R+1]; a map index out of range raises bit 0 of d_err like a source outside the grid.
 bool vhp_sweep_window_supported(int nx, int ny, int radius);
+// ... and the direct route of vhp_visibility_merge_view_batch (kFmtMergeView*), whose CTAs keep their view in a
+// shared-memory tail
+bool vhp_sweep_merge_view_supported(int nx, int ny, int radius);
 cudaError_t vhp_launch_sweep_window_batch(const VhpTilePlanes &pl, int nmaps, int nx, int ny,
                                           const int32_t *d_src_xy, const int32_t *d_src_map, int64_t npairs,
                                           int radius, vhp_dtype dtype, void *d_out, const double *d_rcp2,
@@ -233,14 +237,18 @@ struct VhpMergeDev {
   const int32_t *pair_k = nullptr;     // index of the pair within its group
   const int32_t *pair_map = nullptr;   // map of the pair (its group's)
 };
-// range of vhp_visibility_merge_range_batch: 0 <= radius <= 16383, shape VHP_RANGE_BOX / VHP_RANGE_DISK
+// range of vhp_visibility_merge_range_batch: 0 <= radius <= 16383, shape VHP_RANGE_BOX / VHP_RANGE_DISK.  views:
+// vhp_visibility_merge_view_batch's [pair][5] = (r, ax, ay, bx, by) on the device, indexed like the pairs (null: the
+// range merge)
 struct VhpMergeRange {
   int radius = 0;
   int shape = VHP_RANGE_BOX;
+  const int32_t *views = nullptr;
 };
 // the sweeps fold straight into the group outputs (kFmtMerge*, one CTA per pair); needs thr > 0 and zero-filled
 // vmax / count, -1-filled first.  range: sweep only each pair's box and fold only its cells in range
-// (kFmtMergeRange*; supported where vhp_sweep_window_supported holds)
+// (kFmtMergeRange*; supported where vhp_sweep_window_supported holds); range->views: fold only each pair's cells in
+// its view (kFmtMergeView*, supported where vhp_sweep_merge_view_supported holds; a bad view raises bit 4 of d_err)
 cudaError_t vhp_launch_sweep_merge(const VhpTilePlanes &pl, int nx, int ny, const int32_t *d_src_xy,
                                    const VhpMergeDev &m, int64_t npairs, double thr, const double *d_rcp2,
                                    int *d_err, cudaStream_t st, int64_t *launches,
@@ -256,10 +264,12 @@ cudaError_t vhp_launch_merge_fold(const double *d_field, int64_t p0, int64_t np,
                                   const int32_t *d_src_xy, double thr, const VhpMergeDev &m, int sm_count,
                                   cudaStream_t st, int64_t *launches);
 // the fold of np fp64 windows d_win[np][2R+1][2R+1] of pairs [p0, p0 + np) (vhp_visibility_window_batch's layout)
-// into the group outputs, cells in range only (relaxed red atomics: any order gives the same result)
+// into the group outputs, cells in range only (relaxed red atomics: any order gives the same result); with
+// range.views the cells in each pair's view only (a bad view raises bit 4 of d_err and folds nothing)
 cudaError_t vhp_launch_merge_window_fold(const double *d_win, int64_t p0, int64_t np, int nx, int ny,
                                          const int32_t *d_src_xy, double thr, const VhpMergeRange &range,
-                                         const VhpMergeDev &m, int sm_count, cudaStream_t st, int64_t *launches);
+                                         const VhpMergeDev &m, int *d_err, int sm_count, cudaStream_t st,
+                                         int64_t *launches);
 
 // Greedy coverage placement (vhp_visibility_cover_greedy_batch).  The coverage bits of a candidate at (sx, sy) are
 // stored over its box, clipped to the grid: H = min(2R+1, ny) rows from row y0 and W words (the span rule of
