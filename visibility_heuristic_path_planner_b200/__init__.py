@@ -215,6 +215,16 @@ def _np_ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def _cover_weights(weights, shape):
+    """weights of the weighted cover calls: None, or uint8 of the problems' (nprob, ny, nx)."""
+    if weights is None:
+        return None
+    w = np.asarray(weights)
+    if w.dtype != np.uint8 or w.shape != shape:
+        raise ValueError(f"weights must be uint8 of shape {shape}, got {w.dtype} {w.shape}")
+    return np.ascontiguousarray(w)
+
+
 def _occ_u8(occ):
     """(ny, nx) or (nmaps, ny, nx) -> contiguous uint8 (1 free / 0 occupied)."""
     occ = np.asarray(occ)
@@ -514,23 +524,8 @@ class Context:
         (None: all).  Returns pick (int32 (nprob, k), index within the group, -1 after the last pick), gain (uint32
         (nprob, k), cells newly covered), npicked (int32 (nprob,)) and covered (uint32 (nprob, ny, ceil(nx/32)), the
         bits of the union, see unpack_bits)."""
-        occ = _occ_u8(occ)
-        nmaps, ny, nx = occ.shape
-        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
-        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
-        npb = gp.shape[0] - 1
-        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
-        tb = None if target is None else pack_bits(np.asarray(target, bool).reshape(max(npb, 0), ny, nx))
-        k = int(k)
-        n = max(npb, 0)
-        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint32),
-                 npicked=np.empty(n, np.int32), covered=np.empty((n, ny, (nx + 31) // 32), np.uint32))
-        co = CoverOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "covered")])
-        self._check(self.lib.vhp_visibility_cover_greedy_batch(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy),
-                                                                _np_ptr(gp), _np_ptr(gm), npb, k, int(radius),
-                                                                int(shape), float(threshold), _np_ptr(tb),
-                                                                C.byref(co)))
-        return r
+        return self._cover_host(self.lib.vhp_visibility_cover_greedy_batch, CoverOut, occ, cand_xy, group_ptr, k,
+                                threshold, radius, shape, group_map, target=target)
 
     def visibility_cover_greedy_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape,
                                           pick_t=None, gain_t=None, npicked_t=None, covered_t=None, group_map_t=None,
@@ -538,13 +533,8 @@ class Context:
         """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2),
         group_ptr_t int64 (nprob + 1), target_t int32 (nprob, ny, ceil(nx/32)) packed bits or None; outputs pick_t,
         gain_t int32 (nprob, k), npicked_t int32 (nprob,), covered_t int32 (nprob, ny, ceil(nx/32)); any may be None."""
-        nmaps, ny, nx = occ_t.shape
-        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        co = CoverOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(covered_t))
-        self._check(self.lib.vhp_visibility_cover_greedy_batch_dev(
-            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
-            group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
-            ptr(target_t), C.byref(co)))
+        self._cover_dev(self.lib.vhp_visibility_cover_greedy_batch_dev, CoverOut, occ_t, cand_xy_t, group_ptr_t, k,
+                        threshold, radius, shape, (pick_t, gain_t, npicked_t, covered_t), group_map_t, target_t)
 
     def visibility_cover_greedy_weighted_batch(self, occ, cand_xy, group_ptr, k, threshold, radius, shape,
                                                weights=None, group_map=None):
@@ -553,26 +543,8 @@ class Context:
         summed weight.  weights: uint8 (nprob, ny, nx), the importance of each cell to each problem (None: every cell
         weighs 1).  Returns pick (int32 (nprob, k)), gain (uint64 (nprob, k), summed weight newly covered), npicked
         (int32 (nprob,)) and covered (uint32 (nprob, ny, ceil(nx/32)), the bits of the union, see unpack_bits)."""
-        occ = _occ_u8(occ)
-        nmaps, ny, nx = occ.shape
-        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
-        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
-        npb = gp.shape[0] - 1
-        n = max(npb, 0)
-        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
-        if weights is not None:
-            w = np.asarray(weights)
-            if w.dtype != np.uint8 or w.shape != (n, ny, nx):
-                raise ValueError(f"weights must be uint8 of shape {(n, ny, nx)}, got {w.dtype} {w.shape}")
-            weights = np.ascontiguousarray(w)
-        k = int(k)
-        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint64),
-                 npicked=np.empty(n, np.int32), covered=np.empty((n, ny, (nx + 31) // 32), np.uint32))
-        co = CoverWeightedOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "covered")])
-        self._check(self.lib.vhp_visibility_cover_greedy_weighted_batch(
-            self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp), _np_ptr(gm), npb, k, int(radius),
-            int(shape), float(threshold), _np_ptr(weights), C.byref(co)))
-        return r
+        return self._cover_host(self.lib.vhp_visibility_cover_greedy_weighted_batch, CoverWeightedOut, occ, cand_xy,
+                                group_ptr, k, threshold, radius, shape, group_map, weights=weights)
 
     def visibility_cover_greedy_weighted_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape,
                                                    pick_t=None, gain_t=None, npicked_t=None, covered_t=None,
@@ -581,13 +553,9 @@ class Context:
         group_ptr_t int64 (nprob + 1), weights_t uint8 (nprob, ny, nx) or None; outputs pick_t int32 (nprob, k),
         gain_t int64 / uint64 (nprob, k), npicked_t int32 (nprob,), covered_t int32 (nprob, ny, ceil(nx/32)); any may
         be None."""
-        nmaps, ny, nx = occ_t.shape
-        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        co = CoverWeightedOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(covered_t))
-        self._check(self.lib.vhp_visibility_cover_greedy_weighted_batch_dev(
-            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
-            group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
-            ptr(weights_t), C.byref(co)))
+        self._cover_dev(self.lib.vhp_visibility_cover_greedy_weighted_batch_dev, CoverWeightedOut, occ_t, cand_xy_t,
+                        group_ptr_t, k, threshold, radius, shape, (pick_t, gain_t, npicked_t, covered_t), group_map_t,
+                        weights_t)
 
     def visibility_cover_greedy_mfold_batch(self, occ, cand_xy, group_ptr, k, m, threshold, radius, shape,
                                             weights=None, group_map=None):
@@ -596,26 +564,8 @@ class Context:
         round takes the candidate, not yet picked, whose cells covered fewer than m times weigh the most.  Returns pick
         (int32 (nprob, k)), gain (uint64 (nprob, k), summed weight the pick adds), npicked (int32 (nprob,)) and count
         (uint8 (nprob, ny, nx), min(m, number of picks covering the cell))."""
-        occ = _occ_u8(occ)
-        nmaps, ny, nx = occ.shape
-        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
-        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
-        npb = gp.shape[0] - 1
-        n = max(npb, 0)
-        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
-        if weights is not None:
-            w = np.asarray(weights)
-            if w.dtype != np.uint8 or w.shape != (n, ny, nx):
-                raise ValueError(f"weights must be uint8 of shape {(n, ny, nx)}, got {w.dtype} {w.shape}")
-            weights = np.ascontiguousarray(w)
-        k = int(k)
-        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint64),
-                 npicked=np.empty(n, np.int32), count=np.empty((n, ny, nx), np.uint8))
-        co = CoverMfoldOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "count")])
-        self._check(self.lib.vhp_visibility_cover_greedy_mfold_batch(
-            self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(gp), _np_ptr(gm), npb, k, int(radius),
-            int(shape), float(threshold), _np_ptr(weights), int(m), C.byref(co)))
-        return r
+        return self._cover_host(self.lib.vhp_visibility_cover_greedy_mfold_batch, CoverMfoldOut, occ, cand_xy,
+                                group_ptr, k, threshold, radius, shape, group_map, weights=weights, m=m)
 
     def visibility_cover_greedy_mfold_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, k, m, threshold, radius, shape,
                                                 pick_t=None, gain_t=None, npicked_t=None, count_t=None,
@@ -623,13 +573,9 @@ class Context:
         """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2),
         group_ptr_t int64 (nprob + 1), weights_t uint8 (nprob, ny, nx) or None; outputs pick_t int32 (nprob, k),
         gain_t int64 / uint64 (nprob, k), npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx); any may be None."""
-        nmaps, ny, nx = occ_t.shape
-        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        co = CoverMfoldOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(count_t))
-        self._check(self.lib.vhp_visibility_cover_greedy_mfold_batch_dev(
-            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), group_ptr_t.data_ptr(), ptr(group_map_t),
-            group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape), float(threshold),
-            ptr(weights_t), int(m), C.byref(co)))
+        self._cover_dev(self.lib.vhp_visibility_cover_greedy_mfold_batch_dev, CoverMfoldOut, occ_t, cand_xy_t,
+                        group_ptr_t, k, threshold, radius, shape, (pick_t, gain_t, npicked_t, count_t), group_map_t,
+                        weights_t, m=m)
 
     def visibility_cover_greedy_view_batch(self, occ, cand_xy, views, group_ptr, k, m, threshold, radius, shape,
                                            weights=None, group_map=None):
@@ -638,29 +584,8 @@ class Context:
         (nsrc, 5), (r, ax, ay, bx, by) per candidate: range r (0 <= r <= radius) in the call's shape and the sector
         from a = (ax, ay) to b = (bx, by), in the grid's (x, y) = (column, row); see sensor_views.  Returns pick, gain,
         npicked and count as visibility_cover_greedy_mfold_batch."""
-        occ = _occ_u8(occ)
-        nmaps, ny, nx = occ.shape
-        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
-        vw = np.ascontiguousarray(views, dtype=np.int32).reshape(-1, 5)
-        if vw.shape[0] != xy.shape[0]:
-            raise ValueError(f"views must have one row per candidate ({xy.shape[0]}), got {vw.shape[0]}")
-        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
-        npb = gp.shape[0] - 1
-        n = max(npb, 0)
-        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
-        if weights is not None:
-            w = np.asarray(weights)
-            if w.dtype != np.uint8 or w.shape != (n, ny, nx):
-                raise ValueError(f"weights must be uint8 of shape {(n, ny, nx)}, got {w.dtype} {w.shape}")
-            weights = np.ascontiguousarray(w)
-        k = int(k)
-        r = dict(pick=np.empty((n, max(k, 0)), np.int32), gain=np.empty((n, max(k, 0)), np.uint64),
-                 npicked=np.empty(n, np.int32), count=np.empty((n, ny, nx), np.uint8))
-        co = CoverMfoldOut(*[_np_ptr(r[name]) for name in ("pick", "gain", "npicked", "count")])
-        self._check(self.lib.vhp_visibility_cover_greedy_view_batch(
-            self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), _np_ptr(vw), _np_ptr(gp), _np_ptr(gm), npb, k,
-            int(radius), int(shape), float(threshold), _np_ptr(weights), int(m), C.byref(co)))
-        return r
+        return self._cover_host(self.lib.vhp_visibility_cover_greedy_view_batch, CoverMfoldOut, occ, cand_xy,
+                                group_ptr, k, threshold, radius, shape, group_map, weights=weights, m=m, views=views)
 
     def visibility_cover_greedy_view_batch_dev(self, occ_t, cand_xy_t, views_t, group_ptr_t, k, m, threshold, radius,
                                                shape, pick_t=None, gain_t=None, npicked_t=None, count_t=None,
@@ -669,13 +594,53 @@ class Context:
         int32 (nsrc, 5), group_ptr_t int64 (nprob + 1), weights_t uint8 (nprob, ny, nx) or None; outputs pick_t int32
         (nprob, k), gain_t int64 / uint64 (nprob, k), npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx); any may
         be None.  A bad view is reported by the next synchronising call."""
+        self._cover_dev(self.lib.vhp_visibility_cover_greedy_view_batch_dev, CoverMfoldOut, occ_t, cand_xy_t,
+                        group_ptr_t, k, threshold, radius, shape, (pick_t, gain_t, npicked_t, count_t), group_map_t,
+                        weights_t, m=m, views_t=views_t)
+
+    def _cover_host(self, fn, out_type, occ, cand_xy, group_ptr, k, threshold, radius, shape, group_map, target=None,
+                    weights=None, m=None, views=None):
+        # out_type's fields name the outputs: CoverOut has uint32 gains, the weighted calls' uint64 ones
+        occ = _occ_u8(occ)
+        nmaps, ny, nx = occ.shape
+        xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
+        lead = ()
+        if views is not None:
+            vw = np.ascontiguousarray(views, dtype=np.int32).reshape(-1, 5)
+            if vw.shape[0] != xy.shape[0]:
+                raise ValueError(f"views must have one row per candidate ({xy.shape[0]}), got {vw.shape[0]}")
+            lead = (_np_ptr(vw),)
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        npb = gp.shape[0] - 1
+        n = max(npb, 0)
+        gm = None if group_map is None else np.ascontiguousarray(group_map, dtype=np.int32)
+        if target is not None:
+            extra = pack_bits(np.asarray(target, bool).reshape(n, ny, nx))
+        else:
+            extra = _cover_weights(weights, (n, ny, nx))
+        k = int(k)
+        kinds = dict(pick=((n, max(k, 0)), np.int32),
+                     gain=((n, max(k, 0)), np.uint32 if out_type is CoverOut else np.uint64),
+                     npicked=((n,), np.int32), covered=((n, ny, (nx + 31) // 32), np.uint32),
+                     count=((n, ny, nx), np.uint8))
+        names = [name for name, _ in out_type._fields_]
+        r = {name: np.empty(*kinds[name]) for name in names}
+        co = out_type(*[_np_ptr(r[name]) for name in names])
+        tail = () if m is None else (int(m),)
+        self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), *lead, _np_ptr(gp), _np_ptr(gm), npb, k,
+                       int(radius), int(shape), float(threshold), _np_ptr(extra), *tail, C.byref(co)))
+        return r
+
+    def _cover_dev(self, fn, out_type, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape, outs, group_map_t,
+                   extra_t, m=None, views_t=False):
         nmaps, ny, nx = occ_t.shape
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        co = CoverMfoldOut(ptr(pick_t), ptr(gain_t), ptr(npicked_t), ptr(count_t))
-        self._check(self.lib.vhp_visibility_cover_greedy_view_batch_dev(
-            self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), ptr(views_t), group_ptr_t.data_ptr(),
-            ptr(group_map_t), group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius), int(shape),
-            float(threshold), ptr(weights_t), int(m), C.byref(co)))
+        co = out_type(*[ptr(t) for t in outs])
+        lead = () if views_t is False else (ptr(views_t),)
+        tail = () if m is None else (int(m),)
+        self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), *lead, group_ptr_t.data_ptr(),
+                       ptr(group_map_t), group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius),
+                       int(shape), float(threshold), ptr(extra_t), *tail, C.byref(co)))
 
     def visibility_variant_batch(self, occ, src_xy, model, alpha=1.0, fac=1.0, light_strength=1.0,
                                  cutoff=0.001, src_map=None, dtype=F64):

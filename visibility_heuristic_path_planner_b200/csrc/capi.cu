@@ -8,7 +8,6 @@
 #include <new>
 #include <string>
 #include <thread>
-#include <type_traits>
 #include <vector>
 
 #include "vhp_internal.h"
@@ -979,8 +978,7 @@ vhp_status check_range(vhp_context *ctx, const std::string &what, const VhpMerge
 
 vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
                             const void *group_ptr, int64_t ngroups, int64_t nsrc, double thr, int dtype,
-                            const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false,
-                            const void *views = nullptr) {
+                            const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false) {
   const std::string what = merge_name(range, view);
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
@@ -995,7 +993,7 @@ vhp_status check_merge_args(vhp_context *ctx, const void *occ, int nmaps, int nx
     const vhp_status sr = check_range(ctx, what, *range);
     if (sr != VHP_OK) return sr;
   }
-  if (view && nsrc > 0 && !views) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": views is NULL");
+  if (view && nsrc > 0 && !range->views) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": views is NULL");
   return VHP_OK;
 }
 
@@ -1098,23 +1096,24 @@ vhp_status check_groups_host(vhp_context *ctx, const std::string &what, const in
   return VHP_OK;
 }
 
-// host buffers: validate, upload maps and sources once, then runs of whole groups whose outputs fit 1 GB of device
-// memory (at least one group), each copied back with plain cudaMemcpyAsync (the merged result is already K times
-// smaller than the fields it folds).  view: vhp_visibility_merge_view_batch, views [nsrc][5] uploaded with the
-// sources.
-vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
-                          const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
-                          const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false,
-                          const int32_t *views = nullptr) {
-  const char *what = merge_name(range, view);
-  vhp_status st = check_groups_host(ctx, what, gptr, ngroups);
-  if (st != VHP_OK) return st;
-  const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
-  st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range, view, views);
-  if (st != VHP_OK) return st;
-  if (view && (st = check_views_host(ctx, views, nsrc, range->radius, what, "source")) != VHP_OK) return st;
-  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, what)) != VHP_OK) return st;
-  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, what)) != VHP_OK) return st;
+// The host form of the group calls (merge and cover), after the call's argument checks: check the views (range->views,
+// null but for the view calls), the sources and the group maps, upload maps, sources and views once, then runs of
+// whole groups, as many as fit `budget` at per_src bytes per source plus per_group (at least one).  Each run's
+// group_ptr, rebased, and its group maps go to b_misc / b_map, and run(g0, gc, d_xy, d_gptr, d_gmap, nsrc, range) runs
+// the device form on groups [g0, g0 + gc) and copies their outputs (out_bytes per group) back with plain
+// cudaMemcpyAsync, synchronised: h_ptr and the buffers are reused.  name / item: the call and what a source is called,
+// for the messages.
+template <class Run>
+vhp_status run_groups_host(vhp_context *ctx, const char *name, const char *item, const uint8_t *occ, int nmaps,
+                           int nx, int ny, const int32_t *xy, const int64_t *gptr, const int32_t *gmap,
+                           int64_t ngroups, const VhpMergeRange *range, size_t per_src, size_t per_group,
+                           size_t budget, size_t out_bytes, const char *upload_what, Run run) {
+  const int64_t nsrc = gptr[ngroups];
+  const int32_t *views = range ? range->views : nullptr;
+  vhp_status st;
+  if (views && (st = check_views_host(ctx, views, nsrc, range->radius, name, item)) != VHP_OK) return st;
+  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, name)) != VHP_OK) return st;
+  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, ngroups, nmaps, nx, ny, name)) != VHP_OK) return st;
   ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
   ctx->last_transport_packed = 0;
   if (ngroups == 0) return VHP_OK;
@@ -1123,48 +1122,32 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   // (the group maps are uploaded per run of groups below)
   if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
     return st;
-  if (view && nsrc > 0) {
+  if (views && nsrc > 0) {
     if ((st = ensure(ctx, ctx->b_views, 20 * (size_t)nsrc)) != VHP_OK) return st;
     VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_views.p, views, 20 * (size_t)nsrc, cudaMemcpyHostToDevice, ctx->stream));
   }
-  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
-  const size_t bv = out->vmax ? esz : 0, bf = out->first ? 4 : 0, bc = out->count ? 4 : 0;
-  const int64_t gchunk = std::min<int64_t>(ngroups, std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / (cells * (bv + bf + bc)))));
-  vhp_status result = ensure(ctx, ctx->b_out[0], (size_t)gchunk * cells * (bv + bf + bc));
-  if (result == VHP_OK) result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gchunk + 1));
-  if (result == VHP_OK && gmap) result = ensure(ctx, ctx->b_map, 4 * (size_t)gchunk);
-  std::vector<int64_t> h_ptr((size_t)gchunk + 1);
-  const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
-  for (int64_t g0 = 0; g0 < ngroups && result == VHP_OK; g0 += gchunk) {
-    const int64_t gc = std::min(gchunk, ngroups - g0), a = gptr[g0];
+  auto group_bytes = [&](int64_t g) { return (size_t)(gptr[g + 1] - gptr[g]) * per_src + per_group; };
+  std::vector<int64_t> h_ptr;
+  vhp_status result = VHP_OK;
+  for (int64_t g0 = 0, gc = 0; g0 < ngroups && result == VHP_OK; g0 += gc) {
+    size_t bytes = group_bytes(g0);
+    for (gc = 1; g0 + gc < ngroups && bytes + group_bytes(g0 + gc) <= budget; ++gc) bytes += group_bytes(g0 + gc);
+    const int64_t a = gptr[g0];
+    h_ptr.resize((size_t)gc + 1);
     for (int64_t i = 0; i <= gc; ++i) h_ptr[(size_t)i] = gptr[g0 + i] - a;
-    char *base = (char *)ctx->b_out[0].p;
-    VhpMergeDev m;
-    m.f32 = dtype == VHP_F32;
-    m.vmax = out->vmax ? base : nullptr;
-    m.first = out->first ? (int32_t *)(base + (size_t)gc * cells * bv) : nullptr;
-    m.count = out->count ? (uint32_t *)(base + (size_t)gc * cells * (bv + bf)) : nullptr;
+    if ((result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gc + 1))) != VHP_OK) break;
+    if (gmap && (result = ensure(ctx, ctx->b_map, 4 * (size_t)gc)) != VHP_OK) break;
     cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
                                     ctx->stream);
     if (e == cudaSuccess && gmap)
       e = cudaMemcpyAsync(ctx->b_map.p, gmap + g0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: upload of the group layout"); break; }
+    if (e != cudaSuccess) { result = cuda_fail(ctx, e, upload_what); break; }
     VhpMergeRange run_range;
     if (range) run_range = *range;
-    if (view) run_range.views = (const int32_t *)ctx->b_views.p + 5 * a;
-    result = run_merge_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy + 2 * a,
-                           (const int64_t *)ctx->b_misc.p, gmap ? (const int32_t *)ctx->b_map.p : nullptr, gc,
-                           gptr[g0 + gc] - a, thr, m, range ? &run_range : nullptr);
-    if (result != VHP_OK) break;
-    const size_t n = (size_t)gc * cells, off = (size_t)g0 * cells;
-    if (out->vmax) e = cudaMemcpyAsync((char *)out->vmax + off * esz, m.vmax, n * esz, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && out->first)
-      e = cudaMemcpyAsync(out->first + off, m.first, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && out->count)
-      e = cudaMemcpyAsync(out->count + off, m.count, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "merge: copy of the group outputs"); break; }
-    ctx->last_d2h_bytes += (int64_t)(n * (bv + bf + bc));
+    if (views) run_range.views = (const int32_t *)ctx->b_views.p + 5 * a;
+    result = run(g0, gc, (const int32_t *)ctx->b_src.p + 2 * a, (const int64_t *)ctx->b_misc.p,
+                 gmap ? (const int32_t *)ctx->b_map.p : nullptr, gptr[g0 + gc] - a, range ? &run_range : nullptr);
+    if (result == VHP_OK) ctx->last_d2h_bytes += (int64_t)((size_t)gc * out_bytes);
   }
   cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
   ctx->last_result_bytes = ctx->last_d2h_bytes;
@@ -1173,15 +1156,56 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
   return check_device_error(ctx);
 }
 
+// host buffers: runs of whole groups whose outputs fit 1 GB of device memory (the merged result is already K times
+// smaller than the fields it folds).  view: vhp_visibility_merge_view_batch, range->views [nsrc][5] on the host.
+vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
+                          const int64_t *gptr, const int32_t *gmap, int64_t ngroups, double thr, vhp_dtype dtype,
+                          const vhp_merge_out *out, const VhpMergeRange *range = nullptr, bool view = false) {
+  const char *what = merge_name(range, view);
+  vhp_status st = check_groups_host(ctx, what, gptr, ngroups);
+  if (st != VHP_OK) return st;
+  const int64_t nsrc = (ctx && gptr && ngroups >= 0) ? gptr[ngroups] : 0;
+  st = check_merge_args(ctx, occ, nmaps, nx, ny, xy, gptr, ngroups, nsrc, thr, dtype, out, range, view);
+  if (st != VHP_OK) return st;
+  const size_t cells = (size_t)nx * ny, esz = dtype == VHP_F32 ? 4 : 8;
+  const size_t bv = out->vmax ? esz : 0, bf = out->first ? 4 : 0, bc = out->count ? 4 : 0;
+  const size_t group_bytes = cells * (bv + bf + bc);
+  auto run = [&](int64_t g0, int64_t gc, const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap,
+                 int64_t run_nsrc, const VhpMergeRange *run_range) {
+    vhp_status r = ensure(ctx, ctx->b_out[0], (size_t)gc * group_bytes);
+    if (r != VHP_OK) return r;
+    char *base = (char *)ctx->b_out[0].p;
+    VhpMergeDev m;
+    m.f32 = dtype == VHP_F32;
+    m.vmax = out->vmax ? base : nullptr;
+    m.first = out->first ? (int32_t *)(base + (size_t)gc * cells * bv) : nullptr;
+    m.count = out->count ? (uint32_t *)(base + (size_t)gc * cells * (bv + bf)) : nullptr;
+    r = run_merge_dev(ctx, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy, d_gptr, d_gmap, gc, run_nsrc, thr, m,
+                      run_range);
+    if (r != VHP_OK) return r;
+    const size_t n = (size_t)gc * cells, off = (size_t)g0 * cells;
+    cudaError_t e = cudaSuccess;
+    if (out->vmax) e = cudaMemcpyAsync((char *)out->vmax + off * esz, m.vmax, n * esz, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->first)
+      e = cudaMemcpyAsync(out->first + off, m.first, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->count)
+      e = cudaMemcpyAsync(out->count + off, m.count, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    return e == cudaSuccess ? VHP_OK : cuda_fail(ctx, e, "merge: copy of the group outputs");
+  };
+  return run_groups_host(ctx, what, "source", occ, nmaps, nx, ny, xy, gptr, gmap, ngroups, range, 0, group_bytes,
+                         (size_t)1 << 30, group_bytes, "merge: upload of the group layout", run);
+}
+
 // ---- greedy coverage placement (vhp_visibility_cover_greedy_batch) --------------------------------------
 // Phase 1 stores every candidate's coverage bits over its box (VhpCoverBox): the direct route sweeps the boxes
 // straight into bits (kFmtCoverBits: threshold > 0 and window_direct_route), the fallback folds chunks of fp64
 // windows (run_window_dev, any of its routes) or, where a window would be larger than the map, of whole fields
 // (run_dev) with cover_fold_kernel.  Phase 2 (kernels_cover.cu) runs min(k, nsrc) greedy rounds on the device.
-// The weighted call (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds, the
-// m-fold call (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters, and
-// the view call (vhp_visibility_cover_greedy_view_batch) the m-fold call with each candidate's bits masked by its view
-// in between.
+// Every cover call is a CoverCall through check_cover_args and run_cover_dev (and run_cover_host): the weighted call
+// (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds, the m-fold call
+// (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters, and the view call
+// (vhp_visibility_cover_greedy_view_batch) the m-fold call with each candidate's bits masked by its view in between.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
 const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
 const char *const kCoverMfoldName = "vhp_visibility_cover_greedy_mfold_batch";
@@ -1189,75 +1213,56 @@ const char *const kCoverViewName = "vhp_visibility_cover_greedy_view_batch";
 // the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
 constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
-// the per-cell output of each cover call: the covered bits, or the m-fold call's counts
-void *cover_cells(const vhp_cover_out *o) { return o->covered; }
-void *cover_cells(const vhp_cover_weighted_out *o) { return o->covered; }
-void *cover_cells(const vhp_cover_mfold_out *o) { return o->count; }
+// A cover call and its arguments.  weighted: uint64 gains and uint8 weights; mfold (with weighted): cells count until
+// m picks cover them, `count` instead of `covered`; view (with mfold): range.views masks each candidate's bits.
+// extra: the target ([prob][ny][ceil(nx/32)] uint32) or the weights ([prob][ny][nx] uint8), may be null.
+struct CoverCall {
+  const char *name;
+  bool weighted = false, mfold = false, view = false;
+  int32_t k, m = 1;
+  VhpMergeRange range;
+  double thr;
+  const void *extra;
+  CoverCall(const char *call, int32_t k_, int32_t radius, int32_t shape, double thr_, const void *extra_)
+      : name(call), k(k_), range(radius, shape), thr(thr_), extra(extra_) {}
+};
 
-// Out: vhp_cover_out, vhp_cover_weighted_out or vhp_cover_mfold_out
+// a call's public outputs as VhpCoverOut; a null struct stays null (check_cover_args reports it).  Out: vhp_cover_out
+// or vhp_cover_weighted_out
 template <class Out>
-vhp_status check_cover_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
-                            const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k, const VhpMergeRange &range,
-                            double thr, const Out *out, const char *name = kCoverName) {
-  const std::string what = name;
+const VhpCoverOut *cover_out(const Out *p, VhpCoverOut &o) {
+  if (p) o = {p->pick, p->gain, p->npicked, p->covered, nullptr};
+  return p ? &o : nullptr;
+}
+const VhpCoverOut *cover_out(const vhp_cover_mfold_out *p, VhpCoverOut &o) {
+  if (p) o = {p->pick, p->gain, p->npicked, nullptr, p->count};
+  return p ? &o : nullptr;
+}
+
+// The m-fold and view calls report these under the m-fold call's name, but for "views is NULL".  The weighted key's
+// limit on nsrc is checked before any candidate is read; the views' values by check_views_host, or by bit 3 of d_err
+// on the device.
+vhp_status check_cover_args(vhp_context *ctx, const CoverCall &c, const void *occ, int nmaps, int nx, int ny,
+                            const void *xy, const void *group_ptr, int64_t nprob, int64_t nsrc,
+                            const VhpCoverOut *out) {
+  const std::string what = c.mfold ? kCoverMfoldName : c.name;
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || nprob < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
   if (nprob > INT32_MAX) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": more than 2^31 - 1 problems");
-  const vhp_status st = check_grid_dtype(ctx, nx, ny, VHP_F64);
+  vhp_status st = check_grid_dtype(ctx, nx, ny, VHP_F64);
   if (st != VHP_OK) return st;
-  if (thr != thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
-  if (k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": k < 0");
-  if (!out->pick && !out->gain && !out->npicked && !cover_cells(out))
+  if (c.thr != c.thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
+  if (c.k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": k < 0");
+  if (!out->pick && !out->gain && !out->npicked && !out->covered && !out->count)
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
-  return check_range(ctx, what, range);
-}
-
-// the cover call's checks, then the weighted key's limit on nsrc (before any candidate is read)
-template <class Out>
-vhp_status check_cover_weighted_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
-                                     const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
-                                     const VhpMergeRange &range, double thr, const Out *out,
-                                     const char *name = kCoverWeightedName) {
-  const vhp_status st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr, out,
-                                         name);
-  if (st != VHP_OK) return st;
-  if (nsrc >= kCoverWeightedMaxSrc)
-    return fail(ctx, VHP_ERR_INVALID_ARG, std::string(name) + ": 2^28 or more candidates");
+  if ((st = check_range(ctx, what, c.range)) != VHP_OK) return st;
+  if (c.weighted && nsrc >= kCoverWeightedMaxSrc)
+    return fail(ctx, VHP_ERR_INVALID_ARG, what + ": 2^28 or more candidates");
+  if (c.mfold && (c.m < 1 || c.m > 255)) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": m outside [1, 255]");
+  if (c.view && nsrc > 0 && !c.range.views)
+    return fail(ctx, VHP_ERR_INVALID_ARG, std::string(c.name) + ": views is NULL");
   return VHP_OK;
-}
-
-// the weighted call's checks, then m
-vhp_status check_cover_mfold_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
-                                  const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
-                                  const VhpMergeRange &range, double thr, int32_t m, const vhp_cover_mfold_out *out) {
-  const vhp_status st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr,
-                                                  out, kCoverMfoldName);
-  if (st != VHP_OK) return st;
-  if (m < 1 || m > 255) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverMfoldName) + ": m outside [1, 255]");
-  return VHP_OK;
-}
-
-// the m-fold call's checks, then the views' buffer (their values: check_views_host, or bit 3 of d_err on the device)
-vhp_status check_cover_view_args(vhp_context *ctx, const void *occ, int nmaps, int nx, int ny, const void *xy,
-                                 const void *views, const void *group_ptr, int64_t nprob, int64_t nsrc, int32_t k,
-                                 const VhpMergeRange &range, double thr, int32_t m, const vhp_cover_mfold_out *out) {
-  const vhp_status st = check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, group_ptr, nprob, nsrc, k, range, thr, m,
-                                               out);
-  if (st != VHP_OK) return st;
-  if (nsrc > 0 && !views) return fail(ctx, VHP_ERR_INVALID_ARG, std::string(kCoverViewName) + ": views is NULL");
-  return VHP_OK;
-}
-
-// Out: vhp_cover_out or vhp_cover_weighted_out, Dev: VhpCoverDev or VhpCoverWeightedDev
-template <class Dev, class Out>
-Dev cover_dev_of(const Out &o) {
-  Dev c;
-  c.pick = o.pick;
-  c.gain = o.gain;
-  c.npicked = o.npicked;
-  c.covered = o.covered;
-  return c;
 }
 
 // a workspace buffer of the rounds; a failed allocation names its size
@@ -1277,15 +1282,13 @@ struct CoverBits {
 };
 
 // Phase 1 of the cover calls: the table, the workspace of the rounds (ws_bytes) and every candidate's coverage bits
-vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
-                            const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                            const VhpMergeRange &range, double thr, bool weighted, CoverBits &cb, bool mfold = false,
-                            const char *call = nullptr) {
-  const char *name = call ? call : mfold ? kCoverMfoldName : weighted ? kCoverWeightedName : kCoverName;
-  const int R = std::min(range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
-  const bool disk = range.shape == VHP_RANGE_DISK;
-  const int r2 = range.radius * range.radius;
-  const int64_t rounds = std::min<int64_t>(k, nsrc);
+vhp_status run_cover_phase1(vhp_context *ctx, const CoverCall &c, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                            const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
+                            int64_t nsrc, CoverBits &cb) {
+  const int R = std::min(c.range.radius, std::max(nx, ny) - 1); // the geometry's radius: the same boxes
+  const bool disk = c.range.shape == VHP_RANGE_DISK;
+  const int r2 = c.range.radius * c.range.radius;
+  const int64_t rounds = std::min<int64_t>(c.k, nsrc);
   cb.R = R;
   vhp_status st;
   if (nprob > 0 || nsrc > 0) {
@@ -1297,17 +1300,17 @@ vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, i
                                          ctx->sm_count, ctx->stream, &ctx->launches));
     if (rounds > 0 && nprob > 0) {
       const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
-      if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits", name)) !=
+      if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits", c.name)) !=
           VHP_OK)
         return st;
-      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, weighted, mfold),
-                             "workspace", name)) != VHP_OK)
+      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, c.weighted, c.mfold),
+                             "workspace", c.name)) != VHP_OK)
         return st;
       uint32_t *bits = cb.bits = (uint32_t *)ctx->b_cover.p;
-      if (thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
+      if (c.thr > 0.0 && window_direct_route(ctx, nx, ny, R)) {
         if ((st = ensure_rcp2(ctx, std::min(std::max(nx, ny), R + 1) + 64)) != VHP_OK) return st;
         if ((st = pack_tile(ctx, d_occ, nmaps, nx, ny, false)) != VHP_OK) return st;
-        VHP_CUDA(ctx, vhp_launch_sweep_cover(ctx->tile, nx, ny, d_xy, pm, nsrc, R, thr, bits, ctx->rcp2_table,
+        VHP_CUDA(ctx, vhp_launch_sweep_cover(ctx->tile, nx, ny, d_xy, pm, nsrc, R, c.thr, bits, ctx->rcp2_table,
                                              ctx->d_err, ctx->stream, &ctx->launches));
         if (disk) cb.disk_r2 = r2;
       } else {
@@ -1322,7 +1325,7 @@ vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, i
                    : run_dev(ctx, Op::Sweep, d_occ, nmaps, nx, ny, d_xy + 2 * p0, pm + p0, np, VHP_F64, ctx->b_mwin.p);
           if (st != VHP_OK) return st;
           VHP_CUDA(ctx, vhp_launch_cover_fold((const double *)ctx->b_mwin.p, win ? R : -1, p0, np, nx, ny, R, disk, r2,
-                                              d_xy, thr, bits, ctx->sm_count, ctx->stream, &ctx->launches));
+                                              d_xy, c.thr, bits, ctx->sm_count, ctx->stream, &ctx->launches));
         }
       }
     }
@@ -1330,183 +1333,94 @@ vhp_status run_cover_phase1(vhp_context *ctx, const uint8_t *d_occ, int nmaps, i
   return VHP_OK;
 }
 
-vhp_status run_cover_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
-                         const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                         const VhpMergeRange &range, double thr, const uint32_t *d_target, const VhpCoverDev &out) {
+// Phase 1, the view call's mask of the bits (range r_c in the call's shape, so the rounds apply no disk), then the
+// rounds.  c.extra and c.range.views are on the device.
+vhp_status run_cover_dev(vhp_context *ctx, const CoverCall &c, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                         const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
+                         int64_t nsrc, const VhpCoverOut &out) {
   CoverBits cb;
-  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
-                                         false, cb);
+  const vhp_status st = run_cover_phase1(ctx, c, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, cb);
   if (st != VHP_OK) return st;
-  VHP_CUDA(ctx, vhp_launch_cover_greedy(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk, d_target,
-                                        k, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream, &ctx->launches));
+  if (c.view) {
+    if (cb.bits)
+      VHP_CUDA(ctx, vhp_launch_cover_view(cb.bits, nsrc, nx, ny, cb.R, c.range.radius, c.range.shape == VHP_RANGE_DISK,
+                                          d_xy, c.range.views, ctx->d_err, ctx->sm_count, ctx->stream,
+                                          &ctx->launches));
+    cb.disk_r2 = -1;
+  }
+  VHP_CUDA(ctx, vhp_launch_cover_greedy(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk, c.weighted,
+                                        c.mfold, c.extra, c.k, c.m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
+                                        &ctx->launches));
   return VHP_OK;
 }
 
-vhp_status run_cover_weighted_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
-                                  const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
-                                  int64_t nsrc, int32_t k, const VhpMergeRange &range, double thr,
-                                  const uint8_t *d_weights, const VhpCoverWeightedDev &out) {
-  CoverBits cb;
-  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
-                                         true, cb);
+// the _dev entry point of every cover call
+vhp_status cover_dev_entry(vhp_context *ctx, const CoverCall &c, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                           const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
+                           int64_t nsrc, const VhpCoverOut *out) {
+  const vhp_status st = check_cover_args(ctx, c, d_occ, nmaps, nx, ny, d_xy, d_gptr, nprob, nsrc, out);
   if (st != VHP_OK) return st;
-  VHP_CUDA(ctx, vhp_launch_cover_greedy_weighted(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk,
-                                                 d_weights, k, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
-                                                 &ctx->launches));
-  return VHP_OK;
+  VHP_ON_DEVICE(ctx);
+  return run_cover_dev(ctx, c, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, *out);
 }
 
-vhp_status run_cover_mfold_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
-                               const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob, int64_t nsrc, int32_t k,
-                               const VhpMergeRange &range, double thr, const uint8_t *d_weights, int32_t m,
-                               const VhpCoverMfoldDev &out) {
-  CoverBits cb;
-  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
-                                         true, cb, true);
-  if (st != VHP_OK) return st;
-  VHP_CUDA(ctx, vhp_launch_cover_greedy_mfold(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk,
-                                              d_weights, k, m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
-                                              &ctx->launches));
-  return VHP_OK;
-}
-
-// the view call: phase 1, the bits masked by the views (range r_c in the call's shape, so the rounds apply no disk),
-// then the m-fold rounds
-vhp_status run_cover_view_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny, const int32_t *d_xy,
-                              const int32_t *d_views, const int64_t *d_gptr, const int32_t *d_gmap, int64_t nprob,
-                              int64_t nsrc, int32_t k, const VhpMergeRange &range, double thr,
-                              const uint8_t *d_weights, int32_t m, const VhpCoverMfoldDev &out) {
-  CoverBits cb;
-  const vhp_status st = run_cover_phase1(ctx, d_occ, nmaps, nx, ny, d_xy, d_gptr, d_gmap, nprob, nsrc, k, range, thr,
-                                         true, cb, true, kCoverViewName);
-  if (st != VHP_OK) return st;
-  if (cb.bits)
-    VHP_CUDA(ctx, vhp_launch_cover_view(cb.bits, nsrc, nx, ny, cb.R, range.radius, range.shape == VHP_RANGE_DISK, d_xy,
-                                        d_views, ctx->d_err, ctx->sm_count, ctx->stream, &ctx->launches));
-  VHP_CUDA(ctx, vhp_launch_cover_greedy_mfold(cb.bits, nsrc, nprob, nx, ny, cb.R, -1, d_xy, cb.pg, cb.pk, d_weights,
-                                              k, m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
-                                              &ctx->launches));
-  return VHP_OK;
-}
-
-// host buffers: validate, upload maps and candidates once, then runs of whole problems whose device memory (candidate
-// bits, workspace, outputs) fits 4 GB (at least one problem), each copied back with plain cudaMemcpyAsync.  Out picks
-// the call: vhp_cover_out, extra = target ([prob][ny][ceil(nx/32)] uint32); vhp_cover_weighted_out, extra = weights
-// ([prob][ny][nx] uint8); vhp_cover_mfold_out, extra = weights and m, and count ([prob][ny][nx] uint8) instead of
-// covered.  extra may be null.  view (with vhp_cover_mfold_out): the view call, views [nsrc][5] uploaded with the
-// candidates.
-template <class Out>
-vhp_status run_cover_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny, const int32_t *xy,
-                          const int64_t *gptr, const int32_t *gmap, int64_t nprob, int32_t k,
-                          const VhpMergeRange &range, double thr, const void *extra, const Out *out, int32_t m = 1,
-                          bool view = false, const int32_t *views = nullptr) {
-  constexpr bool kM = std::is_same<Out, vhp_cover_mfold_out>::value;
-  constexpr bool kW = kM || std::is_same<Out, vhp_cover_weighted_out>::value;
-  using Dev = typename std::conditional<
-      kM, VhpCoverMfoldDev, typename std::conditional<kW, VhpCoverWeightedDev, VhpCoverDev>::type>::type;
-  using Gain = typename std::remove_pointer<decltype(Dev::gain)>::type;
-  const char *name = view ? kCoverViewName : kM ? kCoverMfoldName : kW ? kCoverWeightedName : kCoverName;
-  vhp_status st = check_groups_host(ctx, name, gptr, nprob);
+// host buffers: runs of whole problems whose device memory (candidate bits, workspace, outputs) fits 4 GB, each with
+// its slice of c.extra uploaded.  c.range.views: the view call's [nsrc][5] on the host.
+vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *occ, int nmaps, int nx, int ny,
+                          const int32_t *xy, const int64_t *gptr, const int32_t *gmap, int64_t nprob,
+                          const VhpCoverOut *out) {
+  vhp_status st = check_groups_host(ctx, c.name, gptr, nprob);
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
-  if constexpr (kM) {
-    st = view ? check_cover_view_args(ctx, occ, nmaps, nx, ny, xy, views, gptr, nprob, nsrc, k, range, thr, m, out)
-              : check_cover_mfold_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, m, out);
-    if (st == VHP_OK && view) st = check_views_host(ctx, views, nsrc, range.radius, kCoverViewName, "candidate");
-  } else if constexpr (kW)
-    st = check_cover_weighted_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
-  else
-    st = check_cover_args(ctx, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, k, range, thr, out);
-  if (st != VHP_OK) return st;
-  if ((st = check_points(ctx, xy, 2, nullptr, nsrc, nmaps, nx, ny, name)) != VHP_OK) return st;
-  if (gmap && (st = check_points(ctx, nullptr, 0, gmap, nprob, nmaps, nx, ny, name)) != VHP_OK) return st;
-  ctx->last_d2h_bytes = ctx->last_result_bytes = 0;
-  ctx->last_transport_packed = 0;
-  if (nprob == 0) return VHP_OK;
-  VHP_ON_DEVICE(ctx);
-  PlanesGuard planes_guard(ctx);
-  if ((st = stage_host_batch(ctx, occ, nmaps, nx, ny, xy, 8, nsrc, nullptr, sweeps_use_planes(ctx, nx, ny))) != VHP_OK)
-    return st;
-  if (view && nsrc > 0) {
-    if ((st = ensure(ctx, ctx->b_views, 20 * (size_t)nsrc)) != VHP_OK) return st;
-    VHP_CUDA(ctx, cudaMemcpyAsync(ctx->b_views.p, views, 20 * (size_t)nsrc, cudaMemcpyHostToDevice, ctx->stream));
-  }
-  const size_t plane = (size_t)ny * ((nx + 31) / 32);
-  const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(range.radius, std::max(nx, ny) - 1), 0, 0);
-  const size_t box = (size_t)b.H * b.W * 4, budget = (size_t)4 << 30;
-  const size_t bp = out->pick ? 4 * (size_t)k : 0, bg = out->gain ? sizeof(Gain) * (size_t)k : 0;
-  const size_t bn = out->npicked ? 4 : 0, bc = cover_cells(out) ? (kM ? (size_t)ny * nx : plane * 4) : 0;
-  const size_t bt = extra ? (kW ? (size_t)ny * nx : plane * 4) : 0;
+  if ((st = check_cover_args(ctx, c, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, out)) != VHP_OK) return st;
+  const size_t plane = (size_t)ny * ((nx + 31) / 32), gsz = c.weighted ? 8 : 4;
+  const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(c.range.radius, std::max(nx, ny) - 1), 0, 0);
+  const size_t box = (size_t)b.H * b.W * 4;
+  const size_t bp = out->pick ? 4 * (size_t)c.k : 0, bg = out->gain ? gsz * (size_t)c.k : 0;
+  const size_t bn = out->npicked ? 4 : 0, bc = out->covered ? plane * 4 : out->count ? (size_t)ny * nx : 0;
+  const size_t bt = c.extra ? (c.weighted ? (size_t)ny * nx : plane * 4) : 0;
   // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
   // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters; views: 20 bytes)
-  const size_t per_src = box + 12 + sizeof(Gain) + (view ? 20 : 0), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
-                                                             (kW ? plane * 32 : 0) + (kM ? plane * 32 : 0);
-  auto prob_bytes = [&](int64_t q) { return (size_t)(gptr[q + 1] - gptr[q]) * per_src + per_prob; };
-  std::vector<int64_t> h_ptr;
-  const int32_t *d_xy = (const int32_t *)ctx->b_src.p;
-  vhp_status result = VHP_OK;
-  for (int64_t q0 = 0, gc = 0; q0 < nprob && result == VHP_OK; q0 += gc) {
-    size_t bytes = prob_bytes(q0);
-    for (gc = 1; q0 + gc < nprob && bytes + prob_bytes(q0 + gc) <= budget; ++gc) bytes += prob_bytes(q0 + gc);
-    const int64_t a = gptr[q0];
-    h_ptr.resize((size_t)gc + 1);
-    for (int64_t i = 0; i <= gc; ++i) h_ptr[(size_t)i] = gptr[q0 + i] - a;
-    if ((result = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + bn + bc) + 256)) != VHP_OK) break;
-    if ((result = ensure(ctx, ctx->b_misc, 8 * ((size_t)gc + 1))) != VHP_OK) break;
-    if (gmap && (result = ensure(ctx, ctx->b_map, 4 * (size_t)gc)) != VHP_OK) break;
-    if (extra && (result = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) break;
-    char *base = (char *)ctx->b_out[0].p;
-    const size_t o_gain = (gc * bp + sizeof(Gain) - 1) & ~(sizeof(Gain) - 1); // uint64 gains: 8-byte aligned
-    Dev o;
-    o.pick = out->pick ? (int32_t *)base : nullptr;
-    o.gain = out->gain ? (Gain *)(base + o_gain) : nullptr;
-    o.npicked = out->npicked ? (int32_t *)(base + o_gain + gc * bg) : nullptr;
-    char *cells = cover_cells(out) ? base + o_gain + gc * (bg + bn) : nullptr;
-    if constexpr (kM)
-      o.count = (uint8_t *)cells;
-    else
-      o.covered = (uint32_t *)cells;
-    cudaError_t e = cudaMemcpyAsync(ctx->b_misc.p, h_ptr.data(), 8 * ((size_t)gc + 1), cudaMemcpyHostToDevice,
-                                    ctx->stream);
-    if (e == cudaSuccess && gmap)
-      e = cudaMemcpyAsync(ctx->b_map.p, gmap + q0, 4 * (size_t)gc, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess && extra)
-      e = cudaMemcpyAsync(ctx->b_out[1].p, (const char *)extra + (size_t)q0 * bt, (size_t)gc * bt,
+  const size_t per_src = box + 12 + gsz + (c.view ? 20 : 0), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
+                                                                  (c.weighted ? plane * 32 : 0) +
+                                                                  (c.mfold ? plane * 32 : 0);
+  void *const host_cells = out->covered ? (void *)out->covered : (void *)out->count;
+  auto run = [&](int64_t q0, int64_t gc, const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap,
+                 int64_t run_nsrc, const VhpMergeRange *run_range) {
+    vhp_status r;
+    if ((r = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + bn + bc) + 256)) != VHP_OK) return r;
+    if (c.extra && (r = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) return r;
+    cudaError_t e = cudaSuccess;
+    if (c.extra)
+      e = cudaMemcpyAsync(ctx->b_out[1].p, (const char *)c.extra + (size_t)q0 * bt, (size_t)gc * bt,
                           cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: upload of the problems"); break; }
-    const uint8_t *d_occ = (const uint8_t *)ctx->b_occ.p;
-    const int64_t *d_gptr = (const int64_t *)ctx->b_misc.p;
-    const int32_t *d_gmap = gmap ? (const int32_t *)ctx->b_map.p : nullptr;
-    if constexpr (kM)
-      result = view ? run_cover_view_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, (const int32_t *)ctx->b_views.p + 5 * a,
-                                         d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k, range, thr,
-                                         extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o)
-                    : run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc,
-                                          gptr[q0 + gc] - a, k, range, thr,
-                                          extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, m, o);
-    else if constexpr (kW)
-      result = run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a,
-                                      k, range, thr, extra ? (const uint8_t *)ctx->b_out[1].p : nullptr, o);
-    else
-      result = run_cover_dev(ctx, d_occ, nmaps, nx, ny, d_xy + 2 * a, d_gptr, d_gmap, gc, gptr[q0 + gc] - a, k, range,
-                             thr, extra ? (const uint32_t *)ctx->b_out[1].p : nullptr, o);
-    if (result != VHP_OK) break;
-    if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "cover: upload of the problems");
+    char *base = (char *)ctx->b_out[0].p;
+    const size_t o_gain = (gc * bp + gsz - 1) & ~(gsz - 1); // uint64 gains: 8-byte aligned
+    char *cells = base + o_gain + gc * (bg + bn);
+    VhpCoverOut o;
+    o.pick = out->pick ? (int32_t *)base : nullptr;
+    o.gain = out->gain ? base + o_gain : nullptr;
+    o.npicked = out->npicked ? (int32_t *)(base + o_gain + gc * bg) : nullptr;
+    o.covered = out->covered ? (uint32_t *)cells : nullptr;
+    o.count = out->count ? (uint8_t *)cells : nullptr;
+    CoverCall rc = c;
+    rc.range = *run_range;
+    rc.extra = c.extra ? ctx->b_out[1].p : nullptr;
+    r = run_cover_dev(ctx, rc, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy, d_gptr, d_gmap, gc, run_nsrc, o);
+    if (r != VHP_OK) return r;
+    if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * c.k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && out->gain)
-      e = cudaMemcpyAsync(out->gain + q0 * k, o.gain, gc * bg, cudaMemcpyDeviceToHost, ctx->stream);
+      e = cudaMemcpyAsync((char *)out->gain + q0 * bg, o.gain, gc * bg, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && out->npicked)
       e = cudaMemcpyAsync(out->npicked + q0, o.npicked, gc * bn, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && cells)
-      e = cudaMemcpyAsync((char *)cover_cells(out) + q0 * bc, cells, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // h_ptr and the buffers are reused
-    if (e != cudaSuccess) { result = cuda_fail(ctx, e, "cover: copy of the outputs"); break; }
-    ctx->last_d2h_bytes += (int64_t)(gc * (bp + bg + bn + bc));
-  }
-  cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-  ctx->last_result_bytes = ctx->last_d2h_bytes;
-  if (result != VHP_OK) return result;
-  if (e2 != cudaSuccess) return cuda_fail(ctx, e2, "sync stream");
-  return check_device_error(ctx);
+    if (e == cudaSuccess && host_cells)
+      e = cudaMemcpyAsync((char *)host_cells + q0 * bc, cells, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    return e == cudaSuccess ? VHP_OK : cuda_fail(ctx, e, "cover: copy of the outputs");
+  };
+  return run_groups_host(ctx, c.name, "candidate", occ, nmaps, nx, ny, xy, gptr, gmap, nprob, &c.range, per_src,
+                         per_prob, (size_t)4 << 30, bp + bg + bn + bc, "cover: upload of the problems", run);
 }
 
 // ---- opt-in sweep variants ------------------------------------------------------------------------
@@ -2047,9 +1961,7 @@ vhp_status vhp_visibility_merge_range_batch(vhp_context *ctx, const uint8_t *occ
                                             const int32_t *group_map, int64_t ngroups, int32_t radius,
                                             int32_t shape, double threshold, vhp_dtype dtype,
                                             const vhp_merge_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
+  const VhpMergeRange range(radius, shape);
   return run_merge_host(ctx, occ, nmaps, nx, ny, src_xy, group_ptr, group_map, ngroups, threshold, dtype, out,
                         &range);
 }
@@ -2059,9 +1971,7 @@ vhp_status vhp_visibility_merge_range_batch_dev(vhp_context *ctx, const uint8_t 
                                                 const int32_t *d_group_map, int64_t ngroups, int64_t nsrc,
                                                 int32_t radius, int32_t shape, double threshold,
                                                 vhp_dtype dtype, const vhp_merge_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
+  const VhpMergeRange range(radius, shape);
   vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
                                    d_out, &range);
   if (st != VHP_OK) return st;
@@ -2074,11 +1984,9 @@ vhp_status vhp_visibility_merge_view_batch(vhp_context *ctx, const uint8_t *occ,
                                            const int32_t *src_xy, const int32_t *views, const int64_t *group_ptr,
                                            const int32_t *group_map, int64_t ngroups, int32_t radius, int32_t shape,
                                            double threshold, vhp_dtype dtype, const vhp_merge_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
+  const VhpMergeRange range(radius, shape, views);
   return run_merge_host(ctx, occ, nmaps, nx, ny, src_xy, group_ptr, group_map, ngroups, threshold, dtype, out,
-                        &range, true, views);
+                        &range, true);
 }
 
 vhp_status vhp_visibility_merge_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -2086,12 +1994,9 @@ vhp_status vhp_visibility_merge_view_batch_dev(vhp_context *ctx, const uint8_t *
                                                const int64_t *d_group_ptr, const int32_t *d_group_map,
                                                int64_t ngroups, int64_t nsrc, int32_t radius, int32_t shape,
                                                double threshold, vhp_dtype dtype, const vhp_merge_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  range.views = d_views;
+  const VhpMergeRange range(radius, shape, d_views);
   vhp_status st = check_merge_args(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, ngroups, nsrc, threshold, dtype,
-                                   d_out, &range, true, d_views);
+                                   d_out, &range, true);
   if (st != VHP_OK) return st;
   VHP_ON_DEVICE(ctx);
   return run_merge_dev(ctx, d_occ, nmaps, nx, ny, d_src_xy, d_group_ptr, d_group_map, ngroups, nsrc, threshold,
@@ -2103,11 +2008,9 @@ vhp_status vhp_visibility_cover_greedy_batch(vhp_context *ctx, const uint8_t *oc
                                              const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
                                              int32_t shape, double threshold, const uint32_t *target,
                                              const vhp_cover_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, target,
-                        out);
+  const CoverCall c(kCoverName, k, radius, shape, threshold, target);
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
@@ -2115,15 +2018,10 @@ vhp_status vhp_visibility_cover_greedy_batch_dev(vhp_context *ctx, const uint8_t
                                                  const int32_t *d_group_map, int64_t nprob, int64_t nsrc, int32_t k,
                                                  int32_t radius, int32_t shape, double threshold,
                                                  const uint32_t *d_target, const vhp_cover_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  vhp_status st = check_cover_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
-                                   threshold, d_out);
-  if (st != VHP_OK) return st;
-  VHP_ON_DEVICE(ctx);
-  return run_cover_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
-                       threshold, d_target, cover_dev_of<VhpCoverDev>(*d_out));
+  const CoverCall c(kCoverName, k, radius, shape, threshold, d_target);
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_weighted_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
@@ -2131,11 +2029,10 @@ vhp_status vhp_visibility_cover_greedy_weighted_batch(vhp_context *ctx, const ui
                                                       const int32_t *group_map, int64_t nprob, int32_t k,
                                                       int32_t radius, int32_t shape, double threshold,
                                                       const uint8_t *weights, const vhp_cover_weighted_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
-                        out);
+  CoverCall c(kCoverWeightedName, k, radius, shape, threshold, weights);
+  c.weighted = true;
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
@@ -2144,15 +2041,11 @@ vhp_status vhp_visibility_cover_greedy_weighted_batch_dev(vhp_context *ctx, cons
                                                           int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
                                                           int32_t shape, double threshold, const uint8_t *d_weights,
                                                           const vhp_cover_weighted_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  vhp_status st = check_cover_weighted_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
-                                            threshold, d_out);
-  if (st != VHP_OK) return st;
-  VHP_ON_DEVICE(ctx);
-  return run_cover_weighted_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
-                                threshold, d_weights, cover_dev_of<VhpCoverWeightedDev>(*d_out));
+  CoverCall c(kCoverWeightedName, k, radius, shape, threshold, d_weights);
+  c.weighted = true;
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_mfold_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
@@ -2160,11 +2053,11 @@ vhp_status vhp_visibility_cover_greedy_mfold_batch(vhp_context *ctx, const uint8
                                                    const int32_t *group_map, int64_t nprob, int32_t k, int32_t radius,
                                                    int32_t shape, double threshold, const uint8_t *weights, int32_t m,
                                                    const vhp_cover_mfold_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
-                        out, m);
+  CoverCall c(kCoverMfoldName, k, radius, shape, threshold, weights);
+  c.weighted = c.mfold = true;
+  c.m = m;
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
@@ -2173,20 +2066,12 @@ vhp_status vhp_visibility_cover_greedy_mfold_batch_dev(vhp_context *ctx, const u
                                                        int32_t k, int32_t radius, int32_t shape, double threshold,
                                                        const uint8_t *d_weights, int32_t m,
                                                        const vhp_cover_mfold_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  vhp_status st = check_cover_mfold_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, nprob, nsrc, k, range,
-                                         threshold, m, d_out);
-  if (st != VHP_OK) return st;
-  VHP_ON_DEVICE(ctx);
-  VhpCoverMfoldDev o;
-  o.pick = d_out->pick;
-  o.gain = d_out->gain;
-  o.npicked = d_out->npicked;
-  o.count = d_out->count;
-  return run_cover_mfold_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc, k, range,
-                             threshold, d_weights, m, o);
+  CoverCall c(kCoverMfoldName, k, radius, shape, threshold, d_weights);
+  c.weighted = c.mfold = true;
+  c.m = m;
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_view_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
@@ -2194,11 +2079,12 @@ vhp_status vhp_visibility_cover_greedy_view_batch(vhp_context *ctx, const uint8_
                                                   const int64_t *group_ptr, const int32_t *group_map, int64_t nprob,
                                                   int32_t k, int32_t radius, int32_t shape, double threshold,
                                                   const uint8_t *weights, int32_t m, const vhp_cover_mfold_out *out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  return run_cover_host(ctx, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, k, range, threshold, weights,
-                        out, m, true, views);
+  CoverCall c(kCoverViewName, k, radius, shape, threshold, weights);
+  c.weighted = c.mfold = c.view = true;
+  c.m = m;
+  c.range.views = views;
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
 }
 
 vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,
@@ -2207,20 +2093,13 @@ vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const ui
                                                       int64_t nprob, int64_t nsrc, int32_t k, int32_t radius,
                                                       int32_t shape, double threshold, const uint8_t *d_weights,
                                                       int32_t m, const vhp_cover_mfold_out *d_out) {
-  VhpMergeRange range;
-  range.radius = radius;
-  range.shape = shape;
-  vhp_status st = check_cover_view_args(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_views, d_group_ptr, nprob, nsrc, k,
-                                        range, threshold, m, d_out);
-  if (st != VHP_OK) return st;
-  VHP_ON_DEVICE(ctx);
-  VhpCoverMfoldDev o;
-  o.pick = d_out->pick;
-  o.gain = d_out->gain;
-  o.npicked = d_out->npicked;
-  o.count = d_out->count;
-  return run_cover_view_dev(ctx, d_occ, nmaps, nx, ny, d_cand_xy, d_views, d_group_ptr, d_group_map, nprob, nsrc, k,
-                            range, threshold, d_weights, m, o);
+  CoverCall c(kCoverViewName, k, radius, shape, threshold, d_weights);
+  c.weighted = c.mfold = c.view = true;
+  c.m = m;
+  c.range.views = d_views;
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
 }
 
 vhp_status vhp_raycast_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx,

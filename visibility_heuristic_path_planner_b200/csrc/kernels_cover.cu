@@ -655,32 +655,20 @@ size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bo
   return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold, mfold).bytes;
 }
 
-cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
-                                    int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                    const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
-                                    const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches) {
-  return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, d_target,
-                              nullptr, k, 1, d_ws, out, nullptr, sm_count, st, launches);
-}
-
-cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
-                                             int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                             const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, void *d_ws,
-                                             const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
-                                             int64_t *launches) {
-  return launch_rounds<true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
-                             d_weights, k, 1, d_ws, out, nullptr, sm_count, st, launches);
-}
-
-cudaError_t vhp_launch_cover_greedy_mfold(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
-                                          int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                          const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, int m,
-                                          void *d_ws, const VhpCoverMfoldDev &out, int sm_count, cudaStream_t st,
-                                          int64_t *launches) {
-  VhpCoverWeightedDev o;
-  o.pick = out.pick;
-  o.gain = out.gain;
-  o.npicked = out.npicked;
+cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
+                                    const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
+                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m, void *d_ws,
+                                    const VhpCoverOut &out, int sm_count, cudaStream_t st, int64_t *launches) {
+  if (!weighted) {
+    const VhpCoverDevT<uint32_t> o{out.pick, (uint32_t *)out.gain, out.npicked, out.covered};
+    return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k,
+                                (const uint32_t *)d_extra, nullptr, k, 1, d_ws, o, nullptr, sm_count, st, launches);
+  }
+  const VhpCoverDevT<uint64_t> o{out.pick, (uint64_t *)out.gain, out.npicked, out.covered};
+  const uint8_t *d_weights = (const uint8_t *)d_extra;
+  if (!mfold)
+    return launch_rounds<true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
+                               d_weights, k, 1, d_ws, o, nullptr, sm_count, st, launches);
   return launch_rounds<true, true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
                                    d_weights, k, m, d_ws, o, out.count, sm_count, st, launches);
 }

@@ -244,6 +244,8 @@ struct VhpMergeRange {
   int radius = 0;
   int shape = VHP_RANGE_BOX;
   const int32_t *views = nullptr;
+  VhpMergeRange() = default;
+  VhpMergeRange(int r, int s, const int32_t *v = nullptr) : radius(r), shape(s), views(v) {}
 };
 // the sweeps fold straight into the group outputs (kFmtMerge*, one CTA per pair); needs thr > 0 and zero-filled
 // vmax / count, -1-filled first.  range: sweep only each pair's box and fold only its cells in range
@@ -306,7 +308,16 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
                                   bool disk, int r2, const int32_t *d_xy, double thr, uint32_t *d_bits, int sm_count,
                                   cudaStream_t st, int64_t *launches);
 // Phase 2, the greedy rounds over the bits of nsrc candidates (table of vhp_launch_merge_table) of nprob problems.
-// Gain is uint32 (cells) for the cover call, uint64 (summed weights) for the weighted call.
+// The outputs of every cover call (any may be null): gain is uint32 (cells) for the cover call, uint64 (summed
+// weights) for the weighted ones; the m-fold rounds write count instead of covered.
+struct VhpCoverOut {
+  int32_t *pick = nullptr;     // [prob][k]
+  void *gain = nullptr;        // [prob][k]
+  int32_t *npicked = nullptr;  // [prob]
+  uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
+  uint8_t *count = nullptr;    // [prob][ny][nx], min(m, picks whose S covers the cell)
+};
+// cover_apply_kernel's parameter (kernels_cover.cu): the outputs but count, with the gain typed
 template <class Gain>
 struct VhpCoverDevT {
   int32_t *pick = nullptr;   // [prob][k]
@@ -314,36 +325,17 @@ struct VhpCoverDevT {
   int32_t *npicked = nullptr; // [prob]
   uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
 };
-using VhpCoverDev = VhpCoverDevT<uint32_t>;
-using VhpCoverWeightedDev = VhpCoverDevT<uint64_t>;
-// the m-fold call's outputs: gains as the weighted call's, count instead of covered
-struct VhpCoverMfoldDev {
-  int32_t *pick = nullptr;    // [prob][k]
-  uint64_t *gain = nullptr;   // [prob][k]
-  int32_t *npicked = nullptr; // [prob]
-  uint8_t *count = nullptr;   // [prob][ny][nx], min(m, picks whose S covers the cell)
-};
 // workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane; m-fold:
 // those of the weighted rounds and a counter plane of the padded plane's size)
 size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold = false);
 // outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
-// route's sweep stores the whole box); d_target (may be null): [prob][ny][ceil(nx/32)] bits of the cells to cover
-cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
-                                    int ny, int R, int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                    const int32_t *d_pair_k, const uint32_t *d_target, int32_t k, void *d_ws,
-                                    const VhpCoverDev &out, int sm_count, cudaStream_t st, int64_t *launches);
-// the weighted rounds: d_weights (may be null: every cell weighs 1) [prob][ny][nx] uint8; nsrc < 2^28
-cudaError_t vhp_launch_cover_greedy_weighted(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
-                                             int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                             const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, void *d_ws,
-                                             const VhpCoverWeightedDev &out, int sm_count, cudaStream_t st,
-                                             int64_t *launches);
-// the m-fold rounds: the weighted rounds, where a cell's weight counts until m in [1, 255] picks cover it
-cudaError_t vhp_launch_cover_greedy_mfold(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R,
-                                          int disk_r2, const int32_t *d_xy, const int32_t *d_pair_group,
-                                          const int32_t *d_pair_k, const uint8_t *d_weights, int32_t k, int m,
-                                          void *d_ws, const VhpCoverMfoldDev &out, int sm_count, cudaStream_t st,
-                                          int64_t *launches);
+// route's sweep stores the whole box).  d_extra (may be null): [prob][ny][ceil(nx/32)] uint32 bits of the cells to
+// cover, or for the weighted rounds [prob][ny][nx] uint8 weights (null: every cell weighs 1; nsrc < 2^28).  The
+// m-fold rounds (with weighted) are the weighted rounds where a cell's weight counts until m in [1, 255] picks cover it.
+cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
+                                    const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
+                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m, void *d_ws,
+                                    const VhpCoverOut &out, int sm_count, cudaStream_t st, int64_t *launches);
 // the view call, between phase 1 and the m-fold rounds (which then run with disk_r2 = -1): every candidate's bits
 // &= its view, d_views [nsrc][5] = (r, ax, ay, bx, by): range r in [0, radius] in the call's shape (disk or box), and
 // the sector of a and b.  A bad view raises bit 3 of d_err and clears the candidate's bits.
