@@ -401,6 +401,56 @@ vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const ui
                                                       int32_t shape, double threshold, const uint8_t *d_weights,
                                                       int32_t m, const vhp_cover_mfold_out *d_out);
 
+/* Quota sensor placement: the fewest greedy picks that reach a coverage target ("how few cameras cover 95 % of this
+ * floor", "how many sensors until every doorway is seen twice"), with the rounds looping on the device.  The inputs
+ * are those of vhp_visibility_cover_greedy_view_batch (problems, candidates, views, group_map, radius R, shape,
+ * threshold, weights, m, the 2^28 limit), except that views may be NULL (every candidate omnidirectional with r = R:
+ * the call is then vhp_visibility_cover_greedy_mfold_batch), k is kmax, and quota ([prob] uint64, in the units of f)
+ * is new.  With f(A) = sum over x of W_q(x) * min(cnt_A(x), m), problem q runs that call's greedy and stops at the
+ * first of:
+ *   reached    the picks so far have total = sum of gain >= quota[q] (quota 0: no pick);
+ *   exhausted  the argmax gain is 0 (everything coverable is counted);
+ *   capped     kmax picks.
+ * So npicked[q] = min { j : sum_{i<j} gain_i >= quota[q] }, limited by the other two, and since the greedy sequence is
+ * the same for any k the result is exactly a prefix: pick, gain and npicked are those of the view call (views given) or
+ * the m-fold call (views NULL) with k = kmax, cut at npicked[q], and count is that call's count with k = npicked[q].
+ * Every decision is an integer comparison, so the result is exact and order-independent.  quota = UINT64_MAX and
+ * kmax >= the group's size is greedy set cover of the coverable weight.  Outputs (any may be NULL, at least one must be
+ * given):
+ *   pick[q][r]     index within the group of the r-th pick, -1 from npicked on             (int32 [prob][kmax])
+ *   gain[q][r]     what the r-th pick adds to f, 0 from npicked on, non-increasing         (uint64 [prob][kmax])
+ *   npicked[q]                                                                             (int32 [prob])
+ *   count[q]       min(m, number of picks whose S covers the cell)                         (uint8 [prob][ny][nx])
+ *   total[q]       f(picks) = sum of gain; the quota is reached exactly when total >= quota (uint64 [prob])
+ * Routes, phase 1 and the view mask are those of vhp_visibility_cover_greedy_view_batch.  The rounds are the body of a
+ * CUDA-graph WHILE node, built, launched and destroyed by each call (each run of problems of the host form), that runs
+ * until no problem is active or min(kmax, nsrc) rounds have run; the launch count does not depend on the quotas or on
+ * the rounds run, and the _dev form does not synchronise.  Workspace: that of vhp_visibility_cover_greedy_mfold_batch
+ * plus 16 bytes per problem (total and a copy of the quota) and two counters; the host form's 4 GB batches also count
+ * each problem's 8 quota and 8 total bytes.  A failure to build the graph is VHP_ERR_CUDA with the CUDA message.
+ * Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_cover_greedy_view_batch (sizes, NaN threshold, radius and
+ * shape, m outside [1, 255], the 2^28 limit, bad views when views are given), kmax < 0, quota NULL with nprob > 0, no
+ * output.  The host form checks them all before any candidate is read; the _dev form reports a bad view as the view
+ * call does.  kmax == 0 is valid (npicked 0, count and total zero). */
+typedef struct vhp_cover_quota_out {
+  int32_t *pick;     /* [prob][kmax], -1 from npicked on */
+  uint64_t *gain;    /* [prob][kmax], 0 from npicked on, non-increasing */
+  int32_t *npicked;  /* [prob] */
+  uint8_t *count;    /* [prob][ny][nx], min(m, picks covering the cell) */
+  uint64_t *total;   /* [prob], f(picks) = sum of gain; reached <=> total >= quota */
+} vhp_cover_quota_out;
+vhp_status vhp_visibility_cover_quota_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                            const int32_t *cand_xy, const int32_t *views, const int64_t *group_ptr,
+                                            const int32_t *group_map, int64_t nprob, int32_t kmax, int32_t radius,
+                                            int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                            const uint64_t *quota, const vhp_cover_quota_out *out);
+vhp_status vhp_visibility_cover_quota_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                const int32_t *d_cand_xy, const int32_t *d_views,
+                                                const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t nprob,
+                                                int64_t nsrc, int32_t kmax, int32_t radius, int32_t shape,
+                                                double threshold, const uint8_t *d_weights, int32_t m,
+                                                const uint64_t *d_quota, const vhp_cover_quota_out *d_out);
+
 /* Directional merged visibility: what a set of cameras with headings and fields of view covers together, the
  * evaluation counterpart of vhp_visibility_cover_greedy_view_batch.  Everything is vhp_visibility_merge_range_batch
  * (inputs, groups, group_map, radius R, shape, threshold, dtype, the outputs and the "writes" rule), with source k's

@@ -66,6 +66,13 @@ class CoverMfoldOut(C.Structure):
     _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("count", C.c_void_p)]
 
 
+class CoverQuotaOut(C.Structure):
+    """struct vhp_cover_quota_out: pick (int32 [prob][kmax]), gain (uint64 [prob][kmax]), npicked (int32 [prob]), count
+    (uint8 [prob][ny][nx]), total (uint64 [prob]), each may be NULL."""
+    _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("count", C.c_void_p),
+                ("total", C.c_void_p)]
+
+
 class SweepVariant(C.Structure):
     """struct vhp_sweep_variant: model 1 = getAccessibilityMap.m (alpha, fac, light_strength),
     model 2 = computeVisibilityUsingQueue as an order-free rule (cutoff)."""
@@ -164,6 +171,12 @@ def load_library(build_if_missing: bool = True):
     lib.vhp_visibility_cover_greedy_view_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64,
                                                                C.c_int32, C.c_int32, C.c_int32, C.c_double, vp,
                                                                C.c_int32, C.POINTER(CoverMfoldOut)]
+    lib.vhp_visibility_cover_quota_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, C.c_int32, C.c_int32,
+                                                     C.c_int32, C.c_double, vp, C.c_int32, vp,
+                                                     C.POINTER(CoverQuotaOut)]
+    lib.vhp_visibility_cover_quota_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64, C.c_int32,
+                                                         C.c_int32, C.c_int32, C.c_double, vp, C.c_int32, vp,
+                                                         C.POINTER(CoverQuotaOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -223,6 +236,27 @@ def _cover_weights(weights, shape):
     if w.dtype != np.uint8 or w.shape != shape:
         raise ValueError(f"weights must be uint8 of shape {shape}, got {w.dtype} {w.shape}")
     return np.ascontiguousarray(w)
+
+
+def _cover_quota(quota, fraction, m, weights, n, shape):
+    """the quota call's uint64 quotas (n,): quota broadcast, ceil(fraction * m * sum of W_q) in float64, or UINT64_MAX"""
+    if quota is not None and fraction is not None:
+        raise ValueError("give quota or fraction, not both")
+    if fraction is not None:
+        p = float(fraction)
+        if not np.isfinite(p) or p < 0:
+            raise ValueError(f"fraction must be finite and >= 0, got {fraction}")
+        w = np.full(n, shape[0] * shape[1], np.int64) if weights is None else \
+            _cover_weights(weights, (n, *shape)).reshape(n, -1).sum(1, dtype=np.int64)
+        return np.ceil(p * float(int(m)) * w.astype(np.float64)).astype(np.uint64)
+    if quota is None:
+        return np.full(n, np.iinfo(np.uint64).max, np.uint64)
+    q = quota if isinstance(quota, np.ndarray) else np.array(quota, dtype=object)  # Python ints up to UINT64_MAX
+    if q.dtype.kind == "O" and not all(isinstance(v, (int, np.integer)) for v in q.ravel()):
+        raise ValueError("quota must be non-negative integers")
+    if q.dtype.kind not in "iuO" or (q.dtype.kind != "u" and (q < 0).any()):
+        raise ValueError(f"quota must be non-negative integers, got {q.dtype}")
+    return np.ascontiguousarray(np.broadcast_to(q.astype(np.uint64), (n,)))
 
 
 def _occ_u8(occ):
@@ -598,14 +632,49 @@ class Context:
                         group_ptr_t, k, threshold, radius, shape, (pick_t, gain_t, npicked_t, count_t), group_map_t,
                         weights_t, m=m, views_t=views_t)
 
+    def visibility_cover_quota_batch(self, occ, cand_xy, group_ptr, threshold, radius, shape, quota=None,
+                                     fraction=None, m=1, weights=None, views=None, kmax=None, group_map=None):
+        """Quota sensor placement (vhp_visibility_cover_quota_batch): the greedy of visibility_cover_greedy_view_batch
+        (views given) or visibility_cover_greedy_mfold_batch (views None), run per problem until the summed gain
+        reaches the problem's quota, the argmax gain is 0, or kmax picks are made; the result is a prefix of that
+        call's greedy.  quota: uint64 per problem (a scalar is every problem's), in units of
+        f = sum of W(x) * min(count(x), m); fraction=p instead gives quota_q = ceil(p * m * sum of W_q over every cell)
+        in float64.  The fraction counts every cell's weight, so cells that need no coverage, such as walls, should
+        weigh 0 (weights None: every cell weighs 1, walls included).  Neither: UINT64_MAX, greedy set cover of all that
+        can be covered.  kmax None: the largest group's size.  Returns pick (int32 (nprob, kmax)), gain (uint64
+        (nprob, kmax)), npicked (int32 (nprob,)), count (uint8 (nprob, ny, nx)), total (uint64 (nprob,), the summed
+        gain) and reached (bool (nprob,), total >= quota)."""
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        n = max(gp.shape[0] - 1, 0)
+        if kmax is None:
+            kmax = int(np.diff(gp).max()) if n else 0
+        q = _cover_quota(quota, fraction, m, weights, n, _occ_u8(occ).shape[1:])
+        r = self._cover_host(self.lib.vhp_visibility_cover_quota_batch, CoverQuotaOut, occ, cand_xy, gp, kmax,
+                             threshold, radius, shape, group_map, weights=weights, m=m, views=views, quota=q)
+        r["reached"] = r["total"] >= q
+        return r
+
+    def visibility_cover_quota_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, quota_t, kmax, threshold, radius, shape,
+                                         m=1, pick_t=None, gain_t=None, npicked_t=None, count_t=None, total_t=None,
+                                         group_map_t=None, weights_t=None, views_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2), group_ptr_t
+        int64 (nprob + 1), quota_t uint64 / int64 (nprob,) (the bits of a uint64), weights_t uint8 (nprob, ny, nx) or
+        None, views_t int32 (nsrc, 5) or None; outputs pick_t int32 (nprob, kmax), gain_t int64 / uint64 (nprob, kmax),
+        npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx), total_t int64 / uint64 (nprob,); any may be None.  A
+        bad view is reported by the next synchronising call."""
+        self._cover_dev(self.lib.vhp_visibility_cover_quota_batch_dev, CoverQuotaOut, occ_t, cand_xy_t, group_ptr_t,
+                        kmax, threshold, radius, shape, (pick_t, gain_t, npicked_t, count_t, total_t), group_map_t,
+                        weights_t, m=m, views_t=views_t, quota_t=quota_t)
+
     def _cover_host(self, fn, out_type, occ, cand_xy, group_ptr, k, threshold, radius, shape, group_map, target=None,
-                    weights=None, m=None, views=None):
-        # out_type's fields name the outputs: CoverOut has uint32 gains, the weighted calls' uint64 ones
+                    weights=None, m=None, views=False, quota=None):
+        # out_type's fields name the outputs: CoverOut has uint32 gains, the weighted calls' uint64 ones.  views: False
+        # for the calls without views, None for NULL
         occ = _occ_u8(occ)
         nmaps, ny, nx = occ.shape
         xy = np.ascontiguousarray(cand_xy, dtype=np.int32).reshape(-1, 2)
-        lead = ()
-        if views is not None:
+        lead = () if views is False else (None,)
+        if views is not False and views is not None:
             vw = np.ascontiguousarray(views, dtype=np.int32).reshape(-1, 5)
             if vw.shape[0] != xy.shape[0]:
                 raise ValueError(f"views must have one row per candidate ({xy.shape[0]}), got {vw.shape[0]}")
@@ -622,22 +691,26 @@ class Context:
         kinds = dict(pick=((n, max(k, 0)), np.int32),
                      gain=((n, max(k, 0)), np.uint32 if out_type is CoverOut else np.uint64),
                      npicked=((n,), np.int32), covered=((n, ny, (nx + 31) // 32), np.uint32),
-                     count=((n, ny, nx), np.uint8))
+                     count=((n, ny, nx), np.uint8), total=((n,), np.uint64))
         names = [name for name, _ in out_type._fields_]
         r = {name: np.empty(*kinds[name]) for name in names}
         co = out_type(*[_np_ptr(r[name]) for name in names])
         tail = () if m is None else (int(m),)
+        if quota is not None:
+            tail += (_np_ptr(quota),)
         self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), *lead, _np_ptr(gp), _np_ptr(gm), npb, k,
                        int(radius), int(shape), float(threshold), _np_ptr(extra), *tail, C.byref(co)))
         return r
 
     def _cover_dev(self, fn, out_type, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape, outs, group_map_t,
-                   extra_t, m=None, views_t=False):
+                   extra_t, m=None, views_t=False, quota_t=False):
         nmaps, ny, nx = occ_t.shape
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         co = out_type(*[ptr(t) for t in outs])
         lead = () if views_t is False else (ptr(views_t),)
         tail = () if m is None else (int(m),)
+        if quota_t is not False:
+            tail += (ptr(quota_t),)
         self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), *lead, group_ptr_t.data_ptr(),
                        ptr(group_map_t), group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius),
                        int(shape), float(threshold), ptr(extra_t), *tail, C.byref(co)))

@@ -1206,15 +1206,19 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
 // (vhp_visibility_cover_greedy_weighted_batch) runs the same phase 1 and the weighted rounds, the m-fold call
 // (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters, and the view call
 // (vhp_visibility_cover_greedy_view_batch) the m-fold call with each candidate's bits masked by its view in between.
+// The quota call (vhp_visibility_cover_quota_batch) is the view call, or the m-fold call without views, whose rounds
+// loop on the device until each problem's gains reach its quota.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
 const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
 const char *const kCoverMfoldName = "vhp_visibility_cover_greedy_mfold_batch";
 const char *const kCoverViewName = "vhp_visibility_cover_greedy_view_batch";
+const char *const kCoverQuotaName = "vhp_visibility_cover_quota_batch";
 // the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
 constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
 // A cover call and its arguments.  weighted: uint64 gains and uint8 weights; mfold (with weighted): cells count until
-// m picks cover them, `count` instead of `covered`; view (with mfold): range.views masks each candidate's bits.
+// m picks cover them, `count` instead of `covered`; view (with mfold): range.views masks each candidate's bits; quota
+// (with mfold, the quota call): a problem stops once the sum of its gains reaches its quota, k is kmax.
 // extra: the target ([prob][ny][ceil(nx/32)] uint32) or the weights ([prob][ny][nx] uint8), may be null.
 struct CoverCall {
   const char *name;
@@ -1223,6 +1227,7 @@ struct CoverCall {
   VhpMergeRange range;
   double thr;
   const void *extra;
+  const uint64_t *quota = nullptr; // [prob]
   CoverCall(const char *call, int32_t k_, int32_t radius, int32_t shape, double thr_, const void *extra_)
       : name(call), k(k_), range(radius, shape), thr(thr_), extra(extra_) {}
 };
@@ -1238,14 +1243,20 @@ const VhpCoverOut *cover_out(const vhp_cover_mfold_out *p, VhpCoverOut &o) {
   if (p) o = {p->pick, p->gain, p->npicked, nullptr, p->count};
   return p ? &o : nullptr;
 }
+const VhpCoverOut *cover_out(const vhp_cover_quota_out *p, VhpCoverOut &o) {
+  if (p) o = {p->pick, p->gain, p->npicked, nullptr, p->count, p->total};
+  return p ? &o : nullptr;
+}
 
-// The m-fold and view calls report these under the m-fold call's name, but for "views is NULL".  The weighted key's
+// The m-fold and view calls report these under the m-fold call's name, but for "views is NULL"; the quota call under
+// its own name, with "kmax" for k.  The weighted key's
 // limit on nsrc is checked before any candidate is read; the views' values by check_views_host, or by bit 3 of d_err
 // on the device.
 vhp_status check_cover_args(vhp_context *ctx, const CoverCall &c, const void *occ, int nmaps, int nx, int ny,
                             const void *xy, const void *group_ptr, int64_t nprob, int64_t nsrc,
                             const VhpCoverOut *out) {
-  const std::string what = c.mfold ? kCoverMfoldName : c.name;
+  const bool quota = c.name == kCoverQuotaName;
+  const std::string what = c.mfold && !quota ? kCoverMfoldName : c.name;
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
   if (nmaps < 1 || nx < 1 || ny < 1 || nprob < 0 || nsrc < 0) return fail(ctx, VHP_ERR_INVALID_ARG, "bad sizes");
@@ -1253,8 +1264,9 @@ vhp_status check_cover_args(vhp_context *ctx, const CoverCall &c, const void *oc
   vhp_status st = check_grid_dtype(ctx, nx, ny, VHP_F64);
   if (st != VHP_OK) return st;
   if (c.thr != c.thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
-  if (c.k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": k < 0");
-  if (!out->pick && !out->gain && !out->npicked && !out->covered && !out->count)
+  if (c.k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + (quota ? ": kmax < 0" : ": k < 0"));
+  if (quota && nprob > 0 && !c.quota) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": quota is NULL");
+  if (!out->pick && !out->gain && !out->npicked && !out->covered && !out->count && !out->total)
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
   if ((st = check_range(ctx, what, c.range)) != VHP_OK) return st;
   if (c.weighted && nsrc >= kCoverWeightedMaxSrc)
@@ -1303,7 +1315,8 @@ vhp_status run_cover_phase1(vhp_context *ctx, const CoverCall &c, const uint8_t 
       if ((st = ensure_cover(ctx, ctx->b_cover, (size_t)nsrc * b.H * b.W * 4, "candidate coverage bits", c.name)) !=
           VHP_OK)
         return st;
-      if ((st = ensure_cover(ctx, ctx->b_cover_ws, vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, c.weighted, c.mfold),
+      if ((st = ensure_cover(ctx, ctx->b_cover_ws,
+                             vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, c.weighted, c.mfold, c.quota != nullptr),
                              "workspace", c.name)) != VHP_OK)
         return st;
       uint32_t *bits = cb.bits = (uint32_t *)ctx->b_cover.p;
@@ -1349,8 +1362,8 @@ vhp_status run_cover_dev(vhp_context *ctx, const CoverCall &c, const uint8_t *d_
     cb.disk_r2 = -1;
   }
   VHP_CUDA(ctx, vhp_launch_cover_greedy(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk, c.weighted,
-                                        c.mfold, c.extra, c.k, c.m, ctx->b_cover_ws.p, out, ctx->sm_count, ctx->stream,
-                                        &ctx->launches));
+                                        c.mfold, c.extra, c.k, c.m, c.quota, ctx->b_cover_ws.p, out, ctx->sm_count,
+                                        ctx->stream, ctx->copy_stream, &ctx->launches));
   return VHP_OK;
 }
 
@@ -1365,7 +1378,7 @@ vhp_status cover_dev_entry(vhp_context *ctx, const CoverCall &c, const uint8_t *
 }
 
 // host buffers: runs of whole problems whose device memory (candidate bits, workspace, outputs) fits 4 GB, each with
-// its slice of c.extra uploaded.  c.range.views: the view call's [nsrc][5] on the host.
+// its slice of c.extra (and of c.quota) uploaded.  c.range.views: the view call's [nsrc][5] on the host.
 vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *occ, int nmaps, int nx, int ny,
                           const int32_t *xy, const int64_t *gptr, const int32_t *gmap, int64_t nprob,
                           const VhpCoverOut *out) {
@@ -1379,34 +1392,41 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
   const size_t bp = out->pick ? 4 * (size_t)c.k : 0, bg = out->gain ? gsz * (size_t)c.k : 0;
   const size_t bn = out->npicked ? 4 : 0, bc = out->covered ? plane * 4 : out->count ? (size_t)ny * nx : 0;
   const size_t bt = c.extra ? (c.weighted ? (size_t)ny * nx : plane * 4) : 0;
+  const size_t btot = out->total ? 8 : 0, bq = c.quota ? 8 : 0; // the quota call's total and quota
   // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
-  // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters; views: 20 bytes)
+  // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters; views: 20 bytes;
+  // the 64 bytes of per-problem scalars hold the quota rounds' total and quota copy too)
   const size_t per_src = box + 12 + gsz + (c.view ? 20 : 0), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
                                                                   (c.weighted ? plane * 32 : 0) +
-                                                                  (c.mfold ? plane * 32 : 0);
+                                                                  (c.mfold ? plane * 32 : 0) + btot + bq;
   void *const host_cells = out->covered ? (void *)out->covered : (void *)out->count;
   auto run = [&](int64_t q0, int64_t gc, const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap,
                  int64_t run_nsrc, const VhpMergeRange *run_range) {
     vhp_status r;
-    if ((r = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + bn + bc) + 256)) != VHP_OK) return r;
+    if ((r = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + btot + bq + bn + bc) + 256)) != VHP_OK) return r;
     if (c.extra && (r = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) return r;
     cudaError_t e = cudaSuccess;
     if (c.extra)
       e = cudaMemcpyAsync(ctx->b_out[1].p, (const char *)c.extra + (size_t)q0 * bt, (size_t)gc * bt,
                           cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) return cuda_fail(ctx, e, "cover: upload of the problems");
     char *base = (char *)ctx->b_out[0].p;
-    const size_t o_gain = (gc * bp + gsz - 1) & ~(gsz - 1); // uint64 gains: 8-byte aligned
-    char *cells = base + o_gain + gc * (bg + bn);
+    const size_t o_gain = (gc * bp + gsz - 1) & ~(gsz - 1); // uint64 gains, totals and quotas: 8-byte aligned
+    char *tot = base + o_gain + gc * bg, *quota = tot + gc * btot;
+    char *cells = quota + gc * (bq + bn);
+    if (e == cudaSuccess && c.quota)
+      e = cudaMemcpyAsync(quota, c.quota + q0, gc * bq, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "cover: upload of the problems");
     VhpCoverOut o;
     o.pick = out->pick ? (int32_t *)base : nullptr;
     o.gain = out->gain ? base + o_gain : nullptr;
-    o.npicked = out->npicked ? (int32_t *)(base + o_gain + gc * bg) : nullptr;
+    o.npicked = out->npicked ? (int32_t *)(quota + gc * bq) : nullptr;
     o.covered = out->covered ? (uint32_t *)cells : nullptr;
     o.count = out->count ? (uint8_t *)cells : nullptr;
+    o.total = out->total ? (uint64_t *)tot : nullptr;
     CoverCall rc = c;
     rc.range = *run_range;
     rc.extra = c.extra ? ctx->b_out[1].p : nullptr;
+    rc.quota = c.quota ? (const uint64_t *)quota : nullptr;
     r = run_cover_dev(ctx, rc, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy, d_gptr, d_gmap, gc, run_nsrc, o);
     if (r != VHP_OK) return r;
     if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * c.k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
@@ -1416,11 +1436,13 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
       e = cudaMemcpyAsync(out->npicked + q0, o.npicked, gc * bn, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && host_cells)
       e = cudaMemcpyAsync((char *)host_cells + q0 * bc, cells, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->total)
+      e = cudaMemcpyAsync(out->total + q0, o.total, gc * btot, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     return e == cudaSuccess ? VHP_OK : cuda_fail(ctx, e, "cover: copy of the outputs");
   };
   return run_groups_host(ctx, c.name, "candidate", occ, nmaps, nx, ny, xy, gptr, gmap, nprob, &c.range, per_src,
-                         per_prob, (size_t)4 << 30, bp + bg + bn + bc, "cover: upload of the problems", run);
+                         per_prob, (size_t)4 << 30, bp + bg + bn + bc + btot, "cover: upload of the problems", run);
 }
 
 // ---- opt-in sweep variants ------------------------------------------------------------------------
@@ -2097,6 +2119,38 @@ vhp_status vhp_visibility_cover_greedy_view_batch_dev(vhp_context *ctx, const ui
   c.weighted = c.mfold = c.view = true;
   c.m = m;
   c.range.views = d_views;
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
+}
+
+vhp_status vhp_visibility_cover_quota_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                            const int32_t *cand_xy, const int32_t *views, const int64_t *group_ptr,
+                                            const int32_t *group_map, int64_t nprob, int32_t kmax, int32_t radius,
+                                            int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                            const uint64_t *quota, const vhp_cover_quota_out *out) {
+  CoverCall c(kCoverQuotaName, kmax, radius, shape, threshold, weights);
+  c.weighted = c.mfold = true;
+  c.view = views != nullptr;
+  c.m = m;
+  c.range.views = views;
+  c.quota = quota;
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
+}
+
+vhp_status vhp_visibility_cover_quota_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                const int32_t *d_cand_xy, const int32_t *d_views,
+                                                const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t nprob,
+                                                int64_t nsrc, int32_t kmax, int32_t radius, int32_t shape,
+                                                double threshold, const uint8_t *d_weights, int32_t m,
+                                                const uint64_t *d_quota, const vhp_cover_quota_out *d_out) {
+  CoverCall c(kCoverQuotaName, kmax, radius, shape, threshold, d_weights);
+  c.weighted = c.mfold = true;
+  c.view = d_views != nullptr;
+  c.m = m;
+  c.range.views = d_views;
+  c.quota = d_quota;
   VhpCoverOut o;
   return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
                          cover_out(d_out, o));

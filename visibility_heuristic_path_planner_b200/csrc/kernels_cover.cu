@@ -22,6 +22,13 @@
 //
 // The view call (vhp_visibility_cover_greedy_view_batch) narrows every S(c) to its candidate's view once, in place,
 // with cover_view_kernel between phase 1 and the m-fold rounds; the rounds cannot tell masked bits from swept ones.
+//
+// The quota call (vhp_visibility_cover_quota_batch) runs the m-fold rounds (or the view call's) until each problem is
+// done: the apply step instantiated with kQ = true reads the round from device memory, adds each pick's gain to the
+// problem's total and marks the problem done once total >= quota (or at gain 0, or at kmax picks), decrementing a
+// counter of active problems.  The rounds are the body of a CUDA-graph WHILE node, apply, update and
+// cover_quota_step_kernel, which advances the round and keeps the loop going while a problem is active and
+// round < min(kmax, nsrc).
 #include <algorithm>
 #include <cstdint>
 #include <type_traits>
@@ -44,6 +51,12 @@ using GainT = typename std::conditional<kW, uint64_t, uint32_t>::type;
 
 struct CoverGeo {
   int nx, ny, R, nw; // R: the radius clamped for the geometry; nw = ceil(nx / 32)
+};
+
+// the quota call's loop state, in the workspace: total and quota [prob], the active problems and the round
+struct CoverQuotaState {
+  unsigned long long *total = nullptr, *quota = nullptr;
+  int *active = nullptr, *round = nullptr;
 };
 
 // bits lo .. hi of a word (any lo, hi; empty if lo > hi after clamping to [0, 31])
@@ -255,7 +268,9 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
 // problem's state over the pick's box.  kM (m-fold, with kW): cnt += 1 over S(p) saturating at mfold (cnt: the
 // counter plane, wpad's layout), new = the cells that reach mfold now and are not in state, state |= new, and the
 // pick's gain is zeroed (with mfold >= 2 it keeps gain on its own cells).  gain, cnt and mfold are unused otherwise.
-template <bool kW, bool kM>
+// kQ (quota, with kM): the round is *qs.round (r is unused), and a problem is done once its total reaches its quota or
+// r + 1 == k (kmax); every problem that becomes done decrements *qs.active once.  qs is unused otherwise.
+template <bool kW, bool kM, bool kQ = false>
 __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32_t *__restrict__ bits,
                                                                     const int64_t *__restrict__ first, int64_t nsrc,
                                                                     CoverGeo G,
@@ -264,10 +279,12 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
                                                                     int *done, uint32_t *__restrict__ state,
                                                                     uint32_t *__restrict__ newb,
                                                                     VhpCoverDevT<GainT<kW>> out, GainT<kW> *gain,
-                                                                    uint8_t *__restrict__ cnt, int mfold) {
+                                                                    uint8_t *__restrict__ cnt, int mfold,
+                                                                    CoverQuotaState qs) {
   const int64_t q = blockIdx.x;
   if (done[q]) return;
   const unsigned long long key = slot[q];
+  if constexpr (kQ) r = *qs.round;
   __syncthreads(); // every thread has read the slot before thread 0 resets it
   GainT<kW> gn;
   uint32_t idx;
@@ -280,7 +297,10 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
   }
   const int64_t c = first[q] + idx;
   if (gn == 0 || first[q] < 0 || c >= nsrc) { // (the last two: an inconsistent group layout, reported by the table)
-    if (threadIdx.x == 0) done[q] = 1;
+    if (threadIdx.x == 0) {
+      done[q] = 1;
+      if constexpr (kQ) atomicSub(qs.active, 1);
+    }
     return;
   }
   if (threadIdx.x == 0) {
@@ -290,6 +310,14 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
     cur[q] = c;
     slot[q] = 0;
     if constexpr (kM) gain[c] = 0;
+    if constexpr (kQ) {
+      const unsigned long long t = qs.total[q] + gn;
+      qs.total[q] = t;
+      if (t >= qs.quota[q] || r + 1 >= k) {
+        done[q] = 1;
+        atomicSub(qs.active, 1);
+      }
+    }
   }
   const VhpCoverBox b = vhp_cover_box(G.nx, G.ny, G.R, __ldg(xy + 2 * c), __ldg(xy + 2 * c + 1));
   const int hw = b.H * b.W;
@@ -360,6 +388,34 @@ __global__ void cover_count_kernel(const uint8_t *__restrict__ cnt, size_t nrows
         if (x + b < nx) dst[b] = (uint8_t)(w[b >> 2] >> (8 * (b & 3)));
     }
   }
+}
+
+// The quota call, before init: copy the quotas, zero the totals, and start the problems of quota 0 done; *active =
+// the others, *round = 0 (both zeroed before).  The loop is uniform over the warp, so every lane takes part in the ballot.
+__global__ void cover_quota_init_kernel(const unsigned long long *__restrict__ quota, int64_t nprob, int *done,
+                                        CoverQuotaState qs) {
+  const int lane = threadIdx.x & 31;
+  const int64_t step = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x - lane; i0 < nprob; i0 += step) {
+    const int64_t q = i0 + lane;
+    unsigned long long v = 0;
+    if (q < nprob) {
+      v = __ldg(quota + q);
+      qs.quota[q] = v;
+      qs.total[q] = 0;
+      done[q] = v == 0;
+    }
+    const unsigned a = __ballot_sync(kAll, v != 0);
+    if (lane == 0 && a) atomicAdd(qs.active, __popc(a));
+  }
+}
+
+// The quota call's loop control, the last node of the WHILE body: round += 1, and loop again while a problem is
+// active and round < rounds = min(kmax, nsrc).
+__global__ void cover_quota_step_kernel(CoverQuotaState qs, int32_t rounds, cudaGraphConditionalHandle loop) {
+  const int r = *qs.round + 1;
+  *qs.round = r;
+  cudaGraphSetConditional(loop, (*qs.active > 0 && r < rounds) ? 1u : 0u);
 }
 
 // floor and ceiling of n / d, d != 0 (C division truncates toward zero)
@@ -536,7 +592,8 @@ unsigned grid_for(size_t n, int bs, int sm_count) {
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 // workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src] (uint32, weighted uint64), slot [prob],
-// cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]; m-fold (weighted too): cnt, wpad's layout
+// cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]; m-fold (weighted too): cnt, wpad's layout;
+// quota (m-fold too): total [prob], quota [prob], active, round
 struct CoverWs {
   uint32_t *state, *newb;
   void *gain;
@@ -544,18 +601,22 @@ struct CoverWs {
   int64_t *cur, *first;
   int *done;
   uint8_t *wpad, *cnt;
+  CoverQuotaState qs;
   size_t bytes;
 };
-CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold) {
+CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold,
+                 bool quota = false) {
   const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
   const size_t np = (size_t)nprob, plane = (size_t)ny * ((nx + 31) / 32);
   const size_t o_new = align256(np * plane * 4), o_gain = o_new + align256(np * b.H * b.W * 4);
   const size_t o_slot = o_gain + align256((size_t)nsrc * (weighted ? 8 : 4)), o_cur = o_slot + align256(np * 8);
   const size_t o_first = o_cur + align256(np * 8), o_done = o_first + align256(np * 8);
   const size_t o_wpad = o_done + align256(np * 4), o_cnt = o_wpad + (weighted ? align256(np * plane * 32) : 0);
+  const size_t o_total = o_cnt + (mfold ? align256(np * plane * 32) : 0), o_quota = o_total + align256(np * 8);
+  const size_t o_ctl = o_quota + align256(np * 8);
   char *p = static_cast<char *>(base);
   CoverWs w{};
-  w.bytes = o_cnt + (mfold ? align256(np * plane * 32) : 0);
+  w.bytes = quota ? o_ctl + 256 : o_total;
   if (!p) return w;
   w.state = (uint32_t *)p;
   w.newb = (uint32_t *)(p + o_new);
@@ -566,17 +627,61 @@ CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R,
   w.done = (int *)(p + o_done);
   w.wpad = weighted ? (uint8_t *)(p + o_wpad) : nullptr;
   w.cnt = mfold ? (uint8_t *)(p + o_cnt) : nullptr;
+  if (quota) {
+    w.qs.total = (unsigned long long *)(p + o_total);
+    w.qs.quota = (unsigned long long *)(p + o_quota);
+    w.qs.active = (int *)(p + o_ctl);
+    w.qs.round = w.qs.active + 1;
+  }
   return w;
 }
 
-// the rounds of the three calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null:
-// all 1), kM (with kW) counts each cell until mfold picks cover it and writes d_count (may be null) at the end
-template <bool kW, bool kM = false>
+// The quota call's rounds: a graph of one WHILE node whose body, captured on `cap`, is apply, update and the step
+// kernel; the step kernel's condition ends the loop.  The graph is built, launched on st and destroyed here: it holds
+// this call's workspace pointers, so it is never reused (an exec destroyed while in flight is freed on completion).
+template <class Apply, class Update>
+cudaError_t launch_quota_loop(CoverQuotaState qs, int32_t rounds, cudaStream_t st, cudaStream_t cap, Apply apply,
+                              Update update) {
+  cudaGraph_t graph = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  cudaError_t e = cudaGraphCreate(&graph, 0);
+  cudaGraphConditionalHandle handle = 0;
+  if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&handle, graph, 1, cudaGraphCondAssignDefault);
+  cudaGraphNodeParams np = {};
+  np.type = cudaGraphNodeTypeConditional;
+  np.conditional.handle = handle;
+  np.conditional.type = cudaGraphCondTypeWhile;
+  np.conditional.size = 1;
+  cudaGraphNode_t node;
+  if (e == cudaSuccess) e = cudaGraphAddNode(&node, graph, nullptr, 0, &np);
+  if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(cap, np.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                                          cudaStreamCaptureModeRelaxed);
+  if (e == cudaSuccess) {
+    apply(cap);
+    update(cap);
+    cover_quota_step_kernel<<<1, 1, 0, cap>>>(qs, rounds, handle);
+    const cudaError_t el = cudaGetLastError();
+    cudaGraph_t captured = nullptr;
+    e = cudaStreamEndCapture(cap, &captured);
+    if (e == cudaSuccess) e = el;
+  }
+  if (e == cudaSuccess) e = cudaGraphInstantiate(&exec, graph, 0);
+  if (e == cudaSuccess) e = cudaGraphLaunch(exec, st);
+  if (exec) cudaGraphExecDestroy(exec);
+  if (graph) cudaGraphDestroy(graph);
+  return e;
+}
+
+// the rounds of the four calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null:
+// all 1), kM (with kW) counts each cell until mfold picks cover it and writes d_count (may be null) at the end, kQ
+// (with kM) loops until each problem's total reaches d_quota (the graph of launch_quota_loop) and writes d_total
+template <bool kW, bool kM = false, bool kQ = false>
 cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                           const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
                           const uint32_t *d_target, const uint8_t *d_weights, int32_t k, int mfold, void *d_ws,
                           const VhpCoverDevT<GainT<kW>> &out, uint8_t *d_count, int sm_count, cudaStream_t st,
-                          int64_t *launches) {
+                          int64_t *launches, const uint64_t *d_quota = nullptr, uint64_t *d_total = nullptr,
+                          cudaStream_t cap = nullptr) {
   const CoverGeo G{nx, ny, R, (nx + 31) / 32};
   const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
   cudaError_t e = cudaSuccess;
@@ -586,8 +691,9 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   if (e == cudaSuccess && out.covered) e = cudaMemsetAsync(out.covered, 0, np * plane * 4, st);
   const int64_t rounds = std::min<int64_t>(k, nsrc);
   if (e == cudaSuccess && d_count && rounds <= 0) e = cudaMemsetAsync(d_count, 0, np * ny * nx, st); // no pick
+  if (e == cudaSuccess && d_total && rounds <= 0) e = cudaMemsetAsync(d_total, 0, np * 8, st);
   if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
-  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW, kM);
+  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW, kM, kQ);
   GainT<kW> *gain = (GainT<kW> *)ws.gain;
   if (kW) {
     cover_weight_kernel<<<grid_for(np * plane * 8, 256, sm_count), 256, 0, st>>>(d_weights, nprob, G, ws.wpad,
@@ -604,18 +710,39 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0xff, np * 8, st);
   if (e == cudaSuccess && kM) e = cudaMemsetAsync(ws.cnt, 0, np * plane * 32, st);
   if (e != cudaSuccess) return e;
+  if constexpr (kQ) {
+    if ((e = cudaMemsetAsync(ws.qs.active, 0, 8, st)) != cudaSuccess) return e; // active and round
+    cover_quota_init_kernel<<<grid_for(np, 256, sm_count), 256, 0, st>>>(
+        reinterpret_cast<const unsigned long long *>(d_quota), nprob, ws.done, ws.qs);
+    if (launches) *launches += 1;
+  }
   const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
   cover_init_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
                                                       gain, ws.slot, ws.first, ws.wpad);
-  for (int32_t r = 0; r < rounds; ++r) {
-    cover_apply_kernel<kW, kM><<<(unsigned)nprob, kApplyThreads, 0, st>>>(d_bits, ws.first, nsrc, G, d_xy, r, k,
-                                                                          ws.slot, ws.cur, ws.done, ws.state, ws.newb,
-                                                                          out, gain, ws.cnt, mfold);
-    if (r + 1 < rounds)
-      cover_update_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
-                                                            ws.done, ws.newb, gain, ws.slot, ws.wpad);
+  auto apply = [&](int32_t r, cudaStream_t s) {
+    cover_apply_kernel<kW, kM, kQ><<<(unsigned)nprob, kApplyThreads, 0, s>>>(d_bits, ws.first, nsrc, G, d_xy, r, k,
+                                                                             ws.slot, ws.cur, ws.done, ws.state,
+                                                                             ws.newb, out, gain, ws.cnt, mfold, ws.qs);
+  };
+  auto update = [&](cudaStream_t s) {
+    cover_update_kernel<kW><<<cgrid, kWarps * 32, 0, s>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
+                                                         ws.done, ws.newb, gain, ws.slot, ws.wpad);
+  };
+  if constexpr (kQ) {
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = launch_quota_loop(ws.qs, (int32_t)rounds, st, cap, [&](cudaStream_t s) { apply(0, s); }, update)) !=
+        cudaSuccess)
+      return e;
+    if (launches) *launches += 2; // init and the graph
+    if (d_total && (e = cudaMemcpyAsync(d_total, ws.qs.total, np * 8, cudaMemcpyDeviceToDevice, st)) != cudaSuccess)
+      return e;
+  } else {
+    for (int32_t r = 0; r < rounds; ++r) {
+      apply(r, st);
+      if (r + 1 < rounds) update(st);
+    }
+    if (launches) *launches += 2 * rounds;
   }
-  if (launches) *launches += 2 * rounds;
   if (kM && d_count) {
     const size_t nrows = np * ny;
     cover_count_kernel<<<grid_for(nrows * ((nx + 15) / 16), 256, sm_count), 256, 0, st>>>(ws.cnt, nrows, nx, G.nw,
@@ -651,14 +778,15 @@ cudaError_t vhp_launch_cover_view(uint32_t *d_bits, int64_t nsrc, int nx, int ny
   return cudaGetLastError();
 }
 
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold) {
-  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold, mfold).bytes;
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold, bool quota) {
+  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold || quota, mfold || quota, quota).bytes;
 }
 
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                                     const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
-                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m, void *d_ws,
-                                    const VhpCoverOut &out, int sm_count, cudaStream_t st, int64_t *launches) {
+                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m,
+                                    const uint64_t *d_quota, void *d_ws, const VhpCoverOut &out, int sm_count,
+                                    cudaStream_t st, cudaStream_t cap, int64_t *launches) {
   if (!weighted) {
     const VhpCoverDevT<uint32_t> o{out.pick, (uint32_t *)out.gain, out.npicked, out.covered};
     return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k,
@@ -666,6 +794,10 @@ cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t npro
   }
   const VhpCoverDevT<uint64_t> o{out.pick, (uint64_t *)out.gain, out.npicked, out.covered};
   const uint8_t *d_weights = (const uint8_t *)d_extra;
+  if (d_quota)
+    return launch_rounds<true, true, true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k,
+                                           nullptr, d_weights, k, m, d_ws, o, out.count, sm_count, st, launches,
+                                           d_quota, out.total, cap);
   if (!mfold)
     return launch_rounds<true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k, nullptr,
                                d_weights, k, 1, d_ws, o, nullptr, sm_count, st, launches);

@@ -309,13 +309,14 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
                                   cudaStream_t st, int64_t *launches);
 // Phase 2, the greedy rounds over the bits of nsrc candidates (table of vhp_launch_merge_table) of nprob problems.
 // The outputs of every cover call (any may be null): gain is uint32 (cells) for the cover call, uint64 (summed
-// weights) for the weighted ones; the m-fold rounds write count instead of covered.
+// weights) for the weighted ones; the m-fold rounds write count instead of covered, the quota rounds also total.
 struct VhpCoverOut {
   int32_t *pick = nullptr;     // [prob][k]
   void *gain = nullptr;        // [prob][k]
   int32_t *npicked = nullptr;  // [prob]
   uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
   uint8_t *count = nullptr;    // [prob][ny][nx], min(m, picks whose S covers the cell)
+  uint64_t *total = nullptr;   // [prob], the sum of the gains (quota rounds)
 };
 // cover_apply_kernel's parameter (kernels_cover.cu): the outputs but count, with the gain typed
 template <class Gain>
@@ -326,16 +327,22 @@ struct VhpCoverDevT {
   uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
 };
 // workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane; m-fold:
-// those of the weighted rounds and a counter plane of the padded plane's size)
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold = false);
+// those of the weighted rounds and a counter plane of the padded plane's size; quota: those of the m-fold rounds, a
+// total and a quota copy per problem, and the active and round counters)
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold = false,
+                          bool quota = false);
 // outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
 // route's sweep stores the whole box).  d_extra (may be null): [prob][ny][ceil(nx/32)] uint32 bits of the cells to
 // cover, or for the weighted rounds [prob][ny][nx] uint8 weights (null: every cell weighs 1; nsrc < 2^28).  The
 // m-fold rounds (with weighted) are the weighted rounds where a cell's weight counts until m in [1, 255] picks cover it.
+// d_quota (non-null: the quota rounds, weighted and m-fold; k = kmax): [prob] uint64, problem q stops once the sum of
+// its gains reaches d_quota[q]; the rounds then loop in a CUDA graph captured on `cap` and launched on st, and write
+// out.total.  Otherwise the rounds are min(k, nsrc) fixed launches on st and cap is unused.
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                                     const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
-                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m, void *d_ws,
-                                    const VhpCoverOut &out, int sm_count, cudaStream_t st, int64_t *launches);
+                                    bool weighted, bool mfold, const void *d_extra, int32_t k, int m,
+                                    const uint64_t *d_quota, void *d_ws, const VhpCoverOut &out, int sm_count,
+                                    cudaStream_t st, cudaStream_t cap, int64_t *launches);
 // the view call, between phase 1 and the m-fold rounds (which then run with disk_r2 = -1): every candidate's bits
 // &= its view, d_views [nsrc][5] = (r, ax, ay, bx, by): range r in [0, radius] in the call's shape (disk or box), and
 // the sector of a and b.  A bad view raises bit 3 of d_err and clears the candidate's bits.
