@@ -23,6 +23,9 @@ vhp_status fail(vhp_context *ctx, vhp_status st, const std::string &msg) {
 }
 
 vhp_status cuda_fail(vhp_context *ctx, cudaError_t e, const char *what) {
+  // a refused call (e.g. cudaFuncSetAttribute) stays the thread's last error, which the next call's check after a good
+  // launch would report as its own: clear it once it is reported here
+  (void)cudaGetLastError();
   return fail(ctx, VHP_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
 

@@ -78,11 +78,17 @@ struct PlannerParams {
 // batches of 256 x 256 maps -- the epilogue pass wants the threads -- and stay selectable with
 // VHP_PLANNER_WARPS for experiments.  Also measured and dropped: 6 warps x 3 CTAs per SM and 10
 // warps x 2 (both 96 registers: 182k / 180k), 12 warps x 1 (140 registers: 244k, no better).
+// The kernel's static shared memory (s_ctl, s_best; 16-byte aligned each) comes out of the same 227 KB opt-in limit as
+// the dynamic tile state, so the planner's largest map is a little narrower than the tile kernel's
+// (vhp_planner_supported).
+constexpr int kPlannerCtl = 5, kPlannerBest = 32;
+constexpr size_t kPlannerStaticSmem = ((kPlannerCtl * sizeof(int) + 15) & ~(size_t)15) + kPlannerBest * sizeof(Best);
+
 template <int NWK, int MINB = 1>
 __global__ void __launch_bounds__(NWK * 32, MINB) planner_kernel(const PlannerParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  __shared__ int s_ctl[5];              // {done, next x, next y, status, nb_of_sources}
-  __shared__ Best s_best[32];
+  __shared__ int s_ctl[kPlannerCtl];    // {done, next x, next y, status, nb_of_sources}
+  __shared__ Best s_best[kPlannerBest];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, NW = blockDim.x >> 5;
   const int64_t q = blockIdx.x;
   const int nx = p.fp.nx, ny = p.fp.ny;
@@ -474,7 +480,9 @@ cudaError_t vhp_launch_strip_epilogue(int nx, int ny, int y0, int y1, int sx, in
   return cudaGetLastError();
 }
 
-bool vhp_planner_supported(int nx, int ny) { return vhp_sweep_tile_supported(nx, ny); }
+bool vhp_planner_supported(int nx, int ny) {
+  return vhp_sweep_tile_supported(nx, ny) && tile_smem_bytes<double>(nx, ny) + kPlannerStaticSmem <= 227u * 1024u;
+}
 
 size_t vhp_planner_first_ws_bytes(int64_t nprob) {
   return (((size_t)nprob * 8 + 255) & ~(size_t)255) + (((size_t)nprob * 20 + 255) & ~(size_t)255) +
@@ -489,7 +497,7 @@ cudaError_t vhp_launch_planner(const VhpTilePlanes &pl, int nx, int ny, const in
                                int32_t *d_nb, int32_t *d_ls, double *d_path_len, int32_t *d_path_n,
                                int32_t *d_path, float *d_vg32, float *d_vis32, int *d_err,
                                cudaStream_t st, int64_t *launches, void *d_first_ws, int first_rounds) {
-  if (!vhp_sweep_tile_supported(nx, ny)) return cudaErrorInvalidConfiguration;
+  if (!vhp_planner_supported(nx, ny)) return cudaErrorInvalidConfiguration;
   // large batches: every problem's first sweep and epilogue batch-wide (see planner_first_* above)
   const int *resume = nullptr;
   if (d_first_ws) {
