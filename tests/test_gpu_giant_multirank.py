@@ -19,13 +19,13 @@ def _gpus():
     return torch.cuda.device_count()
 
 
-def _run(nproc, size, queries, spr=1, port=29541, p2p=True):
+def _run(nproc, size, queries, spr=1, port=29541, p2p=True, map_kind="random"):
     env = dict(os.environ)
     env["VHP_GIANT_P2P"] = "1" if p2p else "0"
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={nproc}",
            "--master-addr", "127.0.0.1", "--master-port", str(port),
            os.path.join(ROOT, "tools", "giant_multi_gpu.py"), "--size", str(size), "--queries", str(queries),
-           "--spr", str(spr), "--max-iter", "40"]
+           "--spr", str(spr), "--max-iter", "40", "--map", map_kind]
     p = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=env)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-4000:]
     line = [l for l in p.stdout.splitlines() if l.startswith("{")][-1]
@@ -45,6 +45,16 @@ def test_two_ranks_equal_single_gpu():
     assert all(q["peer_handover"] == 0 and q["halo_bytes_sent"] > 0 for q in r["queries"] if q["iterations"] > 0)
     r = _run(2, 1024, 2, spr=3, port=29542)   # remote and local strip boundaries mixed (NCCL hand-over)
     assert r["all_ranks_equal"]
+
+
+def test_two_ranks_ties_across_the_rank_boundary():
+    """A map mirrored about both axes, the middle row rank 0's last: cells mirrored about the start's row tie on
+    h and lie on different ranks, so the all-gathered minimum has to keep the first pushed (peer memory and NCCL)"""
+    if _gpus() < 2:
+        pytest.skip("needs >= 2 GPUs")
+    for port, p2p in ((29546, True), (29547, False)):
+        r = _run(2, 1024, 4, port=port, p2p=p2p, map_kind="mirrored")
+        assert r["n"] == 1025 and r["all_ranks_equal"] and all(q["equal_single_gpu"] for q in r["queries"])
 
 
 def test_all_gpus_equal_single_gpu():

@@ -26,6 +26,7 @@ from test_gpu_merge import expected as merge_expected
 from test_gpu_merge import make_groups
 from test_gpu_merge_range import expected as merge_range_expected
 from test_gpu_planner import check as planner_check
+from test_planner_ties_cpu import LINE_ITER, LINE_THR, SYM_ITER, SYM_THR, line_cases, symmetric_cases
 from test_window_cpu import window_of
 
 pytestmark = pytest.mark.gpu
@@ -231,7 +232,8 @@ def format_case(oracle):
 @pytest.fixture(scope="module")
 def planner_cases(oracle):
     """(occ, start_end, prob_map or None, threshold, max_iter, oracle results): the planner.npz goldens, the random
-    problems of test_random_problems_vs_oracle"""
+    problems of test_random_problems_vs_oracle, and the small tie cases of test_gpu_planner_ties (maps with exact
+    ties on h, where only the push-order half of the arg-min decides)"""
     cases = []
     g = load_golden("planner.npz")
     maps = np.stack([oracle.generate_environment(101, 101, 10, 10, 20, 10, 20, s) for s in range(1, 7)])
@@ -248,6 +250,11 @@ def planner_cases(oracle):
                        rng.integers(0, ny, 8)], axis=1).astype(np.int32)
         thr = float(rng.choice([0.0, 0.2, 0.5, 0.9, 1.0]))
         cases.append((occ, se, None, thr, 12, [planner_ref(oracle, occ, s, thr, 12) for s in se]))
+    for ties, thr, mi in ((symmetric_cases(), SYM_THR, SYM_ITER), (line_cases(), LINE_THR, LINE_ITER)):
+        maps = np.stack([occ for _, occ, _, _ in ties])
+        se = np.array([start + end for _, _, start, end in ties], np.int32)
+        cases.append((maps, se, np.arange(len(ties), dtype=np.int32), thr, mi,
+                      [planner_ref(oracle, maps[k], se[k], thr, mi) for k in range(len(ties))]))
     return cases
 
 

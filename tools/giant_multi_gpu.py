@@ -6,6 +6,9 @@ checks its rows against the single-GPU planner it runs itself, rank 0 prints tim
         --master-port 29533 tools/giant_multi_gpu.py [--size 2048] [--queries 3] [--spr 1]
 
 BASELINE configs[4] shape: --size 8192 (dense random obstacles, multi-source planner).
+--map mirrored: the same obstacles on one quarter, mirrored about the middle row and the middle column (an odd
+side), every query from the centre to a point on one of the two axes: cells mirrored about the start tie on h, so
+the first pushed of them has to win across ranks.  On two ranks of one strip each the middle row is rank 0's last.
 torch.distributed (gloo) only carries the 128-byte NCCL id and the verdicts."""
 import argparse
 import json
@@ -29,6 +32,24 @@ def giant_map(n, seed=8192):
     return occ, g
 
 
+def mirrored_map(n, queries):
+    """(occ, queries): giant_map's obstacles on a quarter, mirrored about both axes of a (2m+1)^2 map, m = n // 2;
+    start at the centre, ends on the axes"""
+    m = n // 2
+    q, g = giant_map(m + 1)
+    occ = np.concatenate([q, q[:, -2::-1]], axis=1)
+    occ = np.concatenate([occ, occ[-2::-1]], axis=0)
+    out = []
+    for k in range(queries):
+        d = int(g.integers(m // 4, m))
+        end = ((m, m + d), (m + d, m), (m, m - d), (m - d, m))[k % 4]
+        out.append(((m, m), end))
+        for x, y in ((m, m), end):
+            occ[y, x] = occ[y, 2 * m - x] = occ[2 * m - y, x] = occ[2 * m - y, 2 * m - x] = 1
+    assert np.array_equal(occ, occ[::-1]) and np.array_equal(occ, occ[:, ::-1])
+    return occ, out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--size", type=int, default=2048)
@@ -38,6 +59,7 @@ def main():
     ap.add_argument("--spr", type=int, default=1, help="strips per rank")
     ap.add_argument("--batch", type=int, default=0, help="iterations per snapshot (0: default)")
     ap.add_argument("--no-check", action="store_true")
+    ap.add_argument("--map", choices=("random", "mirrored"), default="random")
     args = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -48,11 +70,14 @@ def main():
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("gloo")
-    n = args.size
-    occ, g = giant_map(n)
-    free = np.argwhere(occ != 0)
-    picks = free[g.integers(0, len(free), 2 * args.queries)]
-    queries = [((int(a[1]), int(a[0])), (int(b[1]), int(b[0]))) for a, b in zip(picks[::2], picks[1::2])]
+    if args.map == "mirrored":
+        occ, queries = mirrored_map(args.size, args.queries)
+    else:
+        occ, g = giant_map(args.size)
+        free = np.argwhere(occ != 0)
+        picks = free[g.integers(0, len(free), 2 * args.queries)]
+        queries = [((int(a[1]), int(a[0])), (int(b[1]), int(b[0]))) for a, b in zip(picks[::2], picks[1::2])]
+    n = occ.shape[0]
     if world > 1:
         gp = GiantPlanner.from_torch_dist(occ, local, dist, strips_per_rank=args.spr)
     else:
