@@ -451,6 +451,68 @@ vhp_status vhp_visibility_cover_quota_batch_dev(vhp_context *ctx, const uint8_t 
                                                 double threshold, const uint8_t *d_weights, int32_t m,
                                                 const uint64_t *d_quota, const vhp_cover_quota_out *d_out);
 
+/* Budgeted sensor placement: what to buy and where it goes when candidates cost different amounts ("10 000 EUR,
+ * cameras cost 300, lidars 1 800"), greedy by coverage per unit cost.  The inputs are those of
+ * vhp_visibility_cover_quota_batch (problems, candidates, views (NULL: omnidirectional with r = R), group_map, radius
+ * R, shape, threshold, weights, m, kmax, the 2^28 limit), except that quota may be NULL (no quota), and two are new:
+ * cost ([nsrc] uint32, each in [1, 2^32 - 1], the cost of choosing the candidate in any unit) and budget ([prob]
+ * uint64, UINT64_MAX: no budget).  With f(A) = sum over x of W_q(x) * min(cnt_A(x), m) and gain(c) what c adds to f,
+ * problem q starts with spent = 0 and repeats
+ *   eligible(c) = c not picked, gain(c) > 0, cost(c) <= budget[q] - spent;
+ *   stop when no candidate is eligible, kmax picks are made, or (quota given) total >= quota[q];
+ *   otherwise pick p = argmax over eligible c of gain(c) / cost(c) (an exact rational comparison, ties to the smallest
+ *   index in the group), spent += cost(p), total += gain(p), and count the pick as the m-fold call does.
+ * This is the cost-effective greedy of Khuller, Moss and Naor.  A candidate that stops fitting never fits again, so
+ * the rule equals "consider by ratio, skip what does not fit".  The call also returns the best affordable singleton:
+ * single[q] = argmax over c with cost(c) <= budget[q] of f({c}) (ties to the smallest index; -1 when no such c has a
+ * positive gain) and single_gain[q] = f({single}).  max(total, single_gain) >= (1 - 1/e) / 2 * OPT for the monotone
+ * submodular f (Khuller et al. prove 1 - 1/sqrt(e) for m = 1); the call returns both and does not choose.  All costs
+ * 1 and budget B with quota NULL is exactly the view call (views given) or the m-fold call (views NULL) with
+ * k = min(B, kmax); all costs 1 and budget UINT64_MAX is exactly the quota call.  The ratio is compared through the
+ * 128-bit key (floor(gain * 2^64 / cost) << 28) | (2^28 - 1 - index), which orders exactly by ratio and then by
+ * index for gains < 2^36 and costs < 2^32, so the result is exact and order-independent.  Outputs (any may be NULL,
+ * at least one must be given):
+ *   pick[q][r]     index within the group of the r-th pick, -1 from npicked on             (int32 [prob][kmax])
+ *   gain[q][r]     what the r-th pick adds to f, 0 from npicked on; not monotone in general (uint64 [prob][kmax])
+ *   npicked[q]                                                                             (int32 [prob])
+ *   count[q]       min(m, number of picks whose S covers the cell)                         (uint8 [prob][ny][nx])
+ *   total[q]       f(picks) = sum of gain                                                  (uint64 [prob])
+ *   spent[q]       sum of the picks' costs, <= budget[q]                                   (uint64 [prob])
+ *   single[q]      the best affordable singleton, -1: none                                 (int32 [prob])
+ *   single_gain[q] its gain, 0: none                                                       (uint64 [prob])
+ * Routes, phase 1, the view mask and the device loop (a CUDA-graph WHILE node per call) are those of the quota call;
+ * the launch count is that call's plus one and does not depend on costs, budgets, quotas or the rounds run, and the
+ * _dev form does not synchronise.  Workspace: that of the quota call plus 32 bytes per problem (a 16-byte slot, the
+ * remaining budget and the spent cost); the host form's 4 GB batches also count 4 cost bytes per candidate and each
+ * problem's budget and the outputs above.  Errors (VHP_ERR_INVALID_ARG): those of vhp_visibility_cover_quota_batch
+ * except that quota may be NULL, cost NULL with nsrc > 0, budget NULL with nprob > 0, a zero cost.  The host form
+ * checks them all before any candidate is read; the _dev form reports a bad view as the view call does, and a zero
+ * cost by the next synchronising call (that candidate is never picked nor the singleton).  kmax == 0 is valid
+ * (npicked 0, count, total and spent zero, single -1). */
+typedef struct vhp_cover_budget_out {
+  int32_t *pick;         /* [prob][kmax], -1 from npicked on */
+  uint64_t *gain;        /* [prob][kmax], 0 from npicked on */
+  int32_t *npicked;      /* [prob] */
+  uint8_t *count;        /* [prob][ny][nx], min(m, picks covering the cell) */
+  uint64_t *total;       /* [prob], f(picks) = sum of gain */
+  uint64_t *spent;       /* [prob], sum of the picks' costs */
+  int32_t *single;       /* [prob], the best affordable singleton, -1: none */
+  uint64_t *single_gain; /* [prob], its gain */
+} vhp_cover_budget_out;
+vhp_status vhp_visibility_cover_budget_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                             const int32_t *cand_xy, const int32_t *views, const int64_t *group_ptr,
+                                             const int32_t *group_map, int64_t nprob, int32_t kmax, int32_t radius,
+                                             int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                             const uint64_t *quota, const uint32_t *cost, const uint64_t *budget,
+                                             const vhp_cover_budget_out *out);
+vhp_status vhp_visibility_cover_budget_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                 const int32_t *d_cand_xy, const int32_t *d_views,
+                                                 const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t nprob,
+                                                 int64_t nsrc, int32_t kmax, int32_t radius, int32_t shape,
+                                                 double threshold, const uint8_t *d_weights, int32_t m,
+                                                 const uint64_t *d_quota, const uint32_t *d_cost,
+                                                 const uint64_t *d_budget, const vhp_cover_budget_out *d_out);
+
 /* Directional merged visibility: what a set of cameras with headings and fields of view covers together, the
  * evaluation counterpart of vhp_visibility_cover_greedy_view_batch.  Everything is vhp_visibility_merge_range_batch
  * (inputs, groups, group_map, radius R, shape, threshold, dtype, the outputs and the "writes" rule), with source k's

@@ -73,6 +73,14 @@ class CoverQuotaOut(C.Structure):
                 ("total", C.c_void_p)]
 
 
+class CoverBudgetOut(C.Structure):
+    """struct vhp_cover_budget_out: pick (int32 [prob][kmax]), gain (uint64 [prob][kmax]), npicked (int32 [prob]),
+    count (uint8 [prob][ny][nx]), total, spent (uint64 [prob]), single (int32 [prob]), single_gain (uint64 [prob]),
+    each may be NULL."""
+    _fields_ = [("pick", C.c_void_p), ("gain", C.c_void_p), ("npicked", C.c_void_p), ("count", C.c_void_p),
+                ("total", C.c_void_p), ("spent", C.c_void_p), ("single", C.c_void_p), ("single_gain", C.c_void_p)]
+
+
 class SweepVariant(C.Structure):
     """struct vhp_sweep_variant: model 1 = getAccessibilityMap.m (alpha, fac, light_strength),
     model 2 = computeVisibilityUsingQueue as an order-free rule (cutoff)."""
@@ -177,6 +185,12 @@ def load_library(build_if_missing: bool = True):
     lib.vhp_visibility_cover_quota_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64, C.c_int32,
                                                          C.c_int32, C.c_int32, C.c_double, vp, C.c_int32, vp,
                                                          C.POINTER(CoverQuotaOut)]
+    lib.vhp_visibility_cover_budget_batch.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, C.c_int32,
+                                                      C.c_int32, C.c_int32, C.c_double, vp, C.c_int32, vp, vp, vp,
+                                                      C.POINTER(CoverBudgetOut)]
+    lib.vhp_visibility_cover_budget_batch_dev.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp, i64, i64, C.c_int32,
+                                                          C.c_int32, C.c_int32, C.c_double, vp, C.c_int32, vp, vp, vp,
+                                                          C.POINTER(CoverBudgetOut)]
     for name in ("vhp_visibility_window_batch", "vhp_visibility_window_batch_dev"):
         getattr(lib, name).argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, C.c_int32, i32, vp]
     lib.vhp_visibility_batch_packed.argtypes = [vp, vp, i32, i32, i32, vp, vp, i64, i32, C.POINTER(vp)]
@@ -251,12 +265,37 @@ def _cover_quota(quota, fraction, m, weights, n, shape):
         return np.ceil(p * float(int(m)) * w.astype(np.float64)).astype(np.uint64)
     if quota is None:
         return np.full(n, np.iinfo(np.uint64).max, np.uint64)
-    q = quota if isinstance(quota, np.ndarray) else np.array(quota, dtype=object)  # Python ints up to UINT64_MAX
-    if q.dtype.kind == "O" and not all(isinstance(v, (int, np.integer)) for v in q.ravel()):
-        raise ValueError("quota must be non-negative integers")
+    return _cover_u64(quota, n, "quota")
+
+
+def _cover_u64(v, n, what):
+    """non-negative integers (a scalar or one per problem) as contiguous uint64 (n,)"""
+    q = v if isinstance(v, np.ndarray) else np.array(v, dtype=object)  # Python ints up to UINT64_MAX
+    if q.dtype.kind == "O" and not all(isinstance(x, (int, np.integer)) for x in q.ravel()):
+        raise ValueError(f"{what} must be non-negative integers")
     if q.dtype.kind not in "iuO" or (q.dtype.kind != "u" and (q < 0).any()):
-        raise ValueError(f"quota must be non-negative integers, got {q.dtype}")
+        raise ValueError(f"{what} must be non-negative integers, got {q.dtype}")
     return np.ascontiguousarray(np.broadcast_to(q.astype(np.uint64), (n,)))
+
+
+def _cover_cost(cost, nsrc):
+    """the budget call's costs: integers in [0, 2^32 - 1], one per candidate, as contiguous uint32 (a zero is the
+    library's error to report)"""
+    c = np.asarray(cost)
+    if c.shape != (nsrc,):
+        raise ValueError(f"cost must have one value per candidate ({nsrc},), got {c.shape}")
+    if c.dtype.kind == "O":
+        if not all(isinstance(x, (int, np.integer)) for x in c.ravel()):
+            raise ValueError("cost must be integers")
+        c = np.array([int(x) for x in c.ravel()], dtype=object)
+        if any(x < 0 or x > 0xffffffff for x in c):
+            raise ValueError("cost must lie in [1, 2^32 - 1]")
+        return np.ascontiguousarray(c.astype(np.uint32))
+    if c.dtype.kind not in "iu":
+        raise ValueError(f"cost must be integers, got {c.dtype}")
+    if c.size and (int(c.min()) < 0 or int(c.max()) > 0xffffffff):
+        raise ValueError("cost must lie in [1, 2^32 - 1]")
+    return np.ascontiguousarray(c.astype(np.uint32))
 
 
 def _occ_u8(occ):
@@ -666,8 +705,53 @@ class Context:
                         kmax, threshold, radius, shape, (pick_t, gain_t, npicked_t, count_t, total_t), group_map_t,
                         weights_t, m=m, views_t=views_t, quota_t=quota_t)
 
+    def visibility_cover_budget_batch(self, occ, cand_xy, group_ptr, cost, budget, threshold, radius, shape,
+                                      quota=None, fraction=None, m=1, weights=None, views=None, kmax=None,
+                                      group_map=None):
+        """Budgeted sensor placement (vhp_visibility_cover_budget_batch): each problem picks, among the candidates
+        not yet picked whose cost fits what is left of its budget, the one of largest gain / cost (exactly; ties to the
+        smallest index), until none fits or has a positive gain, kmax picks are made, or the quota (when given) is
+        reached.  cost: integers in [1, 2^32 - 1], one per candidate; budget: uint64 per problem (a scalar is every
+        problem's; UINT64_MAX: no budget).  quota / fraction as in visibility_cover_quota_batch, but neither means no
+        quota.  views None: every candidate omnidirectional with r = radius.  kmax None: the largest group's size.
+        Returns pick (int32 (nprob, kmax)), gain (uint64 (nprob, kmax)), npicked (int32 (nprob,)), count (uint8
+        (nprob, ny, nx)), total and spent (uint64 (nprob,)), single (int32 (nprob,), the best affordable singleton, -1:
+        none), single_gain (uint64 (nprob,)), reached (bool (nprob,), total >= quota; False without a quota) and
+        best_single (bool (nprob,), single_gain > total: the singleton is the better answer)."""
+        gp = np.ascontiguousarray(group_ptr, dtype=np.int64)
+        n = max(gp.shape[0] - 1, 0)
+        if kmax is None:
+            kmax = int(np.diff(gp).max()) if n else 0
+        nsrc = np.asarray(cand_xy).reshape(-1, 2).shape[0]
+        c = _cover_cost(cost, nsrc)
+        b = _cover_u64(budget, n, "budget")
+        q = None if quota is None and fraction is None else \
+            _cover_quota(quota, fraction, m, weights, n, _occ_u8(occ).shape[1:])
+        r = self._cover_host(self.lib.vhp_visibility_cover_budget_batch, CoverBudgetOut, occ, cand_xy, gp, kmax,
+                             threshold, radius, shape, group_map, weights=weights, m=m, views=views, quota=q,
+                             cost=c, budget=b)
+        r["reached"] = r["total"] >= q if q is not None else np.zeros(n, bool)
+        r["best_single"] = r["single_gain"] > r["total"]
+        return r
+
+    def visibility_cover_budget_batch_dev(self, occ_t, cand_xy_t, group_ptr_t, cost_t, budget_t, kmax, threshold,
+                                          radius, shape, quota_t=None, m=1, pick_t=None, gain_t=None, npicked_t=None,
+                                          count_t=None, total_t=None, spent_t=None, single_t=None,
+                                          single_gain_t=None, group_map_t=None, weights_t=None, views_t=None):
+        """The same on CUDA tensors (asynchronous): occ_t uint8 (nmaps, ny, nx), cand_xy_t int32 (nsrc, 2),
+        group_ptr_t int64 (nprob + 1), cost_t uint32 / int32 (nsrc,) (the bits of a uint32), budget_t and quota_t
+        uint64 / int64 (nprob,) (the bits of a uint64; quota_t None: no quota), weights_t uint8 (nprob, ny, nx) or
+        None, views_t int32 (nsrc, 5) or None; outputs pick_t int32 (nprob, kmax), gain_t int64 / uint64 (nprob,
+        kmax), npicked_t int32 (nprob,), count_t uint8 (nprob, ny, nx), total_t, spent_t, single_gain_t int64 /
+        uint64 (nprob,), single_t int32 (nprob,); any may be None.  A bad view or a zero cost is reported by the next
+        synchronising call."""
+        self._cover_dev(self.lib.vhp_visibility_cover_budget_batch_dev, CoverBudgetOut, occ_t, cand_xy_t, group_ptr_t,
+                        kmax, threshold, radius, shape,
+                        (pick_t, gain_t, npicked_t, count_t, total_t, spent_t, single_t, single_gain_t), group_map_t,
+                        weights_t, m=m, views_t=views_t, quota_t=quota_t, cost_t=cost_t, budget_t=budget_t)
+
     def _cover_host(self, fn, out_type, occ, cand_xy, group_ptr, k, threshold, radius, shape, group_map, target=None,
-                    weights=None, m=None, views=False, quota=None):
+                    weights=None, m=None, views=False, quota=None, cost=None, budget=None):
         # out_type's fields name the outputs: CoverOut has uint32 gains, the weighted calls' uint64 ones.  views: False
         # for the calls without views, None for NULL
         occ = _occ_u8(occ)
@@ -691,19 +775,22 @@ class Context:
         kinds = dict(pick=((n, max(k, 0)), np.int32),
                      gain=((n, max(k, 0)), np.uint32 if out_type is CoverOut else np.uint64),
                      npicked=((n,), np.int32), covered=((n, ny, (nx + 31) // 32), np.uint32),
-                     count=((n, ny, nx), np.uint8), total=((n,), np.uint64))
+                     count=((n, ny, nx), np.uint8), total=((n,), np.uint64), spent=((n,), np.uint64),
+                     single=((n,), np.int32), single_gain=((n,), np.uint64))
         names = [name for name, _ in out_type._fields_]
         r = {name: np.empty(*kinds[name]) for name in names}
         co = out_type(*[_np_ptr(r[name]) for name in names])
         tail = () if m is None else (int(m),)
-        if quota is not None:
+        if quota is not None or cost is not None:  # the budget call passes NULL for no quota
             tail += (_np_ptr(quota),)
+        if cost is not None:
+            tail += (_np_ptr(cost), _np_ptr(budget))
         self._check(fn(self.h, _np_ptr(occ), nmaps, nx, ny, _np_ptr(xy), *lead, _np_ptr(gp), _np_ptr(gm), npb, k,
                        int(radius), int(shape), float(threshold), _np_ptr(extra), *tail, C.byref(co)))
         return r
 
     def _cover_dev(self, fn, out_type, occ_t, cand_xy_t, group_ptr_t, k, threshold, radius, shape, outs, group_map_t,
-                   extra_t, m=None, views_t=False, quota_t=False):
+                   extra_t, m=None, views_t=False, quota_t=False, cost_t=False, budget_t=None):
         nmaps, ny, nx = occ_t.shape
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         co = out_type(*[ptr(t) for t in outs])
@@ -711,6 +798,8 @@ class Context:
         tail = () if m is None else (int(m),)
         if quota_t is not False:
             tail += (ptr(quota_t),)
+        if cost_t is not False:
+            tail += (ptr(cost_t), ptr(budget_t))
         self._check(fn(self.h, occ_t.data_ptr(), nmaps, nx, ny, cand_xy_t.data_ptr(), *lead, group_ptr_t.data_ptr(),
                        ptr(group_map_t), group_ptr_t.shape[0] - 1, cand_xy_t.shape[0], int(k), int(radius),
                        int(shape), float(threshold), ptr(extra_t), *tail, C.byref(co)))

@@ -167,6 +167,9 @@ vhp_status check_device_error(vhp_context *ctx) {
       return fail(ctx, VHP_ERR_INVALID_ARG,
                   "a source's view (r, ax, ay, bx, by) is invalid: r outside [0, radius], a or b (0, 0), or a "
                   "component outside [-32767, 32767]; that source contributed nothing");
+    if (flag & 32)
+      return fail(ctx, VHP_ERR_INVALID_ARG,
+                  "vhp_visibility_cover_budget_batch_dev: a candidate's cost is 0; that candidate was never picked");
     return fail(ctx, VHP_ERR_INVALID_ARG, "a source / start / end point lies outside the grid");
   }
   return VHP_OK;
@@ -1210,27 +1213,33 @@ vhp_status run_merge_host(vhp_context *ctx, const uint8_t *occ, int nmaps, int n
 // (vhp_visibility_cover_greedy_mfold_batch) the same phase 1 and the weighted rounds with counters, and the view call
 // (vhp_visibility_cover_greedy_view_batch) the m-fold call with each candidate's bits masked by its view in between.
 // The quota call (vhp_visibility_cover_quota_batch) is the view call, or the m-fold call without views, whose rounds
-// loop on the device until each problem's gains reach its quota.
+// loop on the device until each problem's gains reach its quota.  The budget call (vhp_visibility_cover_budget_batch)
+// is the quota call with per-candidate costs and a budget per problem: its rounds pick by gain / cost among the
+// candidates that still fit the budget, and the quota may be null.
 const char *const kCoverName = "vhp_visibility_cover_greedy_batch";
 const char *const kCoverWeightedName = "vhp_visibility_cover_greedy_weighted_batch";
 const char *const kCoverMfoldName = "vhp_visibility_cover_greedy_mfold_batch";
 const char *const kCoverViewName = "vhp_visibility_cover_greedy_view_batch";
 const char *const kCoverQuotaName = "vhp_visibility_cover_quota_batch";
+const char *const kCoverBudgetName = "vhp_visibility_cover_budget_batch";
 // the weighted key keeps 28 bits for the index within the group (kernels_cover.cu)
 constexpr int64_t kCoverWeightedMaxSrc = (int64_t)1 << 28;
 
 // A cover call and its arguments.  weighted: uint64 gains and uint8 weights; mfold (with weighted): cells count until
 // m picks cover them, `count` instead of `covered`; view (with mfold): range.views masks each candidate's bits; quota
-// (with mfold, the quota call): a problem stops once the sum of its gains reaches its quota, k is kmax.
+// (with mfold, the quota call): a problem stops once the sum of its gains reaches its quota, k is kmax; budget (with
+// mfold, the budget call): the picks go by gain / cost within each problem's budget, and quota may be null.
 // extra: the target ([prob][ny][ceil(nx/32)] uint32) or the weights ([prob][ny][nx] uint8), may be null.
 struct CoverCall {
   const char *name;
-  bool weighted = false, mfold = false, view = false;
+  bool weighted = false, mfold = false, view = false, budget = false;
   int32_t k, m = 1;
   VhpMergeRange range;
   double thr;
   const void *extra;
-  const uint64_t *quota = nullptr; // [prob]
+  const uint64_t *quota = nullptr;   // [prob]
+  const uint32_t *cost = nullptr;    // [src], the budget call's
+  const uint64_t *budgets = nullptr; // [prob], the budget call's
   CoverCall(const char *call, int32_t k_, int32_t radius, int32_t shape, double thr_, const void *extra_)
       : name(call), k(k_), range(radius, shape), thr(thr_), extra(extra_) {}
 };
@@ -1250,15 +1259,19 @@ const VhpCoverOut *cover_out(const vhp_cover_quota_out *p, VhpCoverOut &o) {
   if (p) o = {p->pick, p->gain, p->npicked, nullptr, p->count, p->total};
   return p ? &o : nullptr;
 }
+const VhpCoverOut *cover_out(const vhp_cover_budget_out *p, VhpCoverOut &o) {
+  if (p) o = {p->pick, p->gain, p->npicked, nullptr, p->count, p->total, p->spent, p->single, p->single_gain};
+  return p ? &o : nullptr;
+}
 
-// The m-fold and view calls report these under the m-fold call's name, but for "views is NULL"; the quota call under
-// its own name, with "kmax" for k.  The weighted key's
+// The m-fold and view calls report these under the m-fold call's name, but for "views is NULL"; the quota and budget
+// calls under their own names, with "kmax" for k.  The weighted key's
 // limit on nsrc is checked before any candidate is read; the views' values by check_views_host, or by bit 3 of d_err
 // on the device.
 vhp_status check_cover_args(vhp_context *ctx, const CoverCall &c, const void *occ, int nmaps, int nx, int ny,
                             const void *xy, const void *group_ptr, int64_t nprob, int64_t nsrc,
                             const VhpCoverOut *out) {
-  const bool quota = c.name == kCoverQuotaName;
+  const bool quota = c.name == kCoverQuotaName || c.budget;
   const std::string what = c.mfold && !quota ? kCoverMfoldName : c.name;
   if (!ctx) return fail(nullptr, VHP_ERR_INVALID_ARG, "null context");
   if (!occ || !group_ptr || !out || (nsrc > 0 && !xy)) return fail(ctx, VHP_ERR_INVALID_ARG, "null buffer");
@@ -1268,8 +1281,11 @@ vhp_status check_cover_args(vhp_context *ctx, const CoverCall &c, const void *oc
   if (st != VHP_OK) return st;
   if (c.thr != c.thr) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": threshold is NaN");
   if (c.k < 0) return fail(ctx, VHP_ERR_INVALID_ARG, what + (quota ? ": kmax < 0" : ": k < 0"));
-  if (quota && nprob > 0 && !c.quota) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": quota is NULL");
-  if (!out->pick && !out->gain && !out->npicked && !out->covered && !out->count && !out->total)
+  if (quota && !c.budget && nprob > 0 && !c.quota) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": quota is NULL");
+  if (c.budget && nsrc > 0 && !c.cost) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": cost is NULL");
+  if (c.budget && nprob > 0 && !c.budgets) return fail(ctx, VHP_ERR_INVALID_ARG, what + ": budget is NULL");
+  if (!out->pick && !out->gain && !out->npicked && !out->covered && !out->count && !out->total && !out->spent &&
+      !out->single && !out->single_gain)
     return fail(ctx, VHP_ERR_INVALID_ARG, what + ": no output requested");
   if ((st = check_range(ctx, what, c.range)) != VHP_OK) return st;
   if (c.weighted && nsrc >= kCoverWeightedMaxSrc)
@@ -1319,7 +1335,8 @@ vhp_status run_cover_phase1(vhp_context *ctx, const CoverCall &c, const uint8_t 
           VHP_OK)
         return st;
       if ((st = ensure_cover(ctx, ctx->b_cover_ws,
-                             vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, c.weighted, c.mfold, c.quota != nullptr),
+                             vhp_cover_ws_bytes(nprob, nsrc, nx, ny, R, c.weighted, c.mfold, c.quota != nullptr,
+                                                c.budget),
                              "workspace", c.name)) != VHP_OK)
         return st;
       uint32_t *bits = cb.bits = (uint32_t *)ctx->b_cover.p;
@@ -1364,9 +1381,10 @@ vhp_status run_cover_dev(vhp_context *ctx, const CoverCall &c, const uint8_t *d_
                                           &ctx->launches));
     cb.disk_r2 = -1;
   }
+  const VhpCoverBudget bud{c.cost, c.budgets, ctx->d_err};
   VHP_CUDA(ctx, vhp_launch_cover_greedy(cb.bits, nsrc, nprob, nx, ny, cb.R, cb.disk_r2, d_xy, cb.pg, cb.pk, c.weighted,
                                         c.mfold, c.extra, c.k, c.m, c.quota, ctx->b_cover_ws.p, out, ctx->sm_count,
-                                        ctx->stream, ctx->copy_stream, &ctx->launches));
+                                        ctx->stream, ctx->copy_stream, &ctx->launches, c.budget ? &bud : nullptr));
   return VHP_OK;
 }
 
@@ -1381,7 +1399,8 @@ vhp_status cover_dev_entry(vhp_context *ctx, const CoverCall &c, const uint8_t *
 }
 
 // host buffers: runs of whole problems whose device memory (candidate bits, workspace, outputs) fits 4 GB, each with
-// its slice of c.extra (and of c.quota) uploaded.  c.range.views: the view call's [nsrc][5] on the host.
+// its slice of c.extra (and of c.quota, c.cost and c.budgets) uploaded.  c.range.views: the view call's [nsrc][5] on
+// the host.  The budget call's costs are checked for zeros before any candidate is read.
 vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *occ, int nmaps, int nx, int ny,
                           const int32_t *xy, const int64_t *gptr, const int32_t *gmap, int64_t nprob,
                           const VhpCoverOut *out) {
@@ -1389,6 +1408,10 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
   if (st != VHP_OK) return st;
   const int64_t nsrc = (ctx && gptr && nprob >= 0) ? gptr[nprob] : 0;
   if ((st = check_cover_args(ctx, c, occ, nmaps, nx, ny, xy, gptr, nprob, nsrc, out)) != VHP_OK) return st;
+  for (int64_t i = 0; c.budget && i < nsrc; ++i)
+    if (c.cost[i] == 0)
+      return fail(ctx, VHP_ERR_INVALID_ARG, std::string(c.name) + ": the cost of candidate " + std::to_string(i) +
+                                                " is 0");
   const size_t plane = (size_t)ny * ((nx + 31) / 32), gsz = c.weighted ? 8 : 4;
   const VhpCoverBox b = vhp_cover_box(nx, ny, std::min(c.range.radius, std::max(nx, ny) - 1), 0, 0);
   const size_t box = (size_t)b.H * b.W * 4;
@@ -1396,17 +1419,22 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
   const size_t bn = out->npicked ? 4 : 0, bc = out->covered ? plane * 4 : out->count ? (size_t)ny * nx : 0;
   const size_t bt = c.extra ? (c.weighted ? (size_t)ny * nx : plane * 4) : 0;
   const size_t btot = out->total ? 8 : 0, bq = c.quota ? 8 : 0; // the quota call's total and quota
+  // the budget call's spent, single_gain, budget and single outputs and inputs
+  const size_t bsp = out->spent ? 8 : 0, bsg = out->single_gain ? 8 : 0, bb = c.budget ? 8 : 0,
+               bs1 = out->single ? 4 : 0;
   // device bytes of problem q: its candidates' bits, table and gains, state, new, outputs, target or weights (and
   // the weighted rounds' 32-byte rows of weights, and the m-fold rounds' 32-byte rows of counters; views: 20 bytes;
-  // the 64 bytes of per-problem scalars hold the quota rounds' total and quota copy too)
-  const size_t per_src = box + 12 + gsz + (c.view ? 20 : 0), per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 +
-                                                                  (c.weighted ? plane * 32 : 0) +
-                                                                  (c.mfold ? plane * 32 : 0) + btot + bq;
+  // the 64 bytes of per-problem scalars hold the quota rounds' total and quota copy too; the budget call's 4-byte
+  // costs, and its ratio slot, remaining budget and spent cost, 32 bytes)
+  const size_t per_src = box + 12 + gsz + (c.view ? 20 : 0) + (c.budget ? 4 : 0),
+               per_prob = plane * 4 + box + bp + bg + bn + bc + bt + 64 + (c.weighted ? plane * 32 : 0) +
+                          (c.mfold ? plane * 32 : 0) + btot + bq + bsp + bsg + bb + bs1 + (c.budget ? 32 : 0);
   void *const host_cells = out->covered ? (void *)out->covered : (void *)out->count;
   auto run = [&](int64_t q0, int64_t gc, const int32_t *d_xy, const int64_t *d_gptr, const int32_t *d_gmap,
                  int64_t run_nsrc, const VhpMergeRange *run_range) {
     vhp_status r;
-    if ((r = ensure(ctx, ctx->b_out[0], (size_t)gc * (bp + bg + btot + bq + bn + bc) + 256)) != VHP_OK) return r;
+    const size_t bytes = (size_t)gc * (bp + bg + btot + bq + bn + bc + bsp + bsg + bb + bs1) + 256;
+    if ((r = ensure(ctx, ctx->b_out[0], bytes + (c.budget ? 4 * (size_t)run_nsrc : 0))) != VHP_OK) return r;
     if (c.extra && (r = ensure(ctx, ctx->b_out[1], (size_t)gc * bt)) != VHP_OK) return r;
     cudaError_t e = cudaSuccess;
     if (c.extra)
@@ -1414,22 +1442,33 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
                           cudaMemcpyHostToDevice, ctx->stream);
     char *base = (char *)ctx->b_out[0].p;
     const size_t o_gain = (gc * bp + gsz - 1) & ~(gsz - 1); // uint64 gains, totals and quotas: 8-byte aligned
-    char *tot = base + o_gain + gc * bg, *quota = tot + gc * btot;
-    char *cells = quota + gc * (bq + bn);
+    char *tot = base + o_gain + gc * bg, *spent = tot + gc * btot, *sgain = spent + gc * bsp;
+    char *quota = sgain + gc * bsg, *budget = quota + gc * bq, *npk = budget + gc * bb, *single = npk + gc * bn;
+    char *cells = single + gc * bs1;
+    char *cost = base + ((size_t)(cells + gc * bc - base + 3) & ~(size_t)3); // 4-byte aligned, within the 256 spare
     if (e == cudaSuccess && c.quota)
       e = cudaMemcpyAsync(quota, c.quota + q0, gc * bq, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && c.budget)
+      e = cudaMemcpyAsync(budget, c.budgets + q0, gc * bb, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && c.budget && run_nsrc > 0)
+      e = cudaMemcpyAsync(cost, c.cost + gptr[q0], 4 * (size_t)run_nsrc, cudaMemcpyHostToDevice, ctx->stream);
     if (e != cudaSuccess) return cuda_fail(ctx, e, "cover: upload of the problems");
     VhpCoverOut o;
     o.pick = out->pick ? (int32_t *)base : nullptr;
     o.gain = out->gain ? base + o_gain : nullptr;
-    o.npicked = out->npicked ? (int32_t *)(quota + gc * bq) : nullptr;
+    o.npicked = out->npicked ? (int32_t *)npk : nullptr;
     o.covered = out->covered ? (uint32_t *)cells : nullptr;
     o.count = out->count ? (uint8_t *)cells : nullptr;
     o.total = out->total ? (uint64_t *)tot : nullptr;
+    o.spent = out->spent ? (uint64_t *)spent : nullptr;
+    o.single = out->single ? (int32_t *)single : nullptr;
+    o.single_gain = out->single_gain ? (uint64_t *)sgain : nullptr;
     CoverCall rc = c;
     rc.range = *run_range;
     rc.extra = c.extra ? ctx->b_out[1].p : nullptr;
     rc.quota = c.quota ? (const uint64_t *)quota : nullptr;
+    rc.budgets = c.budget ? (const uint64_t *)budget : nullptr;
+    rc.cost = c.budget ? (const uint32_t *)cost : nullptr;
     r = run_cover_dev(ctx, rc, (const uint8_t *)ctx->b_occ.p, nmaps, nx, ny, d_xy, d_gptr, d_gmap, gc, run_nsrc, o);
     if (r != VHP_OK) return r;
     if (out->pick) e = cudaMemcpyAsync(out->pick + q0 * c.k, o.pick, gc * bp, cudaMemcpyDeviceToHost, ctx->stream);
@@ -1441,11 +1480,18 @@ vhp_status run_cover_host(vhp_context *ctx, const CoverCall &c, const uint8_t *o
       e = cudaMemcpyAsync((char *)host_cells + q0 * bc, cells, gc * bc, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && out->total)
       e = cudaMemcpyAsync(out->total + q0, o.total, gc * btot, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->spent)
+      e = cudaMemcpyAsync(out->spent + q0, o.spent, gc * bsp, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->single)
+      e = cudaMemcpyAsync(out->single + q0, o.single, gc * bs1, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && out->single_gain)
+      e = cudaMemcpyAsync(out->single_gain + q0, o.single_gain, gc * bsg, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     return e == cudaSuccess ? VHP_OK : cuda_fail(ctx, e, "cover: copy of the outputs");
   };
   return run_groups_host(ctx, c.name, "candidate", occ, nmaps, nx, ny, xy, gptr, gmap, nprob, &c.range, per_src,
-                         per_prob, (size_t)4 << 30, bp + bg + bn + bc + btot, "cover: upload of the problems", run);
+                         per_prob, (size_t)4 << 30, bp + bg + bn + bc + btot + bsp + bs1 + bsg,
+                         "cover: upload of the problems", run);
 }
 
 // ---- opt-in sweep variants ------------------------------------------------------------------------
@@ -2154,6 +2200,44 @@ vhp_status vhp_visibility_cover_quota_batch_dev(vhp_context *ctx, const uint8_t 
   c.m = m;
   c.range.views = d_views;
   c.quota = d_quota;
+  VhpCoverOut o;
+  return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
+                         cover_out(d_out, o));
+}
+
+vhp_status vhp_visibility_cover_budget_batch(vhp_context *ctx, const uint8_t *occ, int nmaps, int nx, int ny,
+                                             const int32_t *cand_xy, const int32_t *views, const int64_t *group_ptr,
+                                             const int32_t *group_map, int64_t nprob, int32_t kmax, int32_t radius,
+                                             int32_t shape, double threshold, const uint8_t *weights, int32_t m,
+                                             const uint64_t *quota, const uint32_t *cost, const uint64_t *budget,
+                                             const vhp_cover_budget_out *out) {
+  CoverCall c(kCoverBudgetName, kmax, radius, shape, threshold, weights);
+  c.weighted = c.mfold = c.budget = true;
+  c.view = views != nullptr;
+  c.m = m;
+  c.range.views = views;
+  c.quota = quota;
+  c.cost = cost;
+  c.budgets = budget;
+  VhpCoverOut o;
+  return run_cover_host(ctx, c, occ, nmaps, nx, ny, cand_xy, group_ptr, group_map, nprob, cover_out(out, o));
+}
+
+vhp_status vhp_visibility_cover_budget_batch_dev(vhp_context *ctx, const uint8_t *d_occ, int nmaps, int nx, int ny,
+                                                 const int32_t *d_cand_xy, const int32_t *d_views,
+                                                 const int64_t *d_group_ptr, const int32_t *d_group_map, int64_t nprob,
+                                                 int64_t nsrc, int32_t kmax, int32_t radius, int32_t shape,
+                                                 double threshold, const uint8_t *d_weights, int32_t m,
+                                                 const uint64_t *d_quota, const uint32_t *d_cost,
+                                                 const uint64_t *d_budget, const vhp_cover_budget_out *d_out) {
+  CoverCall c(kCoverBudgetName, kmax, radius, shape, threshold, d_weights);
+  c.weighted = c.mfold = c.budget = true;
+  c.view = d_views != nullptr;
+  c.m = m;
+  c.range.views = d_views;
+  c.quota = d_quota;
+  c.cost = d_cost;
+  c.budgets = d_budget;
   VhpCoverOut o;
   return cover_dev_entry(ctx, c, d_occ, nmaps, nx, ny, d_cand_xy, d_group_ptr, d_group_map, nprob, nsrc,
                          cover_out(d_out, o));

@@ -29,6 +29,14 @@
 // counter of active problems.  The rounds are the body of a CUDA-graph WHILE node, apply, update and
 // cover_quota_step_kernel, which advances the round and keeps the loop going while a problem is active and
 // round < min(kmax, nsrc).
+//
+// The budget call (vhp_visibility_cover_budget_batch) runs the quota call's loop with init, apply and update
+// instantiated with kB = true: a candidate keys only while its cost fits the problem's remaining budget, and the key is
+// the 128-bit ratio key (ratio_key), so the slot's max is the exact argmax of gain / cost with ties to the smallest
+// index.  Apply reads the pick's gain from the gain array, spends its cost and stops at the quota (when given) or kmax
+// like the quota call; a problem whose slot is empty (nothing affordable of positive gain) is done.  Init also puts each
+// affordable candidate's round-0 key (key_of) into the 64-bit slot, which the rounds leave alone: after the loop,
+// cover_budget_out_kernel turns it into the best affordable singleton.
 #include <algorithm>
 #include <cstdint>
 #include <type_traits>
@@ -57,6 +65,15 @@ struct CoverGeo {
 struct CoverQuotaState {
   unsigned long long *total = nullptr, *quota = nullptr;
   int *active = nullptr, *round = nullptr;
+};
+
+// the budget call's state, in the workspace but cost: the ratio-key slot, the remaining budget and the spent cost
+// [prob]; cost [src] is the caller's (or the host form's upload), err the context's error word (bit 5: a zero cost)
+struct CoverBudgetState {
+  const uint32_t *cost = nullptr;
+  unsigned __int128 *slot = nullptr;
+  unsigned long long *left = nullptr, *spent = nullptr;
+  int *err = nullptr;
 };
 
 // bits lo .. hi of a word (any lo, hi; empty if lo > hi after clamping to [0, 31])
@@ -121,6 +138,50 @@ __device__ __forceinline__ unsigned long long key_of(uint32_t gain, int32_t k) {
 }
 __device__ __forceinline__ unsigned long long key_of(uint64_t gain, int32_t k) {
   return ((unsigned long long)gain << kIdxBits) | (kIdxMask - (uint32_t)k);
+}
+
+// The budget rounds' key: (floor(gain * 2^64 / cost) << 28) | (2^28 - 1 - k).  With gain < 2^36 and cost < 2^32, two
+// distinct ratios differ by at least 1 / (c1 c2) > 2^-64, so the floor orders them strictly, and equal ratios give equal
+// floors: the key orders by exact ratio, then by smallest index.  The floor is < 2^100, and > 2^32 for gain > 0.  It
+// is gain / cost followed by two 32-bit steps of long division on the remainder (r < cost < 2^32, so r << 32 fits).
+__device__ __forceinline__ unsigned __int128 ratio_key(uint64_t gain, uint32_t cost, int32_t k) {
+  const uint64_t hi = gain / cost, r0 = (gain % cost) << 32;
+  const uint64_t d1 = r0 / cost, d2 = ((r0 % cost) << 32) / cost;
+  const unsigned __int128 f = ((unsigned __int128)hi << 64) | (d1 << 32) | d2;
+  return (f << kIdxBits) | (unsigned __int128)(kIdxMask - (uint32_t)k);
+}
+
+// *a = max(*a, v) by compare-and-swap; the first compare against 0 doubles as an atomic read of the slot
+__device__ __forceinline__ void atomic_max128(unsigned __int128 *a, const unsigned __int128 v) {
+  unsigned __int128 old = 0;
+  while (old < v) {
+    const unsigned __int128 prev = atomicCAS(a, old, v);
+    if (prev == old) return;
+    old = prev;
+  }
+}
+
+// put_keys for the 128-bit slots: the warp's max (as two 64-bit halves) in one compare-and-swap loop when the valid
+// lanes share a problem
+__device__ __forceinline__ void put_keys(const bool valid, const int32_t g, const unsigned __int128 key,
+                                         unsigned __int128 *slot) {
+  const unsigned vm = __ballot_sync(kAll, valid);
+  if (!vm) return;
+  const int lead = __ffs(vm) - 1, lane = threadIdx.x & 31;
+  const int32_t g0 = __shfl_sync(kAll, g, lead);
+  if (__all_sync(kAll, !valid || g == g0)) {
+    unsigned __int128 m = valid ? key : 0;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const unsigned long long h = __shfl_xor_sync(kAll, (unsigned long long)(m >> 64), o);
+      const unsigned long long l = __shfl_xor_sync(kAll, (unsigned long long)m, o);
+      const unsigned __int128 t = ((unsigned __int128)h << 64) | l;
+      m = t > m ? t : m;
+    }
+    if (lane == lead) atomic_max128(slot + g0, m);
+  } else if (valid) {
+    atomic_max128(slot + g, key);
+  }
 }
 
 // Fallback of phase 1: one thread per box word of pairs [p0, p0 + np).
@@ -195,8 +256,10 @@ __global__ void cover_weight_kernel(const uint8_t *__restrict__ wts, int64_t npr
 // gain(c) = |S(c) \ state| of 32 candidates per CTA (a warp per candidate, lanes over rows); disk_r2 >= 0: the disk
 // mask dx^2 + dy^2 <= disk_r2 is applied to the bits in place first.  Then the keys of round 0, and first[q] = the
 // problem's candidate of index 0 (the rounds read no group_ptr: the host form's copy of it may be gone by then).
-// kW: the gain sums the weights of wpad (cover_weight_kernel's plane) instead of counting cells.
-template <bool kW>
+// kW: the gain sums the weights of wpad (cover_weight_kernel's plane) instead of counting cells.  kB (budget, with kW):
+// a candidate of positive gain and cost <= its problem's budget puts its ratio key into bs.slot and its key_of into
+// slot (the singleton); a zero cost raises bit 5 of bs.err and puts neither.  bs is unused otherwise.
+template <bool kW, bool kB = false>
 __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__restrict__ bits, int64_t nsrc, CoverGeo G,
                                                                  int disk_r2, const int32_t *__restrict__ xy,
                                                                  const int32_t *__restrict__ pg,
@@ -204,7 +267,8 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
                                                                  const uint32_t *__restrict__ state,
                                                                  GainT<kW> *__restrict__ gain,
                                                                  unsigned long long *slot, int64_t *first,
-                                                                 const uint8_t *__restrict__ wpad) {
+                                                                 const uint8_t *__restrict__ wpad,
+                                                                 CoverBudgetState bs = {}) {
   __shared__ GainT<kW> sg[kCand];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t base = blockIdx.x * (int64_t)kCand;
@@ -260,7 +324,15 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
     const int32_t kc = g >= 0 ? __ldg(pk + c) : -1;
     if (c < nsrc) gain[c] = gn;
     if (kc == 0) first[g] = c;
-    put_keys(g >= 0, g, key_of(gn, kc), slot);
+    if constexpr (kB) {
+      const uint32_t cost = g >= 0 ? __ldg(bs.cost + c) : 0u;
+      if (g >= 0 && cost == 0) atomicOr(bs.err, 32);
+      const bool fits = g >= 0 && cost != 0 && gn > 0 && cost <= bs.left[g];
+      put_keys(fits, g, key_of(gn, kc), slot);
+      put_keys(fits, g, ratio_key(gn, fits ? cost : 1u, kc), bs.slot);
+    } else {
+      put_keys(g >= 0, g, key_of(gn, kc), slot);
+    }
   }
 }
 
@@ -270,7 +342,9 @@ __global__ void __launch_bounds__(kWarps * 32) cover_init_kernel(uint32_t *__res
 // pick's gain is zeroed (with mfold >= 2 it keeps gain on its own cells).  gain, cnt and mfold are unused otherwise.
 // kQ (quota, with kM): the round is *qs.round (r is unused), and a problem is done once its total reaches its quota or
 // r + 1 == k (kmax); every problem that becomes done decrements *qs.active once.  qs is unused otherwise.
-template <bool kW, bool kM, bool kQ = false>
+// kB (budget, with kQ): the pick is bs.slot's (empty: done) with its gain read from gain; its cost leaves the problem's
+// remaining budget and joins its spent cost.  slot (the singleton's) is left alone.  bs is unused otherwise.
+template <bool kW, bool kM, bool kQ = false, bool kB = false>
 __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32_t *__restrict__ bits,
                                                                     const int64_t *__restrict__ first, int64_t nsrc,
                                                                     CoverGeo G,
@@ -280,15 +354,25 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
                                                                     uint32_t *__restrict__ newb,
                                                                     VhpCoverDevT<GainT<kW>> out, GainT<kW> *gain,
                                                                     uint8_t *__restrict__ cnt, int mfold,
-                                                                    CoverQuotaState qs) {
+                                                                    CoverQuotaState qs, CoverBudgetState bs = {}) {
   const int64_t q = blockIdx.x;
   if (done[q]) return;
-  const unsigned long long key = slot[q];
+  const unsigned long long key = kB ? 0ull : slot[q];
+  GainT<kW> bgn = 0; // kB: the pick's gain, read before thread 0 zeroes it
+  uint32_t bidx = 0;
+  if constexpr (kB) {
+    const unsigned __int128 bkey = bs.slot[q];
+    bidx = (uint32_t)(kIdxMask - (uint64_t)(bkey & kIdxMask));
+    if (bkey != 0 && first[q] >= 0 && first[q] + bidx < nsrc) bgn = gain[first[q] + bidx];
+  }
   if constexpr (kQ) r = *qs.round;
   __syncthreads(); // every thread has read the slot before thread 0 resets it
   GainT<kW> gn;
   uint32_t idx;
-  if constexpr (kW) {
+  if constexpr (kB) {
+    gn = bgn;
+    idx = bidx;
+  } else if constexpr (kW) {
     gn = key >> kIdxBits;
     idx = (uint32_t)(kIdxMask - (key & kIdxMask));
   } else {
@@ -308,7 +392,14 @@ __global__ void __launch_bounds__(kApplyThreads) cover_apply_kernel(const uint32
     if (out.gain) out.gain[q * k + r] = gn;
     if (out.npicked) out.npicked[q] = r + 1;
     cur[q] = c;
-    slot[q] = 0;
+    if constexpr (kB) {
+      bs.slot[q] = 0;
+      const uint32_t cost = __ldg(bs.cost + c);
+      bs.left[q] -= cost;
+      bs.spent[q] += cost;
+    } else {
+      slot[q] = 0;
+    }
     if constexpr (kM) gain[c] = 0;
     if constexpr (kQ) {
       const unsigned long long t = qs.total[q] + gn;
@@ -418,6 +509,43 @@ __global__ void cover_quota_step_kernel(CoverQuotaState qs, int32_t rounds, cuda
   cudaGraphSetConditional(loop, (*qs.active > 0 && r < rounds) ? 1u : 0u);
 }
 
+// The budget call, before init: cover_quota_init_kernel with quota null meaning no quota (UINT64_MAX, which no total
+// reaches), and each problem's remaining budget = its budget, spent = 0.
+__global__ void cover_budget_init_kernel(const unsigned long long *__restrict__ quota,
+                                         const unsigned long long *__restrict__ budget, int64_t nprob, int *done,
+                                         CoverQuotaState qs, CoverBudgetState bs) {
+  const int lane = threadIdx.x & 31;
+  const int64_t step = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x - lane; i0 < nprob; i0 += step) {
+    const int64_t q = i0 + lane;
+    unsigned long long v = 0;
+    if (q < nprob) {
+      v = quota ? __ldg(quota + q) : ~0ull;
+      qs.quota[q] = v;
+      qs.total[q] = 0;
+      bs.left[q] = __ldg(budget + q);
+      bs.spent[q] = 0;
+      done[q] = v == 0;
+    }
+    const unsigned a = __ballot_sync(kAll, v != 0);
+    if (lane == 0 && a) atomicAdd(qs.active, __popc(a));
+  }
+}
+
+// The budget call, after the rounds: the singleton slot as single (-1: empty) and single_gain, and total and spent.
+// Any output may be null.
+__global__ void cover_budget_out_kernel(const unsigned long long *__restrict__ slot, int64_t nprob,
+                                        CoverQuotaState qs, CoverBudgetState bs, uint64_t *total, uint64_t *spent,
+                                        int32_t *single, uint64_t *single_gain) {
+  for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nprob; q += (int64_t)gridDim.x * blockDim.x) {
+    const unsigned long long key = slot[q];
+    if (single) single[q] = key ? (int32_t)(kIdxMask - (key & kIdxMask)) : -1;
+    if (single_gain) single_gain[q] = key >> kIdxBits;
+    if (total) total[q] = qs.total[q];
+    if (spent) spent[q] = bs.spent[q];
+  }
+}
+
 // floor and ceiling of n / d, d != 0 (C division truncates toward zero)
 __device__ __forceinline__ long long floor_div(long long n, long long d) {
   const long long q = n / d;
@@ -505,8 +633,9 @@ __global__ void __launch_bounds__(kWarps * 32) cover_view_kernel(uint32_t *__res
 
 // After round r's apply: exact gain update of the candidates whose box meets their problem's pick, then the keys of
 // round r + 1.  Candidates of finished problems do nothing; a candidate of gain 0 keeps it.  kW: the weights of
-// wpad's words, loaded only for words where S(c) & new is not 0.
-template <bool kW>
+// wpad's words, loaded only for words where S(c) & new is not 0.  kB (budget, with kW): only a candidate of positive
+// gain whose nonzero cost fits the problem's remaining budget puts a key, its ratio key into bs.slot.
+template <bool kW, bool kB = false>
 __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_t *__restrict__ bits, int64_t nsrc,
                                                                    CoverGeo G, const int32_t *__restrict__ xy,
                                                                    const int32_t *__restrict__ pg,
@@ -516,7 +645,8 @@ __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_
                                                                    const uint32_t *__restrict__ newb,
                                                                    GainT<kW> *__restrict__ gain,
                                                                    unsigned long long *slot,
-                                                                   const uint8_t *__restrict__ wpad) {
+                                                                   const uint8_t *__restrict__ wpad,
+                                                                   CoverBudgetState bs = {}) {
   __shared__ GainT<kW> sdec[kCand];
   __shared__ unsigned sov;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -581,7 +711,13 @@ __global__ void __launch_bounds__(kWarps * 32) cover_update_kernel(const uint32_
       gn -= sdec[lane];
       gain[c] = gn;
     }
-    put_keys(valid, g, key_of(gn, valid ? pk[c] : 0), slot);
+    if constexpr (kB) {
+      const uint32_t cost = valid ? __ldg(bs.cost + c) : 0u;
+      const bool fits = valid && gn > 0 && cost != 0 && cost <= bs.left[g];
+      put_keys(fits, g, ratio_key(gn, fits ? cost : 1u, valid ? pk[c] : 0), bs.slot);
+    } else {
+      put_keys(valid, g, key_of(gn, valid ? pk[c] : 0), slot);
+    }
   }
 }
 
@@ -593,7 +729,8 @@ size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 // workspace of the rounds: state [prob][ny][nw], new [prob][H][W], gain [src] (uint32, weighted uint64), slot [prob],
 // cur [prob], first [prob], done [prob]; weighted: wpad [prob][ny][nw][32]; m-fold (weighted too): cnt, wpad's layout;
-// quota (m-fold too): total [prob], quota [prob], active, round
+// quota (m-fold too): total [prob], quota [prob], active, round; budget (quota too): the 16-byte ratio slot, the
+// remaining budget and the spent cost [prob]
 struct CoverWs {
   uint32_t *state, *newb;
   void *gain;
@@ -602,10 +739,11 @@ struct CoverWs {
   int *done;
   uint8_t *wpad, *cnt;
   CoverQuotaState qs;
+  CoverBudgetState bs;
   size_t bytes;
 };
 CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold,
-                 bool quota = false) {
+                 bool quota = false, bool budget = false) {
   const VhpCoverBox b = vhp_cover_box(nx, ny, R, 0, 0);
   const size_t np = (size_t)nprob, plane = (size_t)ny * ((nx + 31) / 32);
   const size_t o_new = align256(np * plane * 4), o_gain = o_new + align256(np * b.H * b.W * 4);
@@ -613,10 +751,11 @@ CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R,
   const size_t o_first = o_cur + align256(np * 8), o_done = o_first + align256(np * 8);
   const size_t o_wpad = o_done + align256(np * 4), o_cnt = o_wpad + (weighted ? align256(np * plane * 32) : 0);
   const size_t o_total = o_cnt + (mfold ? align256(np * plane * 32) : 0), o_quota = o_total + align256(np * 8);
-  const size_t o_ctl = o_quota + align256(np * 8);
+  const size_t o_ctl = o_quota + align256(np * 8), o_bslot = o_ctl + 256;
+  const size_t o_left = o_bslot + align256(np * 16), o_spent = o_left + align256(np * 8);
   char *p = static_cast<char *>(base);
   CoverWs w{};
-  w.bytes = quota ? o_ctl + 256 : o_total;
+  w.bytes = budget ? o_spent + align256(np * 8) : quota ? o_ctl + 256 : o_total;
   if (!p) return w;
   w.state = (uint32_t *)p;
   w.newb = (uint32_t *)(p + o_new);
@@ -632,6 +771,11 @@ CoverWs cover_ws(void *base, int64_t nprob, int64_t nsrc, int nx, int ny, int R,
     w.qs.quota = (unsigned long long *)(p + o_quota);
     w.qs.active = (int *)(p + o_ctl);
     w.qs.round = w.qs.active + 1;
+  }
+  if (budget) {
+    w.bs.slot = (unsigned __int128 *)(p + o_bslot);
+    w.bs.left = (unsigned long long *)(p + o_left);
+    w.bs.spent = (unsigned long long *)(p + o_spent);
   }
   return w;
 }
@@ -674,14 +818,17 @@ cudaError_t launch_quota_loop(CoverQuotaState qs, int32_t rounds, cudaStream_t s
 
 // the rounds of the four calls: kW = false counts cells of d_target (null: all), kW = true sums d_weights (null:
 // all 1), kM (with kW) counts each cell until mfold picks cover it and writes d_count (may be null) at the end, kQ
-// (with kM) loops until each problem's total reaches d_quota (the graph of launch_quota_loop) and writes d_total
-template <bool kW, bool kM = false, bool kQ = false>
+// (with kM) loops until each problem's total reaches d_quota (the graph of launch_quota_loop) and writes d_total, kB
+// (with kQ) picks by gain / cost within each problem's budget (bud; d_quota may be null) and also writes bout's spent,
+// single and single_gain
+template <bool kW, bool kM = false, bool kQ = false, bool kB = false>
 cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                           const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
                           const uint32_t *d_target, const uint8_t *d_weights, int32_t k, int mfold, void *d_ws,
                           const VhpCoverDevT<GainT<kW>> &out, uint8_t *d_count, int sm_count, cudaStream_t st,
                           int64_t *launches, const uint64_t *d_quota = nullptr, uint64_t *d_total = nullptr,
-                          cudaStream_t cap = nullptr) {
+                          cudaStream_t cap = nullptr, const VhpCoverBudget &bud = {},
+                          const VhpCoverOut &bout = {}) {
   const CoverGeo G{nx, ny, R, (nx + 31) / 32};
   const size_t np = (size_t)nprob, plane = (size_t)ny * G.nw;
   cudaError_t e = cudaSuccess;
@@ -692,8 +839,15 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   const int64_t rounds = std::min<int64_t>(k, nsrc);
   if (e == cudaSuccess && d_count && rounds <= 0) e = cudaMemsetAsync(d_count, 0, np * ny * nx, st); // no pick
   if (e == cudaSuccess && d_total && rounds <= 0) e = cudaMemsetAsync(d_total, 0, np * 8, st);
+  if constexpr (kB) {
+    if (e == cudaSuccess && bout.spent && rounds <= 0) e = cudaMemsetAsync(bout.spent, 0, np * 8, st);
+    if (e == cudaSuccess && bout.single && rounds <= 0) e = cudaMemsetAsync(bout.single, 0xff, np * 4, st);
+    if (e == cudaSuccess && bout.single_gain && rounds <= 0) e = cudaMemsetAsync(bout.single_gain, 0, np * 8, st);
+  }
   if (e != cudaSuccess || rounds <= 0 || nprob == 0) return e;
-  const CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW, kM, kQ);
+  CoverWs ws = cover_ws(d_ws, nprob, nsrc, nx, ny, R, kW, kM, kQ, kB);
+  ws.bs.cost = bud.cost;
+  ws.bs.err = bud.err;
   GainT<kW> *gain = (GainT<kW> *)ws.gain;
   if (kW) {
     cover_weight_kernel<<<grid_for(np * plane * 8, 256, sm_count), 256, 0, st>>>(d_weights, nprob, G, ws.wpad,
@@ -712,21 +866,28 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
   if (e != cudaSuccess) return e;
   if constexpr (kQ) {
     if ((e = cudaMemsetAsync(ws.qs.active, 0, 8, st)) != cudaSuccess) return e; // active and round
-    cover_quota_init_kernel<<<grid_for(np, 256, sm_count), 256, 0, st>>>(
-        reinterpret_cast<const unsigned long long *>(d_quota), nprob, ws.done, ws.qs);
+    if constexpr (kB) {
+      if ((e = cudaMemsetAsync(ws.bs.slot, 0, np * 16, st)) != cudaSuccess) return e;
+      cover_budget_init_kernel<<<grid_for(np, 256, sm_count), 256, 0, st>>>(
+          reinterpret_cast<const unsigned long long *>(d_quota),
+          reinterpret_cast<const unsigned long long *>(bud.budget), nprob, ws.done, ws.qs, ws.bs);
+    } else {
+      cover_quota_init_kernel<<<grid_for(np, 256, sm_count), 256, 0, st>>>(
+          reinterpret_cast<const unsigned long long *>(d_quota), nprob, ws.done, ws.qs);
+    }
     if (launches) *launches += 1;
   }
   const unsigned cgrid = (unsigned)((nsrc + kCand - 1) / kCand);
-  cover_init_kernel<kW><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k, ws.state,
-                                                      gain, ws.slot, ws.first, ws.wpad);
+  cover_init_kernel<kW, kB><<<cgrid, kWarps * 32, 0, st>>>(d_bits, nsrc, G, disk_r2, d_xy, d_pair_group, d_pair_k,
+                                                          ws.state, gain, ws.slot, ws.first, ws.wpad, ws.bs);
   auto apply = [&](int32_t r, cudaStream_t s) {
-    cover_apply_kernel<kW, kM, kQ><<<(unsigned)nprob, kApplyThreads, 0, s>>>(d_bits, ws.first, nsrc, G, d_xy, r, k,
-                                                                             ws.slot, ws.cur, ws.done, ws.state,
-                                                                             ws.newb, out, gain, ws.cnt, mfold, ws.qs);
+    cover_apply_kernel<kW, kM, kQ, kB><<<(unsigned)nprob, kApplyThreads, 0, s>>>(
+        d_bits, ws.first, nsrc, G, d_xy, r, k, ws.slot, ws.cur, ws.done, ws.state, ws.newb, out, gain, ws.cnt, mfold,
+        ws.qs, ws.bs);
   };
   auto update = [&](cudaStream_t s) {
-    cover_update_kernel<kW><<<cgrid, kWarps * 32, 0, s>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
-                                                         ws.done, ws.newb, gain, ws.slot, ws.wpad);
+    cover_update_kernel<kW, kB><<<cgrid, kWarps * 32, 0, s>>>(d_bits, nsrc, G, d_xy, d_pair_group, d_pair_k, ws.cur,
+                                                             ws.done, ws.newb, gain, ws.slot, ws.wpad, ws.bs);
   };
   if constexpr (kQ) {
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
@@ -734,8 +895,15 @@ cudaError_t launch_rounds(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx,
         cudaSuccess)
       return e;
     if (launches) *launches += 2; // init and the graph
-    if (d_total && (e = cudaMemcpyAsync(d_total, ws.qs.total, np * 8, cudaMemcpyDeviceToDevice, st)) != cudaSuccess)
+    if constexpr (kB) {
+      cover_budget_out_kernel<<<grid_for(np, 256, sm_count), 256, 0, st>>>(ws.slot, nprob, ws.qs, ws.bs, d_total,
+                                                                            bout.spent, bout.single,
+                                                                            bout.single_gain);
+      if (launches) *launches += 1;
+    } else if (d_total &&
+               (e = cudaMemcpyAsync(d_total, ws.qs.total, np * 8, cudaMemcpyDeviceToDevice, st)) != cudaSuccess) {
       return e;
+    }
   } else {
     for (int32_t r = 0; r < rounds; ++r) {
       apply(r, st);
@@ -778,15 +946,19 @@ cudaError_t vhp_launch_cover_view(uint32_t *d_bits, int64_t nsrc, int nx, int ny
   return cudaGetLastError();
 }
 
-size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold, bool quota) {
-  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold || quota, mfold || quota, quota).bytes;
+size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold, bool quota,
+                          bool budget) {
+  return cover_ws(nullptr, nprob, nsrc, nx, ny, R, weighted || mfold || quota || budget, mfold || quota || budget,
+                  quota || budget, budget)
+      .bytes;
 }
 
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                                     const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
                                     bool weighted, bool mfold, const void *d_extra, int32_t k, int m,
                                     const uint64_t *d_quota, void *d_ws, const VhpCoverOut &out, int sm_count,
-                                    cudaStream_t st, cudaStream_t cap, int64_t *launches) {
+                                    cudaStream_t st, cudaStream_t cap, int64_t *launches,
+                                    const VhpCoverBudget *budget) {
   if (!weighted) {
     const VhpCoverDevT<uint32_t> o{out.pick, (uint32_t *)out.gain, out.npicked, out.covered};
     return launch_rounds<false>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k,
@@ -794,6 +966,10 @@ cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t npro
   }
   const VhpCoverDevT<uint64_t> o{out.pick, (uint64_t *)out.gain, out.npicked, out.covered};
   const uint8_t *d_weights = (const uint8_t *)d_extra;
+  if (budget)
+    return launch_rounds<true, true, true, true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group,
+                                                 d_pair_k, nullptr, d_weights, k, m, d_ws, o, out.count, sm_count, st,
+                                                 launches, d_quota, out.total, cap, *budget, out);
   if (d_quota)
     return launch_rounds<true, true, true>(d_bits, nsrc, nprob, nx, ny, R, disk_r2, d_xy, d_pair_group, d_pair_k,
                                            nullptr, d_weights, k, m, d_ws, o, out.count, sm_count, st, launches,

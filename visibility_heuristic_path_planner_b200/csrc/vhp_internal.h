@@ -105,7 +105,7 @@ struct vhp_context {
   std::string last_error;
   // device-side error word (bit 0: a source / start / end outside the grid, bit 2: inconsistent source groups,
   // bit 3: a bad view of vhp_visibility_cover_greedy_view_batch_dev, bit 4: a bad view of
-  // vhp_visibility_merge_view_batch_dev)
+  // vhp_visibility_merge_view_batch_dev, bit 5: a zero cost of vhp_visibility_cover_budget_batch_dev)
   int *d_err = nullptr;
   // workspace buffers (grown on demand, reused across calls)
   VhpDevBuf b_occ, b_src, b_map, b_out[2], b_scratch, b_planner, b_misc, b_grid, b_bin;
@@ -309,7 +309,8 @@ cudaError_t vhp_launch_cover_fold(const double *d_val, int win_r, int64_t p0, in
                                   cudaStream_t st, int64_t *launches);
 // Phase 2, the greedy rounds over the bits of nsrc candidates (table of vhp_launch_merge_table) of nprob problems.
 // The outputs of every cover call (any may be null): gain is uint32 (cells) for the cover call, uint64 (summed
-// weights) for the weighted ones; the m-fold rounds write count instead of covered, the quota rounds also total.
+// weights) for the weighted ones; the m-fold rounds write count instead of covered, the quota rounds also total, the
+// budget rounds also spent, single and single_gain.
 struct VhpCoverOut {
   int32_t *pick = nullptr;     // [prob][k]
   void *gain = nullptr;        // [prob][k]
@@ -317,6 +318,15 @@ struct VhpCoverOut {
   uint32_t *covered = nullptr; // [prob][ny][ceil(nx/32)]
   uint8_t *count = nullptr;    // [prob][ny][nx], min(m, picks whose S covers the cell)
   uint64_t *total = nullptr;   // [prob], the sum of the gains (quota rounds)
+  uint64_t *spent = nullptr;   // [prob], the sum of the picks' costs (budget rounds)
+  int32_t *single = nullptr;   // [prob], the best affordable singleton, -1: none (budget rounds)
+  uint64_t *single_gain = nullptr; // [prob], its gain (budget rounds)
+};
+// the budget rounds' inputs: cost [src] (uint32, a zero raises bit 5 of err and is never picked), budget [prob]
+struct VhpCoverBudget {
+  const uint32_t *cost = nullptr;
+  const uint64_t *budget = nullptr;
+  int *err = nullptr;
 };
 // cover_apply_kernel's parameter (kernels_cover.cu): the outputs but count, with the gain typed
 template <class Gain>
@@ -328,21 +338,26 @@ struct VhpCoverDevT {
 };
 // workspace bytes of the rounds beyond the candidate bits (weighted: uint64 gains and the padded weight plane; m-fold:
 // those of the weighted rounds and a counter plane of the padded plane's size; quota: those of the m-fold rounds, a
-// total and a quota copy per problem, and the active and round counters)
+// total and a quota copy per problem, and the active and round counters; budget: those of the quota rounds, a 16-byte
+// ratio-key slot, the remaining budget and the spent cost per problem)
 size_t vhp_cover_ws_bytes(int64_t nprob, int64_t nsrc, int nx, int ny, int R, bool weighted, bool mfold = false,
-                          bool quota = false);
+                          bool quota = false, bool budget = false);
 // outputs are filled here; d_bits: the candidates' box bits; disk_r2 >= 0: apply the disk mask first (the direct
 // route's sweep stores the whole box).  d_extra (may be null): [prob][ny][ceil(nx/32)] uint32 bits of the cells to
 // cover, or for the weighted rounds [prob][ny][nx] uint8 weights (null: every cell weighs 1; nsrc < 2^28).  The
 // m-fold rounds (with weighted) are the weighted rounds where a cell's weight counts until m in [1, 255] picks cover it.
 // d_quota (non-null: the quota rounds, weighted and m-fold; k = kmax): [prob] uint64, problem q stops once the sum of
 // its gains reaches d_quota[q]; the rounds then loop in a CUDA graph captured on `cap` and launched on st, and write
-// out.total.  Otherwise the rounds are min(k, nsrc) fixed launches on st and cap is unused.
+// out.total.  Otherwise the rounds are min(k, nsrc) fixed launches on st and cap is unused.  budget (non-null: the
+// budget rounds, weighted and m-fold; d_quota may then be null, no quota): the quota rounds' loop, picking by gain /
+// cost among the candidates whose cost fits the problem's remaining budget; they also write out.spent, out.single and
+// out.single_gain.
 cudaError_t vhp_launch_cover_greedy(uint32_t *d_bits, int64_t nsrc, int64_t nprob, int nx, int ny, int R, int disk_r2,
                                     const int32_t *d_xy, const int32_t *d_pair_group, const int32_t *d_pair_k,
                                     bool weighted, bool mfold, const void *d_extra, int32_t k, int m,
                                     const uint64_t *d_quota, void *d_ws, const VhpCoverOut &out, int sm_count,
-                                    cudaStream_t st, cudaStream_t cap, int64_t *launches);
+                                    cudaStream_t st, cudaStream_t cap, int64_t *launches,
+                                    const VhpCoverBudget *budget = nullptr);
 // the view call, between phase 1 and the m-fold rounds (which then run with disk_r2 = -1): every candidate's bits
 // &= its view, d_views [nsrc][5] = (r, ax, ay, bx, by): range r in [0, radius] in the call's shape (disk or box), and
 // the sector of a and b.  A bad view raises bit 3 of d_err and clears the candidate's bits.
